@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the `fade annotate` realignment hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|c4] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole workload, processed as chunks of --chunk reads
 through the C ABI (libfadegpu.so).  Workloads (BASELINE.json `configs`):
@@ -33,6 +33,12 @@ through the C ABI (libfadegpu.so).  Workloads (BASELINE.json `configs`):
 
 Multi-GPU: launched under torchrun, one rank per GPU, every rank with its own reference copy; no data-path
 collective; value = all ranks' reads / max-over-ranks time.
+
+--dump-outputs DIR: after the K timed steps, the results the last timed pass through the C ABI handed back (per-read
+flags, and each read's record: score, begin / end cells, op count, ops, window start) for a fixed, seeded sample of
+2^18 of rank 0's reads (all of them when there are fewer), one DIR/<name>.npy per field plus DIR/read.npy with the
+sampled read numbers.  The workload is seeded, so the same arguments give the same inputs, and two builds can be
+compared file for file.
 """
 from __future__ import annotations
 
@@ -57,6 +63,9 @@ N_READS = 10_000_000
 CHUNK = 1_000_000
 C3_READS = 100_000_000
 C3_BASES = 3.1e9
+# --dump-outputs: 20 float64 values per sampled read, so 2^18 reads are 40 MiB (inside 64 MB)
+DUMP_READS = 1 << 18
+DUMP_SEED = 3003
 # hg38 chr1-22,X,Y lengths; scaled to sum 3.1 Gbp (SURVEY.md 8d, C3)
 HG38 = [248956422, 242193529, 198295559, 190214555, 181538259, 170805979, 159345973, 145138636, 138394717, 133797422,
         135086622, 133275309, 114364328, 107043718, 101991189, 90338345, 83257441, 80373285, 58617616, 64444167,
@@ -88,7 +97,15 @@ def parse_args():
                          "(what the file drivers use; NOT the default bench line, which produces every record in full)")
     ap.add_argument("--file-reads", type=int, default=1_000_000,
                     help="records of the e2e_file leg (fade-b200 annotate BAM -> BAM on the first reads of the workload; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned for a fixed, seeded sample of rank 0's "
+                         "reads as DIR/<name>.npy (float64), to compare two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and (a.impl == "reference" or a.e2e_path == "arrays"):
+        ap.error("--dump-outputs reads the results the GPU path leaves resident in its batches: "
+                 "it needs --impl fade_b200 and --e2e-path compact or view")
     if a.reads <= 0:
         a.reads = C3_READS if a.workload == "c3" else N_READS
     return a
@@ -206,6 +223,48 @@ class Workload:
             desc += "; FADEGPU_F_TAGS_ONLY (no traceback where the score rules out both accept predicates)"
         return {"workload": desc, "chunk_reads": a.chunk, "resident_chunks": a.group,
                 "l2": "inputs + checkpoint scratch per chunk (>2 GB) exceed the 126 MB L2; no explicit flush"}
+
+
+class OutputSample:
+    """What the path hands a caller (fadegpu_get_results after fadegpu_wait), kept for a fixed, seeded sample of the
+    rank's reads, one row per read.  The records come in an unspecified order, so each is placed through result_index;
+    a read without a record keeps zeros in the record fields, and ops past min(n_ops, MAX_OPS) are zeroed.  float64
+    holds every int32 / uint32 / int64 field exactly."""
+    FIELDS = ("score", "end_query", "end_ref", "beg_query", "beg_ref", "n_ops")
+
+    def __init__(self, n_reads: int, first: int):
+        from fade_b200 import api
+        self.max_ops = api.MAX_OPS
+        if n_reads > DUMP_READS:
+            self.idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n_reads, DUMP_READS, replace=False))
+        else:
+            self.idx = np.arange(n_reads)
+        self.first = first
+        n = len(self.idx)
+        self.out = {k: np.zeros(n) for k in ("flags", *self.FIELDS, "result_flags", "win_start")}
+        self.out["ops"] = np.zeros((n, self.max_ops))
+
+    def take(self, b, first: int):
+        """the sampled reads among [first, first + b.n) of the rank's stream, from batch b's last results"""
+        lo, hi = np.searchsorted(self.idx, [first, first + b.n])
+        k = self.idx[lo:hi] - first
+        rec, ws, ridx = b.results()
+        self.out["flags"][lo:hi] = b.flags[k]
+        r = ridx[k]
+        row = np.arange(lo, hi)[r >= 0]
+        r = r[r >= 0]
+        for f in self.FIELDS:
+            self.out[f][row] = rec[f][r]
+        self.out["result_flags"][row] = rec["flags"][r]
+        self.out["win_start"][row] = ws[r]
+        live = np.arange(self.max_ops)[None, :] < np.minimum(rec["n_ops"][r], self.max_ops)[:, None]
+        self.out["ops"][row] = np.where(live, rec["ops"][r], 0)
+
+    def write(self, d: str):
+        os.makedirs(d, exist_ok=True)
+        np.save(os.path.join(d, "read.npy"), (self.idx + self.first).astype(np.float64))
+        for k, v in self.out.items():
+            np.save(os.path.join(d, f"{k}.npy"), v)
 
 
 def cpu_kind() -> str:
@@ -377,6 +436,7 @@ def main():
     max_over_ranks, sum_over_ranks = red.max, red.sum
 
     wl = Workload(args, rank, world)
+    dump = OutputSample(wl.n, wl.first) if (args.dump_outputs and rank == 0) else None
     from fade_b200 import default_params
     from fade_b200 import api as _api
     # compact results (fadegpu_get_results): fadegpu_wait rebuilds only flags[] and the result index
@@ -537,6 +597,9 @@ def main():
                 agg["d2h"] = agg.get("d2h", 0) + copies["d2h"]
         barrier()
         sampler.window(t_w0, time.time())
+        if dump:        # untimed: the group's last timed pass left every chunk's results in its batch
+            for b, (a, _) in zip(live, bounds):
+                dump.take(b, gfirst - wl.first + a)
         for b in (live if path != "arrays" else batches):
             note_host(b)
         if gi == 0 and rank == 0:
@@ -544,6 +607,8 @@ def main():
             if args.scalar_sample > 0:
                 scalar = cpu_baseline(wl.contigs, rd, args.scalar_sample, host_threads, wl.window, simd=False)
     clocks = sampler.stop() if rank == 0 else None
+    if dump:
+        dump.write(args.dump_outputs)
 
     per_rank = None
     if world > 1:       # every rank's e2e passes (diagnostics of the scaling curve): mean and worst pass in ms
