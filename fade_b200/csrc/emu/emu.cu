@@ -17,7 +17,7 @@ namespace {
 
 template <int R>
 struct ThreadState {
-    uint32_t H[R], E[R], qs[R];
+    uint32_t H[R], E[R], qs[R], qf[R];   // qf: query words of fill_step_f16
     uint32_t hu_prev, fout, M;
 };
 
@@ -48,6 +48,7 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
             const int ca = i < qlen_a ? qa[i] : C_QPAD;
             const int cb = i < qlen_b ? qb[i] : C_QPAD;
             st[g].qs[r] = q_sel(ca, cb);
+            st[g].qf[r] = q_self(ca, cb);
             qc[i] = (uint8_t)(ca | (cb << 4));
         }
     auto init_state = [&](ThreadState<R> &s) {
@@ -56,7 +57,8 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
     };
     for (int g = 0; g < FG; ++g) init_state(st[g]);
 
-    // ---- score-only pass with checkpoints ----
+    // ---- score-only pass with checkpoints (the fp16 step where the scoring allows it, as on the device) ----
+    const bool f16 = k.f16_ok && !(tagged & 8);
     const int CW = ck_words<R>();
     std::vector<uint32_t> ck((size_t)nblk * FG * CW);
     LaneCtl ctl[2];
@@ -74,7 +76,8 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
             for (int g = 0; g < FG; ++g) {
                 const uint32_t ts = tw[t - g + FG];
                 const uint32_t hd = st[g].hu_prev;
-                fill_step<R>(st[g].H, st[g].E, st[g].qs, st[g].M, ts, hd, fin[g], st[g].fout, k);
+                if (f16) fill_step_f16<R>(st[g].H, st[g].E, st[g].qf, st[g].M, ts, hd, fin[g], st[g].fout, k);
+                else fill_step<R>(st[g].H, st[g].E, st[g].qs, st[g].M, ts, hd, fin[g], st[g].fout, k);
                 st[g].hu_prev = hu[g];
             }
         }
@@ -185,6 +188,7 @@ extern "C" int fadeemu_align_pair(int R, const uint8_t *qa, int qlen_a, const ui
 {
     SwConsts k = make_consts(open, extend, match, mismatch);
     k.shortcut = (tagged & 2) ? 0 : 1;   // bit 1 of `tagged`: disable the ungapped-diagonal shortcut
+                                         // bit 3: integer score-only step even where the fp16 one is exact
 #define CASE(RR)                                                                                   \
     case RR:                                                                                       \
         return align_pair<RR>(qa, qlen_a, ta, tlen_a, qb, qlen_b, tb, tlen_b, k, extra_blocks,    \
@@ -200,3 +204,8 @@ extern "C" int fadeemu_align_pair(int R, const uint8_t *qa, int qlen_a, const ui
 extern "C" int fadeemu_comp_code_of_nt16(int nib) { return comp_code_of_nt16(nib); }
 extern "C" uint32_t fadeemu_prmt(uint32_t a, uint32_t b, uint32_t s) { return prmt_sx(a, b, s); }
 extern "C" int fadeemu_sizeof_alnout(void) { return (int)sizeof(AlnOut); }
+extern "C" int fadeemu_f16_ok(int open, int extend, int match, int mismatch) { return make_consts(open, extend, match, mismatch).f16_ok; }
+extern "C" void fadeemu_fma_f16x2(const uint32_t *a, const uint32_t *b, const uint32_t *c, uint32_t *out, int64_t n)
+{
+    for (int64_t i = 0; i < n; ++i) out[i] = fma_f16x2(a[i], b[i], c[i]);
+}

@@ -40,7 +40,8 @@ __device__ __forceinline__ uint32_t stage_targets(const KernelArgs &a, const Aln
     return w;
 }
 
-template <int R>
+// F16: query words for fill_step_f16 (q_self) instead of fill_step (q_sel)
+template <int R, bool F16>
 __device__ __forceinline__ void stage_pair(const KernelArgs &a, const AlnDesc &da, const AlnDesc &db,
                                            int g, int nblk, uint16_t *tw, uint32_t (&qs)[R],
                                            uint8_t *qc, uint32_t &wild)
@@ -54,7 +55,7 @@ __device__ __forceinline__ void stage_pair(const KernelArgs &a, const AlnDesc &d
         if (i < da.qlen) ca = rc_query_code(sa, da.qlen, i);
         if (i < db.qlen) cb = rc_query_code(sb, db.qlen, i);
         w |= (ca == C_WILD ? 1u : 0u) | (cb == C_WILD ? 2u : 0u);
-        qs[r] = q_sel(ca, cb);
+        qs[r] = F16 ? q_self(ca, cb) : q_sel(ca, cb);
         if (qc) qc[i] = (uint8_t)(ca | (cb << 4));
     }
     wild = w;
@@ -68,10 +69,19 @@ __device__ __forceinline__ AlnDesc load_desc(const KernelArgs &a, int idx)
     return d;
 }
 
+// score-only step: fill_step_f16 (scorings with k.f16_ok, query words from q_self) or fill_step (q_sel)
+template <int R, bool F16>
+__device__ __forceinline__ void score_step(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R], uint32_t &M,
+                                           uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out, const SwConsts &k)
+{
+    if (F16) fill_step_f16<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
+    else fill_step<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
+}
+
 // ------------------------------------------------------------------------------------------------
 // score-only wavefront with checkpoints
 // ------------------------------------------------------------------------------------------------
-template <int R>
+template <int R, bool F16>
 __global__ void __launch_bounds__(FILL_THREADS, (R <= 19 ? 5 : 1)) sw_fill_kernel(const KernelArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -88,7 +98,7 @@ __global__ void __launch_bounds__(FILL_THREADS, (R <= 19 ? 5 : 1)) sw_fill_kerne
 
     uint32_t H[R], E[R], qs[R];
     uint32_t wild;
-    stage_pair<R>(a, da, db, g, nblk, tw, qs, nullptr, wild);
+    stage_pair<R, F16>(a, da, db, g, nblk, tw, qs, nullptr, wild);
 #pragma unroll
     for (int r = 0; r < R; ++r) { H[r] = 0u; E[r] = k.neg_o; }
     uint32_t hu_prev = 0u, fout = k.neg_o, M = 0u, Mprev = 0u;
@@ -115,7 +125,7 @@ __global__ void __launch_bounds__(FILL_THREADS, (R <= 19 ? 5 : 1)) sw_fill_kerne
             uint32_t fin = __shfl_up_sync(FULL, fout, 1, FG);
             if (g == 0) { hu = 0u; fin = k.neg_o; }
             const uint32_t ts = twp[t];
-            fill_step<R>(H, E, qs, M, ts, hu_prev, fin, fout, k);
+            score_step<R, F16>(H, E, qs, M, ts, hu_prev, fin, fout, k);
             hu_prev = hu;
         }
         if (c + 1 < nblk) {
@@ -202,7 +212,8 @@ __global__ void FADE_SMALL_KERNEL trace_init_kernel(const KernelArgs a)
 
 // MODE 0: tagged trace recording, 1: plain trace recording, 2: scan only (round 0: find the end cell,
 // no trace tile; the traceback then tries the ungapped-diagonal proof before asking for a traced replay)
-template <int R, int MODE>
+// with the score-only step, fill_step_f16 when F16
+template <int R, int MODE, bool F16 = false>
 __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, unsigned warp0, unsigned nwarps,
                                              uint16_t (*tws_all)[40])
 {
@@ -273,7 +284,7 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
                 const int i = g * R + r;
                 const int ca = i < d[0].qlen ? rc_query_code(s0, d[0].qlen, i) : C_QPAD;
                 const int cb = i < d[1].qlen ? rc_query_code(s1, d[1].qlen, i) : C_QPAD;
-                qs[r] = q_sel(ca, cb);
+                qs[r] = F16 ? q_self(ca, cb) : q_sel(ca, cb);
             }
             __syncwarp();   // previous iteration's readers of tws are done
             for (int x = g; x < FBLK + FG - 1; x += FG) {
@@ -296,7 +307,7 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
             const uint32_t ts = twp[u];
             uint32_t cmax = 0u;
             if (SCAN_ONLY) {
-                fill_step<R>(H, E, qs, cmax, ts, hu_prev, fin, fout, k);
+                score_step<R, F16>(H, E, qs, cmax, ts, hu_prev, fin, fout, k);
             } else {
                 uint32_t trw[RW];
                 if (TAGGED) trace_step_tagged<R>(H, E, qs, ts, hu_prev, fin, fout, k, trw, cmax);
@@ -328,12 +339,12 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
     }
 }
 
-template <int R, int MODE>
+template <int R, int MODE, bool F16 = false>
 __global__ void __launch_bounds__(128) trace_replay_kernel(const KernelArgs a)
 {
     __shared__ uint16_t tws_all[16][40];
     if (blockIdx.x == 0 && threadIdx.x == 0) a.qcount[(a.round & 1) ^ 1] = 0u;   // next round's queue starts empty
-    replay_round<R, MODE>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
+    replay_round<R, MODE, F16>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
                             gridDim.x * (blockDim.x >> 5), tws_all);
 }
 
@@ -910,16 +921,22 @@ int tw_stride_for(int nblk_max) { return (FBLK * std::min(nblk_max, FILL_CHUNK_B
 
 size_t fill_smem_bytes(int tw_stride) { return (size_t)(FILL_THREADS / FG) * tw_stride * 2; }
 
-template <int R>
-static cudaError_t launch_fill_t(const KernelArgs &a, cudaStream_t s)
+template <int R, bool F16>
+static cudaError_t launch_fill_tf(const KernelArgs &a, cudaStream_t s)
 {
     const size_t smem = fill_smem_bytes(a.tw_stride);
-    cudaError_t e = cudaFuncSetAttribute(sw_fill_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(sw_fill_kernel<R, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const int wpb = FILL_THREADS / 32;
     const int grid = (a.n_items + wpb - 1) / wpb;
-    sw_fill_kernel<R><<<grid, FILL_THREADS, smem, s>>>(a);
+    sw_fill_kernel<R, F16><<<grid, FILL_THREADS, smem, s>>>(a);
     return cudaGetLastError();
+}
+
+template <int R>
+static cudaError_t launch_fill_t(const KernelArgs &a, cudaStream_t s)
+{
+    return a.k.f16_ok ? launch_fill_tf<R, true>(a, s) : launch_fill_tf<R, false>(a, s);
 }
 
 template <int R, bool TAGGED>
@@ -944,7 +961,10 @@ static cudaError_t launch_trace_tt(KernelArgs a, cudaStream_t s, int sm_count, i
             cudaMemcpy(qc, a.qcount, sizeof(qc), cudaMemcpyDeviceToHost);
             fprintf(stderr, "[fadegpu] round %d: %u requests (n_aln %d)\n", r, qc[r & 1], n);
         }
-        if (r == 0 && a.k.shortcut) trace_replay_kernel<R, 2><<<std::max(g1, 1), 128, 0, s>>>(a);
+        if (r == 0 && a.k.shortcut) {
+            if (a.k.f16_ok) trace_replay_kernel<R, 2, true><<<std::max(g1, 1), 128, 0, s>>>(a);
+            else trace_replay_kernel<R, 2, false><<<std::max(g1, 1), 128, 0, s>>>(a);
+        }
         else trace_replay_kernel<R, TAGGED ? 0 : 1><<<std::max(g1, 1), 128, 0, s>>>(a);
         trace_advance_kernel<R><<<std::max(g2, 1), 128, 0, s>>>(a);
         nl += 2;

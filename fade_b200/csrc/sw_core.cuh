@@ -46,31 +46,9 @@ struct SwConsts {
     uint32_t neg_e16_f;         // packed -16*extend + 2 (F extension tag)
     int32_t tagged_ok;          // scoring fits the tagged encoding
     int32_t shortcut;           // traceback may use the ungapped-diagonal proof instead of a replay
+    uint32_t flut0, flut1;      // byte LUT of the fp16 score words of fill_step_f16
+    int32_t f16_ok;             // fill_step_f16 is exact for this scoring (checked in make_consts)
 };
-
-FD SwConsts make_consts(int open, int extend, int match, int mismatch)
-{
-    SwConsts k;
-    const uint32_t m = (uint32_t)(match & 0xff), x = (uint32_t)(mismatch & 0xff);
-    k.lut0 = m | (x << 8) | (x << 16) | (x << 24);
-    k.lut1 = x | (x << 8) | (x << 16) | (x << 24);
-    const uint32_t no = (uint32_t)((-open) & 0xffff), ne = (uint32_t)((-extend) & 0xffff);
-    k.neg_o = no | (no << 16);
-    k.neg_e = ne | (ne << 16);
-    k.open = open; k.extend = extend; k.match = match; k.mismatch = mismatch;
-    const int tm = 16 * match + 8, tx = 16 * mismatch + 8;
-    k.tagged_ok = (tm <= 127 && tx >= -128 && open <= 1000) ? 1 : 0;
-    const uint32_t bm = (uint32_t)(tm & 0xff), bx = (uint32_t)(tx & 0xff);
-    k.tlut0 = bm | (bx << 8) | (bx << 16) | (bx << 24);
-    k.tlut1 = bx | (bx << 8) | (bx << 16) | (bx << 24);
-    const uint32_t o16 = (uint32_t)((-16 * open) & 0xffff);
-    const uint32_t ee = (uint32_t)((-16 * extend + 1) & 0xffff), ef = (uint32_t)((-16 * extend + 2) & 0xffff);
-    k.neg_o16 = o16 | (o16 << 16);
-    k.neg_e16_e = ee | (ee << 16);
-    k.neg_e16_f = ef | (ef << 16);
-    k.shortcut = 1;
-    return k;
-}
 
 // ---- packed helpers -------------------------------------------------------------------------
 FD int lane_lo(uint32_t w) { return (int)(int16_t)(w & 0xffffu); }
@@ -101,6 +79,135 @@ FD uint32_t prmt_sx(uint32_t a, uint32_t b, uint32_t sel)
 FD uint32_t q_sel(int ca, int cb) { return (uint32_t)(ca * 0x11) | ((uint32_t)(cb * 0x11) << 8); }
 FD uint32_t t_sel(int ca, int cb) { return (uint32_t)(ca * 0x11 | 0x80) | ((uint32_t)(cb * 0x11 | 0x80) << 8); }
 FD uint32_t score_word(uint32_t qs, uint32_t ts, const SwConsts &k) { return prmt_sx(k.lut0, k.lut1, qs ^ ts); }
+
+// ---- fp16x2 arithmetic on score words ----------------------------------------------------------
+// A non-negative score n <= 2047 has the same bit pattern as int16 and as the fp16 number n * 2^-24
+// (subnormals and the first normal binade both have ulp 2^-24), so HFMA2 and the DPX int16
+// instructions can work on the same registers.  A negative fp16 result is sign-magnitude (0x8000 | m),
+// i.e. negative as an int16, and a .RELU DPX instruction that consumes it clamps it to 0, as it clamps a
+// two's-complement negative.  fp16 never carries from one lane into the other (an int16x2 IMAD does,
+// which is why the integer step cannot use the FMA pipe this way; DESIGN.md 4.1).
+//
+// Host branch: exact emulation of one lane of fma.rn.f16 on finite operands: exact product and sum, one
+// round-to-nearest-even to fp16, overflow to infinity, IEEE signs of zero results.
+FD uint32_t f16_fma_lane(uint32_t a, uint32_t b, uint32_t c)
+{
+    struct Dec { int neg, m, e; };   // |value| = m * 2^(e - 24)
+    auto dec = [](uint32_t x) {
+        const int ex = (int)((x >> 10) & 31), fr = (int)(x & 1023);
+        return Dec{ (int)((x >> 15) & 1), ex ? (fr | 1024) : fr, ex ? ex - 1 : 0 };
+    };
+    const Dec da = dec(a), db = dec(b), dc = dec(c);
+    // exact values in units of 2^-48: |product| < 2^80, |c| < 2^64
+    const __int128 p = (__int128)((int64_t)da.m * db.m) << (da.e + db.e);
+    const __int128 q = (__int128)dc.m << (dc.e + 24);
+    const __int128 v = ((da.neg ^ db.neg) ? -p : p) + (dc.neg ? -q : q);
+    if (v == 0) return (p == 0 && q == 0 && (da.neg ^ db.neg) && dc.neg) ? 0x8000u : 0u;
+    const uint32_t sign = v < 0 ? 0x8000u : 0u;
+    const __int128 av = v < 0 ? -v : v;
+    int e = 0;
+    while (e < 30 && (av >> (24 + e)) >= 2048) ++e;
+    const int sh = 24 + e;
+    __int128 m = av >> sh;
+    const __int128 rem = av - (m << sh), half = (__int128)1 << (sh - 1);
+    if (rem > half || (rem == half && (m & 1))) ++m;
+    if (m == 2048) { m = 1024; ++e; }
+    if (e > 29) return sign | 0x7c00u;
+    if (m < 1024) return sign | (uint32_t)m;                          // subnormal (e == 0)
+    return sign | ((uint32_t)(e + 1) << 10) | (uint32_t)(m - 1024);
+}
+
+// fma.rn.f16x2 without .ftz: the subnormals are the scores, they must not flush
+FD uint32_t fma_f16x2(uint32_t a, uint32_t b, uint32_t c)
+{
+#if defined(__CUDA_ARCH__)
+    uint32_t d;
+    asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+    return d;
+#else
+    return f16_fma_lane(a & 0xffffu, b & 0xffffu, c & 0xffffu) | (f16_fma_lane(a >> 16, b >> 16, c >> 16) << 16);
+#endif
+}
+
+// packed fp16 2^-24: fma_f16x2(s, F16_UNIT, h) adds the fp16 number s to h in units of the score grid
+constexpr uint32_t F16_UNIT = 0x00010001u;
+
+// Query words of the fp16 step: against the same t_sel target words, sel = q_self ^ t_sel has nibbles
+// (xa|8, xa, xb|8, xb), so each lane is (LUT byte in the high half, its sign replicated in the low half).
+FD uint32_t q_self(int ca, int cb) { return (uint32_t)(ca * 0x11 | 0x88) | ((uint32_t)(cb * 0x11 | 0x88) << 8); }
+FD uint32_t score_word_f16(uint32_t qs, uint32_t ts, const SwConsts &k) { return prmt_sx(k.flut0, k.flut1, qs ^ ts); }
+
+// fp16 word (b:00 for b < 0x80, b:FF otherwise -- what score_word_f16 produces from LUT byte b) in units of 2^-25
+FD int64_t f16_byte_word_x2(uint32_t b)
+{
+    const uint32_t w = b < 0x80 ? (b << 8) : ((b << 8) | 0xffu);
+    const int ex = (int)((w >> 10) & 31), fr = (int)(w & 1023);
+    const int64_t mag = ex ? (int64_t)(fr | 1024) << ex : (int64_t)fr * 2;
+    return (w & 0x8000u) ? -mag : mag;
+}
+
+// LUT byte for score v: the one whose word is nearest to v (+2 -> 0x40 = 2.0, -3 -> 0xC1 = -2.998).  Adding a
+// word within half a unit of v to an integer n rounds to exactly n + v; make_consts checks it (f16_step_exact).
+FD uint32_t f16_score_byte(int v)
+{
+    uint32_t best = 0;
+    int64_t bd = -1;
+    for (uint32_t b = 0; b < 256; ++b) {
+        if ((b & 0x7c) == 0x7c) continue;   // infinity / NaN
+        const int64_t d = f16_byte_word_x2(b) - ((int64_t)v << 25);
+        const int64_t ad = d < 0 ? -d : d;
+        if (bd < 0 || ad < bd) { bd = ad; best = b; }
+    }
+    return best;
+}
+
+// Is fill_step_f16 exact for this scoring?  On the packed kernels (at most FG * 38 = 304 query rows) H stays
+// within [0, max(match, mismatch) * 304].  For every H in that range the fp16 diagonal add must give H + s,
+// or a word that is negative as an int16 where H + s < 0 (the .RELU max clamps it).
+FD bool f16_step_exact(const SwConsts &k)
+{
+    const int top = (k.match > k.mismatch ? k.match : k.mismatch) * FG * 38;
+    if (top > 2047) return false;
+    const int sc[2] = { k.match, k.mismatch };
+    const uint32_t sel[2] = { q_self(0, 0) ^ t_sel(0, 0), q_self(0, 0) ^ t_sel(1, 1) };   // codes equal / different
+    for (int n = 0; n <= top; ++n) {
+        for (int i = 0; i < 2; ++i) {
+            const int want = n + sc[i];
+            const uint32_t s = prmt_sx(k.flut0, k.flut1, sel[i]);
+            const uint32_t d = fma_f16x2(s, F16_UNIT, (uint32_t)n * 0x10001u);
+            if (want >= 0 ? d != (uint32_t)want * 0x10001u : (lane_lo(d) > 0 || lane_hi(d) > 0)) return false;
+        }
+    }
+    return true;
+}
+
+FD SwConsts make_consts(int open, int extend, int match, int mismatch)
+{
+    SwConsts k;
+    const uint32_t m = (uint32_t)(match & 0xff), x = (uint32_t)(mismatch & 0xff);
+    k.lut0 = m | (x << 8) | (x << 16) | (x << 24);
+    k.lut1 = x | (x << 8) | (x << 16) | (x << 24);
+    const uint32_t no = (uint32_t)((-open) & 0xffff), ne = (uint32_t)((-extend) & 0xffff);
+    k.neg_o = no | (no << 16);
+    k.neg_e = ne | (ne << 16);
+    k.open = open; k.extend = extend; k.match = match; k.mismatch = mismatch;
+    const int tm = 16 * match + 8, tx = 16 * mismatch + 8;
+    k.tagged_ok = (tm <= 127 && tx >= -128 && open <= 1000) ? 1 : 0;
+    const uint32_t bm = (uint32_t)(tm & 0xff), bx = (uint32_t)(tx & 0xff);
+    k.tlut0 = bm | (bx << 8) | (bx << 16) | (bx << 24);
+    k.tlut1 = bx | (bx << 8) | (bx << 16) | (bx << 24);
+    const uint32_t o16 = (uint32_t)((-16 * open) & 0xffff);
+    const uint32_t ee = (uint32_t)((-16 * extend + 1) & 0xffff), ef = (uint32_t)((-16 * extend + 2) & 0xffff);
+    k.neg_o16 = o16 | (o16 << 16);
+    k.neg_e16_e = ee | (ee << 16);
+    k.neg_e16_f = ef | (ef << 16);
+    k.shortcut = 1;
+    const uint32_t fm = f16_score_byte(match), fx = f16_score_byte(mismatch);
+    k.flut0 = fm | (fx << 8) | (fx << 16) | (fx << 24);
+    k.flut1 = fx | (fx << 8) | (fx << 16) | (fx << 24);
+    k.f16_ok = f16_step_exact(k) ? 1 : 0;
+    return k;
+}
 
 // ---- reference / read decoding ----------------------------------------------------------------
 // Device-resident reference: 2-bit plane (16 bases / word, code order A C T G), N plane and
@@ -188,9 +295,10 @@ FD uint32_t FADE_VIADDMAX_RELU(uint32_t a, uint32_t b, uint32_t c)
 //     H = max(0, Hdiag + s, E, F).
 // Per packed cell pair: LOP3 + PRMT (score), VIADDMNMX.RELU, VIMNMX, VIADD (H-open), 2x VIADDMNMX and
 // half a VIMNMX3 (running maximum over two rows) = 7.5 ALU-pipe instructions, all of them issued at
-// 64 threads / clk / SM (profiles/r01_ubench_b200.txt).  Moving H-open to the FMA pipe as IMAD in a
-// biased domain needs one more max for the zero floor and does not reduce the ALU-pipe time; see
-// DESIGN.md 4.1.
+// 64 threads / clk / SM (profiles/r01_ubench_b200.txt).  The score-only pass uses it for scorings that
+// fill_step_f16 below cannot take exactly (SwConsts::f16_ok == 0).  Moving H-open to the FMA pipe as a
+// 32-bit IMAD needs a biased domain (a negative low lane borrows from the high lane), in which the .RELU
+// zero floor no longer works; fp16x2 has neither problem (DESIGN.md 4.1).
 template <int R>
 FD void fill_step(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R], uint32_t &M,
                   uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out, const SwConsts &k)
@@ -201,6 +309,40 @@ FD void fill_step(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R], u
         const uint32_t s = score_word(qs[r], ts, k);
         const uint32_t t1 = FADE_VIADDMAX_RELU(hdiag, s, E[r]);
         const uint32_t h = FADE_VMAX(t1, f);
+        hdiag = H[r];
+        H[r] = h;
+        const uint32_t ho = FADE_VADD(h, k.neg_o);
+        E[r] = FADE_VIADDMAX(E[r], k.neg_e, ho);
+        f = FADE_VIADDMAX(f, k.neg_e, ho);
+        M = FADE_VMAX(M, h);
+    }
+    f_out = f;
+}
+
+FD uint32_t FADE_VMAX3_RELU(uint32_t a, uint32_t b, uint32_t c)
+{
+#if defined(__CUDA_ARCH__)
+    return __vimax3_s16x2_relu(a, b, c);
+#else
+    return FADE_VMAX(FADE_VMAX3(a, b, c), 0u);
+#endif
+}
+
+// fill_step with the diagonal add on the FMA pipe, for scorings with k.f16_ok (query words from q_self): Hdiag + s
+// is one HFMA2 on the fp16 score word (exact, see the fp16 section above; a negative sum reads as a negative int16),
+// and max(0, Hdiag + s, E, F) one VIMNMX3.RELU, which replaces VIADDMNMX.RELU + VIMNMX.  H, E and F, and so the
+// checkpoints, are bit-identical to fill_step's.  Moving H - open to the FMA pipe as well (HADD2, with E' and F'
+// clamped at 0) was measured no faster: VIADD.16x2 already co-issues with the DPX max instructions
+// (profiles/r03_ubench_b200.txt).
+template <int R>
+FD void fill_step_f16(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R], uint32_t &M,
+                      uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out, const SwConsts &k)
+{
+    uint32_t f = f_in;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const uint32_t d = fma_f16x2(score_word_f16(qs[r], ts, k), F16_UNIT, hdiag);
+        const uint32_t h = FADE_VMAX3_RELU(d, E[r], f);
         hdiag = H[r];
         H[r] = h;
         const uint32_t ho = FADE_VADD(h, k.neg_o);

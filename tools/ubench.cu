@@ -1,9 +1,40 @@
 // ubench.cu -- instruction-throughput microbenchmarks for the INT16x2 DP instruction mix on B200.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o ubench ubench.cu ; run on the GPU box.
-// Prints thread-instructions / clk / SM for each kernel (8 independent chains per thread unless noted).
+// Prints thread-instructions / clk / SM for each kernel (8 independent chains per thread unless noted), then the
+// score-only DP step of the fill kernel (sw_core.cuh) in cells / clk / SM.
 #include <cstdio>
 #include <cstdint>
 #include <cuda_runtime.h>
+#include "../fade_b200/csrc/sw_core.cuh"
+
+__device__ __forceinline__ uint32_t add_f16x2(uint32_t a, uint32_t b)
+{
+    uint32_t d;
+    asm("add.rn.f16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
+    return d;
+}
+
+// fade::fill_step_f16 with H - open as HADD2 on the FMA pipe too: its negative results are sign-magnitude, so E' and
+// F' take the .RELU max (clamped at 0; H and the trace decisions would not change).  Measured here, not used.
+template <int R>
+__device__ __forceinline__ void fill_step_f16_ho(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R], uint32_t &M,
+                                                 uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out,
+                                                 const fade::SwConsts &k, uint32_t neg_o_f16)
+{
+    uint32_t f = f_in;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const uint32_t d = fade::fma_f16x2(fade::score_word_f16(qs[r], ts, k), fade::F16_UNIT, hdiag);
+        const uint32_t h = __vimax3_s16x2_relu(d, E[r], f);
+        hdiag = H[r];
+        H[r] = h;
+        const uint32_t ho = add_f16x2(h, neg_o_f16);
+        E[r] = __viaddmax_s16x2_relu(E[r], k.neg_e, ho);
+        f = __viaddmax_s16x2_relu(f, k.neg_e, ho);
+        M = __vmaxs2(M, h);
+    }
+    f_out = f;
+}
 
 #define CHK(x) do { cudaError_t e = (x); if (e != cudaSuccess) { printf("CUDA error %s at %d\n", cudaGetErrorString(e), __LINE__); return 1; } } while (0)
 
@@ -37,6 +68,11 @@ __global__ void __launch_bounds__(256) k(uint32_t *out, int iters, uint32_t c1, 
                 if (KIND == 11) { x[i] = __viaddmax_s16x2(x[i], c1, y[i]); y[i] = __viaddmax_s16x2(y[i], c2, x[i]); } // 3 register operands
                 if (KIND == 12) { x[i] = __vmaxs2(x[i], y[i]); y[i] = y[i] * one + c1; }
                 if (KIND == 13) x[i] = __vimax3_s16x2_relu(x[i], c1, c2);
+                // fp16x2 on integer score words (sw_core.cuh): c1 / c2 are small subnormals
+                if (KIND == 14) x[i] = fade::fma_f16x2(x[i], c1, c2);                                // HFMA2
+                if (KIND == 15) x[i] = add_f16x2(x[i], c1);                                    // HADD2
+                if (KIND == 16) { x[i] = __viaddmax_s16x2(x[i], c1, c2); y[i] = fade::fma_f16x2(y[i], c1, c2); }
+                if (KIND == 17) { x[i] = __vimax3_s16x2_relu(x[i], c1, c2); y[i] = fade::fma_f16x2(y[i], c1, c2); }
             }
         }
     }
@@ -70,6 +106,65 @@ int run(const char *name, int per_iter, int sms, double mhz)
     return 0;
 }
 
+// The score-only step of sw_fill_kernel<19> on register data: 19 rows x 2 lanes per thread and step, the target
+// word from 8 registers, the diagonal H from the thread's own bottom row (no shuffle, no memory traffic).
+// V = 0: fill_step, 1: fill_step_f16 (diagonal add on the FMA pipe), 2: fill_step_f16 with H - open there too.
+template <int V>
+__global__ void __launch_bounds__(128, 5) step_k(uint32_t *out, int iters, fade::SwConsts k)
+{
+    constexpr int R = 19;
+    uint32_t H[R], E[R], qs[R], ts[8];
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const int ca = (threadIdx.x + 5 * r) & 3, cb = (threadIdx.x * 3 + r) & 3;
+        qs[r] = V ? fade::q_self(ca, cb) : fade::q_sel(ca, cb);
+        H[r] = 0u; E[r] = k.neg_o;
+    }
+#pragma unroll
+    for (int i = 0; i < 8; ++i) ts[i] = fade::t_sel((threadIdx.x * 3 + i) & 3, (7 * i + threadIdx.x) & 3);
+    uint32_t M = 0u, f = k.neg_o, hu_prev = 0u;
+    for (int it = 0; it < iters; ++it) {
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+            const uint32_t hu = H[R - 1];
+            if (V == 0) fade::fill_step<R>(H, E, qs, M, ts[u], hu_prev, f, f, k);
+            if (V == 1) fade::fill_step_f16<R>(H, E, qs, M, ts[u], hu_prev, f, f, k);
+            if (V == 2) fill_step_f16_ho<R>(H, E, qs, M, ts[u], hu_prev, f, f, k, 0x800a800au);   // fp16 -10 (open)
+            hu_prev = hu;
+        }
+    }
+    uint32_t r = M ^ f;
+#pragma unroll
+    for (int i = 0; i < R; ++i) r ^= H[i] ^ E[i];
+    if (r == 0x12345678u) out[0] = r;
+}
+
+// returns the best time in ms (the first row is the baseline of the speed-up column), < 0 on an error
+template <int V>
+float run_step(const char *name, int sms, double mhz, double base_ms)
+{
+    uint32_t *d;
+    if (cudaMalloc(&d, 64) != cudaSuccess) return -1.f;
+    const fade::SwConsts kc = fade::make_consts(10, 2, 2, -3);
+    const int blocks = sms * 5 * 4, threads = 128, iters = 512;
+    cudaEvent_t e0, e1;
+    cudaEventCreate(&e0); cudaEventCreate(&e1);
+    float best = 1e30f;
+    for (int rep = 0; rep < 4; ++rep) {
+        cudaEventRecord(e0);
+        step_k<V><<<blocks, threads>>>(d, iters, kc);
+        cudaEventRecord(e1);
+        if (cudaEventSynchronize(e1) != cudaSuccess) return -1.f;
+        float ms; cudaEventElapsedTime(&ms, e0, e1);
+        if (rep && ms < best) best = ms;
+    }
+    const double cells = (double)blocks * threads * iters * 8.0 * 2 * 19;
+    printf("%-44s %8.3f ms  %6.2f cells/clk/SM  %5.3fx\n", name, best, cells / (best * 1e-3) / (mhz * 1e6) / sms,
+           base_ms > 0 ? base_ms / best : 1.0);
+    cudaFree(d);
+    return best;
+}
+
 int main()
 {
     cudaDeviceProp p; CHK(cudaGetDeviceProperties(&p, 0));
@@ -91,5 +186,12 @@ int main()
     run<10>("VIADDMNMX + LOP3 (2 per iter)", 2, s, mhz);
     run<11>("VIADDMNMX 3-reg x2 (2 per iter)", 2, s, mhz);
     run<12>("VIMNMX + IMAD (2 per iter)", 2, s, mhz);
+    run<14>("HFMA2", 1, s, mhz);
+    run<15>("HADD2", 1, s, mhz);
+    run<16>("VIADDMNMX + HFMA2 (2 per iter)", 2, s, mhz);
+    run<17>("VIMNMX3.RELU + HFMA2 (2 per iter)", 2, s, mhz);
+    const float base = run_step<0>("fill_step<19> (integer)", s, mhz, 0.0);
+    run_step<1>("fill_step_f16<19> diagonal add on FMA (A)", s, mhz, base);
+    run_step<2>("fill_step_f16<19> + H-open on FMA (A+B)", s, mhz, base);
     return 0;
 }
