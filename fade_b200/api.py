@@ -8,7 +8,7 @@ from dataclasses import dataclass, field
 
 import numpy as np
 
-from ._lib import BatchView, FadeGpuError, HostRecord, Inputs, Params, Result, ResultsView, Stats, lib
+from ._lib import BatchView, FadeGpuError, HostRecord, Inputs, PairResult, PairsIn, Params, Result, ResultsView, Stats, lib
 
 MAX_OPS = 10
 R_ALIGNED, R_ART_LEFT, R_ART_RIGHT, R_OPS_TRUNC, R_GENERIC, R_OVERSIZE, R_SCORE_ONLY = 1, 2, 4, 8, 16, 32, 64
@@ -26,6 +26,61 @@ META_DTYPE = np.dtype([("pos", "<i8"), ("seq_off", "<u4"), ("l_qseq", "<i4"), ("
                        ("clip_left", "<u4"), ("clip_right", "<u4")])
 assert META_DTYPE.itemsize == 32
 OPCHARS = "MIDNSHP=XB"
+# fadegpu_pair_result: one record of Context.align_pairs, in pair order
+PAIR_RESULT_DTYPE = np.dtype([("score", "<i4"), ("end_query", "<i4"), ("end_ref", "<i4"), ("beg_query", "<i4"),
+                              ("beg_ref", "<i4"), ("n_ops", "<i4"), ("flags", "<u4"), ("reserved", "<i4")])
+assert PAIR_RESULT_DTYPE.itemsize == 32
+
+
+def _pack_side(seqs, offsets=None):
+    """One side of a pair call as (uint8 buffer, int64 offsets[n+1]): a list of str / bytes, or one bytes / uint8 buffer
+    plus its offsets."""
+    if offsets is not None:
+        buf = np.frombuffer(seqs, dtype=np.uint8) if isinstance(seqs, (bytes, bytearray)) else np.asarray(seqs)
+        if buf.dtype != np.uint8 or buf.ndim != 1:
+            raise TypeError("a sequence buffer must be bytes or a 1-d uint8 array")
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        if off.ndim != 1 or len(off) < 1:
+            raise ValueError("offsets must be a 1-d array of n+1 entries")
+        if len(off) > 1 and (off[0] < 0 or off[-1] > len(buf)):
+            raise ValueError("offsets exceed the sequence buffer")
+        return np.ascontiguousarray(buf), off
+    parts = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+    off = np.zeros(len(parts) + 1, dtype=np.int64)
+    if parts:
+        np.cumsum([len(p) for p in parts], out=off[1:])
+    return np.frombuffer(b"".join(parts), dtype=np.uint8).copy(), off
+
+
+def pack_pairs(queries, targets, query_offsets=None, target_offsets=None):
+    """(query buffer, query offsets, target buffer, target offsets) as fadegpu_align_pairs reads them"""
+    q, qo = _pack_side(queries, query_offsets)
+    t, to = _pack_side(targets, target_offsets)
+    if len(qo) != len(to):
+        raise ValueError(f"{len(qo) - 1} queries but {len(to) - 1} targets")
+    return q, qo, t, to
+
+
+def default_max_ops(query_offsets) -> int:
+    """3 * the longest query: no CIGAR of a local alignment can be longer (see fadegpu_align_pairs in fadegpu.h)"""
+    qo = np.asarray(query_offsets, dtype=np.int64)
+    return int(3 * np.diff(qo).max()) if len(qo) > 1 else 0
+
+
+@dataclass
+class PairResults:
+    """Context.align_pairs: records[n] (PAIR_RESULT_DTYPE) and ops[n, max_ops] in pair order, and the call's stats."""
+    records: np.ndarray
+    ops: np.ndarray
+    stats: Stats
+
+    def __len__(self):
+        return len(self.records)
+
+    def cigar(self, k: int) -> str:
+        """forward CIGAR of pair k (its first max_ops ops when the record has R_OPS_TRUNC)"""
+        n = min(int(self.records["n_ops"][k]), self.ops.shape[1])
+        return "".join(f"{int(o) >> 4}{OPCHARS[int(o) & 0xf]}" for o in self.ops[k, :n])
 
 
 def default_params(**kw) -> Params:
@@ -108,6 +163,26 @@ class Context:
         ms = C.c_float()
         self._check(lib().fadegpu_replay_batches(self._h, arr, len(batches), iters, C.byref(ms)))
         return ms.value
+
+    def align_pairs(self, queries, targets, max_ops: int | None = None, *, query_offsets=None,
+                    target_offsets=None) -> PairResults:
+        """fadegpu_align_pairs: Smith-Waterman with traceback of query k against target k, with the ctx's scoring.
+
+        queries / targets: lists of str or bytes, or one bytes / uint8 buffer each with query_offsets /
+        target_offsets (n+1 int64 entries).  Queries are taken as given (no reverse complement) and must use the
+        nt16 letters =ACMGRSVTWYHKDBN; targets may hold any letter.  max_ops defaults to 3 * the longest query,
+        which never truncates a CIGAR."""
+        q, qo, t, to = pack_pairs(queries, targets, query_offsets, target_offsets)
+        n = len(qo) - 1
+        if max_ops is None:
+            max_ops = default_max_ops(qo)
+        rec = np.zeros(n, dtype=PAIR_RESULT_DTYPE)
+        ops = np.zeros((n, max_ops), dtype=np.uint32)
+        st = Stats()
+        pin = PairsIn(q.ctypes.data, qo.ctypes.data, t.ctypes.data, to.ctypes.data)
+        self._check(lib().fadegpu_align_pairs(self._h, n, C.byref(pin), max_ops, rec.ctypes.data,
+                                              ops.ctypes.data if max_ops > 0 else None, C.byref(st)))
+        return PairResults(rec, ops, st)
 
     def alloc_batch(self, max_reads: int, max_seq_bytes: int) -> "Batch":
         return Batch(self, max_reads, max_seq_bytes)

@@ -26,7 +26,7 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
                const uint8_t *qb, int qlen_b, const uint8_t *tb, int tlen_b,
                const SwConsts &k, int extra_blocks, int tagged, int32_t min_length,
                uint32_t clipl_a, uint32_t clipr_a, uint32_t clipl_b, uint32_t clipr_b,
-               AlnOut *out_a, AlnOut *out_b)
+               AlnOut *out_a, AlnOut *out_b, int ops_cap = 0, uint32_t *ops_a = nullptr, uint32_t *ops_b = nullptr)
 {
     const int rows = FG * R;
     if (qlen_a > rows || qlen_b > rows) return -1;
@@ -101,6 +101,11 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
     constexpr int RW = trace_words<R>();
     std::vector<uint32_t> tr((size_t)tile_words<R>());
     const bool tg = (tagged & 1) && k.tagged_ok;
+    // ops_cap > 0: the walkers also spill every op into rings of ops_cap words, as the device does for
+    // fadegpu_align_pairs, and ops_a / ops_b receive the first ops_cap forward ops assembled from them
+    std::vector<uint32_t> spill[2];
+    for (auto &v : spill) v.assign((size_t)(ops_cap > 0 ? ops_cap : 1), 0u);
+    uint32_t *sp0 = ops_cap > 0 ? spill[0].data() : nullptr, *sp1 = ops_cap > 0 ? spill[1].data() : nullptr;
     int guard = 0;
     bool first_iter = true;
     while (ctl[0].phase != 2 || ctl[1].phase != 2) {
@@ -169,12 +174,21 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
                 if (scan[L][g] && !found[L][g]) return -3;  // a candidate must find its cell
         // bit 2 of `tagged`: the first (scan) replay of a lane records no trace, like round 0 on the device
         const bool so0 = (tagged & 4) && ctl[0].phase == 0 && first_iter, so1 = (tagged & 4) && ctl[1].phase == 0 && first_iter;
-        ctl_advance<R>(ctl[0], so0 ? nullptr : tr.data(), 0, StagedAcc{ tw.data(), qc.data(), 0 }, k);
-        ctl_advance<R>(ctl[1], so1 ? nullptr : tr.data(), 1, StagedAcc{ tw.data(), qc.data(), 1 }, k);
+        ctl_advance<R>(ctl[0], so0 ? nullptr : tr.data(), 0, StagedAcc{ tw.data(), qc.data(), 0 }, k, sp0, ops_cap);
+        ctl_advance<R>(ctl[1], so1 ? nullptr : tr.data(), 1, StagedAcc{ tw.data(), qc.data(), 1 }, k, sp1, ops_cap);
         first_iter = false;
     }
     finalize_result(ctl[0], *out_a, 0, clipl_a, clipr_a, min_length);
     finalize_result(ctl[1], *out_b, 1, clipl_b, clipr_b, min_length);
+    if (ops_cap > 0) {
+        const LaneCtl *cl[2] = { &ctl[0], &ctl[1] };
+        uint32_t *dst[2] = { ops_a, ops_b };
+        for (int L = 0; L < 2; ++L) {
+            const LaneCtl &c = *cl[L];
+            if (c.S <= 0 || c.nrev == 0) { for (int w = 0; w < ops_cap; ++w) dst[L][w] = 0; continue; }
+            forward_ops(spill[L].data(), ops_cap, c.nrev, c.i + 1, c.qlen - 1 - c.end_i, dst[L]);
+        }
+    }
     return 0;
 }
 
@@ -193,6 +207,26 @@ extern "C" int fadeemu_align_pair(int R, const uint8_t *qa, int qlen_a, const ui
     case RR:                                                                                       \
         return align_pair<RR>(qa, qlen_a, ta, tlen_a, qb, qlen_b, tb, tlen_b, k, extra_blocks,    \
                               tagged, min_length, clips[0], clips[1], clips[2], clips[3], out_a, out_b);
+    switch (R) {
+        CASE(1) CASE(2) CASE(3) CASE(5) CASE(13) CASE(19) CASE(25) CASE(32) CASE(38)
+    default: return -10;
+    }
+#undef CASE
+}
+
+// The same with the full-CIGAR spill of fadegpu_align_pairs: ops_a / ops_b receive the first ops_cap forward ops.
+extern "C" int fadeemu_align_pair_ops(int R, const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
+                                      const uint8_t *qb, int qlen_b, const uint8_t *tb, int tlen_b,
+                                      int open, int extend, int match, int mismatch, int tagged, int ops_cap,
+                                      AlnOut *out_a, AlnOut *out_b, uint32_t *ops_a, uint32_t *ops_b)
+{
+    if (ops_cap <= 0) return -11;
+    SwConsts k = make_consts(open, extend, match, mismatch);
+    k.shortcut = (tagged & 2) ? 0 : 1;
+#define CASE(RR)                                                                                   \
+    case RR:                                                                                       \
+        return align_pair<RR>(qa, qlen_a, ta, tlen_a, qb, qlen_b, tb, tlen_b, k, 0, tagged, 0, 0, 0, 0, 0, \
+                              out_a, out_b, ops_cap, ops_a, ops_b);
     switch (R) {
         CASE(1) CASE(2) CASE(3) CASE(5) CASE(13) CASE(19) CASE(25) CASE(32) CASE(38)
     default: return -10;

@@ -34,6 +34,8 @@ using namespace fade;
 static_assert(FADEGPU_MAX_OPS == OPS_CAP, "ABI ops capacity must match the kernels");
 static_assert(sizeof(AlnOut) == 32 + 4 * OPS_CAP, "AlnOut layout");
 static_assert(sizeof(AlnDesc) == 40, "AlnDesc layout");
+static_assert(sizeof(PairResult) == sizeof(fadegpu_pair_result) && sizeof(fadegpu_pair_result) == 32, "fadegpu_pair_result layout");
+static_assert(PAIR_R_OVERSIZE == FADEGPU_R_OVERSIZE, "oversize flag");
 
 static thread_local std::string g_last_error;
 
@@ -89,6 +91,26 @@ struct fadegpu_ctx {
     std::deque<std::pair<fadegpu_batch *, int64_t>> jobs;
     bool worker_stop = false, worker_busy = false;
     std::mutex submit_mu;                 // one submit body at a time (they size shared scratch and order the streams)
+    std::vector<fadegpu_batch *> batches; // the caller's batches (guarded by q_mu): fadegpu_align_pairs refuses to run while
+                                          // one of them is in flight
+    // fadegpu_align_pairs: an internal batch (descriptors, binning arrays, result records) that grows with use, the
+    // targets packed as a reference of their own, and the staging of the raw ASCII
+    struct PairBufs {
+        fadegpu_batch *b = nullptr;
+        char *h_stage = nullptr, *d_raw = nullptr;          // pinned staging / device copy of offsets + ASCII
+        size_t stage_bytes = 0, raw_bytes = 0;
+        uint32_t *d_two = nullptr, *d_n = nullptr, *d_x = nullptr, *d_chunk_x = nullptr;
+        size_t two_bytes = 0, n_bytes = 0, x_bytes = 0, chunk_bytes = 0;
+        int64_t *d_xpos = nullptr, *d_clen = nullptr, *d_coff = nullptr;
+        size_t xpos_bytes = 0, clen_bytes = 0, coff_bytes = 0;
+        uint8_t *d_xchr = nullptr;
+        size_t xchr_bytes = 0;
+        uint32_t *d_spill = nullptr, *d_ops = nullptr;
+        size_t spill_bytes = 0, ops_bytes = 0;
+        fadegpu_pair_result *d_res = nullptr;
+        size_t res_bytes = 0;
+        int32_t *d_bad = nullptr;
+    } pairs;
 };
 
 struct AlnTmp {       // a read that needs SW, captured in read order (sequential pass), before sorting
@@ -355,7 +377,23 @@ int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *c
 // start of a timed replay), traceback + generic on c->tstream, consecutive launches on alternating
 // scratch sets.  On return b->ev_kernels marks the end of the batch's kernels; the caller joins it.
 // With stage timers every launch is synchronised.
-int run_plan(fadegpu_ctx *c, fadegpu_batch *b, float *fill_ms, float *trace_ms, float *gen_ms, int *launches, cudaEvent_t dep)
+// What a plan runs against: the resident reference (submits) or the packed targets of a pair call, whether alignments
+// whose score rules out both predicates skip the traceback (FADEGPU_F_TAGS_ONLY), and the optional full-CIGAR spill
+// rings (ops_cap words per alignment of the batch, in its sorted order).
+struct PlanTarget {
+    RefDev ref;
+    int tags_only;
+    uint32_t *ops_spill;
+    int ops_cap;
+};
+
+PlanTarget batch_target(const fadegpu_ctx *c)
+{
+    return PlanTarget{ ref_dev(c), (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0, nullptr, 0 };
+}
+
+int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill_ms, float *trace_ms, float *gen_ms,
+             int *launches, cudaEvent_t dep)
 {
     const bool timed = fill_ms != nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
@@ -379,7 +417,7 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, float *fill_ms, float *trace_ms, 
             a.items = b->d_items + L.item_first;
             a.n_items = L.n_items;
             a.seq = seq;
-            a.ref = ref_dev(c);
+            a.ref = pt.ref;
             a.ck = ln.d_ck;
             a.fillres = b->d_fillres + (size_t)L.item_first * 32;
             a.aln_flags = b->d_flags + L.aln_first;
@@ -396,8 +434,10 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, float *fill_ms, float *trace_ms, 
                 a.qcount = ln.d_qcount;
                 a.round = 0;
                 a.max_rounds = L.nblk_max + FG;   // each round scans one candidate block or walks one block
-                a.tags_only = (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0;
+                a.tags_only = pt.tags_only;
             }
+            a.ops_spill = pt.ops_spill ? pt.ops_spill + (size_t)L.aln_first * pt.ops_cap : nullptr;
+            a.ops_cap = pt.ops_cap;
             CU(c, cudaMemsetAsync(a.aln_flags, 0, (size_t)L.n_aln * sizeof(uint32_t), sf));
             CU(c, cudaMemsetAsync(ln.d_qcount, 0, 2 * sizeof(unsigned int), sf));
             if (timed) CU(c, cudaEventRecord(e0, sf));
@@ -416,7 +456,8 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, float *fill_ms, float *trace_ms, 
             ga.n_slots = (int)std::max<size_t>(1, std::min<size_t>(GEN_SLOTS_MAX, ln.gen_bytes / (size_t)ga.slot_bytes));
             ga.chunk = 64;
             ga.open = c->p.gap_open; ga.extend = c->p.gap_extend; ga.match = c->p.match; ga.mismatch = c->p.mismatch;
-            ga.min_length = c->p.min_length; ga.tags_only = (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0;
+            ga.min_length = c->p.min_length; ga.tags_only = pt.tags_only;
+            ga.ops_spill = a.ops_spill; ga.ops_cap = a.ops_cap;
             if (timed) CU(c, cudaEventRecord(e2, st));
             CU(c, cudaMemsetAsync(ln.d_cursor, 0, sizeof(unsigned int), st));
             CU(c, launch_generic(ga, ga.n_slots, st));
@@ -436,14 +477,16 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, float *fill_ms, float *trace_ms, 
         } else {
             GenericArgs ga;
             ga.aln = b->d_aln + L.aln_first; ga.n_aln = L.n_aln; ga.aln_flags = nullptr; ga.seq = seq;
-            ga.ref = ref_dev(c); ga.out = b->d_out + L.aln_first; ga.cursor = ln.d_cursor; ga.scratch = ln.d_gen;
+            ga.ref = pt.ref; ga.out = b->d_out + L.aln_first; ga.cursor = ln.d_cursor; ga.scratch = ln.d_gen;
             ga.qmax = L.qmax; ga.tmax = L.tmax;
             ga.slot_bytes = (int64_t)gen_slot_bytes(L.qmax, L.tmax);
             ga.n_slots = (int)std::max<size_t>(1, std::min<size_t>(GEN_SLOTS_MAX, ln.gen_bytes / (size_t)ga.slot_bytes));
             ga.n_slots = std::min(ga.n_slots, std::max(L.n_aln, 1));
             ga.chunk = 1;
             ga.open = c->p.gap_open; ga.extend = c->p.gap_extend; ga.match = c->p.match; ga.mismatch = c->p.mismatch;
-            ga.min_length = c->p.min_length; ga.tags_only = (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0;
+            ga.min_length = c->p.min_length; ga.tags_only = pt.tags_only;
+            ga.ops_spill = pt.ops_spill ? pt.ops_spill + (size_t)L.aln_first * pt.ops_cap : nullptr;
+            ga.ops_cap = pt.ops_cap;
             CU(c, cudaEventRecord(ln.ev_fill, sf));        // (orders tstream after dep and the set's previous traceback)
             CU(c, cudaStreamWaitEvent(st, ln.ev_fill, 0));
             if (timed) CU(c, cudaEventRecord(e0, st));
@@ -589,6 +632,14 @@ void fadegpu_destroy(fadegpu_ctx *c)
         c->worker.join();                 // finishes the queued submits first
     }
     cudaSetDevice(c->device);
+    {
+        fadegpu_ctx::PairBufs &pb = c->pairs;
+        if (pb.b) fadegpu_free_batch(pb.b);
+        free_host(pb.h_stage);
+        free_dev(pb.d_raw); free_dev(pb.d_two); free_dev(pb.d_n); free_dev(pb.d_x); free_dev(pb.d_chunk_x);
+        free_dev(pb.d_xpos); free_dev(pb.d_xchr); free_dev(pb.d_clen); free_dev(pb.d_coff); free_dev(pb.d_spill);
+        free_dev(pb.d_ops); free_dev(pb.d_res); free_dev(pb.d_bad);
+    }
     if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->stream2) { cudaStreamSynchronize(c->stream2); cudaStreamDestroy(c->stream2); }
     if (c->stream3) { cudaStreamSynchronize(c->stream3); cudaStreamDestroy(c->stream3); }
@@ -741,7 +792,11 @@ void fadegpu_free_batch(fadegpu_batch *b)
 {
     if (!b) return;
     fadegpu_ctx *c = b->ctx;
-    if (c) { std::unique_lock<std::mutex> lk(c->q_mu); c->done_cv.wait(lk, [&] { return !b->queued; }); }
+    if (c) {
+        std::unique_lock<std::mutex> lk(c->q_mu);
+        c->done_cv.wait(lk, [&] { return !b->queued; });
+        c->batches.erase(std::remove(c->batches.begin(), c->batches.end(), b), c->batches.end());
+    }
     if (c) { cudaSetDevice(c->device); if (c->stream) cudaStreamSynchronize(c->stream); if (c->tstream) cudaStreamSynchronize(c->tstream); if (c->stream2) cudaStreamSynchronize(c->stream2); if (c->stream3) cudaStreamSynchronize(c->stream3); }
     fadegpu_batch_view &v = b->v;
     free_host(v.seq4); free_host(v.seq_off); free_host(v.l_qseq); free_host(v.tid); free_host(v.pos);
@@ -821,6 +876,7 @@ int fadegpu_alloc_batch(fadegpu_ctx *c, int64_t max_reads, int64_t max_seq_bytes
         fadegpu_free_batch(b);
         return rc;
     }
+    { std::lock_guard<std::mutex> lk(c->q_mu); c->batches.push_back(b); }
     *out = b;
     return FADEGPU_OK;
 }
@@ -1063,7 +1119,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
     CU(c, cudaEventRecord(b->ev[1], c->stream));
     int nl = 0;
-    { int rc = run_plan(c, b, nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
+    { int rc = run_plan(c, b, batch_target(c), nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
     b->st.kernel_launches = nl;
     { int rc = join_kernels(c, b, c->stream3); if (rc) return rc; }
     CU(c, cudaEventRecord(b->ev[2], c->stream3));
@@ -1158,6 +1214,32 @@ enum SubmitMode : int {
     MODE_COMPACT = 2     // fadegpu_submit_compact: one gate byte per read is DMA'd, the GPU fetches the rest it needs
 };
 
+// Launch plan from the binning histogram of the device (b->h_hist, b->h_stats) that classified n_aln alignments; also
+// fills b->h_keybase, the first sorted position of every key, for bin_scatter_kernel.
+static int plan_from_histogram(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln)
+{
+    int64_t cls_first[N_ROW_CLASSES + 2];
+    std::vector<int32_t> &stl = b->sorted_tlen;
+    stl.resize((size_t)n_aln);
+    int64_t run = 0;
+    for (int rk = 0; rk <= N_ROW_CLASSES; ++rk) {
+        cls_first[rk] = run;
+        const int k0 = rk * KEYS_PER_CLASS, k1 = k0 + KEYS_PER_CLASS;
+        for (int key = k0; key < k1; ++key) {
+            const int32_t cnt = b->h_hist[key];
+            b->h_keybase[key] = (int32_t)run;
+            if (!cnt) continue;
+            const int tl = rk == N_ROW_CLASSES ? (int)b->h_stats[5] : key_tlen(key - k0);
+            std::fill(stl.begin() + run, stl.begin() + run + cnt, tl);
+            run += cnt;
+        }
+    }
+    cls_first[N_ROW_CLASSES + 1] = run;
+    if (run != n_aln) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: internal error (histogram does not add up)");
+    return build_plan(c, b, n_aln, cls_first, stl.data(), std::max(1, (int)b->h_stats[2]), std::max(1, (int)b->h_stats[3]),
+                      std::max(1, (int)b->h_stats[4]), std::max(1, (int)b->h_stats[5]));
+}
+
 // Stage B: the inputs go to the GPU, a classify kernel applies the length floor (analysis.d:34) and the window
 // arithmetic (analysis.d:45-59) and histograms the reads that need SW by (row class, window length), the host
 // turns the 96 KB histogram into the launch plan, a scatter kernel writes the sorted descriptors, the GPU pulls the
@@ -1228,29 +1310,7 @@ static int submit_device_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_rea
         const auto t_sort = std::chrono::steady_clock::now();
         n_aln = (int64_t)b->h_stats[1];
         b->st.cells = (int64_t)b->h_stats[0];
-        int64_t cls_first[N_ROW_CLASSES + 2];
-        std::vector<int32_t> &stl = b->sorted_tlen;
-        stl.resize((size_t)n_aln);
-        int64_t run = 0;
-        for (int rk = 0; rk <= N_ROW_CLASSES; ++rk) {
-            cls_first[rk] = run;
-            const int k0 = rk * KEYS_PER_CLASS, k1 = k0 + KEYS_PER_CLASS;
-            for (int key = k0; key < k1; ++key) {
-                const int32_t cnt = b->h_hist[key];
-                b->h_keybase[key] = (int32_t)run;
-                if (!cnt) continue;
-                const int tl = rk == N_ROW_CLASSES ? (int)b->h_stats[5] : key_tlen(key - k0);
-                std::fill(stl.begin() + run, stl.begin() + run + cnt, tl);
-                run += cnt;
-            }
-        }
-        cls_first[N_ROW_CLASSES + 1] = run;
-        if (run != n_aln) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: internal error (histogram does not add up)");
-        {
-            int rc = build_plan(c, b, n_aln, cls_first, stl.data(), std::max(1, (int)b->h_stats[2]), std::max(1, (int)b->h_stats[3]),
-                                std::max(1, (int)b->h_stats[4]), std::max(1, (int)b->h_stats[5]));
-            if (rc) return rc;
-        }
+        { int rc = plan_from_histogram(c, b, n_aln); if (rc) return rc; }
         b->st.host_sort_ms = ms_since(t_sort);
         if (n_aln > 0) {
             CU(c, up(b->d_keybase, b->h_keybase, (size_t)BIN_KEYS * 4));
@@ -1269,7 +1329,7 @@ static int submit_device_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_rea
     CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
     CU(c, cudaEventRecord(b->ev[1], c->stream));
     int nl = 0;
-    { int rc = run_plan(c, b, nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
+    { int rc = run_plan(c, b, batch_target(c), nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
     b->st.kernel_launches = nl + (n > 0 ? 1 : 0) + (n_aln > 0 ? (pull ? 3 : 2) : 0);
     cudaStream_t s3 = c->stream3;                    // results go home while the next batch computes
     { int rc = join_kernels(c, b, s3); if (rc) return rc; }
@@ -1539,7 +1599,7 @@ static int replay_pass(fadegpu_ctx *c, fadegpu_batch *b)
 {
     cudaEvent_t dep = nullptr;
     { int rc = replay_binning(c, b, &dep); if (rc) return rc; }
-    { int rc = run_plan(c, b, nullptr, nullptr, nullptr, nullptr, dep); if (rc) return rc; }
+    { int rc = run_plan(c, b, batch_target(c), nullptr, nullptr, nullptr, nullptr, dep); if (rc) return rc; }
     return 0;
 }
 
@@ -1590,12 +1650,221 @@ int fadegpu_replay_kernels(fadegpu_ctx *c, fadegpu_batch *b, int32_t iters, floa
         std::lock_guard<std::mutex> submit_guard(c->submit_mu);
         CU(c, cudaSetDevice(c->device));
         float f = 0, t = 0, g = 0;
-        int rc = run_plan(c, b, &f, &t, &g, nullptr, nullptr);
+        int rc = run_plan(c, b, batch_target(c), &f, &t, &g, nullptr, nullptr);
         if (rc) return rc;
         b->st.fill_ms = f; b->st.trace_ms = t; b->st.generic_ms = g;
     }
     fadegpu_batch *one[1] = { b };
     return fadegpu_replay_batches(c, one, 1, iters, ms_out);
+}
+
+// copy with the ctx's host threads (the caller's arrays are pageable; the staging is pinned)
+static void parallel_copy(char *dst, const char *src, size_t bytes, int nthr)
+{
+    const int T = (int)std::max<size_t>(1, std::min<size_t>((size_t)std::max(1, nthr), bytes >> 20));
+#pragma omp parallel for schedule(static, 1) num_threads(T) if (T > 1)
+    for (int t = 0; t < T; ++t) {
+        const size_t lo = bytes * (size_t)t / (size_t)T, hi = bytes * (size_t)(t + 1) / (size_t)T;
+        memcpy(dst + lo, src + lo, hi - lo);
+    }
+}
+
+// Pairs: the raw ASCII goes to the device through pinned staging on stream2, where pair_prep_kernel writes the per-pair
+// binning inputs and the queries (nt16, reverse-complemented) and pair_pack_targets_kernel the target planes; the
+// binning, the launch plan and run_plan are those of a device-binned submit, on the ctx's internal pair batch, with
+// the targets as the reference, every alignment traced back and the full CIGARs spilled; the records come back in
+// pair order on stream3.
+int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
+                        fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+{
+    if (!c) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_align_pairs: null ctx");
+    if (n_pairs < 0 || n_pairs > ((int64_t)1 << 30) || max_ops < 0)
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: n_pairs or max_ops out of range");
+    if (n_pairs > 0 && (!in || !in->query_off || !in->target_off || !out || (max_ops > 0 && !ops_out)))
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null argument");
+    {
+        std::lock_guard<std::mutex> lk(c->q_mu);
+        for (const fadegpu_batch *b : c->batches)
+            if (b->in_flight)
+                return fail(c, FADEGPU_E_STATE, "fadegpu_align_pairs: a batch of this ctx is in flight (call fadegpu_wait)");
+    }
+    const auto t_begin = std::chrono::steady_clock::now();
+    const int64_t n = n_pairs;
+    int64_t qbytes = 0, tbytes = 0, n_over = 0;
+    if (n > 0) {
+        const int64_t *qo = in->query_off, *to = in->target_off;
+        if (qo[0] < 0 || to[0] < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: negative offset");
+        for (int64_t k = 0; k < n; ++k) {
+            const int64_t ql = qo[k + 1] - qo[k], tl = to[k + 1] - to[k];
+            if (ql < 0 || tl < 0)
+                return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: offsets decrease at pair " + std::to_string(k));
+            if (ql > 0 && tl > 0 && (tl > 0x7fffffff || ql * tl > PAIR_MAX_CELLS)) ++n_over;
+        }
+        qbytes = qo[n] - qo[0]; tbytes = to[n] - to[0];
+        if ((qbytes > 0 && !in->query) || (tbytes > 0 && !in->target))
+            return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null sequence array");
+    }
+    fadegpu_stats st{};
+    st.n_reads = n;
+    st.n_oversize = n_over;
+    if (n == 0) {
+        if (stats_out) *stats_out = st;
+        return FADEGPU_OK;
+    }
+    std::lock_guard<std::mutex> submit_guard(c->submit_mu);
+    CU(c, cudaSetDevice(c->device));
+    fadegpu_ctx::PairBufs &pb = c->pairs;
+    if (!pb.b || pb.b->v.max_reads < n || pb.b->v.max_seq_bytes < qbytes + 16) {
+        int64_t nr = n, sb = qbytes + 16;
+        if (pb.b) {
+            nr = std::max(nr, pb.b->v.max_reads); sb = std::max(sb, pb.b->v.max_seq_bytes);
+            fadegpu_free_batch(pb.b);
+            pb.b = nullptr;
+        }
+        int rc = fadegpu_alloc_batch(c, nr, sb, &pb.b);
+        if (rc) return rc;
+    }
+    fadegpu_batch *b = pb.b;
+    // ---- staging: [query_off][target_off] rebased to 0, then the query and the target letters ----
+    auto a16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+    const size_t o_toff = a16((size_t)(n + 1) * 8), o_q = o_toff + a16((size_t)(n + 1) * 8), o_t = o_q + a16((size_t)qbytes);
+    const size_t raw = o_t + a16((size_t)tbytes);
+    if (pb.stage_bytes < raw) {
+        free_host(pb.h_stage);
+        pb.stage_bytes = 0;
+        CU(c, cudaHostAlloc((void **)&pb.h_stage, raw, cudaHostAllocDefault));
+        pb.stage_bytes = raw;
+    }
+    {
+        int64_t *hq = reinterpret_cast<int64_t *>(pb.h_stage), *ht = reinterpret_cast<int64_t *>(pb.h_stage + o_toff);
+        const int64_t q0 = in->query_off[0], t0 = in->target_off[0];
+        for (int64_t k = 0; k <= n; ++k) { hq[k] = in->query_off[k] - q0; ht[k] = in->target_off[k] - t0; }
+        if (qbytes) parallel_copy(pb.h_stage + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
+        if (tbytes) parallel_copy(pb.h_stage + o_t, in->target + t0, (size_t)tbytes, c->host_threads);
+    }
+    const int64_t n_words = n + (tbytes >> 5) + 2;   // target k starts at 32 * (k + toff[k] / 32)
+    const int64_t n_chunks = (n_words + PAIR_CHUNK_WORDS - 1) / PAIR_CHUNK_WORDS;
+    {
+        int rc = 0;
+        auto grow = [&](auto **p, size_t *have, size_t bytes) { if (!rc) rc = ensure_dev(c, (void **)p, have, std::max<size_t>(bytes, 16)); };
+        grow(&pb.d_raw, &pb.raw_bytes, raw);
+        grow(&pb.d_two, &pb.two_bytes, (size_t)n_words * 8); grow(&pb.d_n, &pb.n_bytes, (size_t)n_words * 4);
+        grow(&pb.d_x, &pb.x_bytes, (size_t)n_words * 4); grow(&pb.d_chunk_x, &pb.chunk_bytes, (size_t)n_chunks * 4);
+        grow(&pb.d_clen, &pb.clen_bytes, (size_t)n * 8); grow(&pb.d_coff, &pb.coff_bytes, (size_t)n * 8);
+        grow(&pb.d_res, &pb.res_bytes, (size_t)n * sizeof(fadegpu_pair_result));
+        if (max_ops > 0) {
+            grow(&pb.d_spill, &pb.spill_bytes, (size_t)n * (size_t)max_ops * 4);
+            grow(&pb.d_ops, &pb.ops_bytes, (size_t)n * (size_t)max_ops * 4);
+        }
+        if (rc) return rc;
+        if (!pb.d_bad) CU(c, cudaMalloc((void **)&pb.d_bad, sizeof(int32_t)));
+    }
+    // ---- upload, packing and binning on stream2 ----
+    b->n_reads = n;
+    b->plan.clear();
+    b->dev_binning = true;
+    b->ba_valid = false;
+    b->n_aln = 0; b->n_items = 0;
+    memset(&b->st, 0, sizeof(b->st));
+    memset(b->h_stats, 0, 128);
+    cudaStream_t s2 = c->stream2;
+    CU(c, cudaEventRecord(b->ev[0], s2));
+    CU(c, cudaMemcpyAsync(pb.d_raw, pb.h_stage, raw, cudaMemcpyHostToDevice, s2));
+    int64_t h2d = (int64_t)raw;
+    CU(c, cudaEventRecord(b->ev[4], s2));
+    PairArgs pa{};
+    pa.n = n;
+    pa.qoff = reinterpret_cast<const int64_t *>(pb.d_raw); pa.toff = reinterpret_cast<const int64_t *>(pb.d_raw + o_toff);
+    pa.query = pb.d_raw + o_q; pa.target = pb.d_raw + o_t;
+    pa.seq_off = b->d_in_seq_off; pa.pos = b->d_in_pos; pa.l_qseq = b->d_in_lq; pa.tid = b->d_in_tid;
+    pa.aligned_len = b->d_in_alen; pa.clip_left = b->d_in_cl; pa.clip_right = b->d_in_cr;
+    pa.clen = pb.d_clen; pa.coff = pb.d_coff; pa.seq4 = b->d_in_seq4; pa.bad = pb.d_bad;
+    pa.two = pb.d_two; pa.nmask = pb.d_n; pa.xmask = pb.d_x; pa.n_words = n_words;
+    pa.chunk_x = pb.d_chunk_x; pa.n_x = b->d_stats + 12;
+    CU(c, cudaMemsetAsync(b->d_hist, 0, (size_t)BIN_KEYS * 4, s2));
+    CU(c, cudaMemsetAsync(b->d_cursor, 0, (size_t)BIN_KEYS * 4, s2));
+    CU(c, cudaMemsetAsync(b->d_stats, 0, 128, s2));
+    CU(c, cudaMemsetAsync(pb.d_bad, 0x7f, sizeof(int32_t), s2));   // > any pair index
+    CU(c, launch_pair_prep(pa, c->sm_count, s2));
+    CU(c, launch_pair_pack_targets(pa, s2));
+    BinArgs ba{};
+    ba.seq4 = b->d_in_seq4; ba.seq_off = b->d_in_seq_off; ba.l_qseq = b->d_in_lq; ba.tid = b->d_in_tid; ba.pos = b->d_in_pos;
+    ba.aligned_len = b->d_in_alen; ba.clip_left = b->d_in_cl; ba.clip_right = b->d_in_cr;
+    ba.read = nullptr; ba.seq_cursor = nullptr; ba.src_off = b->d_src_off; ba.gate = nullptr; ba.host_meta = nullptr;
+    ba.over_list = b->d_over;
+    // contigs = targets, window 0 and floor 0: the window of pair k is its whole target, every non-empty pair is aligned
+    ba.n = n; ba.seq_total = qbytes; ba.clen = pb.d_clen; ba.coff = pb.d_coff; ba.n_contigs = (int32_t)n;
+    ba.window = 0; ba.min_length = 0; ba.flags = c->p.flags;
+    ba.key = b->d_key; ba.tlen = b->d_tlen; ba.start = b->d_start; ba.hist = b->d_hist; ba.stats = b->d_stats;
+    ba.keybase = b->d_keybase; ba.cursor = b->d_cursor; ba.aln = b->d_aln; ba.aln_start = b->d_aln_start;
+    CU(c, launch_bin_classify(ba, c->sm_count, s2));
+    CU(c, cudaMemcpyAsync(b->h_hist, b->d_hist, (size_t)BIN_KEYS * 4, cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaMemcpyAsync(b->h_stats, b->d_stats, 128, cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaMemcpyAsync(b->h_over, pb.d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaEventRecord(b->ev_prep, s2));
+    CU(c, cudaEventSynchronize(b->ev_prep));
+    const int32_t bad = b->h_over[0];
+    if (bad >= 0 && bad < n)
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: the query of pair " + std::to_string(bad) +
+                                          " holds a letter outside the BAM nt16 alphabet =ACMGRSVTWYHKDBN");
+    if (b->h_stats[6] & 1ull) return fail(c, FADEGPU_E_CUDA, "fadegpu_align_pairs: internal error (query offsets)");
+    const int64_t n_aln = (int64_t)b->h_stats[1], n_x = (int64_t)b->h_stats[12];
+    {
+        int rc = ensure_dev(c, (void **)&pb.d_xpos, &pb.xpos_bytes, std::max<size_t>(16, (size_t)n_x * 8));
+        if (!rc) rc = ensure_dev(c, (void **)&pb.d_xchr, &pb.xchr_bytes, std::max<size_t>(16, (size_t)n_x));
+        if (rc) return rc;
+    }
+    pa.xpos = pb.d_xpos; pa.xchr = pb.d_xchr;
+    if (n_x > 0) CU(c, launch_pair_xlist(pa, s2));
+    { int rc = plan_from_histogram(c, b, n_aln); if (rc) return rc; }
+    if (n_aln > 0) {
+        CU(c, cudaMemcpyAsync(b->d_keybase, b->h_keybase, (size_t)BIN_KEYS * 4, cudaMemcpyHostToDevice, s2));
+        if (b->n_items > 0)
+            CU(c, cudaMemcpyAsync(b->d_items, b->h_items, (size_t)b->n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, s2));
+        h2d += (int64_t)BIN_KEYS * 4 + b->n_items * (int64_t)sizeof(WarpItem);
+        CU(c, launch_bin_scatter(ba, c->sm_count, s2));
+    }
+    CU(c, cudaEventRecord(b->ev_ready, s2));
+    // ---- SW kernels: the batch's plan against the packed targets ----
+    CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
+    CU(c, cudaEventRecord(b->ev[1], c->stream));
+    PlanTarget pt{};
+    pt.ref.planes.two = pb.d_two; pt.ref.planes.nmask = pb.d_n; pt.ref.planes.xmask = pb.d_x;
+    pt.ref.xpos = pb.d_xpos; pt.ref.xchr = pb.d_xchr; pt.ref.n_x = n_x;
+    pt.tags_only = 0;   // every pair is traced back, whatever the ctx's FADEGPU_F_TAGS_ONLY
+    pt.ops_spill = max_ops > 0 ? pb.d_spill : nullptr;
+    pt.ops_cap = max_ops;
+    int nl = 0;
+    { int rc = run_plan(c, b, pt, nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
+    // ---- records in pair order, home on stream3 ----
+    cudaStream_t s3 = c->stream3;
+    { int rc = join_kernels(c, b, s3); if (rc) return rc; }
+    CU(c, cudaEventRecord(b->ev[2], s3));
+    CU(c, launch_pair_results(pa, b->d_aln, b->d_out, (int)n_aln, pb.d_spill, max_ops, reinterpret_cast<PairResult *>(pb.d_res), pb.d_ops, b->d_stats + 7,
+                              c->sm_count, s3));
+    CU(c, cudaMemcpyAsync(out, pb.d_res, (size_t)n * sizeof(fadegpu_pair_result), cudaMemcpyDeviceToHost, s3));
+    if (max_ops > 0)
+        CU(c, cudaMemcpyAsync(ops_out, pb.d_ops, (size_t)n * (size_t)max_ops * 4, cudaMemcpyDeviceToHost, s3));
+    CU(c, cudaMemcpyAsync(b->h_stats + 7, b->d_stats + 7, 8, cudaMemcpyDeviceToHost, s3));
+    CU(c, cudaEventRecord(b->ev[3], s3));
+    CU(c, cudaEventSynchronize(b->ev[3]));
+    if ((int64_t)b->h_stats[7] != n_aln)
+        return fail(c, FADEGPU_E_CUDA, "fadegpu_align_pairs: a kernel did not produce a result record (internal error)");
+    st.n_aligned = n_aln;
+    st.n_generic = b->st.n_generic;
+    st.cells = (int64_t)b->h_stats[0];
+    st.h2d_bytes = h2d;
+    st.d2h_bytes = n * (int64_t)(sizeof(fadegpu_pair_result) + 4 * (size_t)max_ops) + (int64_t)BIN_KEYS * 4 + 128 + 4 + 8;
+    st.kernel_launches = nl + 3 + (n_x > 0 ? 1 : 0) + (n_aln > 0 ? 2 : 1);
+    st.scratch_bytes = b->st.scratch_bytes;
+    float t;
+    if (cudaEventElapsedTime(&t, b->ev[1], b->ev[2]) == cudaSuccess) st.kernel_ms = t;
+    if (cudaEventElapsedTime(&t, b->ev[0], b->ev[3]) == cudaSuccess) st.total_ms = t;
+    st.host_threads = c->host_threads;
+    st.host_submit_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    b->st = st;
+    if (stats_out) *stats_out = st;
+    return FADEGPU_OK;
 }
 
 int fadegpu_measure_alu_peak(fadegpu_ctx *c, double *ops_per_sec_out, double *sm_clock_mhz_out)

@@ -360,7 +360,9 @@ struct AdvanceSmem {
 };
 static_assert(sizeof(LaneCtl) % 4 == 0 && sizeof(AlnOut) % 4 == 0, "word-copyable");
 
-template <int R>
+// SPILL: the launch may carry a full-CIGAR spill ring (a.ops_spill, checked at run time); without it the walker is
+// compiled exactly as for the annotate path
+template <int R, bool SPILL>
 __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, unsigned warp0, unsigned nwarps,
                                               AdvanceSmem *smem_all)
 {
@@ -411,7 +413,13 @@ __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, un
             const int cur_blk = __shfl_sync(FULL, cur_blk_, 0);
             auto push_n = [&](uint32_t op, int n) {
                 if (cur != 0 && (cur & 0xf) == op) { cur += 16u * (uint32_t)n; return; }
-                if (cur != 0) { if (l == 0) c.ring[nrev % OPS_CAP] = cur; ++nrev; }
+                if (cur != 0) {
+                    if (l == 0) {
+                        c.ring[nrev % OPS_CAP] = cur;
+                        if (SPILL && a.ops_spill) a.ops_spill[(size_t)aln * a.ops_cap + nrev % a.ops_cap] = cur;
+                    }
+                    ++nrev;
+                }
                 cur = ((uint32_t)n << 4) | op;
             };
             int forced = 0;   // > 0: the next `forced` steps are DIAG by the ungapped-diagonal proof
@@ -519,7 +527,13 @@ __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, un
                     }
                 }
             }
-            if (done && cur != 0) { if (l == 0) c.ring[nrev % OPS_CAP] = cur; ++nrev; cur = 0; }
+            if (done && cur != 0) {
+                if (l == 0) {
+                    c.ring[nrev % OPS_CAP] = cur;
+                    if (SPILL && a.ops_spill) a.ops_spill[(size_t)aln * a.ops_cap + nrev % a.ops_cap] = cur;
+                }
+                ++nrev; cur = 0;
+            }
             if (l == 0) {
                 c.i = i; c.j = j; c.mode = mode; c.hval = hval; c.gval = gval; c.cur = cur; c.nrev = nrev;
                 if (done) { c.phase = 2; c.next_blk = -1; } else c.next_blk = need;
@@ -548,11 +562,11 @@ __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, un
     }
 }
 
-template <int R>
+template <int R, bool SPILL>
 __global__ void FADE_SMALL_KERNEL trace_advance_kernel(const KernelArgs a)
 {
     __shared__ AdvanceSmem adv[4];
-    advance_round<R>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5), adv);
+    advance_round<R, SPILL>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5), adv);
 }
 
 // The few alignments still unfinished after the full-grid rounds (very long paths): one block
@@ -570,7 +584,7 @@ __global__ void __launch_bounds__(128) trace_tail_kernel(const KernelArgs a)
         replay_round<R, TAGGED ? 0 : 1>(a, r, threadIdx.x >> 5, blockDim.x >> 5, tws_all);
         __threadfence_block();
         __syncthreads();
-        advance_round<R>(a, r, threadIdx.x >> 5, blockDim.x >> 5, adv);
+        advance_round<R, true>(a, r, threadIdx.x >> 5, blockDim.x >> 5, adv);   // (rarely reached: spill checked at run time)
         __threadfence_block();
         __syncthreads();
     }
@@ -711,11 +725,19 @@ __global__ void __launch_bounds__(128) sw_generic_kernel(const GenericArgs a)
             }
             if (cur != 0 && (cur & 0xf) == op) cur += 16;
             else {
-                if (cur != 0) { ring[nrev % OPS_CAP] = cur; ++nrev; }
+                if (cur != 0) {
+                    ring[nrev % OPS_CAP] = cur;
+                    if (a.ops_spill) a.ops_spill[(size_t)cur_idx * a.ops_cap + nrev % a.ops_cap] = cur;
+                    ++nrev;
+                }
                 cur = (1u << 4) | op;
             }
         }
-        if (cur != 0) { ring[nrev % OPS_CAP] = cur; ++nrev; }
+        if (cur != 0) {
+            ring[nrev % OPS_CAP] = cur;
+            if (a.ops_spill) a.ops_spill[(size_t)cur_idx * a.ops_cap + nrev % a.ops_cap] = cur;
+            ++nrev;
+        }
         out.end_query = bi; out.end_ref = bj; out.beg_query = i + 1; out.beg_ref = j + 1;
         const int lead = i + 1, trail = qlen - 1 - bi;
         const int n = (lead > 0) + nrev + (trail > 0);
@@ -896,6 +918,217 @@ __global__ void FADE_SMALL_KERNEL result_index_kernel(const AlnOut *out, int n_a
 }
 
 // ------------------------------------------------------------------------------------------------
+// pairs of caller-supplied sequences (fadegpu_align_pairs): pack the raw ASCII into the formats the
+// binning and the SW kernels read, then put the records back into pair order
+// ------------------------------------------------------------------------------------------------
+// ASCII -> BAM nt16 code of "=ACMGRSVTWYHKDBN" (either case), 16 = not in the alphabet
+__device__ __forceinline__ int nt16_of_ascii(int ch)
+{
+    if (ch >= 'a' && ch <= 'z') ch -= 32;
+    switch (ch) {
+    case '=': return 0; case 'A': return 1; case 'C': return 2; case 'M': return 3;
+    case 'G': return 4; case 'R': return 5; case 'S': return 6; case 'V': return 7;
+    case 'T': return 8; case 'W': return 9; case 'Y': return 10; case 'H': return 11;
+    case 'K': return 12; case 'D': return 13; case 'B': return 14; case 'N': return 15;
+    default: return 16;
+    }
+}
+
+// One warp per pair: lane 0 writes the pair's binning inputs, the lanes write the query as nt16 nibbles in REVERSE
+// COMPLEMENT, two bases per byte.  The kernels reverse-complement a read as they load it (source/util.d:18-34), which
+// restores the forward query; nt16 complement is an involution, so IUPAC letters come back unchanged.
+__global__ void FADE_SMALL_KERNEL pair_prep_kernel(const PairArgs a)
+{
+    const uint8_t comp16[16] = { 0, 8, 4, 12, 2, 10, 6, 14, 1, 9, 5, 13, 3, 11, 7, 15 };
+    const int l = threadIdx.x & 31;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < a.n; k += nwarps) {
+        const int64_t q0 = a.qoff[k], qlen = a.qoff[k + 1] - q0;
+        const int64_t t0 = a.toff[k], tlen = a.toff[k + 1] - t0;
+        const bool over = tlen > 0x7fffffff || qlen * tlen > PAIR_MAX_CELLS;   // left unaligned, reported
+        if (l == 0) {
+            a.seq_off[k] = q0;
+            a.pos[k] = 0;
+            a.l_qseq[k] = (int32_t)qlen;
+            a.tid[k] = (int32_t)k;
+            a.aligned_len[k] = over ? 0 : (int32_t)tlen;
+            a.clip_left[k] = over ? 0 : (int32_t)qlen;   // the length floor (0) passes every non-empty query
+            a.clip_right[k] = 0;
+            a.clen[k] = tlen;
+            a.coff[k] = 32 * (k + (t0 >> 5));
+        }
+        bool bad = false;
+        const char *q = a.query + q0;
+        for (int64_t b = l; b < (qlen + 1) / 2; b += 32) {
+            uint32_t byte = 0;
+            for (int h = 0; h < 2; ++h) {
+                const int64_t i = 2 * b + h;   // base i of the reverse complement = complement of base qlen-1-i
+                if (i >= qlen) break;
+                const int c = nt16_of_ascii((unsigned char)q[qlen - 1 - i]);
+                bad |= c > 15;
+                byte |= (uint32_t)comp16[c & 15] << (h ? 0 : 4);
+            }
+            a.seq4[q0 + b] = (uint8_t)byte;
+        }
+        if (__any_sync(0xffffffffu, bad) && l == 0) atomicMin(a.bad, (int32_t)k);
+    }
+}
+
+// the pair whose target holds global base p (targets start on 32-base boundaries, coff strictly increasing)
+__device__ __forceinline__ int64_t pair_of_base(const PairArgs &a, int64_t p)
+{
+    int64_t lo = 0, hi = a.n - 1;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi + 1) >> 1;
+        if (a.coff[mid] <= p) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// One block per chunk of PAIR_CHUNK_WORDS 32-base words (4 consecutive words per thread): the 2-bit, N and wildcard
+// planes of the targets, as fadegpu_load_reference packs contigs, and the chunk's number of wildcard letters.
+constexpr int PAIR_WORDS_PER_THREAD = PAIR_CHUNK_WORDS / 256;
+__global__ void __launch_bounds__(256) pair_pack_targets_kernel(const PairArgs a)
+{
+    __shared__ int warp_x[8];
+    int nx = 0;
+    for (int u = 0; u < PAIR_WORDS_PER_THREAD; ++u) {
+        const int64_t w = (int64_t)blockIdx.x * PAIR_CHUNK_WORDS + threadIdx.x * PAIR_WORDS_PER_THREAD + u;
+        if (w >= a.n_words) break;
+        uint32_t a0 = 0, a1 = 0, nm = 0, xm = 0;
+        if (a.n > 0) {
+            const int64_t p0 = 32 * w, k = pair_of_base(a, p0);
+            const int64_t local = p0 - a.coff[k], tlen = a.clen[k];
+            if (local >= 0 && local < tlen) {
+                const char *t = a.target + a.toff[k] + local;
+                const int lim = (int)min((int64_t)32, tlen - local);
+                for (int b = 0; b < lim; ++b) {
+                    int ch = (unsigned char)t[b];
+                    if (ch >= 'a' && ch <= 'z') ch -= 32;
+                    const uint32_t code = ch == 'A' ? 0u : ch == 'C' ? 1u : ch == 'T' ? 2u : ch == 'G' ? 3u : 0u;
+                    if (b < 16) a0 |= code << (2 * b); else a1 |= code << (2 * (b - 16));
+                    if (ch == 'N') nm |= 1u << b;
+                    else if (ch != 'A' && ch != 'C' && ch != 'G' && ch != 'T') xm |= 1u << b;
+                }
+            }
+        }
+        a.two[2 * w] = a0; a.two[2 * w + 1] = a1; a.nmask[w] = nm; a.xmask[w] = xm;
+        nx += __popc(xm);
+    }
+    nx = __reduce_add_sync(FULL, nx);
+    if ((threadIdx.x & 31) == 0) warp_x[threadIdx.x >> 5] = nx;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int t = 0;
+        for (int i = 0; i < 8; ++i) t += warp_x[i];
+        a.chunk_x[blockIdx.x] = (uint32_t)t;
+        if (t) atomicAdd(a.n_x, (unsigned long long)t);
+    }
+}
+
+// exclusive prefix of v over a block of 256 threads; *total receives the sum
+__device__ __forceinline__ uint32_t block_exclusive_256(uint32_t v, uint32_t *total)
+{
+    __shared__ uint32_t warp_sum[8];
+    const int l = threadIdx.x & 31, wi = threadIdx.x >> 5;
+    uint32_t inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t y = __shfl_up_sync(FULL, inc, o);
+        if (l >= o) inc += y;
+    }
+    if (l == 31) warp_sum[wi] = inc;
+    __syncthreads();
+    uint32_t before = 0, all = 0;
+    for (int i = 0; i < 8; ++i) { if (i < wi) before += warp_sum[i]; all += warp_sum[i]; }
+    __syncthreads();
+    *total = all;
+    return before + inc - v;
+}
+
+// Order-preserving compaction of the wildcard letters into the sorted (position, upper-cased letter) list that the
+// generic kernel searches (RefDev::xpos / xchr).  Chunk b starts at the sum of chunk_x over the chunks before it.
+__global__ void __launch_bounds__(256) pair_xlist_kernel(const PairArgs a)
+{
+    __shared__ uint32_t chunk_base;
+    if (a.chunk_x[blockIdx.x] == 0) return;   // (uniform over the block)
+    if (threadIdx.x == 0) chunk_base = 0;
+    __syncthreads();
+    {   // chunk_x is small (one word per 32768 target bases): the block adds up its predecessors
+        uint32_t part = 0;
+        for (int64_t c = threadIdx.x; c < blockIdx.x; c += blockDim.x) part += a.chunk_x[c];
+        part = __reduce_add_sync(FULL, part);
+        if ((threadIdx.x & 31) == 0 && part) atomicAdd(&chunk_base, part);
+    }
+    __syncthreads();
+    const int64_t w0 = (int64_t)blockIdx.x * PAIR_CHUNK_WORDS + threadIdx.x * PAIR_WORDS_PER_THREAD;
+    uint32_t xm[PAIR_WORDS_PER_THREAD], cnt = 0;
+    for (int u = 0; u < PAIR_WORDS_PER_THREAD; ++u) {
+        xm[u] = w0 + u < a.n_words ? a.xmask[w0 + u] : 0u;
+        cnt += __popc(xm[u]);
+    }
+    uint32_t total;
+    int64_t slot = (int64_t)chunk_base + block_exclusive_256(cnt, &total);
+    for (int u = 0; u < PAIR_WORDS_PER_THREAD; ++u) {
+        if (!xm[u]) continue;
+        const int64_t p0 = 32 * (w0 + u), k = pair_of_base(a, p0);
+        const char *t = a.target + a.toff[k] + (p0 - a.coff[k]);
+        for (uint32_t m = xm[u]; m; m &= m - 1) {
+            const int b = __ffs(m) - 1;
+            int ch = (unsigned char)t[b];
+            if (ch >= 'a' && ch <= 'z') ch -= 32;
+            a.xpos[slot] = p0 + b;
+            a.xchr[slot] = (uint8_t)ch;
+            ++slot;
+        }
+    }
+}
+
+__global__ void FADE_SMALL_KERNEL pair_results_init_kernel(const PairArgs a, PairResult *res)
+{
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < a.n; k += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t qlen = a.qoff[k + 1] - a.qoff[k], tlen = a.toff[k + 1] - a.toff[k];
+        PairResult r;
+        r.score = r.end_query = r.end_ref = r.beg_query = r.beg_ref = r.n_ops = 0;
+        r.reserved = 0;
+        r.flags = (qlen > 0 && tlen > 0 && (tlen > 0x7fffffff || qlen * tlen > PAIR_MAX_CELLS)) ? PAIR_R_OVERSIZE : 0u;
+        res[k] = r;
+    }
+}
+
+// one thread per alignment: its record goes to the pair's slot, its forward CIGAR (P5) is assembled from the spill ring
+__global__ void FADE_SMALL_KERNEL pair_results_kernel(const AlnDesc *aln, const AlnOut *out, int n_aln, int64_t n,
+                                                      const uint32_t *spill, int max_ops, PairResult *res, uint32_t *ops,
+                                                      unsigned long long *n_ok)
+{
+    int ok = 0;
+    for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < n_aln; idx += gridDim.x * blockDim.x) {
+        const AlnOut o = out[idx];
+        const int64_t k = o.read;
+        if (k < 0 || k >= n || !(o.flags & R_ALIGNED) || (o.flags & 0x80000000u)) continue;
+        ++ok;
+        PairResult r;
+        r.score = o.score; r.end_query = o.end_query; r.end_ref = o.end_ref; r.beg_query = o.beg_query; r.beg_ref = o.beg_ref;
+        r.n_ops = o.n_ops;
+        r.flags = (o.flags & (R_ALIGNED | R_GENERIC)) | (o.n_ops > max_ops ? R_OPS_TRUNC : 0u);
+        r.reserved = 0;
+        res[k] = r;
+        if (max_ops > 0) {
+            uint32_t *dst = ops + (size_t)k * max_ops;
+            if (o.n_ops == 0) {
+                for (int w = 0; w < max_ops; ++w) dst[w] = 0;
+            } else {
+                const int lead = o.beg_query, trail = aln[idx].qlen - 1 - o.end_query;
+                const int nrev = o.n_ops - (lead > 0) - (trail > 0);
+                forward_ops(spill + (size_t)idx * max_ops, max_ops, nrev, lead, trail, dst);
+            }
+        }
+    }
+    ok = __reduce_add_sync(FULL, ok);
+    if ((threadIdx.x & 31) == 0 && ok) atomicAdd(n_ok, (unsigned long long)ok);
+}
+
+// ------------------------------------------------------------------------------------------------
 // INT16x2 ALU issue-rate microbenchmark: 8 independent VIADDMNMX.S16x2 chains per thread
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) alu_peak_kernel(uint32_t *out, int iters)
@@ -966,7 +1199,8 @@ static cudaError_t launch_trace_tt(KernelArgs a, cudaStream_t s, int sm_count, i
             else trace_replay_kernel<R, 2, false><<<std::max(g1, 1), 128, 0, s>>>(a);
         }
         else trace_replay_kernel<R, TAGGED ? 0 : 1><<<std::max(g1, 1), 128, 0, s>>>(a);
-        trace_advance_kernel<R><<<std::max(g2, 1), 128, 0, s>>>(a);
+        if (a.ops_spill) trace_advance_kernel<R, true><<<std::max(g2, 1), 128, 0, s>>>(a);
+        else trace_advance_kernel<R, false><<<std::max(g2, 1), 128, 0, s>>>(a);
         nl += 2;
     }
     if (r < a.max_rounds) {
@@ -1062,6 +1296,40 @@ cudaError_t launch_generic(const GenericArgs &a, int n_slots, cudaStream_t s)
     const int grid = (n_slots + threads - 1) / threads;
     if (a.n_slots != n_slots || a.chunk <= 0) return cudaErrorInvalidValue;
     sw_generic_kernel<<<grid, threads, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pair_prep(const PairArgs &a, int sm_count, cudaStream_t s)
+{
+    if (a.n <= 0) return cudaSuccess;
+    const int grid = (int)std::min<int64_t>((a.n * 32 + 127) / 128, (int64_t)sm_count * 16);
+    pair_prep_kernel<<<grid, 128, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pair_pack_targets(const PairArgs &a, cudaStream_t s)
+{
+    if (a.n_words <= 0) return cudaSuccess;
+    pair_pack_targets_kernel<<<(unsigned)((a.n_words + PAIR_CHUNK_WORDS - 1) / PAIR_CHUNK_WORDS), 256, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pair_xlist(const PairArgs &a, cudaStream_t s)
+{
+    if (a.n_words <= 0) return cudaSuccess;
+    pair_xlist_kernel<<<(unsigned)((a.n_words + PAIR_CHUNK_WORDS - 1) / PAIR_CHUNK_WORDS), 256, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pair_results(const PairArgs &a, const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill,
+                                int max_ops, PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count,
+                                cudaStream_t s)
+{
+    if (a.n <= 0) return cudaSuccess;
+    pair_results_init_kernel<<<(int)std::min<int64_t>((a.n + 127) / 128, (int64_t)sm_count * 16), 128, 0, s>>>(a, res);
+    if (n_aln > 0)
+        pair_results_kernel<<<std::min((n_aln + 127) / 128, sm_count * 16), 128, 0, s>>>(aln, out, n_aln, a.n, spill, max_ops,
+                                                                                       res, ops, n_ok);
     return cudaGetLastError();
 }
 

@@ -5,6 +5,8 @@
 //                        S padding and accept predicates                            (P3-P5, F9)
 //   sw_generic_kernel    exact int32 fallback ON THE DEVICE for wildcard letters and sizes the
 //                        packed kernels do not cover (thread per alignment)
+//   pair_*_kernel        fadegpu_align_pairs: pack caller-supplied ASCII pairs into the read / reference formats
+//                        above, and put the records back into pair order
 //   alu_peak_kernel      INT16x2 ALU issue-rate microbenchmark (roofline denominator)
 //
 // Window gather (source/analysis.d:45-64) and reverse complement (source/util.d:18-34) happen
@@ -65,6 +67,8 @@ struct KernelArgs {
     uint32_t *tiles;           // [ceil(n_aln/2)] trace tiles of the current round
     int32_t round, max_rounds;
     int32_t tags_only;         // FADEGPU_F_TAGS_ONLY
+    uint32_t *ops_spill;       // [n_aln * ops_cap] full reversed-op ring per alignment (ctl_advance); nullptr = none
+    int32_t ops_cap;
 };
 
 struct GenericArgs {
@@ -82,6 +86,8 @@ struct GenericArgs {
     int32_t chunk;             // work items claimed per atomic
     int32_t open, extend, match, mismatch, min_length;
     int32_t tags_only;         // FADEGPU_F_TAGS_ONLY
+    uint32_t *ops_spill;       // as KernelArgs::ops_spill
+    int32_t ops_cap;
 };
 
 // ---- binning on the device (pinned-view submits): classify reads, histogram by (class, window
@@ -120,6 +126,44 @@ struct BinArgs {
     unsigned long long *seq_cursor; // device byte cursor into the compact sequence buffer; nullptr = seq_off is final
     int64_t *src_off;               // [n_aln] offset of each alignment's bases in the pinned view
 };
+
+// ---- pairs of caller-supplied sequences (fadegpu_align_pairs): the raw ASCII is packed on the device into the
+//      formats the binning and the SW kernels read -- the targets become the "contigs" of a reference of their own ----
+struct PairArgs {
+    int64_t n;
+    const char *query, *target;     // concatenated ASCII
+    const int64_t *qoff, *toff;     // [n+1], starting at 0
+    // per-pair inputs of the binning (tid = k, pos = 0, aligned_len = tlen, clip_left = qlen, clip_right = 0)
+    int64_t *seq_off, *pos;
+    int32_t *l_qseq, *tid, *aligned_len, *clip_left, *clip_right;
+    int64_t *clen, *coff;           // contig table: target k starts at coff[k] = 32 * (k + toff[k] / 32)
+    uint8_t *seq4;                  // queries as BAM nt16 nibbles, reverse-complemented, query k at byte qoff[k]
+    int32_t *bad;                   // lowest pair whose query holds a letter outside nt16 (atomicMin; starts at n)
+    // target planes (DESIGN 3) and the sorted wildcard list
+    uint32_t *two, *nmask, *xmask;
+    int64_t n_words;                // 32-base words of the planes
+    uint32_t *chunk_x;              // [n_chunks] wildcard letters per chunk of PAIR_CHUNK_WORDS words
+    unsigned long long *n_x;        // their total
+    int64_t *xpos;
+    uint8_t *xchr;
+};
+constexpr int PAIR_CHUNK_WORDS = 1024;
+// qlen * tlen above this is not aligned (FADEGPU_R_OVERSIZE), as for reads
+constexpr int64_t PAIR_MAX_CELLS = (int64_t)1 << 31;
+constexpr uint32_t PAIR_R_OVERSIZE = 32u;   // FADEGPU_R_OVERSIZE
+cudaError_t launch_pair_prep(const PairArgs &a, int sm_count, cudaStream_t s);
+cudaError_t launch_pair_pack_targets(const PairArgs &a, cudaStream_t s);   // planes + chunk_x + n_x
+cudaError_t launch_pair_xlist(const PairArgs &a, cudaStream_t s);          // xpos / xchr (after n_x is known)
+// pair-ordered result records: zeros (or FADEGPU_R_OVERSIZE) for every pair, then the records of the alignments with
+// their full forward CIGARs assembled from the spill rings; n_ok counts the records the SW kernels produced
+struct PairResult {   // == fadegpu_pair_result
+    int32_t score, end_query, end_ref, beg_query, beg_ref, n_ops;
+    uint32_t flags;
+    int32_t reserved;
+};
+cudaError_t launch_pair_results(const PairArgs &a, const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill,
+                                int max_ops, PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count,
+                                cudaStream_t s);
 
 constexpr int FILL_THREADS = 128;
 constexpr int OVER_CAP = 256;        // oversize reads listed per batch (all of them are counted)

@@ -550,8 +550,12 @@ FD bool ctl_select_end(LaneCtl &c)
     return true;
 }
 
+// spill (optional): a second ring of `spill_cap` words in global storage that receives every op the walker completes,
+// at ring[nrev % spill_cap], so that CIGARs longer than OPS_CAP can be assembled in full (fadegpu_align_pairs).
+// c.ring is written as before either way.
 template <int R, class Acc>
-FD void ctl_advance(LaneCtl &c, const uint32_t *tile, int lane, const Acc &acc, const SwConsts &k)
+FD void ctl_advance(LaneCtl &c, const uint32_t *tile, int lane, const Acc &acc, const SwConsts &k,
+                    uint32_t *spill = nullptr, int spill_cap = 0)
 {
     if (c.phase == 2) return;
     c.cur_blk = c.next_blk;
@@ -564,7 +568,7 @@ FD void ctl_advance(LaneCtl &c, const uint32_t *tile, int lane, const Acc &acc, 
     int need = -1;
     auto push = [&](uint32_t op) {
         if (cur != 0 && (cur & 0xf) == op) { cur += 16; return; }
-        if (cur != 0) { c.ring[nrev % OPS_CAP] = cur; ++nrev; }
+        if (cur != 0) { c.ring[nrev % OPS_CAP] = cur; if (spill) spill[nrev % spill_cap] = cur; ++nrev; }
         cur = (1u << 4) | op;
     };
     for (;;) {
@@ -617,7 +621,11 @@ FD void ctl_advance(LaneCtl &c, const uint32_t *tile, int lane, const Acc &acc, 
         }
     }
     c.i = i; c.j = j; c.mode = mode; c.hval = hval; c.gval = gval;
-    if (done && cur != 0) { c.ring[nrev % OPS_CAP] = cur; ++nrev; cur = 0; }   // flush the last op
+    if (done && cur != 0) {   // flush the last op
+        c.ring[nrev % OPS_CAP] = cur;
+        if (spill) spill[nrev % spill_cap] = cur;
+        ++nrev; cur = 0;
+    }
     c.cur = cur; c.nrev = nrev;
     if (!done) { c.next_blk = need; return; }
     c.phase = 2;
@@ -671,6 +679,23 @@ FD bool score_may_accept(int score, uint32_t clip_left, uint32_t clip_right, int
     return false;
 }
 
+// P5 (dparasail wrapper): forward CIGAR = [S lead] + reversed ring + [S trail].  `ring` holds the last `cap` of the
+// nrev reversed ops the walker pushed (entry nrev % cap), i.e. the first ones of the forward CIGAR; dst receives the
+// first min(n_ops, cap) forward ops, zero-padded to cap.  finalize_result and sw_generic_kernel do the same for their
+// 10-entry rings.
+FD void forward_ops(const uint32_t *ring, int cap, int nrev, int lead, int trail, uint32_t *dst)
+{
+    const int n = (lead > 0) + nrev + (trail > 0);
+    int w = 0;
+    if (lead > 0) dst[w++] = ((uint32_t)lead << 4) | OP_S;
+    for (int k = nrev - 1; k >= 0 && w < cap; --k) {
+        if (nrev - k > cap) break;  // older entries were overwritten in the ring
+        dst[w++] = ring[k % cap];
+    }
+    if (trail > 0 && w < cap && w == n - 1) dst[w++] = ((uint32_t)trail << 4) | OP_S;
+    for (int k = w; k < cap; ++k) dst[k] = 0;
+}
+
 // P5 (dparasail wrapper): forward CIGAR = [S lead] + reversed ring + [S trail]; then predicates.
 FD void finalize_result(const LaneCtl &c, AlnOut &o, int read, uint32_t clip_left, uint32_t clip_right,
                         int32_t min_length)
@@ -691,7 +716,7 @@ FD void finalize_result(const LaneCtl &c, AlnOut &o, int read, uint32_t clip_lef
     const int lead = o.beg_query, trail = c.qlen - 1 - c.end_i;
     const int n = (lead > 0) + c.nrev + (trail > 0);
     o.n_ops = n;
-    int w = 0;
+    int w = 0;   // (forward_ops with cap OPS_CAP, written out so that the annotate kernels compile as they always have)
     if (lead > 0) o.ops[w++] = ((uint32_t)lead << 4) | OP_S;
     for (int k = c.nrev - 1; k >= 0 && w < OPS_CAP; --k) {
         if (c.nrev - k > OPS_CAP) break;  // older entries were overwritten in the ring

@@ -240,6 +240,50 @@ int fadegpu_replay_kernels(fadegpu_ctx *ctx, fadegpu_batch *b, int32_t iters, fl
 int fadegpu_replay_batches(fadegpu_ctx *ctx, fadegpu_batch *const *batches, int32_t n_batches, int32_t iters,
                            float *ms_out);
 
+/* ---- Pairwise Smith-Waterman with traceback on caller-supplied sequences ----
+ * Pair k is query[query_off[k] .. query_off[k+1]) against target[target_off[k] .. target_off[k+1]).
+ *
+ * Alignment semantics: exactly P1-P5 (SURVEY 8a) with the ctx's scoring, the query taken as given (no reverse
+ *   complement) and the whole target as the window.  Query and target are upper-cased, as the reference path does
+ *   (toUpper, source/analysis.d:63).
+ * Target letters: any byte -- ACGT, N as a real symbol, everything else a wildcard, as in fadegpu_load_reference.
+ * Query letters: they must lie in the BAM nt16 alphabet =ACMGRSVTWYHKDBN, in either case (the kernels read queries as
+ *   nt16 codes).  Any other letter fails the call with FADEGPU_E_ARG, and fadegpu_last_error names the first pair
+ *   holding one.
+ * Scoring: from the ctx (fadegpu_params); a ctx used only for pairs needs no fadegpu_load_reference.  The ctx's
+ *   FADEGPU_F_FORCE_GENERIC applies; FADEGPU_F_TAGS_ONLY does not: every pair is traced back.
+ * CIGAR ops: n_ops is always exact.  ops_out[k * max_ops ..] holds the first min(n_ops, max_ops) ops of pair k's forward
+ *   CIGAR (BAM-encoded, S padding included, zero-filled), and FADEGPU_R_OPS_TRUNC is set when n_ops > max_ops -- the
+ *   convention of the 10-op records.  max_ops = 3 * max(query length) never truncates: a local alignment starts and
+ *   ends with a diagonal step, every =/X run holds one, between two of them lie at most one I and one D run, plus at
+ *   most two S ops.  ops_out may be NULL iff max_ops == 0.
+ * Empty pairs: a pair with an empty query or target gets flags = 0 and a zero record.
+ * Oversize pairs: a pair with query length * target length > 2^31 is not aligned; it gets FADEGPU_R_OVERSIZE and is
+ *   counted in stats_out->n_oversize.  FADEGPU_R_ART_* and FADEGPU_R_SCORE_ONLY are never set.
+ * In-flight batches: while a batch of the ctx is submitted and not yet waited for, the call fails with
+ *   FADEGPU_E_STATE.
+ * No side effects on batches: the results of waited batches (fadegpu_get_results) stay valid, and
+ *   fadegpu_replay_kernels / fadegpu_replay_batches of existing batches keep working.
+ *
+ * Synchronous.  The arrays are host memory (pageable is fine) and only read during the call.  out[n_pairs] receives
+ * the records in PAIR ORDER.  stats_out (may be NULL) receives, for this call: n_reads = n_pairs, n_aligned, n_generic,
+ * cells, n_oversize, kernel_launches, h2d / d2h bytes, kernel_ms (the SW kernels: fills, traceback, generic) and
+ * total_ms (upload to results home); the per-stage fill / trace / generic times are not taken (0). */
+typedef struct fadegpu_pairs {
+    const char *query;  const int64_t *query_off;    /* [n+1] ASCII queries, concatenated */
+    const char *target; const int64_t *target_off;   /* [n+1] ASCII targets, concatenated */
+} fadegpu_pairs;                                     /* 32 bytes */
+
+typedef struct fadegpu_pair_result {
+    int32_t score, end_query, end_ref, beg_query, beg_ref;  /* as fadegpu_result; beg_ref == res.position */
+    int32_t n_ops;                                          /* full length of the forward CIGAR, S padding included (P5) */
+    uint32_t flags;         /* FADEGPU_R_ALIGNED | FADEGPU_R_GENERIC | FADEGPU_R_OPS_TRUNC | FADEGPU_R_OVERSIZE only */
+    int32_t reserved;
+} fadegpu_pair_result;                                      /* 32 bytes */
+
+int fadegpu_align_pairs(fadegpu_ctx *ctx, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
+                        fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out);
+
 /* INT16x2 ALU roofline denominator (SURVEY 8d): measures packed VIMNMX/VIADDMNMX issue rate.
  * ops_per_sec_out = packed (2-lane) instructions * 32 threads per second over the whole GPU. */
 int fadegpu_measure_alu_peak(fadegpu_ctx *ctx, double *ops_per_sec_out, double *sm_clock_mhz_out);
