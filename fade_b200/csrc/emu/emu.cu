@@ -17,7 +17,7 @@ namespace {
 
 template <int R>
 struct ThreadState {
-    uint32_t H[R], E[R], qs[R], qf[R];   // qf: query words of fill_step_f16
+    uint32_t H[R], E[R], qs[R], qf[R], qp[(R + 1) / 2];   // qf / qp: query words of fill_step_f16 / fill_step_f16x2
     uint32_t hu_prev, fout, M;
 };
 
@@ -48,7 +48,8 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
             const int ca = i < qlen_a ? qa[i] : C_QPAD;
             const int cb = i < qlen_b ? qb[i] : C_QPAD;
             st[g].qs[r] = q_sel(ca, cb);
-            st[g].qf[r] = q_self(ca, cb);
+            set_query<1>(st[g].qf, r, ca, cb);
+            set_query<2>(st[g].qp, r, ca, cb);
             qc[i] = (uint8_t)(ca | (cb << 4));
         }
     auto init_state = [&](ThreadState<R> &s) {
@@ -57,8 +58,8 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
     };
     for (int g = 0; g < FG; ++g) init_state(st[g]);
 
-    // ---- score-only pass with checkpoints (the fp16 step where the scoring allows it, as on the device) ----
-    const bool f16 = k.f16_ok && !(tagged & 8);
+    // ---- score-only pass with checkpoints (the step make_consts chose, as on the device) ----
+    const int step = (tagged & 8) ? 0 : ((tagged & 16) && k.f16_ok ? 1 : score_step_for(k));
     const int CW = ck_words<R>();
     std::vector<uint32_t> ck((size_t)nblk * FG * CW);
     LaneCtl ctl[2];
@@ -76,8 +77,9 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
             for (int g = 0; g < FG; ++g) {
                 const uint32_t ts = tw[t - g + FG];
                 const uint32_t hd = st[g].hu_prev;
-                if (f16) fill_step_f16<R>(st[g].H, st[g].E, st[g].qf, st[g].M, ts, hd, fin[g], st[g].fout, k);
-                else fill_step<R>(st[g].H, st[g].E, st[g].qs, st[g].M, ts, hd, fin[g], st[g].fout, k);
+                if (step == 2) score_step<R, 2>(st[g].H, st[g].E, st[g].qp, st[g].M, ts, hd, fin[g], st[g].fout, k);
+                else if (step == 1) score_step<R, 1>(st[g].H, st[g].E, st[g].qf, st[g].M, ts, hd, fin[g], st[g].fout, k);
+                else score_step<R, 0>(st[g].H, st[g].E, st[g].qs, st[g].M, ts, hd, fin[g], st[g].fout, k);
                 st[g].hu_prev = hu[g];
             }
         }
@@ -203,6 +205,7 @@ extern "C" int fadeemu_align_pair(int R, const uint8_t *qa, int qlen_a, const ui
     SwConsts k = make_consts(open, extend, match, mismatch);
     k.shortcut = (tagged & 2) ? 0 : 1;   // bit 1 of `tagged`: disable the ungapped-diagonal shortcut
                                          // bit 3: integer score-only step even where the fp16 one is exact
+                                         // bit 4: fill_step_f16 even where fill_step_f16x2 is exact
 #define CASE(RR)                                                                                   \
     case RR:                                                                                       \
         return align_pair<RR>(qa, qlen_a, ta, tlen_a, qb, qlen_b, tb, tlen_b, k, extra_blocks,    \
@@ -239,6 +242,21 @@ extern "C" int fadeemu_comp_code_of_nt16(int nib) { return comp_code_of_nt16(nib
 extern "C" uint32_t fadeemu_prmt(uint32_t a, uint32_t b, uint32_t s) { return prmt_sx(a, b, s); }
 extern "C" int fadeemu_sizeof_alnout(void) { return (int)sizeof(AlnOut); }
 extern "C" int fadeemu_f16_ok(int open, int extend, int match, int mismatch) { return make_consts(open, extend, match, mismatch).f16_ok; }
+// make_consts' choice for fill_step_f16x2: out = { f16_pair_ok, high byte of match, of mismatch, IMAD addend c }
+extern "C" void fadeemu_f16_pair(int open, int extend, int match, int mismatch, uint32_t *out)
+{
+    const SwConsts k = make_consts(open, extend, match, mismatch);
+    out[0] = (uint32_t)k.f16_pair_ok; out[1] = k.plut0 & 0xffu; out[2] = (k.plut0 >> 8) & 0xffu; out[3] = k.pair_c;
+}
+// f16_step_exact(pair = true) for the given high bytes and addend
+extern "C" int fadeemu_f16_pair_exact(int open, int extend, int match, int mismatch, uint32_t pm, uint32_t px, uint32_t c)
+{
+    SwConsts k = make_consts(open, extend, match, mismatch);
+    k.plut0 = pm | (px << 8) | (px << 16) | (px << 24);
+    k.plut1 = px * 0x01010101u;
+    k.pair_c = c;
+    return f16_step_exact(k, true) ? 1 : 0;
+}
 extern "C" void fadeemu_fma_f16x2(const uint32_t *a, const uint32_t *b, const uint32_t *c, uint32_t *out, int64_t n)
 {
     for (int64_t i = 0; i < n; ++i) out[i] = fma_f16x2(a[i], b[i], c[i]);

@@ -40,10 +40,10 @@ __device__ __forceinline__ uint32_t stage_targets(const KernelArgs &a, const Aln
     return w;
 }
 
-// F16: query words for fill_step_f16 (q_self) instead of fill_step (q_sel)
-template <int R, bool F16>
+// STEP: query words of that score-only step (score_step, sw_core.cuh)
+template <int R, int STEP>
 __device__ __forceinline__ void stage_pair(const KernelArgs &a, const AlnDesc &da, const AlnDesc &db,
-                                           int g, int nblk, uint16_t *tw, uint32_t (&qs)[R],
+                                           int g, int nblk, uint16_t *tw, uint32_t (&qs)[query_words<R, STEP>()],
                                            uint8_t *qc, uint32_t &wild)
 {
     uint32_t w = stage_targets(a, da, db, g, 0, FBLK * min(nblk, FILL_CHUNK_BLOCKS), tw);
@@ -55,7 +55,7 @@ __device__ __forceinline__ void stage_pair(const KernelArgs &a, const AlnDesc &d
         if (i < da.qlen) ca = rc_query_code(sa, da.qlen, i);
         if (i < db.qlen) cb = rc_query_code(sb, db.qlen, i);
         w |= (ca == C_WILD ? 1u : 0u) | (cb == C_WILD ? 2u : 0u);
-        qs[r] = F16 ? q_self(ca, cb) : q_sel(ca, cb);
+        set_query<STEP>(qs, r, ca, cb);
         if (qc) qc[i] = (uint8_t)(ca | (cb << 4));
     }
     wild = w;
@@ -69,19 +69,10 @@ __device__ __forceinline__ AlnDesc load_desc(const KernelArgs &a, int idx)
     return d;
 }
 
-// score-only step: fill_step_f16 (scorings with k.f16_ok, query words from q_self) or fill_step (q_sel)
-template <int R, bool F16>
-__device__ __forceinline__ void score_step(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R], uint32_t &M,
-                                           uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out, const SwConsts &k)
-{
-    if (F16) fill_step_f16<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
-    else fill_step<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
-}
-
 // ------------------------------------------------------------------------------------------------
 // score-only wavefront with checkpoints
 // ------------------------------------------------------------------------------------------------
-template <int R, bool F16>
+template <int R, int STEP>
 __global__ void __launch_bounds__(FILL_THREADS, (R <= 19 ? 5 : 1)) sw_fill_kernel(const KernelArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -96,9 +87,9 @@ __global__ void __launch_bounds__(FILL_THREADS, (R <= 19 ? 5 : 1)) sw_fill_kerne
     const int nblk = item.nblk;
     const SwConsts k = a.k;
 
-    uint32_t H[R], E[R], qs[R];
+    uint32_t H[R], E[R], qs[query_words<R, STEP>()];
     uint32_t wild;
-    stage_pair<R, F16>(a, da, db, g, nblk, tw, qs, nullptr, wild);
+    stage_pair<R, STEP>(a, da, db, g, nblk, tw, qs, nullptr, wild);
 #pragma unroll
     for (int r = 0; r < R; ++r) { H[r] = 0u; E[r] = k.neg_o; }
     uint32_t hu_prev = 0u, fout = k.neg_o, M = 0u, Mprev = 0u;
@@ -125,7 +116,7 @@ __global__ void __launch_bounds__(FILL_THREADS, (R <= 19 ? 5 : 1)) sw_fill_kerne
             uint32_t fin = __shfl_up_sync(FULL, fout, 1, FG);
             if (g == 0) { hu = 0u; fin = k.neg_o; }
             const uint32_t ts = twp[t];
-            score_step<R, F16>(H, E, qs, M, ts, hu_prev, fin, fout, k);
+            score_step<R, STEP>(H, E, qs, M, ts, hu_prev, fin, fout, k);
             hu_prev = hu;
         }
         if (c + 1 < nblk) {
@@ -212,8 +203,8 @@ __global__ void FADE_SMALL_KERNEL trace_init_kernel(const KernelArgs a)
 
 // MODE 0: tagged trace recording, 1: plain trace recording, 2: scan only (round 0: find the end cell,
 // no trace tile; the traceback then tries the ungapped-diagonal proof before asking for a traced replay)
-// with the score-only step, fill_step_f16 when F16
-template <int R, int MODE, bool F16 = false>
+// with the score-only step STEP (score_step)
+template <int R, int MODE, int STEP = 0>
 __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, unsigned warp0, unsigned nwarps,
                                              uint16_t (*tws_all)[40])
 {
@@ -258,7 +249,7 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
             }
         }
         // ---- wavefront state of the requested blocks (checkpoints are in the plain domain) ----
-        uint32_t H[R], E[R], qs[R], hu_prev, fout;
+        uint32_t H[R], E[R], qs[query_words<R, STEP>()], hu_prev, fout;
         {
             const uint32_t *p0 = ckp[0] + (size_t)(blk[0] > 0 ? blk[0] - 1 : 0) * CW * 32;
             const uint32_t *p1 = ckp[1] + (size_t)(blk[1] > 0 ? blk[1] - 1 : 0) * CW * 32;
@@ -284,7 +275,7 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
                 const int i = g * R + r;
                 const int ca = i < d[0].qlen ? rc_query_code(s0, d[0].qlen, i) : C_QPAD;
                 const int cb = i < d[1].qlen ? rc_query_code(s1, d[1].qlen, i) : C_QPAD;
-                qs[r] = F16 ? q_self(ca, cb) : q_sel(ca, cb);
+                set_query<STEP>(qs, r, ca, cb);
             }
             __syncwarp();   // previous iteration's readers of tws are done
             for (int x = g; x < FBLK + FG - 1; x += FG) {
@@ -306,8 +297,8 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
             if (g == 0) { hu = 0u; fin = e_init; }
             const uint32_t ts = twp[u];
             uint32_t cmax = 0u;
-            if (SCAN_ONLY) {
-                score_step<R, F16>(H, E, qs, cmax, ts, hu_prev, fin, fout, k);
+            if constexpr (SCAN_ONLY) {
+                score_step<R, STEP>(H, E, qs, cmax, ts, hu_prev, fin, fout, k);
             } else {
                 uint32_t trw[RW];
                 if (TAGGED) trace_step_tagged<R>(H, E, qs, ts, hu_prev, fin, fout, k, trw, cmax);
@@ -339,13 +330,13 @@ __device__ __forceinline__ void replay_round(const KernelArgs &a, int round, uns
     }
 }
 
-template <int R, int MODE, bool F16 = false>
+template <int R, int MODE, int STEP = 0>
 __global__ void __launch_bounds__(128) trace_replay_kernel(const KernelArgs a)
 {
     __shared__ uint16_t tws_all[16][40];
     if (blockIdx.x == 0 && threadIdx.x == 0) a.qcount[(a.round & 1) ^ 1] = 0u;   // next round's queue starts empty
-    replay_round<R, MODE, F16>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
-                            gridDim.x * (blockDim.x >> 5), tws_all);
+    replay_round<R, MODE, STEP>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
+                                gridDim.x * (blockDim.x >> 5), tws_all);
 }
 
 // One WARP per request.  The traceback is a pointer chase; to avoid one L2 round trip per step the
@@ -1154,22 +1145,26 @@ int tw_stride_for(int nblk_max) { return (FBLK * std::min(nblk_max, FILL_CHUNK_B
 
 size_t fill_smem_bytes(int tw_stride) { return (size_t)(FILL_THREADS / FG) * tw_stride * 2; }
 
-template <int R, bool F16>
+template <int R, int STEP>
 static cudaError_t launch_fill_tf(const KernelArgs &a, cudaStream_t s)
 {
     const size_t smem = fill_smem_bytes(a.tw_stride);
-    cudaError_t e = cudaFuncSetAttribute(sw_fill_kernel<R, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(sw_fill_kernel<R, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const int wpb = FILL_THREADS / 32;
     const int grid = (a.n_items + wpb - 1) / wpb;
-    sw_fill_kernel<R, F16><<<grid, FILL_THREADS, smem, s>>>(a);
+    sw_fill_kernel<R, STEP><<<grid, FILL_THREADS, smem, s>>>(a);
     return cudaGetLastError();
 }
 
 template <int R>
 static cudaError_t launch_fill_t(const KernelArgs &a, cudaStream_t s)
 {
-    return a.k.f16_ok ? launch_fill_tf<R, true>(a, s) : launch_fill_tf<R, false>(a, s);
+    switch (score_step_for(a.k)) {
+    case 2: return launch_fill_tf<R, 2>(a, s);
+    case 1: return launch_fill_tf<R, 1>(a, s);
+    default: return launch_fill_tf<R, 0>(a, s);
+    }
 }
 
 template <int R, bool TAGGED>
@@ -1195,8 +1190,10 @@ static cudaError_t launch_trace_tt(KernelArgs a, cudaStream_t s, int sm_count, i
             fprintf(stderr, "[fadegpu] round %d: %u requests (n_aln %d)\n", r, qc[r & 1], n);
         }
         if (r == 0 && a.k.shortcut) {
-            if (a.k.f16_ok) trace_replay_kernel<R, 2, true><<<std::max(g1, 1), 128, 0, s>>>(a);
-            else trace_replay_kernel<R, 2, false><<<std::max(g1, 1), 128, 0, s>>>(a);
+            const int step = score_step_for(a.k);
+            if (step == 2) trace_replay_kernel<R, 2, 2><<<std::max(g1, 1), 128, 0, s>>>(a);
+            else if (step == 1) trace_replay_kernel<R, 2, 1><<<std::max(g1, 1), 128, 0, s>>>(a);
+            else trace_replay_kernel<R, 2, 0><<<std::max(g1, 1), 128, 0, s>>>(a);
         }
         else trace_replay_kernel<R, TAGGED ? 0 : 1><<<std::max(g1, 1), 128, 0, s>>>(a);
         if (a.ops_spill) trace_advance_kernel<R, true><<<std::max(g2, 1), 128, 0, s>>>(a);

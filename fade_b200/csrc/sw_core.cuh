@@ -48,6 +48,9 @@ struct SwConsts {
     int32_t shortcut;           // traceback may use the ungapped-diagonal proof instead of a replay
     uint32_t flut0, flut1;      // byte LUT of the fp16 score words of fill_step_f16
     int32_t f16_ok;             // fill_step_f16 is exact for this scoring (checked in make_consts)
+    uint32_t plut0, plut1;      // byte LUT of the row-pair score words of fill_step_f16x2
+    uint32_t pair_c;            // IMAD addend that forms the second row's word of a pair (see fill_step_f16x2)
+    int32_t f16_pair_ok;        // fill_step_f16x2 is exact for this scoring (checked in make_consts)
 };
 
 // ---- packed helpers -------------------------------------------------------------------------
@@ -137,13 +140,32 @@ constexpr uint32_t F16_UNIT = 0x00010001u;
 FD uint32_t q_self(int ca, int cb) { return (uint32_t)(ca * 0x11 | 0x88) | ((uint32_t)(cb * 0x11 | 0x88) << 8); }
 FD uint32_t score_word_f16(uint32_t qs, uint32_t ts, const SwConsts &k) { return prmt_sx(k.flut0, k.flut1, qs ^ ts); }
 
-// fp16 word (b:00 for b < 0x80, b:FF otherwise -- what score_word_f16 produces from LUT byte b) in units of 2^-25
-FD int64_t f16_byte_word_x2(uint32_t b)
+// Query word of a row pair for fill_step_f16x2: against the same t_sel target words, sel = q_pair ^ t_sel has nibbles
+// (xa1, xa0, xb1, xb0) (x = q ^ t of lane a / b in the pair's first row 0 and second row 1), so one PRMT yields
+// [sa1, sa0, sb1, sb0]: the first row's fp16 word in both lanes, with the second row's bytes as its low bytes.
+FD uint32_t q_pair(int ca0, int cb0, int ca1, int cb1)
 {
-    const uint32_t w = b < 0x80 ? (b << 8) : ((b << 8) | 0xffu);
+    return (uint32_t)(ca1 | (ca0 | 8) << 4) | ((uint32_t)(cb1 | (cb0 | 8) << 4) << 8);
+}
+
+// fp16 word w (16 bits) in units of 2^-25
+FD int64_t f16_word_x2(uint32_t w)
+{
     const int ex = (int)((w >> 10) & 31), fr = (int)(w & 1023);
     const int64_t mag = ex ? (int64_t)(fr | 1024) << ex : (int64_t)fr * 2;
     return (w & 0x8000u) ? -mag : mag;
+}
+
+// fp16 word (b:00 for b < 0x80, b:FF otherwise -- what score_word_f16 produces from LUT byte b) in units of 2^-25
+FD int64_t f16_byte_word_x2(uint32_t b) { return f16_word_x2(b < 0x80 ? (b << 8) : ((b << 8) | 0xffu)); }
+
+// How far inside half a unit of the score v the finite fp16 word hb:lb lies, in units of 2^-25 (> 0: it rounds to v
+// when added to an integer; make_consts still checks the choice with f16_step_exact)
+FD int64_t f16_pair_margin(uint32_t hb, uint32_t lb, int v)
+{
+    if ((hb & 0x7c) == 0x7c) return -1;   // infinity / NaN
+    const int64_t d = f16_word_x2((hb << 8) | lb) - ((int64_t)v << 25);
+    return ((int64_t)1 << 24) - (d < 0 ? -d : d);
 }
 
 // LUT byte for score v: the one whose word is nearest to v (+2 -> 0x40 = 2.0, -3 -> 0xC1 = -2.998).  Adding a
@@ -161,21 +183,26 @@ FD uint32_t f16_score_byte(int v)
     return best;
 }
 
-// Is fill_step_f16 exact for this scoring?  On the packed kernels (at most FG * 38 = 304 query rows) H stays
-// within [0, max(match, mismatch) * 304].  For every H in that range the fp16 diagonal add must give H + s,
-// or a word that is negative as an int16 where H + s < 0 (the .RELU max clamps it).
-FD bool f16_step_exact(const SwConsts &k)
+// Is fill_step_f16 (pair == false) or fill_step_f16x2 (pair == true) exact for this scoring?  On the packed kernels
+// (at most FG * 38 = 304 query rows) H stays within [0, max(match, mismatch) * 304].  For every H in that range and
+// every score word the step can form, the fp16 diagonal add must give H + s where H + s > 0, and a word that is not
+// positive as an int16 where H + s <= 0 (the .RELU max clamps it to 0).  fill_step_f16's words are a flut byte with
+// its sign replicated below it; fill_step_f16x2's are a plut byte with any of the low bytes {fm, fx, pair_c} below it.
+FD bool f16_step_exact(const SwConsts &k, bool pair = false)
 {
     const int top = (k.match > k.mismatch ? k.match : k.mismatch) * FG * 38;
     if (top > 2047) return false;
     const int sc[2] = { k.match, k.mismatch };
     const uint32_t sel[2] = { q_self(0, 0) ^ t_sel(0, 0), q_self(0, 0) ^ t_sel(1, 1) };   // codes equal / different
-    for (int n = 0; n <= top; ++n) {
-        for (int i = 0; i < 2; ++i) {
-            const int want = n + sc[i];
-            const uint32_t s = prmt_sx(k.flut0, k.flut1, sel[i]);
-            const uint32_t d = fma_f16x2(s, F16_UNIT, (uint32_t)n * 0x10001u);
-            if (want >= 0 ? d != (uint32_t)want * 0x10001u : (lane_lo(d) > 0 || lane_hi(d) > 0)) return false;
+    const uint32_t low[3] = { k.plut0 & 0xffu, (k.plut0 >> 8) & 0xffu, k.pair_c & 0xffu };
+    for (int i = 0; i < 2; ++i) {
+        for (int l = 0; l < (pair ? 3 : 1); ++l) {
+            const uint32_t s = pair ? ((low[i] << 8) | low[l]) * 0x10001u : prmt_sx(k.flut0, k.flut1, sel[i]);
+            for (int n = 0; n <= top; ++n) {
+                const int want = n + sc[i];
+                const uint32_t d = fma_f16x2(s, F16_UNIT, (uint32_t)n * 0x10001u);
+                if (want > 0 ? d != (uint32_t)want * 0x10001u : (lane_lo(d) > 0 || lane_hi(d) > 0)) return false;
+            }
         }
     }
     return true;
@@ -206,6 +233,31 @@ FD SwConsts make_consts(int open, int extend, int match, int mismatch)
     k.flut0 = fm | (fx << 8) | (fx << 16) | (fx << 24);
     k.flut1 = fx | (fx << 8) | (fx << 16) | (fx << 24);
     k.f16_ok = f16_step_exact(k) ? 1 : 0;
+    // fill_step_f16x2: the high bytes pm / px and the addend c with the largest smallest margin over the words hb:lb,
+    // hb in {pm, px}, lb in {pm, px, c} (default scoring: 0x3F = 1.75 + lb / 1024, 0xC1 = -2.5 - lb / 512, c = 0x3F;
+    // 0xC1 with c = 0 would form -2.5, a tie).  The choice is then checked exactly.
+    uint32_t pm = 0, px = 0, pc = 0;
+    int64_t best = 0;
+    for (uint32_t bm = 0; bm < 256; ++bm) {
+        const int64_t m0 = f16_pair_margin(bm, bm, match);
+        if (m0 <= best) continue;
+        for (uint32_t bx = 0; bx < 256; ++bx) {
+            int64_t m1 = m0;
+            const int64_t mm[3] = { f16_pair_margin(bm, bx, match), f16_pair_margin(bx, bm, mismatch),
+                                    f16_pair_margin(bx, bx, mismatch) };
+            for (int i = 0; i < 3; ++i) m1 = mm[i] < m1 ? mm[i] : m1;
+            if (m1 <= best) continue;
+            for (uint32_t c = 0; c < 256; ++c) {
+                const int64_t a = f16_pair_margin(bm, c, match), b = f16_pair_margin(bx, c, mismatch);
+                const int64_t m2 = a < b ? (a < m1 ? a : m1) : (b < m1 ? b : m1);
+                if (m2 > best) { best = m2; pm = bm; px = bx; pc = c; }
+            }
+        }
+    }
+    k.plut0 = pm | (px << 8) | (px << 16) | (px << 24);
+    k.plut1 = px | (px << 8) | (px << 16) | (px << 24);
+    k.pair_c = pc;
+    k.f16_pair_ok = (best > 0 && f16_step_exact(k, true)) ? 1 : 0;
     return k;
 }
 
@@ -351,6 +403,59 @@ FD void fill_step_f16(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[R
         M = FADE_VMAX(M, h);
     }
     f_out = f;
+}
+
+// fill_step_f16 with one substitution lookup for every two rows, for scorings with k.f16_pair_ok (query words from
+// q_pair, ceil(R/2) of them).  One LOP3 + PRMT gives w = [sa1, sa0, sb1, sb0], which is the first row's score word in
+// both lanes (its low bytes sa1 / sb1 are don't-cares); one IMAD gives w * 256 + c = [c, sa1, sa0, sb1], the second
+// row's word (low bytes c and sa0).  make_consts picks the LUT bytes and c so that every such low byte leaves the
+// word within half a unit of its score.  The IMAD runs on the FMA pipe beside the DPX maxima (c is not a compile-time
+// constant, so the multiply-add stays an IMAD rather than a shift on the ALU pipe).  An odd R pairs its last row with
+// a padding code.  H, E and F are bit-identical to fill_step's (DESIGN.md 4.1).
+template <int R>
+FD void fill_step_f16x2(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qp)[(R + 1) / 2], uint32_t &M,
+                        uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out, const SwConsts &k)
+{
+    uint32_t f = f_in, w = 0;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        uint32_t s;
+        if ((r & 1) == 0) s = w = prmt_sx(k.plut0, k.plut1, qp[r >> 1] ^ ts);
+        else s = w * 256u + k.pair_c;
+        const uint32_t d = fma_f16x2(s, F16_UNIT, hdiag);
+        const uint32_t h = FADE_VMAX3_RELU(d, E[r], f);
+        hdiag = H[r];
+        H[r] = h;
+        const uint32_t ho = FADE_VADD(h, k.neg_o);
+        E[r] = FADE_VIADDMAX(E[r], k.neg_e, ho);
+        f = FADE_VIADDMAX(f, k.neg_e, ho);
+        M = FADE_VMAX(M, h);
+    }
+    f_out = f;
+}
+
+// The score-only steps: STEP 0 fill_step, 1 fill_step_f16, 2 fill_step_f16x2 (make_consts decides which is exact:
+// score_step_for).  Their query words: one per row (q_sel / q_self) or one per row pair (q_pair).
+FD int score_step_for(const SwConsts &k) { return k.f16_pair_ok ? 2 : (k.f16_ok ? 1 : 0); }
+template <int R, int STEP> FD constexpr int query_words() { return STEP == 2 ? (R + 1) / 2 : R; }
+
+// Set the query word(s) of row r (rows in order: the first row of a pair also writes the padding code of a second row)
+template <int STEP, int N>
+FD void set_query(uint32_t (&qs)[N], int r, int ca, int cb)
+{
+    if (STEP == 0) qs[r] = q_sel(ca, cb);
+    else if (STEP == 1) qs[r] = q_self(ca, cb);
+    else if ((r & 1) == 0) qs[r >> 1] = q_pair(ca, cb, C_QPAD, C_QPAD);
+    else qs[r >> 1] = (qs[r >> 1] & 0xf0f0u) | (uint32_t)ca | ((uint32_t)cb << 8);
+}
+
+template <int R, int STEP>
+FD void score_step(uint32_t (&H)[R], uint32_t (&E)[R], const uint32_t (&qs)[query_words<R, STEP>()], uint32_t &M,
+                   uint32_t ts, uint32_t hdiag, uint32_t f_in, uint32_t &f_out, const SwConsts &k)
+{
+    if constexpr (STEP == 2) fill_step_f16x2<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
+    else if constexpr (STEP == 1) fill_step_f16<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
+    else fill_step<R>(H, E, qs, M, ts, hdiag, f_in, f_out, k);
 }
 
 // Trace nibble of cell (i,j) (one per int16 lane):

@@ -73,6 +73,10 @@ __global__ void __launch_bounds__(256) k(uint32_t *out, int iters, uint32_t c1, 
                 if (KIND == 15) x[i] = add_f16x2(x[i], c1);                                    // HADD2
                 if (KIND == 16) { x[i] = __viaddmax_s16x2(x[i], c1, c2); y[i] = fade::fma_f16x2(y[i], c1, c2); }
                 if (KIND == 17) { x[i] = __vimax3_s16x2_relu(x[i], c1, c2); y[i] = fade::fma_f16x2(y[i], c1, c2); }
+                // co-issue with independent chains (the r02 LOP3 row, KIND 10, is a dependent pair and latency-bound)
+                if (KIND == 18) { x[i] = __viaddmax_s16x2(x[i], c1, c2); y[i] = __byte_perm(y[i], x[i], c2); }
+                if (KIND == 19) { x[i] = __viaddmax_s16x2(x[i], c1, c2); y[i] = (y[i] ^ x[i]) & c1; }
+                if (KIND == 20) { x[i] = fade::fma_f16x2(x[i], c1, c2); y[i] = y[i] * one + c1; }
             }
         }
     }
@@ -107,29 +111,36 @@ int run(const char *name, int per_iter, int sms, double mhz)
 }
 
 // The score-only step of sw_fill_kernel<19> on register data: 19 rows x 2 lanes per thread and step, the target
-// word from 8 registers, the diagonal H from the thread's own bottom row (no shuffle, no memory traffic).
-// V = 0: fill_step, 1: fill_step_f16 (diagonal add on the FMA pipe), 2: fill_step_f16 with H - open there too.
+// word from 8 registers, the diagonal H from the thread's own bottom row (no shuffle, no memory traffic).  The target
+// codes change with the iteration (rot), so the substitution lookups cannot be hoisted out of the loop.
+// V = 0: fill_step, 1: fill_step_f16 (diagonal add on the FMA pipe), 2: fill_step_f16 with H - open there too,
+// 3: fill_step_f16x2 (one lookup per row pair).
 template <int V>
 __global__ void __launch_bounds__(128, 5) step_k(uint32_t *out, int iters, fade::SwConsts k)
 {
     constexpr int R = 19;
-    uint32_t H[R], E[R], qs[R], ts[8];
+    constexpr int STEP = V == 3 ? 2 : (V ? 1 : 0);
+    uint32_t H[R], E[R], qs[fade::query_words<R, STEP>()], ts[8];
 #pragma unroll
     for (int r = 0; r < R; ++r) {
-        const int ca = (threadIdx.x + 5 * r) & 3, cb = (threadIdx.x * 3 + r) & 3;
-        qs[r] = V ? fade::q_self(ca, cb) : fade::q_sel(ca, cb);
+        // codes the compiler cannot prove equal, so it cannot share lookups between rows
+        const int ca = (int)((threadIdx.x * 2654435761u) >> (r + 3)) & 3, cb = (int)((threadIdx.x * 2246822519u) >> (r + 5)) & 3;
+        fade::set_query<STEP>(qs, r, ca, cb);
         H[r] = 0u; E[r] = k.neg_o;
     }
 #pragma unroll
-    for (int i = 0; i < 8; ++i) ts[i] = fade::t_sel((threadIdx.x * 3 + i) & 3, (7 * i + threadIdx.x) & 3);
+    for (int i = 0; i < 8; ++i)
+        ts[i] = fade::t_sel((int)((threadIdx.x * 3266489917u) >> (i + 7)) & 3, (int)((threadIdx.x * 668265263u) >> (i + 9)) & 3);
     uint32_t M = 0u, f = k.neg_o, hu_prev = 0u;
     for (int it = 0; it < iters; ++it) {
+        const uint32_t rot = (uint32_t)(it & 3) * 0x1111u;   // target codes c ^ (it & 3), still in 0..3
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
             const uint32_t hu = H[R - 1];
-            if (V == 0) fade::fill_step<R>(H, E, qs, M, ts[u], hu_prev, f, f, k);
-            if (V == 1) fade::fill_step_f16<R>(H, E, qs, M, ts[u], hu_prev, f, f, k);
-            if (V == 2) fill_step_f16_ho<R>(H, E, qs, M, ts[u], hu_prev, f, f, k, 0x800a800au);   // fp16 -10 (open)
+            if constexpr (V == 0) fade::fill_step<R>(H, E, qs, M, ts[u] ^ rot, hu_prev, f, f, k);
+            else if constexpr (V == 1) fade::fill_step_f16<R>(H, E, qs, M, ts[u] ^ rot, hu_prev, f, f, k);
+            else if constexpr (V == 2) fill_step_f16_ho<R>(H, E, qs, M, ts[u] ^ rot, hu_prev, f, f, k, 0x800a800au);   // fp16 -10 (open)
+            else fade::fill_step_f16x2<R>(H, E, qs, M, ts[u] ^ rot, hu_prev, f, f, k);
             hu_prev = hu;
         }
     }
@@ -190,8 +201,12 @@ int main()
     run<15>("HADD2", 1, s, mhz);
     run<16>("VIADDMNMX + HFMA2 (2 per iter)", 2, s, mhz);
     run<17>("VIMNMX3.RELU + HFMA2 (2 per iter)", 2, s, mhz);
+    run<18>("VIADDMNMX + PRMT (2 per iter)", 2, s, mhz);
+    run<19>("VIADDMNMX + LOP3 indep. (2 per iter)", 2, s, mhz);
+    run<20>("HFMA2 + IMAD (2 per iter)", 2, s, mhz);
     const float base = run_step<0>("fill_step<19> (integer)", s, mhz, 0.0);
     run_step<1>("fill_step_f16<19> diagonal add on FMA (A)", s, mhz, base);
     run_step<2>("fill_step_f16<19> + H-open on FMA (A+B)", s, mhz, base);
+    run_step<3>("fill_step_f16x2<19> one lookup per row pair", s, mhz, base);
     return 0;
 }
