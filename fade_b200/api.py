@@ -8,7 +8,8 @@ from dataclasses import dataclass, field
 
 import numpy as np
 
-from ._lib import BatchView, FadeGpuError, HostRecord, Inputs, PairResult, PairsIn, Params, Result, ResultsView, Stats, lib
+from ._lib import (BatchView, FadeGpuError, HostRecord, Inputs, PairResult, PairsIn, Params, RegionsIn, Result,
+                   ResultsView, Stats, lib)
 
 MAX_OPS = 10
 R_ALIGNED, R_ART_LEFT, R_ART_RIGHT, R_OPS_TRUNC, R_GENERIC, R_OVERSIZE, R_SCORE_ONLY = 1, 2, 4, 8, 16, 32, 64
@@ -61,6 +62,27 @@ def pack_pairs(queries, targets, query_offsets=None, target_offsets=None):
     return q, qo, t, to
 
 
+def _region_array(x, dtype, n, name):
+    """one per-region array of Context.align_regions in its ABI dtype: n entries whose values survive the conversion"""
+    a = np.asarray(x)
+    if a.ndim != 1 or len(a) != n:
+        raise ValueError(f"{name} must be a 1-d array of {n} entries (one per query), not of shape {a.shape}")
+    out = np.ascontiguousarray(a, dtype=dtype)
+    if n and not np.array_equal(out, a):
+        raise ValueError(f"{name} holds values outside {np.dtype(dtype).name}")
+    return out
+
+
+def pack_regions(queries, tids, starts, ends, strands=None, query_offsets=None):
+    """(query buffer, query offsets, tid int32, start int64, end int64, strand uint8) as fadegpu_align_regions reads
+    them; strands None means all 0 (the queries as given)"""
+    q, qo = _pack_side(queries, query_offsets)
+    n = len(qo) - 1
+    strands = np.zeros(n, np.uint8) if strands is None else strands
+    return (q, qo, _region_array(tids, np.int32, n, "tids"), _region_array(starts, np.int64, n, "starts"),
+            _region_array(ends, np.int64, n, "ends"), _region_array(strands, np.uint8, n, "strands"))
+
+
 def default_max_ops(query_offsets) -> int:
     """3 * the longest query: no CIGAR of a local alignment can be longer (see fadegpu_align_pairs in fadegpu.h)"""
     qo = np.asarray(query_offsets, dtype=np.int64)
@@ -69,7 +91,8 @@ def default_max_ops(query_offsets) -> int:
 
 @dataclass
 class PairResults:
-    """Context.align_pairs: records[n] (PAIR_RESULT_DTYPE) and ops[n, max_ops] in pair order, and the call's stats."""
+    """Context.align_pairs / align_regions: records[n] (PAIR_RESULT_DTYPE) and ops[n, max_ops] in pair / region order,
+    and the call's stats."""
     records: np.ndarray
     ops: np.ndarray
     stats: Stats
@@ -182,6 +205,27 @@ class Context:
         pin = PairsIn(q.ctypes.data, qo.ctypes.data, t.ctypes.data, to.ctypes.data)
         self._check(lib().fadegpu_align_pairs(self._h, n, C.byref(pin), max_ops, rec.ctypes.data,
                                               ops.ctypes.data if max_ops > 0 else None, C.byref(st)))
+        return PairResults(rec, ops, st)
+
+    def align_regions(self, queries, tids, starts, ends, strands=None, max_ops: int | None = None, *,
+                      query_offsets=None) -> PairResults:
+        """fadegpu_align_regions: Smith-Waterman with traceback of query k against [starts[k], ends[k]) of the loaded
+        contig tids[k], with the ctx's scoring.
+
+        queries: as in align_pairs (nt16 letters).  strands[k] = 1 aligns the reverse complement of query k (its
+        beg_query / end_query then index the reverse complement); None means all 0.  beg_ref / end_ref are relative to
+        starts[k].  max_ops defaults to 3 * the longest query, which never truncates a CIGAR."""
+        q, qo, tid, start, end, strand = pack_regions(queries, tids, starts, ends, strands, query_offsets)
+        n = len(qo) - 1
+        if max_ops is None:
+            max_ops = default_max_ops(qo)
+        rec = np.zeros(n, dtype=PAIR_RESULT_DTYPE)
+        ops = np.zeros((n, max_ops), dtype=np.uint32)
+        st = Stats()
+        rin = RegionsIn(q.ctypes.data, qo.ctypes.data, tid.ctypes.data, start.ctypes.data, end.ctypes.data,
+                        strand.ctypes.data)
+        self._check(lib().fadegpu_align_regions(self._h, n, C.byref(rin), max_ops, rec.ctypes.data,
+                                                ops.ctypes.data if max_ops > 0 else None, C.byref(st)))
         return PairResults(rec, ops, st)
 
     def alloc_batch(self, max_reads: int, max_seq_bytes: int) -> "Batch":

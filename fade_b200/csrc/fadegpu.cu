@@ -18,6 +18,7 @@
 #include <chrono>
 #include <condition_variable>
 #include <deque>
+#include <functional>
 #include <exception>
 #include <mutex>
 #include <thread>
@@ -91,10 +92,10 @@ struct fadegpu_ctx {
     std::deque<std::pair<fadegpu_batch *, int64_t>> jobs;
     bool worker_stop = false, worker_busy = false;
     std::mutex submit_mu;                 // one submit body at a time (they size shared scratch and order the streams)
-    std::vector<fadegpu_batch *> batches; // the caller's batches (guarded by q_mu): fadegpu_align_pairs refuses to run while
-                                          // one of them is in flight
-    // fadegpu_align_pairs: an internal batch (descriptors, binning arrays, result records) that grows with use, the
-    // targets packed as a reference of their own, and the staging of the raw ASCII
+    std::vector<fadegpu_batch *> batches; // the caller's batches (guarded by q_mu): fadegpu_align_pairs / _regions refuse to
+                                          // run while one of them is in flight
+    // fadegpu_align_pairs / fadegpu_align_regions: an internal batch (descriptors, binning arrays, result records) that
+    // grows with use, the staging of the raw inputs, and the targets of a pair call packed as a reference of their own
     struct PairBufs {
         fadegpu_batch *b = nullptr;
         char *h_stage = nullptr, *d_raw = nullptr;          // pinned staging / device copy of offsets + ASCII
@@ -1669,44 +1670,46 @@ static void parallel_copy(char *dst, const char *src, size_t bytes, int nthr)
     }
 }
 
-// Pairs: the raw ASCII goes to the device through pinned staging on stream2, where pair_prep_kernel writes the per-pair
-// binning inputs and the queries (nt16, reverse-complemented) and pair_pack_targets_kernel the target planes; the
-// binning, the launch plan and run_plan are those of a device-binned submit, on the ctx's internal pair batch, with
-// the targets as the reference, every alignment traced back and the full CIGARs spilled; the records come back in
-// pair order on stream3.
-int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
-                        fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+static size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// FADEGPU_E_STATE while a batch of the ctx is submitted and not yet waited for
+static int refuse_in_flight(fadegpu_ctx *c, const char *fn)
 {
-    if (!c) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_align_pairs: null ctx");
-    if (n_pairs < 0 || n_pairs > ((int64_t)1 << 30) || max_ops < 0)
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: n_pairs or max_ops out of range");
-    if (n_pairs > 0 && (!in || !in->query_off || !in->target_off || !out || (max_ops > 0 && !ops_out)))
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null argument");
-    {
-        std::lock_guard<std::mutex> lk(c->q_mu);
-        for (const fadegpu_batch *b : c->batches)
-            if (b->in_flight)
-                return fail(c, FADEGPU_E_STATE, "fadegpu_align_pairs: a batch of this ctx is in flight (call fadegpu_wait)");
-    }
-    const auto t_begin = std::chrono::steady_clock::now();
-    const int64_t n = n_pairs;
-    int64_t qbytes = 0, tbytes = 0, n_over = 0;
-    if (n > 0) {
-        const int64_t *qo = in->query_off, *to = in->target_off;
-        if (qo[0] < 0 || to[0] < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: negative offset");
-        for (int64_t k = 0; k < n; ++k) {
-            const int64_t ql = qo[k + 1] - qo[k], tl = to[k + 1] - to[k];
-            if (ql < 0 || tl < 0)
-                return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: offsets decrease at pair " + std::to_string(k));
-            if (ql > 0 && tl > 0 && (tl > 0x7fffffff || ql * tl > PAIR_MAX_CELLS)) ++n_over;
-        }
-        qbytes = qo[n] - qo[0]; tbytes = to[n] - to[0];
-        if ((qbytes > 0 && !in->query) || (tbytes > 0 && !in->target))
-            return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null sequence array");
-    }
+    std::lock_guard<std::mutex> lk(c->q_mu);
+    for (const fadegpu_batch *b : c->batches)
+        if (b->in_flight)
+            return fail(c, FADEGPU_E_STATE, std::string(fn) + ": a batch of this ctx is in flight (call fadegpu_wait)");
+    return 0;
+}
+
+// What a pair call and a region call do differently around their shared body (align_staged).  Both stage the query
+// offsets at byte 0 of the upload; the rest of the layout is the caller's.
+struct StagedCall {
+    const char *fn, *item;        // the call's and an item's name, for messages
+    int64_t n, qbytes, n_over;    // items, query letters, oversize items (counted by the host validation)
+    int32_t max_ops;
+    size_t raw;                   // bytes staged and uploaded
+    size_t o_tbeg, o_tend;        // byte offsets of the int64 window bounds of every item in the upload (results init)
+    std::function<void(char *h_stage)> stage;
+    // on stream2, after the upload: the binning inputs and the queries of b (failures reported to *d_bad), and ba's
+    // contig table; counts its launches
+    std::function<int(fadegpu_batch *b, const char *d_raw, BinArgs &ba, int *launches)> prep;
+    // after the binning histogram is home: the reference the SW kernels read; counts its launches
+    std::function<int(fadegpu_batch *b, RefDev *ref, int *launches)> reference;
+};
+
+// The raw inputs go to the device through pinned staging on stream2, where the caller's prep kernels write the
+// per-item binning inputs and the queries; the binning, the launch plan and run_plan are those of a device-binned
+// submit, on the ctx's internal pair batch, with every alignment traced back and the full CIGARs spilled; the records
+// come back in item order on stream3.
+static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_result *out, uint32_t *ops_out,
+                        fadegpu_stats *stats_out, std::chrono::steady_clock::time_point t_begin)
+{
+    const int64_t n = sc.n, qbytes = sc.qbytes;
+    const int32_t max_ops = sc.max_ops;
     fadegpu_stats st{};
     st.n_reads = n;
-    st.n_oversize = n_over;
+    st.n_oversize = sc.n_over;
     if (n == 0) {
         if (stats_out) *stats_out = st;
         return FADEGPU_OK;
@@ -1725,32 +1728,18 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
         if (rc) return rc;
     }
     fadegpu_batch *b = pb.b;
-    // ---- staging: [query_off][target_off] rebased to 0, then the query and the target letters ----
-    auto a16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
-    const size_t o_toff = a16((size_t)(n + 1) * 8), o_q = o_toff + a16((size_t)(n + 1) * 8), o_t = o_q + a16((size_t)qbytes);
-    const size_t raw = o_t + a16((size_t)tbytes);
+    const size_t raw = sc.raw;
     if (pb.stage_bytes < raw) {
         free_host(pb.h_stage);
         pb.stage_bytes = 0;
         CU(c, cudaHostAlloc((void **)&pb.h_stage, raw, cudaHostAllocDefault));
         pb.stage_bytes = raw;
     }
-    {
-        int64_t *hq = reinterpret_cast<int64_t *>(pb.h_stage), *ht = reinterpret_cast<int64_t *>(pb.h_stage + o_toff);
-        const int64_t q0 = in->query_off[0], t0 = in->target_off[0];
-        for (int64_t k = 0; k <= n; ++k) { hq[k] = in->query_off[k] - q0; ht[k] = in->target_off[k] - t0; }
-        if (qbytes) parallel_copy(pb.h_stage + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
-        if (tbytes) parallel_copy(pb.h_stage + o_t, in->target + t0, (size_t)tbytes, c->host_threads);
-    }
-    const int64_t n_words = n + (tbytes >> 5) + 2;   // target k starts at 32 * (k + toff[k] / 32)
-    const int64_t n_chunks = (n_words + PAIR_CHUNK_WORDS - 1) / PAIR_CHUNK_WORDS;
+    sc.stage(pb.h_stage);
     {
         int rc = 0;
         auto grow = [&](auto **p, size_t *have, size_t bytes) { if (!rc) rc = ensure_dev(c, (void **)p, have, std::max<size_t>(bytes, 16)); };
         grow(&pb.d_raw, &pb.raw_bytes, raw);
-        grow(&pb.d_two, &pb.two_bytes, (size_t)n_words * 8); grow(&pb.d_n, &pb.n_bytes, (size_t)n_words * 4);
-        grow(&pb.d_x, &pb.x_bytes, (size_t)n_words * 4); grow(&pb.d_chunk_x, &pb.chunk_bytes, (size_t)n_chunks * 4);
-        grow(&pb.d_clen, &pb.clen_bytes, (size_t)n * 8); grow(&pb.d_coff, &pb.coff_bytes, (size_t)n * 8);
         grow(&pb.d_res, &pb.res_bytes, (size_t)n * sizeof(fadegpu_pair_result));
         if (max_ops > 0) {
             grow(&pb.d_spill, &pb.spill_bytes, (size_t)n * (size_t)max_ops * 4);
@@ -1772,31 +1761,21 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
     CU(c, cudaMemcpyAsync(pb.d_raw, pb.h_stage, raw, cudaMemcpyHostToDevice, s2));
     int64_t h2d = (int64_t)raw;
     CU(c, cudaEventRecord(b->ev[4], s2));
-    PairArgs pa{};
-    pa.n = n;
-    pa.qoff = reinterpret_cast<const int64_t *>(pb.d_raw); pa.toff = reinterpret_cast<const int64_t *>(pb.d_raw + o_toff);
-    pa.query = pb.d_raw + o_q; pa.target = pb.d_raw + o_t;
-    pa.seq_off = b->d_in_seq_off; pa.pos = b->d_in_pos; pa.l_qseq = b->d_in_lq; pa.tid = b->d_in_tid;
-    pa.aligned_len = b->d_in_alen; pa.clip_left = b->d_in_cl; pa.clip_right = b->d_in_cr;
-    pa.clen = pb.d_clen; pa.coff = pb.d_coff; pa.seq4 = b->d_in_seq4; pa.bad = pb.d_bad;
-    pa.two = pb.d_two; pa.nmask = pb.d_n; pa.xmask = pb.d_x; pa.n_words = n_words;
-    pa.chunk_x = pb.d_chunk_x; pa.n_x = b->d_stats + 12;
     CU(c, cudaMemsetAsync(b->d_hist, 0, (size_t)BIN_KEYS * 4, s2));
     CU(c, cudaMemsetAsync(b->d_cursor, 0, (size_t)BIN_KEYS * 4, s2));
     CU(c, cudaMemsetAsync(b->d_stats, 0, 128, s2));
-    CU(c, cudaMemsetAsync(pb.d_bad, 0x7f, sizeof(int32_t), s2));   // > any pair index
-    CU(c, launch_pair_prep(pa, c->sm_count, s2));
-    CU(c, launch_pair_pack_targets(pa, s2));
+    CU(c, cudaMemsetAsync(pb.d_bad, 0x7f, sizeof(int32_t), s2));   // > any item index
     BinArgs ba{};
     ba.seq4 = b->d_in_seq4; ba.seq_off = b->d_in_seq_off; ba.l_qseq = b->d_in_lq; ba.tid = b->d_in_tid; ba.pos = b->d_in_pos;
     ba.aligned_len = b->d_in_alen; ba.clip_left = b->d_in_cl; ba.clip_right = b->d_in_cr;
     ba.read = nullptr; ba.seq_cursor = nullptr; ba.src_off = b->d_src_off; ba.gate = nullptr; ba.host_meta = nullptr;
     ba.over_list = b->d_over;
-    // contigs = targets, window 0 and floor 0: the window of pair k is its whole target, every non-empty pair is aligned
-    ba.n = n; ba.seq_total = qbytes; ba.clen = pb.d_clen; ba.coff = pb.d_coff; ba.n_contigs = (int32_t)n;
-    ba.window = 0; ba.min_length = 0; ba.flags = c->p.flags;
+    // window 0 and floor 0: the window of item k is exactly its target / interval, every non-empty item is aligned
+    ba.n = n; ba.seq_total = qbytes; ba.window = 0; ba.min_length = 0; ba.flags = c->p.flags;
     ba.key = b->d_key; ba.tlen = b->d_tlen; ba.start = b->d_start; ba.hist = b->d_hist; ba.stats = b->d_stats;
     ba.keybase = b->d_keybase; ba.cursor = b->d_cursor; ba.aln = b->d_aln; ba.aln_start = b->d_aln_start;
+    int n_prep = 0;
+    { int rc = sc.prep(b, pb.d_raw, ba, &n_prep); if (rc) return rc; }
     CU(c, launch_bin_classify(ba, c->sm_count, s2));
     CU(c, cudaMemcpyAsync(b->h_hist, b->d_hist, (size_t)BIN_KEYS * 4, cudaMemcpyDeviceToHost, s2));
     CU(c, cudaMemcpyAsync(b->h_stats, b->d_stats, 128, cudaMemcpyDeviceToHost, s2));
@@ -1805,17 +1784,12 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
     CU(c, cudaEventSynchronize(b->ev_prep));
     const int32_t bad = b->h_over[0];
     if (bad >= 0 && bad < n)
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: the query of pair " + std::to_string(bad) +
+        return fail(c, FADEGPU_E_ARG, std::string(sc.fn) + ": the query of " + sc.item + " " + std::to_string(bad) +
                                           " holds a letter outside the BAM nt16 alphabet =ACMGRSVTWYHKDBN");
-    if (b->h_stats[6] & 1ull) return fail(c, FADEGPU_E_CUDA, "fadegpu_align_pairs: internal error (query offsets)");
-    const int64_t n_aln = (int64_t)b->h_stats[1], n_x = (int64_t)b->h_stats[12];
-    {
-        int rc = ensure_dev(c, (void **)&pb.d_xpos, &pb.xpos_bytes, std::max<size_t>(16, (size_t)n_x * 8));
-        if (!rc) rc = ensure_dev(c, (void **)&pb.d_xchr, &pb.xchr_bytes, std::max<size_t>(16, (size_t)n_x));
-        if (rc) return rc;
-    }
-    pa.xpos = pb.d_xpos; pa.xchr = pb.d_xchr;
-    if (n_x > 0) CU(c, launch_pair_xlist(pa, s2));
+    if (b->h_stats[6] & 1ull) return fail(c, FADEGPU_E_CUDA, std::string(sc.fn) + ": internal error (query offsets)");
+    const int64_t n_aln = (int64_t)b->h_stats[1];
+    PlanTarget pt{};
+    { int rc = sc.reference(b, &pt.ref, &n_prep); if (rc) return rc; }
     { int rc = plan_from_histogram(c, b, n_aln); if (rc) return rc; }
     if (n_aln > 0) {
         CU(c, cudaMemcpyAsync(b->d_keybase, b->h_keybase, (size_t)BIN_KEYS * 4, cudaMemcpyHostToDevice, s2));
@@ -1825,23 +1799,21 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
         CU(c, launch_bin_scatter(ba, c->sm_count, s2));
     }
     CU(c, cudaEventRecord(b->ev_ready, s2));
-    // ---- SW kernels: the batch's plan against the packed targets ----
+    // ---- SW kernels: the batch's plan against the caller's reference ----
     CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
     CU(c, cudaEventRecord(b->ev[1], c->stream));
-    PlanTarget pt{};
-    pt.ref.planes.two = pb.d_two; pt.ref.planes.nmask = pb.d_n; pt.ref.planes.xmask = pb.d_x;
-    pt.ref.xpos = pb.d_xpos; pt.ref.xchr = pb.d_xchr; pt.ref.n_x = n_x;
-    pt.tags_only = 0;   // every pair is traced back, whatever the ctx's FADEGPU_F_TAGS_ONLY
+    pt.tags_only = 0;   // every item is traced back, whatever the ctx's FADEGPU_F_TAGS_ONLY
     pt.ops_spill = max_ops > 0 ? pb.d_spill : nullptr;
     pt.ops_cap = max_ops;
     int nl = 0;
     { int rc = run_plan(c, b, pt, nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
-    // ---- records in pair order, home on stream3 ----
+    // ---- records in item order, home on stream3 ----
     cudaStream_t s3 = c->stream3;
     { int rc = join_kernels(c, b, s3); if (rc) return rc; }
     CU(c, cudaEventRecord(b->ev[2], s3));
-    CU(c, launch_pair_results(pa, b->d_aln, b->d_out, (int)n_aln, pb.d_spill, max_ops, reinterpret_cast<PairResult *>(pb.d_res), pb.d_ops, b->d_stats + 7,
-                              c->sm_count, s3));
+    CU(c, launch_pair_results(n, reinterpret_cast<const int64_t *>(pb.d_raw), reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tbeg),
+                              reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tend), b->d_aln, b->d_out, (int)n_aln, pb.d_spill,
+                              max_ops, reinterpret_cast<PairResult *>(pb.d_res), pb.d_ops, b->d_stats + 7, c->sm_count, s3));
     CU(c, cudaMemcpyAsync(out, pb.d_res, (size_t)n * sizeof(fadegpu_pair_result), cudaMemcpyDeviceToHost, s3));
     if (max_ops > 0)
         CU(c, cudaMemcpyAsync(ops_out, pb.d_ops, (size_t)n * (size_t)max_ops * 4, cudaMemcpyDeviceToHost, s3));
@@ -1849,13 +1821,13 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
     CU(c, cudaEventRecord(b->ev[3], s3));
     CU(c, cudaEventSynchronize(b->ev[3]));
     if ((int64_t)b->h_stats[7] != n_aln)
-        return fail(c, FADEGPU_E_CUDA, "fadegpu_align_pairs: a kernel did not produce a result record (internal error)");
+        return fail(c, FADEGPU_E_CUDA, std::string(sc.fn) + ": a kernel did not produce a result record (internal error)");
     st.n_aligned = n_aln;
     st.n_generic = b->st.n_generic;
     st.cells = (int64_t)b->h_stats[0];
     st.h2d_bytes = h2d;
     st.d2h_bytes = n * (int64_t)(sizeof(fadegpu_pair_result) + 4 * (size_t)max_ops) + (int64_t)BIN_KEYS * 4 + 128 + 4 + 8;
-    st.kernel_launches = nl + 3 + (n_x > 0 ? 1 : 0) + (n_aln > 0 ? 2 : 1);
+    st.kernel_launches = nl + n_prep + 1 + (n_aln > 0 ? 2 : 1);
     st.scratch_bytes = b->st.scratch_bytes;
     float t;
     if (cudaEventElapsedTime(&t, b->ev[1], b->ev[2]) == cudaSuccess) st.kernel_ms = t;
@@ -1865,6 +1837,167 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
     b->st = st;
     if (stats_out) *stats_out = st;
     return FADEGPU_OK;
+}
+
+// Pairs: pair_prep_kernel writes the per-pair binning inputs and the queries (nt16, reverse-complemented),
+// pair_pack_targets_kernel and pair_xlist_kernel pack the targets as a reference of their own, whose contigs the
+// targets are.
+int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
+                        fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+{
+    if (!c) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_align_pairs: null ctx");
+    if (n_pairs < 0 || n_pairs > ((int64_t)1 << 30) || max_ops < 0)
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: n_pairs or max_ops out of range");
+    if (n_pairs > 0 && (!in || !in->query_off || !in->target_off || !out || (max_ops > 0 && !ops_out)))
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null argument");
+    { int rc = refuse_in_flight(c, "fadegpu_align_pairs"); if (rc) return rc; }
+    const auto t_begin = std::chrono::steady_clock::now();
+    const int64_t n = n_pairs;
+    int64_t qbytes = 0, tbytes = 0, n_over = 0;
+    if (n > 0) {
+        const int64_t *qo = in->query_off, *to = in->target_off;
+        if (qo[0] < 0 || to[0] < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: negative offset");
+        for (int64_t k = 0; k < n; ++k) {
+            const int64_t ql = qo[k + 1] - qo[k], tl = to[k + 1] - to[k];
+            if (ql < 0 || tl < 0)
+                return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: offsets decrease at pair " + std::to_string(k));
+            if (ql > 0 && tl > 0 && (tl > 0x7fffffff || ql * tl > PAIR_MAX_CELLS)) ++n_over;
+        }
+        qbytes = qo[n] - qo[0]; tbytes = to[n] - to[0];
+        if ((qbytes > 0 && !in->query) || (tbytes > 0 && !in->target))
+            return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null sequence array");
+    }
+    // ---- staging: [query_off][target_off] rebased to 0, then the query and the target letters ----
+    const size_t o_toff = align16((size_t)(n + 1) * 8), o_q = o_toff + align16((size_t)(n + 1) * 8);
+    const size_t o_t = o_q + align16((size_t)qbytes);
+    const int64_t n_words = n + (tbytes >> 5) + 2;   // target k starts at 32 * (k + toff[k] / 32)
+    const int64_t n_chunks = (n_words + PAIR_CHUNK_WORDS - 1) / PAIR_CHUNK_WORDS;
+    fadegpu_ctx::PairBufs &pb = c->pairs;
+    PairArgs pa{};
+    StagedCall sc;
+    sc.fn = "fadegpu_align_pairs"; sc.item = "pair";
+    sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops;
+    sc.raw = o_t + align16((size_t)tbytes);
+    sc.o_tbeg = o_toff; sc.o_tend = o_toff + 8;   // target k spans toff[k] .. toff[k + 1]
+    sc.stage = [&](char *h) {
+        int64_t *hq = reinterpret_cast<int64_t *>(h), *ht = reinterpret_cast<int64_t *>(h + o_toff);
+        const int64_t q0 = in->query_off[0], t0 = in->target_off[0];
+        for (int64_t k = 0; k <= n; ++k) { hq[k] = in->query_off[k] - q0; ht[k] = in->target_off[k] - t0; }
+        if (qbytes) parallel_copy(h + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
+        if (tbytes) parallel_copy(h + o_t, in->target + t0, (size_t)tbytes, c->host_threads);
+    };
+    sc.prep = [&](fadegpu_batch *b, const char *d, BinArgs &ba, int *launches) -> int {
+        int rc = 0;
+        auto grow = [&](auto **p, size_t *have, size_t bytes) { if (!rc) rc = ensure_dev(c, (void **)p, have, std::max<size_t>(bytes, 16)); };
+        grow(&pb.d_two, &pb.two_bytes, (size_t)n_words * 8); grow(&pb.d_n, &pb.n_bytes, (size_t)n_words * 4);
+        grow(&pb.d_x, &pb.x_bytes, (size_t)n_words * 4); grow(&pb.d_chunk_x, &pb.chunk_bytes, (size_t)n_chunks * 4);
+        grow(&pb.d_clen, &pb.clen_bytes, (size_t)n * 8); grow(&pb.d_coff, &pb.coff_bytes, (size_t)n * 8);
+        if (rc) return rc;
+        pa.n = n;
+        pa.qoff = reinterpret_cast<const int64_t *>(d); pa.toff = reinterpret_cast<const int64_t *>(d + o_toff);
+        pa.query = d + o_q; pa.target = d + o_t;
+        pa.seq_off = b->d_in_seq_off; pa.pos = b->d_in_pos; pa.l_qseq = b->d_in_lq; pa.tid = b->d_in_tid;
+        pa.aligned_len = b->d_in_alen; pa.clip_left = b->d_in_cl; pa.clip_right = b->d_in_cr;
+        pa.clen = pb.d_clen; pa.coff = pb.d_coff; pa.seq4 = b->d_in_seq4; pa.bad = pb.d_bad;
+        pa.two = pb.d_two; pa.nmask = pb.d_n; pa.xmask = pb.d_x; pa.n_words = n_words;
+        pa.chunk_x = pb.d_chunk_x; pa.n_x = b->d_stats + 12;
+        CU(c, launch_pair_prep(pa, c->sm_count, c->stream2));
+        CU(c, launch_pair_pack_targets(pa, c->stream2));
+        *launches += 2;
+        ba.clen = pb.d_clen; ba.coff = pb.d_coff; ba.n_contigs = (int32_t)n;   // contigs = targets
+        return 0;
+    };
+    sc.reference = [&](fadegpu_batch *b, RefDev *ref, int *launches) -> int {
+        const int64_t n_x = (int64_t)b->h_stats[12];
+        int rc = ensure_dev(c, (void **)&pb.d_xpos, &pb.xpos_bytes, std::max<size_t>(16, (size_t)n_x * 8));
+        if (!rc) rc = ensure_dev(c, (void **)&pb.d_xchr, &pb.xchr_bytes, std::max<size_t>(16, (size_t)n_x));
+        if (rc) return rc;
+        pa.xpos = pb.d_xpos; pa.xchr = pb.d_xchr;
+        if (n_x > 0) { CU(c, launch_pair_xlist(pa, c->stream2)); ++*launches; }
+        ref->planes.two = pb.d_two; ref->planes.nmask = pb.d_n; ref->planes.xmask = pb.d_x;
+        ref->xpos = pb.d_xpos; ref->xchr = pb.d_xchr; ref->n_x = n_x;
+        return 0;
+    };
+    return align_staged(c, sc, out, ops_out, stats_out, t_begin);
+}
+
+// Regions: only the queries and the intervals are staged; region_prep_kernel writes the per-region binning inputs and
+// the queries, the binning runs on the ctx's contig table and the SW kernels read the resident reference.
+int fadegpu_align_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regions *in, int32_t max_ops,
+                          fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+{
+    if (!c) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_align_regions: null ctx");
+    if (n_regions < 0 || n_regions > ((int64_t)1 << 30) || max_ops < 0)
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: n_regions or max_ops out of range");
+    if (n_regions > 0 && (!in || !in->query_off || !in->tid || !in->start || !in->end || !in->strand || !out ||
+                          (max_ops > 0 && !ops_out)))
+        return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: null argument");
+    { int rc = refuse_in_flight(c, "fadegpu_align_regions"); if (rc) return rc; }
+    if (c->n_contigs <= 0) return fail(c, FADEGPU_E_STATE, "fadegpu_align_regions: no reference is loaded");
+    const auto t_begin = std::chrono::steady_clock::now();
+    const int64_t n = n_regions;
+    int64_t qbytes = 0, n_over = 0;
+    if (n > 0) {
+        const int64_t *qo = in->query_off;
+        if (qo[0] < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: negative offset");
+        for (int64_t k = 0; k < n; ++k) {
+            const int64_t ql = qo[k + 1] - qo[k];
+            if (ql < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: offsets decrease at region " + std::to_string(k));
+            const int32_t tid = in->tid[k];
+            const int64_t s = in->start[k], e = in->end[k];
+            if (tid < 0 || tid >= c->n_contigs || s < 0 || s > e || e > c->clen[(size_t)tid] || in->strand[k] > 1) {
+                const std::string at = "fadegpu_align_regions: region " + std::to_string(k) + ": ";
+                if (tid < 0 || tid >= c->n_contigs)
+                    return fail(c, FADEGPU_E_ARG, at + "tid " + std::to_string(tid) + " is not a contig of the reference");
+                if (s < 0 || s > e || e > c->clen[(size_t)tid])
+                    return fail(c, FADEGPU_E_ARG, at + "[" + std::to_string(s) + ", " + std::to_string(e) +
+                                                      ") is not an interval of contig " + std::to_string(tid) + " (length " +
+                                                      std::to_string(c->clen[(size_t)tid]) + ")");
+                return fail(c, FADEGPU_E_ARG, at + "strand " + std::to_string(in->strand[k]) + " is neither 0 nor 1");
+            }
+            const int64_t tl = e - s;
+            if (ql > 0 && tl > 0 && (tl > 0x7fffffff || ql * tl > PAIR_MAX_CELLS)) ++n_over;
+        }
+        qbytes = qo[n] - qo[0];
+        if (qbytes > 0 && !in->query) return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: null sequence array");
+    }
+    // ---- staging: [query_off rebased to 0][tid][start][end][strand], then the query letters ----
+    const size_t o_tid = align16((size_t)(n + 1) * 8), o_start = o_tid + align16((size_t)n * 4);
+    const size_t o_end = o_start + align16((size_t)n * 8), o_strand = o_end + align16((size_t)n * 8);
+    const size_t o_q = o_strand + align16((size_t)n);
+    StagedCall sc;
+    sc.fn = "fadegpu_align_regions"; sc.item = "region";
+    sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops;
+    sc.raw = o_q + align16((size_t)qbytes);
+    sc.o_tbeg = o_start; sc.o_tend = o_end;
+    sc.stage = [&](char *h) {
+        int64_t *hq = reinterpret_cast<int64_t *>(h);
+        const int64_t q0 = in->query_off[0];
+        for (int64_t k = 0; k <= n; ++k) hq[k] = in->query_off[k] - q0;
+        memcpy(h + o_tid, in->tid, (size_t)n * 4);
+        memcpy(h + o_start, in->start, (size_t)n * 8);
+        memcpy(h + o_end, in->end, (size_t)n * 8);
+        memcpy(h + o_strand, in->strand, (size_t)n);
+        if (qbytes) parallel_copy(h + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
+    };
+    sc.prep = [&](fadegpu_batch *b, const char *d, BinArgs &ba, int *launches) -> int {
+        RegionArgs ra{};
+        ra.n = n;
+        ra.query = d + o_q; ra.qoff = reinterpret_cast<const int64_t *>(d);
+        ra.rtid = reinterpret_cast<const int32_t *>(d + o_tid);
+        ra.start = reinterpret_cast<const int64_t *>(d + o_start); ra.end = reinterpret_cast<const int64_t *>(d + o_end);
+        ra.strand = reinterpret_cast<const uint8_t *>(d + o_strand);
+        ra.seq_off = b->d_in_seq_off; ra.pos = b->d_in_pos; ra.l_qseq = b->d_in_lq; ra.tid = b->d_in_tid;
+        ra.aligned_len = b->d_in_alen; ra.clip_left = b->d_in_cl; ra.clip_right = b->d_in_cr;
+        ra.seq4 = b->d_in_seq4; ra.bad = c->pairs.d_bad;
+        CU(c, launch_region_prep(ra, c->sm_count, c->stream2));
+        *launches += 1;
+        // the intervals were validated above, so the window arithmetic clamps nothing: gstart = coff[tid] + start
+        ba.clen = c->d_clen; ba.coff = c->d_coff; ba.n_contigs = c->n_contigs;
+        return 0;
+    };
+    sc.reference = [&](fadegpu_batch *, RefDev *ref, int *) -> int { *ref = ref_dev(c); return 0; };
+    return align_staged(c, sc, out, ops_out, stats_out, t_begin);
 }
 
 int fadegpu_measure_alu_peak(fadegpu_ctx *c, double *ops_per_sec_out, double *sm_clock_mhz_out)

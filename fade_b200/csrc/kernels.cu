@@ -925,12 +925,31 @@ __device__ __forceinline__ int nt16_of_ascii(int ch)
     }
 }
 
+// The lanes of a warp write the qlen ASCII letters q as nt16 nibbles, two bases per byte, at dst: in REVERSE
+// COMPLEMENT when rc.  True when the lane met a letter outside nt16.
+__device__ __forceinline__ bool pack_query_nt16(const char *q, int64_t qlen, bool rc, uint8_t *dst, int l)
+{
+    const uint8_t comp16[16] = { 0, 8, 4, 12, 2, 10, 6, 14, 1, 9, 5, 13, 3, 11, 7, 15 };
+    bool bad = false;
+    for (int64_t b = l; b < (qlen + 1) / 2; b += 32) {
+        uint32_t byte = 0;
+        for (int h = 0; h < 2; ++h) {
+            const int64_t i = 2 * b + h;   // base i of the reverse complement = complement of base qlen-1-i
+            if (i >= qlen) break;
+            const int c = nt16_of_ascii((unsigned char)q[rc ? qlen - 1 - i : i]);
+            bad |= c > 15;
+            byte |= (uint32_t)(rc ? comp16[c & 15] : c & 15) << (h ? 0 : 4);
+        }
+        dst[b] = (uint8_t)byte;
+    }
+    return bad;
+}
+
 // One warp per pair: lane 0 writes the pair's binning inputs, the lanes write the query as nt16 nibbles in REVERSE
 // COMPLEMENT, two bases per byte.  The kernels reverse-complement a read as they load it (source/util.d:18-34), which
 // restores the forward query; nt16 complement is an involution, so IUPAC letters come back unchanged.
 __global__ void FADE_SMALL_KERNEL pair_prep_kernel(const PairArgs a)
 {
-    const uint8_t comp16[16] = { 0, 8, 4, 12, 2, 10, 6, 14, 1, 9, 5, 13, 3, 11, 7, 15 };
     const int l = threadIdx.x & 31;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < a.n; k += nwarps) {
@@ -948,19 +967,32 @@ __global__ void FADE_SMALL_KERNEL pair_prep_kernel(const PairArgs a)
             a.clen[k] = tlen;
             a.coff[k] = 32 * (k + (t0 >> 5));
         }
-        bool bad = false;
-        const char *q = a.query + q0;
-        for (int64_t b = l; b < (qlen + 1) / 2; b += 32) {
-            uint32_t byte = 0;
-            for (int h = 0; h < 2; ++h) {
-                const int64_t i = 2 * b + h;   // base i of the reverse complement = complement of base qlen-1-i
-                if (i >= qlen) break;
-                const int c = nt16_of_ascii((unsigned char)q[qlen - 1 - i]);
-                bad |= c > 15;
-                byte |= (uint32_t)comp16[c & 15] << (h ? 0 : 4);
-            }
-            a.seq4[q0 + b] = (uint8_t)byte;
+        const bool bad = pack_query_nt16(a.query + q0, qlen, true, a.seq4 + q0, l);
+        if (__any_sync(0xffffffffu, bad) && l == 0) atomicMin(a.bad, (int32_t)k);
+    }
+}
+
+// One warp per region, as pair_prep_kernel: the window of region k is [start, end) of contig tid (window 0 in the
+// binning).  Strand 0 stores the query reverse-complemented and strand 1 as given, so that the kernels' reverse
+// complement aligns the query itself or its reverse complement.
+__global__ void FADE_SMALL_KERNEL region_prep_kernel(const RegionArgs a)
+{
+    const int l = threadIdx.x & 31;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < a.n; k += nwarps) {
+        const int64_t q0 = a.qoff[k], qlen = a.qoff[k + 1] - q0;
+        const int64_t tlen = a.end[k] - a.start[k];
+        const bool over = tlen > 0x7fffffff || qlen * tlen > PAIR_MAX_CELLS;   // left unaligned, reported
+        if (l == 0) {
+            a.seq_off[k] = q0;
+            a.pos[k] = a.start[k];
+            a.l_qseq[k] = (int32_t)qlen;
+            a.tid[k] = a.rtid[k];
+            a.aligned_len[k] = over ? 0 : (int32_t)tlen;
+            a.clip_left[k] = over ? 0 : (int32_t)qlen;   // the length floor (0) passes every non-empty query
+            a.clip_right[k] = 0;
         }
+        const bool bad = pack_query_nt16(a.query + q0, qlen, a.strand[k] == 0, a.seq4 + q0, l);
         if (__any_sync(0xffffffffu, bad) && l == 0) atomicMin(a.bad, (int32_t)k);
     }
 }
@@ -1075,10 +1107,11 @@ __global__ void __launch_bounds__(256) pair_xlist_kernel(const PairArgs a)
     }
 }
 
-__global__ void FADE_SMALL_KERNEL pair_results_init_kernel(const PairArgs a, PairResult *res)
+__global__ void FADE_SMALL_KERNEL pair_results_init_kernel(int64_t n, const int64_t *qoff, const int64_t *t_beg,
+                                                           const int64_t *t_end, PairResult *res)
 {
-    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < a.n; k += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t qlen = a.qoff[k + 1] - a.qoff[k], tlen = a.toff[k + 1] - a.toff[k];
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t qlen = qoff[k + 1] - qoff[k], tlen = t_end[k] - t_beg[k];
         PairResult r;
         r.score = r.end_query = r.end_ref = r.beg_query = r.beg_ref = r.n_ops = 0;
         r.reserved = 0;
@@ -1318,14 +1351,23 @@ cudaError_t launch_pair_xlist(const PairArgs &a, cudaStream_t s)
     return cudaGetLastError();
 }
 
-cudaError_t launch_pair_results(const PairArgs &a, const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill,
-                                int max_ops, PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count,
-                                cudaStream_t s)
+cudaError_t launch_region_prep(const RegionArgs &a, int sm_count, cudaStream_t s)
 {
     if (a.n <= 0) return cudaSuccess;
-    pair_results_init_kernel<<<(int)std::min<int64_t>((a.n + 127) / 128, (int64_t)sm_count * 16), 128, 0, s>>>(a, res);
+    const int grid = (int)std::min<int64_t>((a.n * 32 + 127) / 128, (int64_t)sm_count * 16);
+    region_prep_kernel<<<grid, 128, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pair_results(int64_t n, const int64_t *qoff, const int64_t *t_beg, const int64_t *t_end,
+                                const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill, int max_ops,
+                                PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count, cudaStream_t s)
+{
+    if (n <= 0) return cudaSuccess;
+    pair_results_init_kernel<<<(int)std::min<int64_t>((n + 127) / 128, (int64_t)sm_count * 16), 128, 0, s>>>(n, qoff, t_beg,
+                                                                                                             t_end, res);
     if (n_aln > 0)
-        pair_results_kernel<<<std::min((n_aln + 127) / 128, sm_count * 16), 128, 0, s>>>(aln, out, n_aln, a.n, spill, max_ops,
+        pair_results_kernel<<<std::min((n_aln + 127) / 128, sm_count * 16), 128, 0, s>>>(aln, out, n_aln, n, spill, max_ops,
                                                                                        res, ops, n_ok);
     return cudaGetLastError();
 }

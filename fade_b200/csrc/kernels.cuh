@@ -6,7 +6,8 @@
 //   sw_generic_kernel    exact int32 fallback ON THE DEVICE for wildcard letters and sizes the
 //                        packed kernels do not cover (thread per alignment)
 //   pair_*_kernel        fadegpu_align_pairs: pack caller-supplied ASCII pairs into the read / reference formats
-//                        above, and put the records back into pair order
+//                        above, and put the records back into pair order (also for regions)
+//   region_prep_kernel   fadegpu_align_regions: pack caller-supplied queries against intervals of the reference
 //   alu_peak_kernel      INT16x2 ALU issue-rate microbenchmark (roofline denominator)
 //
 // Window gather (source/analysis.d:45-64) and reverse complement (source/util.d:18-34) happen
@@ -154,16 +155,35 @@ constexpr uint32_t PAIR_R_OVERSIZE = 32u;   // FADEGPU_R_OVERSIZE
 cudaError_t launch_pair_prep(const PairArgs &a, int sm_count, cudaStream_t s);
 cudaError_t launch_pair_pack_targets(const PairArgs &a, cudaStream_t s);   // planes + chunk_x + n_x
 cudaError_t launch_pair_xlist(const PairArgs &a, cudaStream_t s);          // xpos / xchr (after n_x is known)
-// pair-ordered result records: zeros (or FADEGPU_R_OVERSIZE) for every pair, then the records of the alignments with
-// their full forward CIGARs assembled from the spill rings; n_ok counts the records the SW kernels produced
+// ---- caller-supplied queries against intervals of the resident reference (fadegpu_align_regions): only the queries
+//      are packed; the binning runs on the ctx's own contig table ----
+struct RegionArgs {
+    int64_t n;
+    const char *query;              // concatenated ASCII
+    const int64_t *qoff;            // [n+1], starting at 0
+    const int32_t *rtid;            // [n] contig of the interval
+    const int64_t *start, *end;     // [n] interval [start, end) on the contig (validated by the host)
+    const uint8_t *strand;          // [n] 0: the query as given, 1: its reverse complement
+    // per-region inputs of the binning (pos = start, aligned_len = end - start, clip_left = qlen, clip_right = 0)
+    int64_t *seq_off, *pos;
+    int32_t *l_qseq, *tid, *aligned_len, *clip_left, *clip_right;
+    uint8_t *seq4;                  // queries as BAM nt16 nibbles, stored so that the kernels' reverse complement gives
+                                    // the strand's letters, query k at byte qoff[k]
+    int32_t *bad;                   // lowest region whose query holds a letter outside nt16 (atomicMin; starts at n)
+};
+cudaError_t launch_region_prep(const RegionArgs &a, int sm_count, cudaStream_t s);
+// item-ordered result records (pairs or regions): zeros (or FADEGPU_R_OVERSIZE) for every item k, whose query is
+// qoff[k] .. qoff[k+1] and whose window spans t_beg[k] .. t_end[k] (pairs: toff, toff + 1; regions: start, end), then
+// the records of the alignments with their full forward CIGARs assembled from the spill rings; n_ok counts the records
+// the SW kernels produced
 struct PairResult {   // == fadegpu_pair_result
     int32_t score, end_query, end_ref, beg_query, beg_ref, n_ops;
     uint32_t flags;
     int32_t reserved;
 };
-cudaError_t launch_pair_results(const PairArgs &a, const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill,
-                                int max_ops, PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count,
-                                cudaStream_t s);
+cudaError_t launch_pair_results(int64_t n, const int64_t *qoff, const int64_t *t_beg, const int64_t *t_end,
+                                const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill, int max_ops,
+                                PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count, cudaStream_t s);
 
 constexpr int FILL_THREADS = 128;
 constexpr int OVER_CAP = 256;        // oversize reads listed per batch (all of them are counted)

@@ -284,6 +284,43 @@ typedef struct fadegpu_pair_result {
 int fadegpu_align_pairs(fadegpu_ctx *ctx, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
                         fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out);
 
+/* ---- Smith-Waterman with traceback of caller-supplied queries against intervals of the resident reference ----
+ * Region k is query[query_off[k] .. query_off[k+1]) against [start[k], end[k]) of contig tid[k] (the index into the
+ * contigs of fadegpu_load_reference), on strand[k]: 0 aligns the query as given, 1 its reverse complement.
+ *
+ * Alignment semantics: exactly P1-P5 (SURVEY 8a) with the ctx's scoring and the interval as the window, upper-cased as
+ *   every window is.  The reverse complement of strand 1 is the nt16 complement (source/util.d:18-34), so IUPAC
+ *   letters stay valid.  beg_query / end_query index the query as it was aligned (for strand 1: its reverse
+ *   complement, as the annotate records do); beg_ref / end_ref are relative to start, so the reference position of
+ *   the alignment is start + beg_ref.
+ * Query letters: as fadegpu_align_pairs; a letter outside nt16 fails the call with FADEGPU_E_ARG naming the first
+ *   region holding one (checked on the device).
+ * Scoring: from the ctx; FADEGPU_F_FORCE_GENERIC applies, FADEGPU_F_TAGS_ONLY does not: every region is traced back.
+ *   No length floor and no accept predicate applies.
+ * Records and CIGAR ops: as fadegpu_align_pairs, in REGION ORDER: n_ops is always exact, max_ops / ops_out /
+ *   FADEGPU_R_OPS_TRUNC follow the same rules, flags hold only ALIGNED | GENERIC | OPS_TRUNC | OVERSIZE.
+ * Empty regions: an empty query or an empty interval gives flags = 0 and a zero record.
+ * Oversize regions: query length * (end - start) > 2^31, or end - start > 0x7fffffff: not aligned, FADEGPU_R_OVERSIZE,
+ *   counted in stats_out->n_oversize.
+ * Argument errors (FADEGPU_E_ARG, checked on the host before anything is uploaded; fadegpu_last_error names the first
+ *   offending region): tid outside [0, n_contigs), start < 0, start > end, end > the contig's length, strand other
+ *   than 0 or 1, decreasing query offsets, null arrays.
+ * State errors (FADEGPU_E_STATE): no reference is loaded, or a batch of the ctx is in flight.  Waited batches keep
+ *   their results, and fadegpu_replay_kernels / fadegpu_replay_batches of existing batches keep working.
+ *
+ * Synchronous.  The arrays are host memory (pageable is fine) and only read during the call.  stats_out (may be NULL)
+ * receives the fields of fadegpu_align_pairs; h2d_bytes counts what was staged: the query offsets, the per-region
+ * arrays and the query letters (no reference letters), plus the launch plan. */
+typedef struct fadegpu_regions {
+    const char *query; const int64_t *query_off;    /* [n+1] ASCII queries, concatenated */
+    const int32_t *tid;                             /* [n] contig index of fadegpu_load_reference */
+    const int64_t *start, *end;                     /* [n] 0-based half-open interval [start, end) on contig tid */
+    const uint8_t *strand;                          /* [n] 0: the query as given, 1: its reverse complement */
+} fadegpu_regions;                                  /* 48 bytes */
+
+int fadegpu_align_regions(fadegpu_ctx *ctx, int64_t n_regions, const fadegpu_regions *in, int32_t max_ops,
+                          fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out);
+
 /* INT16x2 ALU roofline denominator (SURVEY 8d): measures packed VIMNMX/VIADDMNMX issue rate.
  * ops_per_sec_out = packed (2-lane) instructions * 32 threads per second over the whole GPU. */
 int fadegpu_measure_alu_peak(fadegpu_ctx *ctx, double *ops_per_sec_out, double *sm_clock_mhz_out);
