@@ -7,4 +7,4 @@ CPU fallback: importing works anywhere, computing needs the built library and a 
 """
 from ._lib import FadeGpuError, build, lib, lib_path  # noqa: F401
 from .api import (Batch, Context, Params, Record, annotate_records, default_params,  # noqa: F401
-                  MAX_OPS, PairResults, PAIR_RESULT_DTYPE)
+                  MAX_OPS, PairResults, PAIR_RESULT_DTYPE, ScoreResults)

@@ -78,12 +78,12 @@ class Stats(C.Structure):
 
 
 class PairsIn(C.Structure):
-    """fadegpu_pairs: host arrays of one fadegpu_align_pairs call"""
+    """fadegpu_pairs: host arrays of one fadegpu_align_pairs / fadegpu_score_pairs call"""
     _fields_ = [("query", C.c_void_p), ("query_off", C.c_void_p), ("target", C.c_void_p), ("target_off", C.c_void_p)]
 
 
 class RegionsIn(C.Structure):
-    """fadegpu_regions: host arrays of one fadegpu_align_regions call"""
+    """fadegpu_regions: host arrays of one fadegpu_align_regions / fadegpu_score_regions call"""
     _fields_ = [("query", C.c_void_p), ("query_off", C.c_void_p), ("tid", C.c_void_p), ("start", C.c_void_p),
                 ("end", C.c_void_p), ("strand", C.c_void_p)]
 
@@ -105,7 +105,8 @@ ABI_SYMBOLS = [
     "fadegpu_destroy", "fadegpu_last_error", "fadegpu_load_reference", "fadegpu_share_reference",
     "fadegpu_reference_info", "fadegpu_alloc_batch", "fadegpu_get_batch_view", "fadegpu_free_batch",
     "fadegpu_submit", "fadegpu_submit_compact", "fadegpu_submit_inputs", "fadegpu_wait", "fadegpu_get_results", "fadegpu_get_stats", "fadegpu_get_timeline", "fadegpu_replay_kernels", "fadegpu_replay_batches",
-    "fadegpu_align_pairs", "fadegpu_align_regions", "fadegpu_measure_alu_peak",
+    "fadegpu_align_pairs", "fadegpu_align_regions", "fadegpu_score_pairs", "fadegpu_score_regions",
+    "fadegpu_measure_alu_peak",
     "fadehost_parse_clips", "fadehost_aligned_length", "fadehost_prepare", "fadehost_finish",
 ]
 
@@ -146,6 +147,8 @@ def lib():
     L.fadegpu_replay_batches.argtypes = [vp, C.POINTER(vp), i32, i32, C.POINTER(C.c_float)]
     L.fadegpu_align_pairs.argtypes = [vp, i64, C.POINTER(PairsIn), i32, vp, vp, C.POINTER(Stats)]
     L.fadegpu_align_regions.argtypes = [vp, i64, C.POINTER(RegionsIn), i32, vp, vp, C.POINTER(Stats)]
+    L.fadegpu_score_pairs.argtypes = [vp, i64, C.POINTER(PairsIn), vp, C.POINTER(Stats)]
+    L.fadegpu_score_regions.argtypes = [vp, i64, C.POINTER(RegionsIn), vp, C.POINTER(Stats)]
     L.fadegpu_measure_alu_peak.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.fadehost_parse_clips.argtypes = [C.POINTER(C.c_uint32), i32, C.POINTER(C.c_uint32)]
     L.fadehost_parse_clips.restype = None

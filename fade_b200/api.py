@@ -106,6 +106,17 @@ class PairResults:
         return "".join(f"{int(o) >> 4}{OPCHARS[int(o) & 0xf]}" for o in self.ops[k, :n])
 
 
+@dataclass
+class ScoreResults:
+    """Context.score_pairs / score_regions: records[n] (PAIR_RESULT_DTYPE) in pair / region order -- score, end_query,
+    end_ref and flags; beg_query, beg_ref and n_ops are 0, there is no CIGAR -- and the call's stats."""
+    records: np.ndarray
+    stats: Stats
+
+    def __len__(self):
+        return len(self.records)
+
+
 def default_params(**kw) -> Params:
     p = Params()
     rc = lib().fadegpu_default_params(C.byref(p))
@@ -227,6 +238,29 @@ class Context:
         self._check(lib().fadegpu_align_regions(self._h, n, C.byref(rin), max_ops, rec.ctypes.data,
                                                 ops.ctypes.data if max_ops > 0 else None, C.byref(st)))
         return PairResults(rec, ops, st)
+
+    def score_pairs(self, queries, targets, *, query_offsets=None, target_offsets=None) -> ScoreResults:
+        """fadegpu_score_pairs: score and end cell of query k against target k, without traceback.  Inputs as in
+        align_pairs; score, end_query and end_ref equal align_pairs' on the same inputs."""
+        q, qo, t, to = pack_pairs(queries, targets, query_offsets, target_offsets)
+        n = len(qo) - 1
+        rec = np.zeros(n, dtype=PAIR_RESULT_DTYPE)
+        st = Stats()
+        pin = PairsIn(q.ctypes.data, qo.ctypes.data, t.ctypes.data, to.ctypes.data)
+        self._check(lib().fadegpu_score_pairs(self._h, n, C.byref(pin), rec.ctypes.data, C.byref(st)))
+        return ScoreResults(rec, st)
+
+    def score_regions(self, queries, tids, starts, ends, strands=None, *, query_offsets=None) -> ScoreResults:
+        """fadegpu_score_regions: score and end cell of query k against [starts[k], ends[k]) of contig tids[k], without
+        traceback.  Inputs as in align_regions; score, end_query and end_ref equal align_regions' on the same inputs."""
+        q, qo, tid, start, end, strand = pack_regions(queries, tids, starts, ends, strands, query_offsets)
+        n = len(qo) - 1
+        rec = np.zeros(n, dtype=PAIR_RESULT_DTYPE)
+        st = Stats()
+        rin = RegionsIn(q.ctypes.data, qo.ctypes.data, tid.ctypes.data, start.ctypes.data, end.ctypes.data,
+                        strand.ctypes.data)
+        self._check(lib().fadegpu_score_regions(self._h, n, C.byref(rin), rec.ctypes.data, C.byref(st)))
+        return ScoreResults(rec, st)
 
     def alloc_batch(self, max_reads: int, max_seq_bytes: int) -> "Batch":
         return Batch(self, max_reads, max_seq_bytes)

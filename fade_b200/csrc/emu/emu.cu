@@ -26,7 +26,8 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
                const uint8_t *qb, int qlen_b, const uint8_t *tb, int tlen_b,
                const SwConsts &k, int extra_blocks, int tagged, int32_t min_length,
                uint32_t clipl_a, uint32_t clipr_a, uint32_t clipl_b, uint32_t clipr_b,
-               AlnOut *out_a, AlnOut *out_b, int ops_cap = 0, uint32_t *ops_a = nullptr, uint32_t *ops_b = nullptr)
+               AlnOut *out_a, AlnOut *out_b, int ops_cap = 0, uint32_t *ops_a = nullptr, uint32_t *ops_b = nullptr,
+               int32_t *scan_info = nullptr)
 {
     const int rows = FG * R;
     if (qlen_a > rows || qlen_b > rows) return -1;
@@ -102,7 +103,12 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
     ctl_init(ctl[1], qlen_b, tlen_b);
     constexpr int RW = trace_words<R>();
     std::vector<uint32_t> tr((size_t)tile_words<R>());
-    const bool tg = (tagged & 1) && k.tagged_ok;
+    // bit 5 of `tagged`: score-only calls -- every replay is a scan with the score-only step (no trace), the walkers stop
+    // at the end cell; scan_info[2 L ..] receives lane L's number of scan replays and its first candidate block
+    const bool end_only = (tagged & 32) != 0;
+    const bool tg = !end_only && (tagged & 1) && k.tagged_ok;
+    int32_t scans[2] = { 0, 0 }, first_blk[2];
+    for (int L = 0; L < 2; ++L) first_blk[L] = ctl[L].phase == 0 ? ctl[L].next_blk : -1;
     // ops_cap > 0: the walkers also spill every op into rings of ops_cap words, as the device does for
     // fadegpu_align_pairs, and ops_a / ops_b receive the first ops_cap forward ops assembled from them
     std::vector<uint32_t> spill[2];
@@ -151,10 +157,16 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
                 const uint32_t ts = (tw[t0 - g + FG] & 0x00ffu) | (tw[t1 - g + FG] & 0xff00u);
                 uint32_t cmax = 0;
                 uint32_t trw[RW];
-                if (tg) trace_step_tagged<R>(st[g].H, st[g].E, st[g].qs, ts, st[g].hu_prev, fin[g], st[g].fout, k, trw, cmax);
-                else trace_step_plain<R>(st[g].H, st[g].E, st[g].qs, ts, st[g].hu_prev, fin[g], st[g].fout, k, trw, cmax);
+                if (end_only) {
+                    if (step == 2) score_step<R, 2>(st[g].H, st[g].E, st[g].qp, cmax, ts, st[g].hu_prev, fin[g], st[g].fout, k);
+                    else if (step == 1) score_step<R, 1>(st[g].H, st[g].E, st[g].qf, cmax, ts, st[g].hu_prev, fin[g], st[g].fout, k);
+                    else score_step<R, 0>(st[g].H, st[g].E, st[g].qs, cmax, ts, st[g].hu_prev, fin[g], st[g].fout, k);
+                } else {
+                    if (tg) trace_step_tagged<R>(st[g].H, st[g].E, st[g].qs, ts, st[g].hu_prev, fin[g], st[g].fout, k, trw, cmax);
+                    else trace_step_plain<R>(st[g].H, st[g].E, st[g].qs, ts, st[g].hu_prev, fin[g], st[g].fout, k, trw, cmax);
+                    for (int w = 0; w < RW; ++w) tr[(size_t)tile_index<R>(u, g, w)] = trw[w];
+                }
                 st[g].hu_prev = hu[g];
-                for (int w = 0; w < RW; ++w) tr[(size_t)tile_index<R>(u, g, w)] = trw[w];
                 for (int L = 0; L < 2; ++L) {
                     if (!scan[L][g] || found[L][g]) continue;
                     const int cm = L == 0 ? lane_lo(cmax) : lane_hi(cmax);
@@ -175,10 +187,19 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
             for (int g = 0; g < FG; ++g)
                 if (scan[L][g] && !found[L][g]) return -3;  // a candidate must find its cell
         // bit 2 of `tagged`: the first (scan) replay of a lane records no trace, like round 0 on the device
-        const bool so0 = (tagged & 4) && ctl[0].phase == 0 && first_iter, so1 = (tagged & 4) && ctl[1].phase == 0 && first_iter;
-        ctl_advance<R>(ctl[0], so0 ? nullptr : tr.data(), 0, StagedAcc{ tw.data(), qc.data(), 0 }, k, sp0, ops_cap);
-        ctl_advance<R>(ctl[1], so1 ? nullptr : tr.data(), 1, StagedAcc{ tw.data(), qc.data(), 1 }, k, sp1, ops_cap);
+        const bool so0 = end_only || ((tagged & 4) && ctl[0].phase == 0 && first_iter);
+        const bool so1 = end_only || ((tagged & 4) && ctl[1].phase == 0 && first_iter);
+        for (int L = 0; L < 2; ++L) scans[L] += ctl[L].phase == 0;
+        ctl_advance<R>(ctl[0], so0 ? nullptr : tr.data(), 0, StagedAcc{ tw.data(), qc.data(), 0 }, k, sp0, ops_cap, end_only);
+        ctl_advance<R>(ctl[1], so1 ? nullptr : tr.data(), 1, StagedAcc{ tw.data(), qc.data(), 1 }, k, sp1, ops_cap, end_only);
         first_iter = false;
+    }
+    if (scan_info)
+        for (int L = 0; L < 2; ++L) { scan_info[2 * L] = scans[L]; scan_info[2 * L + 1] = first_blk[L]; }
+    if (end_only) {
+        finalize_end(ctl[0], *out_a, 0);
+        finalize_end(ctl[1], *out_b, 1);
+        return 0;
     }
     finalize_result(ctl[0], *out_a, 0, clipl_a, clipr_a, min_length);
     finalize_result(ctl[1], *out_b, 1, clipl_b, clipr_b, min_length);
@@ -230,6 +251,27 @@ extern "C" int fadeemu_align_pair_ops(int R, const uint8_t *qa, int qlen_a, cons
     case RR:                                                                                       \
         return align_pair<RR>(qa, qlen_a, ta, tlen_a, qb, qlen_b, tb, tlen_b, k, 0, tagged, 0, 0, 0, 0, 0, \
                               out_a, out_b, ops_cap, ops_a, ops_b);
+    switch (R) {
+        CASE(1) CASE(2) CASE(3) CASE(5) CASE(13) CASE(19) CASE(25) CASE(32) CASE(38)
+    default: return -10;
+    }
+#undef CASE
+}
+
+// The score-only calls (fadegpu_score_pairs / _regions): scan-only replays with the score-only step, walkers that stop
+// at the end cell, finalize_end records.  scan_info[4]: per lane, the number of scan replays and the first candidate
+// block (-1: no scan).  `tagged` bits 1, 3 and 4 as above.
+extern "C" int fadeemu_score_pair(int R, const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
+                                  const uint8_t *qb, int qlen_b, const uint8_t *tb, int tlen_b,
+                                  int open, int extend, int match, int mismatch, int extra_blocks, int tagged,
+                                  AlnOut *out_a, AlnOut *out_b, int32_t *scan_info)
+{
+    SwConsts k = make_consts(open, extend, match, mismatch);
+    k.shortcut = (tagged & 2) ? 0 : 1;
+#define CASE(RR)                                                                                   \
+    case RR:                                                                                       \
+        return align_pair<RR>(qa, qlen_a, ta, tlen_a, qb, qlen_b, tb, tlen_b, k, extra_blocks,    \
+                              tagged | 32, 0, 0, 0, 0, 0, out_a, out_b, 0, nullptr, nullptr, scan_info);
     switch (R) {
         CASE(1) CASE(2) CASE(3) CASE(5) CASE(13) CASE(19) CASE(25) CASE(32) CASE(38)
     default: return -10;

@@ -380,17 +380,19 @@ int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *c
 // With stage timers every launch is synchronised.
 // What a plan runs against: the resident reference (submits) or the packed targets of a pair call, whether alignments
 // whose score rules out both predicates skip the traceback (FADEGPU_F_TAGS_ONLY), and the optional full-CIGAR spill
-// rings (ops_cap words per alignment of the batch, in its sorted order).
+// rings (ops_cap words per alignment of the batch, in its sorted order).  end_only (score-only calls): no alignment is
+// traced back; the traceback launches only find the end cell.
 struct PlanTarget {
     RefDev ref;
     int tags_only;
     uint32_t *ops_spill;
     int ops_cap;
+    bool end_only;
 };
 
 PlanTarget batch_target(const fadegpu_ctx *c)
 {
-    return PlanTarget{ ref_dev(c), (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0, nullptr, 0 };
+    return PlanTarget{ ref_dev(c), (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0, nullptr, 0, false };
 }
 
 int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill_ms, float *trace_ms, float *gen_ms,
@@ -447,7 +449,7 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill
             CU(c, cudaEventRecord(ln.ev_fill, sf));
             CU(c, cudaStreamWaitEvent(st, ln.ev_fill, 0));
             nl += 1;   // the fill kernel; launch_trace adds its own launches
-            CU(c, launch_trace(L.R, a, st, c->sm_count, &nl));
+            CU(c, launch_trace(L.R, a, pt.end_only, st, c->sm_count, &nl));
             // wildcard letters found by the packed kernels -> generic kernel over the flagged ones
             GenericArgs ga;
             ga.aln = a.aln; ga.n_aln = L.n_aln; ga.aln_flags = a.aln_flags; ga.seq = a.seq; ga.ref = a.ref;
@@ -1688,6 +1690,7 @@ struct StagedCall {
     const char *fn, *item;        // the call's and an item's name, for messages
     int64_t n, qbytes, n_over;    // items, query letters, oversize items (counted by the host validation)
     int32_t max_ops;
+    bool score_only;              // fadegpu_score_*: score and end cell, no traceback (max_ops is 0)
     size_t raw;                   // bytes staged and uploaded
     size_t o_tbeg, o_tend;        // byte offsets of the int64 window bounds of every item in the upload (results init)
     std::function<void(char *h_stage)> stage;
@@ -1700,8 +1703,8 @@ struct StagedCall {
 
 // The raw inputs go to the device through pinned staging on stream2, where the caller's prep kernels write the
 // per-item binning inputs and the queries; the binning, the launch plan and run_plan are those of a device-binned
-// submit, on the ctx's internal pair batch, with every alignment traced back and the full CIGARs spilled; the records
-// come back in item order on stream3.
+// submit, on the ctx's internal pair batch, with every alignment traced back and the full CIGARs spilled (score-only
+// calls: only the end cell is found, nothing is spilled); the records come back in item order on stream3.
 static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_result *out, uint32_t *ops_out,
                         fadegpu_stats *stats_out, std::chrono::steady_clock::time_point t_begin)
 {
@@ -1802,9 +1805,10 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
     // ---- SW kernels: the batch's plan against the caller's reference ----
     CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
     CU(c, cudaEventRecord(b->ev[1], c->stream));
-    pt.tags_only = 0;   // every item is traced back, whatever the ctx's FADEGPU_F_TAGS_ONLY
+    pt.tags_only = 0;   // every item is traced back (or has its end cell found), whatever the ctx's FADEGPU_F_TAGS_ONLY
     pt.ops_spill = max_ops > 0 ? pb.d_spill : nullptr;
     pt.ops_cap = max_ops;
+    pt.end_only = sc.score_only;
     int nl = 0;
     { int rc = run_plan(c, b, pt, nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
     // ---- records in item order, home on stream3 ----
@@ -1812,8 +1816,9 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
     { int rc = join_kernels(c, b, s3); if (rc) return rc; }
     CU(c, cudaEventRecord(b->ev[2], s3));
     CU(c, launch_pair_results(n, reinterpret_cast<const int64_t *>(pb.d_raw), reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tbeg),
-                              reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tend), b->d_aln, b->d_out, (int)n_aln, pb.d_spill,
-                              max_ops, reinterpret_cast<PairResult *>(pb.d_res), pb.d_ops, b->d_stats + 7, c->sm_count, s3));
+                              reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tend), b->d_aln, b->d_out, (int)n_aln,
+                              sc.score_only, pb.d_spill, max_ops, reinterpret_cast<PairResult *>(pb.d_res), pb.d_ops,
+                              b->d_stats + 7, c->sm_count, s3));
     CU(c, cudaMemcpyAsync(out, pb.d_res, (size_t)n * sizeof(fadegpu_pair_result), cudaMemcpyDeviceToHost, s3));
     if (max_ops > 0)
         CU(c, cudaMemcpyAsync(ops_out, pb.d_ops, (size_t)n * (size_t)max_ops * 4, cudaMemcpyDeviceToHost, s3));
@@ -1842,30 +1847,31 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
 // Pairs: pair_prep_kernel writes the per-pair binning inputs and the queries (nt16, reverse-complemented),
 // pair_pack_targets_kernel and pair_xlist_kernel pack the targets as a reference of their own, whose contigs the
 // targets are.
-int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
-                        fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+static int pairs_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n_pairs, const fadegpu_pairs *in,
+                      int32_t max_ops, fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
 {
-    if (!c) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_align_pairs: null ctx");
+    const std::string at = std::string(fn) + ": ";
+    if (!c) return fail(nullptr, FADEGPU_E_ARG, at + "null ctx");
     if (n_pairs < 0 || n_pairs > ((int64_t)1 << 30) || max_ops < 0)
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: n_pairs or max_ops out of range");
+        return fail(c, FADEGPU_E_ARG, at + "n_pairs or max_ops out of range");
     if (n_pairs > 0 && (!in || !in->query_off || !in->target_off || !out || (max_ops > 0 && !ops_out)))
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null argument");
-    { int rc = refuse_in_flight(c, "fadegpu_align_pairs"); if (rc) return rc; }
+        return fail(c, FADEGPU_E_ARG, at + "null argument");
+    { int rc = refuse_in_flight(c, fn); if (rc) return rc; }
     const auto t_begin = std::chrono::steady_clock::now();
     const int64_t n = n_pairs;
     int64_t qbytes = 0, tbytes = 0, n_over = 0;
     if (n > 0) {
         const int64_t *qo = in->query_off, *to = in->target_off;
-        if (qo[0] < 0 || to[0] < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: negative offset");
+        if (qo[0] < 0 || to[0] < 0) return fail(c, FADEGPU_E_ARG, at + "negative offset");
         for (int64_t k = 0; k < n; ++k) {
             const int64_t ql = qo[k + 1] - qo[k], tl = to[k + 1] - to[k];
             if (ql < 0 || tl < 0)
-                return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: offsets decrease at pair " + std::to_string(k));
+                return fail(c, FADEGPU_E_ARG, at + "offsets decrease at pair " + std::to_string(k));
             if (ql > 0 && tl > 0 && (tl > 0x7fffffff || ql * tl > PAIR_MAX_CELLS)) ++n_over;
         }
         qbytes = qo[n] - qo[0]; tbytes = to[n] - to[0];
         if ((qbytes > 0 && !in->query) || (tbytes > 0 && !in->target))
-            return fail(c, FADEGPU_E_ARG, "fadegpu_align_pairs: null sequence array");
+            return fail(c, FADEGPU_E_ARG, at + "null sequence array");
     }
     // ---- staging: [query_off][target_off] rebased to 0, then the query and the target letters ----
     const size_t o_toff = align16((size_t)(n + 1) * 8), o_q = o_toff + align16((size_t)(n + 1) * 8);
@@ -1875,8 +1881,8 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
     fadegpu_ctx::PairBufs &pb = c->pairs;
     PairArgs pa{};
     StagedCall sc;
-    sc.fn = "fadegpu_align_pairs"; sc.item = "pair";
-    sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops;
+    sc.fn = fn; sc.item = "pair";
+    sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops; sc.score_only = score_only;
     sc.raw = o_t + align16((size_t)tbytes);
     sc.o_tbeg = o_toff; sc.o_tend = o_toff + 8;   // target k spans toff[k] .. toff[k + 1]
     sc.stage = [&](char *h) {
@@ -1921,32 +1927,45 @@ int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in
     return align_staged(c, sc, out, ops_out, stats_out, t_begin);
 }
 
+int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
+                        fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+{
+    return pairs_call(c, "fadegpu_align_pairs", false, n_pairs, in, max_ops, out, ops_out, stats_out);
+}
+
+int fadegpu_score_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, fadegpu_pair_result *out,
+                        fadegpu_stats *stats_out)
+{
+    return pairs_call(c, "fadegpu_score_pairs", true, n_pairs, in, 0, out, nullptr, stats_out);
+}
+
 // Regions: only the queries and the intervals are staged; region_prep_kernel writes the per-region binning inputs and
 // the queries, the binning runs on the ctx's contig table and the SW kernels read the resident reference.
-int fadegpu_align_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regions *in, int32_t max_ops,
-                          fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+static int regions_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n_regions, const fadegpu_regions *in,
+                        int32_t max_ops, fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
 {
-    if (!c) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_align_regions: null ctx");
+    const std::string at0 = std::string(fn) + ": ";
+    if (!c) return fail(nullptr, FADEGPU_E_ARG, at0 + "null ctx");
     if (n_regions < 0 || n_regions > ((int64_t)1 << 30) || max_ops < 0)
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: n_regions or max_ops out of range");
+        return fail(c, FADEGPU_E_ARG, at0 + "n_regions or max_ops out of range");
     if (n_regions > 0 && (!in || !in->query_off || !in->tid || !in->start || !in->end || !in->strand || !out ||
                           (max_ops > 0 && !ops_out)))
-        return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: null argument");
-    { int rc = refuse_in_flight(c, "fadegpu_align_regions"); if (rc) return rc; }
-    if (c->n_contigs <= 0) return fail(c, FADEGPU_E_STATE, "fadegpu_align_regions: no reference is loaded");
+        return fail(c, FADEGPU_E_ARG, at0 + "null argument");
+    { int rc = refuse_in_flight(c, fn); if (rc) return rc; }
+    if (c->n_contigs <= 0) return fail(c, FADEGPU_E_STATE, at0 + "no reference is loaded");
     const auto t_begin = std::chrono::steady_clock::now();
     const int64_t n = n_regions;
     int64_t qbytes = 0, n_over = 0;
     if (n > 0) {
         const int64_t *qo = in->query_off;
-        if (qo[0] < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: negative offset");
+        if (qo[0] < 0) return fail(c, FADEGPU_E_ARG, at0 + "negative offset");
         for (int64_t k = 0; k < n; ++k) {
             const int64_t ql = qo[k + 1] - qo[k];
-            if (ql < 0) return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: offsets decrease at region " + std::to_string(k));
+            if (ql < 0) return fail(c, FADEGPU_E_ARG, at0 + "offsets decrease at region " + std::to_string(k));
             const int32_t tid = in->tid[k];
             const int64_t s = in->start[k], e = in->end[k];
             if (tid < 0 || tid >= c->n_contigs || s < 0 || s > e || e > c->clen[(size_t)tid] || in->strand[k] > 1) {
-                const std::string at = "fadegpu_align_regions: region " + std::to_string(k) + ": ";
+                const std::string at = at0 + "region " + std::to_string(k) + ": ";
                 if (tid < 0 || tid >= c->n_contigs)
                     return fail(c, FADEGPU_E_ARG, at + "tid " + std::to_string(tid) + " is not a contig of the reference");
                 if (s < 0 || s > e || e > c->clen[(size_t)tid])
@@ -1959,15 +1978,15 @@ int fadegpu_align_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regio
             if (ql > 0 && tl > 0 && (tl > 0x7fffffff || ql * tl > PAIR_MAX_CELLS)) ++n_over;
         }
         qbytes = qo[n] - qo[0];
-        if (qbytes > 0 && !in->query) return fail(c, FADEGPU_E_ARG, "fadegpu_align_regions: null sequence array");
+        if (qbytes > 0 && !in->query) return fail(c, FADEGPU_E_ARG, at0 + "null sequence array");
     }
     // ---- staging: [query_off rebased to 0][tid][start][end][strand], then the query letters ----
     const size_t o_tid = align16((size_t)(n + 1) * 8), o_start = o_tid + align16((size_t)n * 4);
     const size_t o_end = o_start + align16((size_t)n * 8), o_strand = o_end + align16((size_t)n * 8);
     const size_t o_q = o_strand + align16((size_t)n);
     StagedCall sc;
-    sc.fn = "fadegpu_align_regions"; sc.item = "region";
-    sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops;
+    sc.fn = fn; sc.item = "region";
+    sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops; sc.score_only = score_only;
     sc.raw = o_q + align16((size_t)qbytes);
     sc.o_tbeg = o_start; sc.o_tend = o_end;
     sc.stage = [&](char *h) {
@@ -1998,6 +2017,18 @@ int fadegpu_align_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regio
     };
     sc.reference = [&](fadegpu_batch *, RefDev *ref, int *) -> int { *ref = ref_dev(c); return 0; };
     return align_staged(c, sc, out, ops_out, stats_out, t_begin);
+}
+
+int fadegpu_align_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regions *in, int32_t max_ops,
+                          fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+{
+    return regions_call(c, "fadegpu_align_regions", false, n_regions, in, max_ops, out, ops_out, stats_out);
+}
+
+int fadegpu_score_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regions *in, fadegpu_pair_result *out,
+                          fadegpu_stats *stats_out)
+{
+    return regions_call(c, "fadegpu_score_regions", true, n_regions, in, 0, out, nullptr, stats_out);
 }
 
 int fadegpu_measure_alu_peak(fadegpu_ctx *c, double *ops_per_sec_out, double *sm_clock_mhz_out)

@@ -352,8 +352,9 @@ struct AdvanceSmem {
 static_assert(sizeof(LaneCtl) % 4 == 0 && sizeof(AlnOut) % 4 == 0, "word-copyable");
 
 // SPILL: the launch may carry a full-CIGAR spill ring (a.ops_spill, checked at run time); without it the walker is
-// compiled exactly as for the annotate path
-template <int R, bool SPILL>
+// compiled exactly as for the annotate path.  END_ONLY (score-only calls): an alignment is done once its end cell is
+// selected -- no walk, no traced replay requested, a finalize_end record.
+template <int R, bool SPILL, bool END_ONLY = false>
 __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, unsigned warp0, unsigned nwarps,
                                               AdvanceSmem *smem_all)
 {
@@ -386,6 +387,9 @@ __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, un
         if (l == 0) {
             c.cur_blk = c.next_blk;
             if (c.phase == 0 && !ctl_select_end<R>(c)) go = 0;
+            if constexpr (END_ONLY) {
+                if (go) { c.phase = 2; c.next_blk = -1; go = 0; }
+            }
         }
         go = __shfl_sync(FULL, go, 0);
         __syncwarp();
@@ -533,8 +537,10 @@ __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, un
         __syncwarp();
         const bool fin = c.phase == 2;
         if (l == 0) {
-            if (fin) finalize_result(c, sm.out, d.read, d.clip_left, d.clip_right, a.min_length);
-            else if (round + 1 < a.max_rounds) {
+            if (fin) {
+                if constexpr (END_ONLY) finalize_end(c, sm.out, d.read);
+                else finalize_result(c, sm.out, d.read, d.clip_left, d.clip_right, a.min_length);
+            } else if (round + 1 < a.max_rounds) {
                 const unsigned slot = atomicAdd(&a.qcount[rin ^ 1], 1u);
                 a.queue[rin ^ 1][slot] = pack_req(aln, c.next_blk, ctl_scanmask(c));
             }   // else: out[aln] keeps its "no result" marker and fadegpu_wait reports the error
@@ -553,11 +559,11 @@ __device__ __forceinline__ void advance_round(const KernelArgs &a, int round, un
     }
 }
 
-template <int R, bool SPILL>
+template <int R, bool SPILL, bool END_ONLY = false>
 __global__ void FADE_SMALL_KERNEL trace_advance_kernel(const KernelArgs a)
 {
     __shared__ AdvanceSmem adv[4];
-    advance_round<R, SPILL>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5), adv);
+    advance_round<R, SPILL, END_ONLY>(a, a.round, blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), gridDim.x * (blockDim.x >> 5), adv);
 }
 
 // The few alignments still unfinished after the full-grid rounds (very long paths): one block
@@ -1152,6 +1158,27 @@ __global__ void FADE_SMALL_KERNEL pair_results_kernel(const AlnDesc *aln, const 
     if ((threadIdx.x & 31) == 0 && ok) atomicAdd(n_ok, (unsigned long long)ok);
 }
 
+// score-only calls: the same, without the begin cell and the CIGAR (the generic kernel's are dropped here)
+__global__ void FADE_SMALL_KERNEL pair_score_results_kernel(const AlnOut *out, int n_aln, int64_t n, PairResult *res,
+                                                            unsigned long long *n_ok)
+{
+    int ok = 0;
+    for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < n_aln; idx += gridDim.x * blockDim.x) {
+        const AlnOut o = out[idx];
+        const int64_t k = o.read;
+        if (k < 0 || k >= n || !(o.flags & R_ALIGNED) || (o.flags & 0x80000000u)) continue;
+        ++ok;
+        PairResult r;
+        r.score = o.score; r.end_query = o.end_query; r.end_ref = o.end_ref;
+        r.beg_query = r.beg_ref = r.n_ops = 0;
+        r.flags = o.flags & (R_ALIGNED | R_GENERIC);
+        r.reserved = 0;
+        res[k] = r;
+    }
+    ok = __reduce_add_sync(FULL, ok);
+    if ((threadIdx.x & 31) == 0 && ok) atomicAdd(n_ok, (unsigned long long)ok);
+}
+
 // ------------------------------------------------------------------------------------------------
 // INT16x2 ALU issue-rate microbenchmark: 8 independent VIADDMNMX.S16x2 chains per thread
 // ------------------------------------------------------------------------------------------------
@@ -1242,9 +1269,38 @@ static cudaError_t launch_trace_tt(KernelArgs a, cudaStream_t s, int sm_count, i
     return cudaGetLastError();
 }
 
-template <int R>
-static cudaError_t launch_trace_t(const KernelArgs &a, cudaStream_t s, int sm_count, int *launches)
+// Score-only calls: trace_init_kernel as above, then rounds of scan-only replays (MODE 2, no trace tile) and advances
+// that stop at the end cell.  Each round scans one candidate block of every unfinished alignment and marks every
+// candidate thread whose maximum was first reached in it; an alignment has at most FG candidate threads, so FG rounds
+// finish all of them and no tail kernel is needed.
+template <int R, int STEP>
+static cudaError_t launch_end_scan_ts(KernelArgs a, cudaStream_t s, int sm_count, int *launches)
 {
+    const int n = a.n_aln;
+    trace_init_kernel<R><<<std::min((n + 127) / 128, sm_count * 8), 128, 0, s>>>(a);
+    const int quads = (n + 7) / 8;
+    a.max_rounds = FG;   // an alignment left after them keeps its "no result" marker, and the call reports it
+    for (int r = 0; r < a.max_rounds; ++r) {
+        a.round = r;
+        const int g1 = std::min((quads + 3) / 4, r < 3 ? sm_count * 4 : sm_count);
+        const int g2 = std::min((n + 3) / 4, r < 3 ? sm_count * 16 : sm_count * 2);
+        trace_replay_kernel<R, 2, STEP><<<std::max(g1, 1), 128, 0, s>>>(a);
+        trace_advance_kernel<R, false, true><<<std::max(g2, 1), 128, 0, s>>>(a);
+    }
+    if (launches) *launches += 1 + 2 * a.max_rounds;
+    return cudaGetLastError();
+}
+
+template <int R>
+static cudaError_t launch_trace_t(const KernelArgs &a, bool end_only, cudaStream_t s, int sm_count, int *launches)
+{
+    if (end_only) {
+        switch (score_step_for(a.k)) {
+        case 2: return launch_end_scan_ts<R, 2>(a, s, sm_count, launches);
+        case 1: return launch_end_scan_ts<R, 1>(a, s, sm_count, launches);
+        default: return launch_end_scan_ts<R, 0>(a, s, sm_count, launches);
+        }
+    }
     return a.k.tagged_ok ? launch_trace_tt<R, true>(a, s, sm_count, launches)
                          : launch_trace_tt<R, false>(a, s, sm_count, launches);
 }
@@ -1262,15 +1318,15 @@ cudaError_t launch_fill(int R, const KernelArgs &a, cudaStream_t s)
     }
 }
 
-cudaError_t launch_trace(int R, const KernelArgs &a, cudaStream_t s, int sm_count, int *launches)
+cudaError_t launch_trace(int R, const KernelArgs &a, bool end_only, cudaStream_t s, int sm_count, int *launches)
 {
     if (a.n_items <= 0) return cudaSuccess;
     switch (R) {
-    case 13: return launch_trace_t<13>(a, s, sm_count, launches);
-    case 19: return launch_trace_t<19>(a, s, sm_count, launches);
-    case 25: return launch_trace_t<25>(a, s, sm_count, launches);
-    case 32: return launch_trace_t<32>(a, s, sm_count, launches);
-    case 38: return launch_trace_t<38>(a, s, sm_count, launches);
+    case 13: return launch_trace_t<13>(a, end_only, s, sm_count, launches);
+    case 19: return launch_trace_t<19>(a, end_only, s, sm_count, launches);
+    case 25: return launch_trace_t<25>(a, end_only, s, sm_count, launches);
+    case 32: return launch_trace_t<32>(a, end_only, s, sm_count, launches);
+    case 38: return launch_trace_t<38>(a, end_only, s, sm_count, launches);
     default: return cudaErrorInvalidValue;
     }
 }
@@ -1360,13 +1416,16 @@ cudaError_t launch_region_prep(const RegionArgs &a, int sm_count, cudaStream_t s
 }
 
 cudaError_t launch_pair_results(int64_t n, const int64_t *qoff, const int64_t *t_beg, const int64_t *t_end,
-                                const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill, int max_ops,
-                                PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count, cudaStream_t s)
+                                const AlnDesc *aln, const AlnOut *out, int n_aln, bool score_only, const uint32_t *spill,
+                                int max_ops, PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count,
+                                cudaStream_t s)
 {
     if (n <= 0) return cudaSuccess;
     pair_results_init_kernel<<<(int)std::min<int64_t>((n + 127) / 128, (int64_t)sm_count * 16), 128, 0, s>>>(n, qoff, t_beg,
                                                                                                              t_end, res);
-    if (n_aln > 0)
+    if (n_aln > 0 && score_only)
+        pair_score_results_kernel<<<std::min((n_aln + 127) / 128, sm_count * 16), 128, 0, s>>>(out, n_aln, n, res, n_ok);
+    else if (n_aln > 0)
         pair_results_kernel<<<std::min((n_aln + 127) / 128, sm_count * 16), 128, 0, s>>>(aln, out, n_aln, n, spill, max_ops,
                                                                                        res, ops, n_ok);
     return cudaGetLastError();

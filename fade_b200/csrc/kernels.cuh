@@ -6,7 +6,7 @@
 //   sw_generic_kernel    exact int32 fallback ON THE DEVICE for wildcard letters and sizes the
 //                        packed kernels do not cover (thread per alignment)
 //   pair_*_kernel        fadegpu_align_pairs: pack caller-supplied ASCII pairs into the read / reference formats
-//                        above, and put the records back into pair order (also for regions)
+//                        above, and put the records back into pair order (also for regions and the score-only calls)
 //   region_prep_kernel   fadegpu_align_regions: pack caller-supplied queries against intervals of the reference
 //   alu_peak_kernel      INT16x2 ALU issue-rate microbenchmark (roofline denominator)
 //
@@ -174,16 +174,17 @@ struct RegionArgs {
 cudaError_t launch_region_prep(const RegionArgs &a, int sm_count, cudaStream_t s);
 // item-ordered result records (pairs or regions): zeros (or FADEGPU_R_OVERSIZE) for every item k, whose query is
 // qoff[k] .. qoff[k+1] and whose window spans t_beg[k] .. t_end[k] (pairs: toff, toff + 1; regions: start, end), then
-// the records of the alignments with their full forward CIGARs assembled from the spill rings; n_ok counts the records
-// the SW kernels produced
+// the records of the alignments with their full forward CIGARs assembled from the spill rings (score_only: score and end
+// cell only, no spill rings, max_ops = 0); n_ok counts the records the SW kernels produced
 struct PairResult {   // == fadegpu_pair_result
     int32_t score, end_query, end_ref, beg_query, beg_ref, n_ops;
     uint32_t flags;
     int32_t reserved;
 };
 cudaError_t launch_pair_results(int64_t n, const int64_t *qoff, const int64_t *t_beg, const int64_t *t_end,
-                                const AlnDesc *aln, const AlnOut *out, int n_aln, const uint32_t *spill, int max_ops,
-                                PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count, cudaStream_t s);
+                                const AlnDesc *aln, const AlnOut *out, int n_aln, bool score_only, const uint32_t *spill,
+                                int max_ops, PairResult *res, uint32_t *ops, unsigned long long *n_ok, int sm_count,
+                                cudaStream_t s);
 
 constexpr int FILL_THREADS = 128;
 constexpr int OVER_CAP = 256;        // oversize reads listed per batch (all of them are counted)
@@ -233,7 +234,8 @@ cudaError_t launch_seq_pull(const uint8_t *host_seq4, const AlnDesc *aln, const 
 cudaError_t launch_result_index(const AlnOut *out, int n_aln, int64_t n_reads, uint8_t *flags, int32_t *ridx, unsigned long long *n_ok,
                                 int sm_count, cudaStream_t s);
 cudaError_t launch_fill(int R, const KernelArgs &a, cudaStream_t s);
-cudaError_t launch_trace(int R, const KernelArgs &a, cudaStream_t s, int sm_count, int *launches);
+// end_only (score-only calls): scan-only rounds that stop at the end cell, no traceback
+cudaError_t launch_trace(int R, const KernelArgs &a, bool end_only, cudaStream_t s, int sm_count, int *launches);
 cudaError_t launch_generic(const GenericArgs &a, int n_slots, cudaStream_t s);
 cudaError_t launch_alu_peak(uint32_t *out, int iters, int blocks, int threads, cudaStream_t s);
 

@@ -658,13 +658,15 @@ FD bool ctl_select_end(LaneCtl &c)
 // spill (optional): a second ring of `spill_cap` words in global storage that receives every op the walker completes,
 // at ring[nrev % spill_cap], so that CIGARs longer than OPS_CAP can be assembled in full (fadegpu_align_pairs).
 // c.ring is written as before either way.
+// end_only (fadegpu_score_pairs / _regions): the alignment is done once its end cell is selected; no walk (finalize_end).
 template <int R, class Acc>
 FD void ctl_advance(LaneCtl &c, const uint32_t *tile, int lane, const Acc &acc, const SwConsts &k,
-                    uint32_t *spill = nullptr, int spill_cap = 0)
+                    uint32_t *spill = nullptr, int spill_cap = 0, bool end_only = false)
 {
     if (c.phase == 2) return;
     c.cur_blk = c.next_blk;
     if (c.phase == 0 && !ctl_select_end<R>(c)) return;
+    if (end_only) { c.phase = 2; c.next_blk = -1; return; }
     // P4: walk while the current cell lies in the replayed block (hot fields in registers)
     int i = c.i, j = c.j, mode = c.mode, hval = c.hval, gval = c.gval, nrev = c.nrev;
     uint32_t cur = c.cur;
@@ -837,6 +839,20 @@ FD void finalize_result(const LaneCtl &c, AlnOut &o, int read, uint32_t clip_lef
     if (accept_side(true, c.S, n, first_op, last_op, lead, trail, clip_left, min_length)) flags |= R_ART_LEFT;
     if (accept_side(false, c.S, n, first_op, last_op, lead, trail, clip_right, min_length)) flags |= R_ART_RIGHT;
     o.flags = flags;
+}
+
+// Score-only record (fadegpu_score_pairs / _regions): the score and the end cell P3 selected, no begin cell and no
+// CIGAR.  Equal, field for field, to what finalize_result writes for score and end cell.
+FD void finalize_end(const LaneCtl &c, AlnOut &o, int read)
+{
+    o.read = read;
+    o.score = c.S;
+    o.end_query = c.S > 0 ? c.end_i : 0;
+    o.end_ref = c.S > 0 ? c.end_j : 0;
+    o.beg_query = o.beg_ref = 0;
+    o.n_ops = 0;
+    o.flags = R_ALIGNED;
+    for (int k = 0; k < OPS_CAP; ++k) o.ops[k] = 0;
 }
 
 }  // namespace fade

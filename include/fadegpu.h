@@ -321,6 +321,30 @@ typedef struct fadegpu_regions {
 int fadegpu_align_regions(fadegpu_ctx *ctx, int64_t n_regions, const fadegpu_regions *in, int32_t max_ops,
                           fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out);
 
+/* ---- Score-only Smith-Waterman of pairs and regions: score and end cell, no traceback ----
+ * fadegpu_score_pairs / fadegpu_score_regions take exactly the inputs of fadegpu_align_pairs / fadegpu_align_regions
+ * (without max_ops and ops_out) and validate them the same way: the same letter rules, the same FADEGPU_E_ARG cases and
+ * messages naming the first offending pair or region (with the calling function's name), FADEGPU_E_STATE while a batch
+ * of the ctx is in flight and, for regions, when no reference is loaded.  The ctx's scoring and FADEGPU_F_FORCE_GENERIC
+ * apply, FADEGPU_F_TAGS_ONLY does not, and FADEGPU_F_NO_SHORTCUT changes no record.
+ *
+ * Records, in PAIR / REGION ORDER: score, end_query and end_ref equal, field for field, those of the traced call on the
+ *   same input (P1-P3: the end cell is the first column, then the first row, holding the score); beg_query, beg_ref and
+ *   n_ops are 0; flags hold only ALIGNED | GENERIC | OVERSIZE (FADEGPU_R_SCORE_ONLY keeps its annotate meaning and is
+ *   not set).  Empty items give flags = 0 and a zero record; oversize items are not aligned, get FADEGPU_R_OVERSIZE and
+ *   are counted in stats_out->n_oversize, as in the traced calls.
+ * What it saves: the traceback rounds after the end cell is found (no traced block replay, no walk), the CIGAR spill
+ *   and the ops copy home.
+ * No side effects on batches: waited batches keep their results, and fadegpu_replay_kernels / fadegpu_replay_batches
+ *   keep working.
+ *
+ * Synchronous; host arrays, only read during the call.  stats_out (may be NULL) receives the fields the traced calls
+ * fill; d2h_bytes counts the 32-byte records and the binning histogram, no ops. */
+int fadegpu_score_pairs(fadegpu_ctx *ctx, int64_t n_pairs, const fadegpu_pairs *in,
+                        fadegpu_pair_result *out, fadegpu_stats *stats_out);
+int fadegpu_score_regions(fadegpu_ctx *ctx, int64_t n_regions, const fadegpu_regions *in,
+                          fadegpu_pair_result *out, fadegpu_stats *stats_out);
+
 /* INT16x2 ALU roofline denominator (SURVEY 8d): measures packed VIMNMX/VIADDMNMX issue rate.
  * ops_per_sec_out = packed (2-lane) instructions * 32 threads per second over the whole GPU. */
 int fadegpu_measure_alu_peak(fadegpu_ctx *ctx, double *ops_per_sec_out, double *sm_clock_mhz_out);

@@ -1,5 +1,5 @@
-"""Throughput of fadegpu_align_regions on read-shaped regions, beside fadegpu_align_pairs and the annotate path on the
-same alignments.
+"""Throughput of fadegpu_align_regions on read-shaped regions, beside fadegpu_align_pairs, the score-only calls
+(fadegpu_score_regions / fadegpu_score_pairs) and the annotate path on the same alignments.
 
 The alignments are those of BASELINE configs[1] (c2), as in tools/pairs_bench.py: the first --reads simulated 2x150
 reads against the synthetic 100 Mbp chromosome (seeds as bench.py), and for every read the annotate path aligns, its
@@ -7,10 +7,13 @@ forward letters on strand 1 against its window [win_start, window end) of the re
 of the same reads is submitted and waited for; then, --rounds times in alternation:
   * regions: one Context.align_regions call from host arrays to host results (wall clock), with its kernel ms (the SW
     kernels), total device ms, H2D / D2H bytes and launches from the call's stats;
+  * score_regions: the same for one Context.score_regions call on the same inputs (score and end cell, no traceback);
   * pairs: the same for one Context.align_pairs call on (RC(read), window letters);
+  * score_pairs: the same for one Context.score_pairs call on those pairs;
   * batch: fadegpu_replay_kernels of the annotate batch (binning + the same SW kernels, nothing copied).
-Every round checks that the region and pair records equal each other and the annotate batch's.  The card's name,
-power limit and SM clock are printed beside the numbers.
+Every round checks that the region and pair records equal each other and the annotate batch's, and that the score-only
+legs' score, end_query and end_ref equal their traced legs'.  The card's name, power limit and SM clock are printed
+beside the numbers.
 
     python tools/regions_bench.py [--reads 1000000] [--max-ops 32]
 """
@@ -80,15 +83,25 @@ def main():
         def pairs():
             return ctx.align_pairs(q, t, a.max_ops, query_offsets=qo, target_offsets=to)
 
-        reg, pr = regions(), pairs()                                                          # warm-up
+        def score_regions():
+            return ctx.score_regions(rq, tids, starts, ends, strands, query_offsets=rqo)
+
+        def score_pairs():
+            return ctx.score_pairs(q, t, query_offsets=qo, target_offsets=to)
+
+        def timed(name, rnd, call):
+            t1 = time.perf_counter()
+            res = call()
+            line(name, rnd, n, time.perf_counter() - t1, res.stats)
+            return res
+
+        reg, pr, sreg, spr = regions(), pairs(), score_regions(), score_pairs()               # warm-up
         b.replay_kernels(1)
         for rnd in range(a.rounds):
-            t1 = time.perf_counter()
-            reg = regions()
-            line("regions", rnd, n, time.perf_counter() - t1, reg.stats)
-            t1 = time.perf_counter()
-            pr = pairs()
-            line("pairs", rnd, n, time.perf_counter() - t1, pr.stats)
+            reg = timed("regions", rnd, regions)
+            sreg = timed("score_regions", rnd, score_regions)
+            pr = timed("pairs", rnd, pairs)
+            spr = timed("score_pairs", rnd, score_pairs)
             ms = b.replay_kernels(a.replay_iters) / a.replay_iters
             bst = b.stats()
             print(f"round {rnd} batch: replay_kernels {ms:.3f} ms per pass ({bst.cells / (ms * 1e6):.1f} GCUPS, "
@@ -97,6 +110,10 @@ def main():
             same_batch = all(np.array_equal(reg.records[f], getattr(b, f)[al]) for f in FIELDS)
             print(f"round {rnd} records: regions == pairs (records and ops): {same_pairs}; "
                   f"regions == annotate batch ({', '.join(FIELDS)}): {same_batch}")
+            same_score = [all(np.array_equal(s.records[f], tr.records[f]) for f in ("score", "end_query", "end_ref"))
+                          for s, tr in ((sreg, reg), (spr, pr))]
+            print(f"round {rnd} score-only records (score, end_query, end_ref): score_regions == regions: "
+                  f"{same_score[0]}; score_pairs == pairs: {same_score[1]}")
         b.close()
 
 
