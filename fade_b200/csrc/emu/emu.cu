@@ -106,7 +106,7 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
     // bit 5 of `tagged`: score-only calls -- every replay is a scan with the score-only step (no trace), the walkers stop
     // at the end cell; scan_info[2 L ..] receives lane L's number of scan replays and its first candidate block
     const bool end_only = (tagged & 32) != 0;
-    const bool tg = !end_only && (tagged & 1) && k.tagged_ok;
+    const bool tg_trace = !end_only && (tagged & 1) && k.tagged_ok;
     int32_t scans[2] = { 0, 0 }, first_blk[2];
     for (int L = 0; L < 2; ++L) first_blk[L] = ctl[L].phase == 0 ? ctl[L].next_blk : -1;
     // ops_cap > 0: the walkers also spill every op into rings of ops_cap words, as the device does for
@@ -118,6 +118,10 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
     bool first_iter = true;
     while (ctl[0].phase != 2 || ctl[1].phase != 2) {
         if (++guard > 4 * nblk + 16) return -2;
+        // bit 2 of `tagged`: the first replay is a scan with the score-only step in the plain / fp16 domain and records
+        // no trace, like round 0 on the device (trace_replay_kernel<R, 2, STEP>)
+        const bool scan_only = end_only || ((tagged & 4) && first_iter);
+        const bool tg = tg_trace && !scan_only;
         int blk[2];
         for (int L = 0; L < 2; ++L) blk[L] = (ctl[L].phase != 2 && ctl[L].next_blk >= 0) ? ctl[L].next_blk : 0;
         bool scan[2][FG];
@@ -157,7 +161,7 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
                 const uint32_t ts = (tw[t0 - g + FG] & 0x00ffu) | (tw[t1 - g + FG] & 0xff00u);
                 uint32_t cmax = 0;
                 uint32_t trw[RW];
-                if (end_only) {
+                if (scan_only) {
                     if (step == 2) score_step<R, 2>(st[g].H, st[g].E, st[g].qp, cmax, ts, st[g].hu_prev, fin[g], st[g].fout, k);
                     else if (step == 1) score_step<R, 1>(st[g].H, st[g].E, st[g].qf, cmax, ts, st[g].hu_prev, fin[g], st[g].fout, k);
                     else score_step<R, 0>(st[g].H, st[g].E, st[g].qs, cmax, ts, st[g].hu_prev, fin[g], st[g].fout, k);
@@ -186,12 +190,10 @@ int align_pair(const uint8_t *qa, int qlen_a, const uint8_t *ta, int tlen_a,
         for (int L = 0; L < 2; ++L)
             for (int g = 0; g < FG; ++g)
                 if (scan[L][g] && !found[L][g]) return -3;  // a candidate must find its cell
-        // bit 2 of `tagged`: the first (scan) replay of a lane records no trace, like round 0 on the device
-        const bool so0 = end_only || ((tagged & 4) && ctl[0].phase == 0 && first_iter);
-        const bool so1 = end_only || ((tagged & 4) && ctl[1].phase == 0 && first_iter);
         for (int L = 0; L < 2; ++L) scans[L] += ctl[L].phase == 0;
-        ctl_advance<R>(ctl[0], so0 ? nullptr : tr.data(), 0, StagedAcc{ tw.data(), qc.data(), 0 }, k, sp0, ops_cap, end_only);
-        ctl_advance<R>(ctl[1], so1 ? nullptr : tr.data(), 1, StagedAcc{ tw.data(), qc.data(), 1 }, k, sp1, ops_cap, end_only);
+        const uint32_t *tile = scan_only ? nullptr : tr.data();
+        ctl_advance<R>(ctl[0], tile, 0, StagedAcc{ tw.data(), qc.data(), 0 }, k, sp0, ops_cap, end_only);
+        ctl_advance<R>(ctl[1], tile, 1, StagedAcc{ tw.data(), qc.data(), 1 }, k, sp1, ops_cap, end_only);
         first_iter = false;
     }
     if (scan_info)
@@ -284,6 +286,7 @@ extern "C" int fadeemu_comp_code_of_nt16(int nib) { return comp_code_of_nt16(nib
 extern "C" uint32_t fadeemu_prmt(uint32_t a, uint32_t b, uint32_t s) { return prmt_sx(a, b, s); }
 extern "C" int fadeemu_sizeof_alnout(void) { return (int)sizeof(AlnOut); }
 extern "C" int fadeemu_f16_ok(int open, int extend, int match, int mismatch) { return make_consts(open, extend, match, mismatch).f16_ok; }
+extern "C" int fadeemu_tagged_ok(int open, int extend, int match, int mismatch) { return make_consts(open, extend, match, mismatch).tagged_ok; }
 // make_consts' choice for fill_step_f16x2: out = { f16_pair_ok, high byte of match, of mismatch, IMAD addend c }
 extern "C" void fadeemu_f16_pair(int open, int extend, int match, int mismatch, uint32_t *out)
 {

@@ -218,8 +218,12 @@ FD SwConsts make_consts(int open, int extend, int match, int mismatch)
     k.neg_o = no | (no << 16);
     k.neg_e = ne | (ne << 16);
     k.open = open; k.extend = extend; k.match = match; k.mismatch = mismatch;
+    // The tagged recorder needs its DIAG candidates 16*s + 8 as signed LUT bytes, 16*(-open - extend) + 2 in an int16
+    // lane, and 16*H + 15 in an int16 lane for every H of the tallest packed query (FG * 38 rows): H <= match * 304 <=
+    // 2047.  Past that bound (match >= 7) 16*H wraps on queries of 2048 / match rows or more, so the plain recorder
+    // (MODE 1) takes the scoring.
     const int tm = 16 * match + 8, tx = 16 * mismatch + 8;
-    k.tagged_ok = (tm <= 127 && tx >= -128 && open <= 1000) ? 1 : 0;
+    k.tagged_ok = (tm <= 127 && tx >= -128 && open <= 1000 && match * FG * 38 <= 2047) ? 1 : 0;
     const uint32_t bm = (uint32_t)(tm & 0xff), bx = (uint32_t)(tx & 0xff);
     k.tlut0 = bm | (bx << 8) | (bx << 16) | (bx << 24);
     k.tlut1 = bx | (bx << 8) | (bx << 16) | (bx << 24);

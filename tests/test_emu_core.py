@@ -58,7 +58,9 @@ def got(x):
             [x.ops[k] for k in range(min(x.n_ops, E.OPS_CAP))])
 
 
-@pytest.mark.parametrize("tagged", [1, 0, 3, 2, 5])   # bit 0: tagged trace, 1: no diagonal shortcut, 2: scan-only first replay
+# bit 0: tagged trace, 1: no diagonal shortcut, 2: the first replay scans with the score-only step and records no trace
+# (round 0 on the device)
+@pytest.mark.parametrize("tagged", [1, 0, 3, 2, 5])
 @pytest.mark.parametrize("R,maxq,maxt,iters", [(1, 8, 40, 300), (2, 16, 90, 300), (3, 24, 120, 200),
                                                (5, 40, 200, 120), (13, 104, 300, 40), (19, 152, 400, 40),
                                                (25, 200, 400, 10), (32, 256, 500, 12), (38, 304, 500, 8)])
