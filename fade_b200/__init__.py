@@ -6,5 +6,5 @@ mirrors the reference's `annotate` loop (source/anno.d:16-110) on top of the C A
 CPU fallback: importing works anywhere, computing needs the built library and a CUDA device.
 """
 from ._lib import FadeGpuError, build, lib, lib_path  # noqa: F401
-from .api import (Batch, Context, Params, Record, annotate_records, default_params,  # noqa: F401
+from .api import (Batch, Context, Job, Params, Record, annotate_records, default_params,  # noqa: F401
                   MAX_OPS, PairResults, PAIR_RESULT_DTYPE, ScoreResults)

@@ -93,6 +93,12 @@ class PairResult(C.Structure):
                 ("beg_ref", C.c_int32), ("n_ops", C.c_int32), ("flags", C.c_uint32), ("reserved", C.c_int32)]
 
 
+class JobResults(C.Structure):
+    """fadegpu_job_results: the records and ops of a waited job, in pinned memory the job owns"""
+    _fields_ = [("n", C.c_int64), ("records", C.c_void_p), ("ops", C.c_void_p), ("max_ops", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 class HostRecord(C.Structure):
     _fields_ = [("flag", C.c_int32), ("has_sa", C.c_int32), ("cigar", C.POINTER(C.c_uint32)),
                 ("n_cigar", C.c_int32), ("seq4", C.POINTER(C.c_uint8)), ("qual", C.POINTER(C.c_uint8)),
@@ -106,6 +112,8 @@ ABI_SYMBOLS = [
     "fadegpu_reference_info", "fadegpu_alloc_batch", "fadegpu_get_batch_view", "fadegpu_free_batch",
     "fadegpu_submit", "fadegpu_submit_compact", "fadegpu_submit_inputs", "fadegpu_wait", "fadegpu_get_results", "fadegpu_get_stats", "fadegpu_get_timeline", "fadegpu_replay_kernels", "fadegpu_replay_batches",
     "fadegpu_align_pairs", "fadegpu_align_regions", "fadegpu_score_pairs", "fadegpu_score_regions",
+    "fadegpu_job_create", "fadegpu_job_destroy", "fadegpu_submit_pairs", "fadegpu_submit_regions", "fadegpu_job_wait",
+    "fadegpu_job_results_view",
     "fadegpu_measure_alu_peak",
     "fadehost_parse_clips", "fadehost_aligned_length", "fadehost_prepare", "fadehost_finish",
 ]
@@ -149,6 +157,13 @@ def lib():
     L.fadegpu_align_regions.argtypes = [vp, i64, C.POINTER(RegionsIn), i32, vp, vp, C.POINTER(Stats)]
     L.fadegpu_score_pairs.argtypes = [vp, i64, C.POINTER(PairsIn), vp, C.POINTER(Stats)]
     L.fadegpu_score_regions.argtypes = [vp, i64, C.POINTER(RegionsIn), vp, C.POINTER(Stats)]
+    L.fadegpu_job_create.argtypes = [vp, C.POINTER(vp)]
+    L.fadegpu_job_destroy.argtypes = [vp]
+    L.fadegpu_job_destroy.restype = None
+    L.fadegpu_submit_pairs.argtypes = [vp, vp, i64, C.POINTER(PairsIn), i32, C.c_uint32]
+    L.fadegpu_submit_regions.argtypes = [vp, vp, i64, C.POINTER(RegionsIn), i32, C.c_uint32]
+    L.fadegpu_job_wait.argtypes = [vp, vp, C.POINTER(Stats)]
+    L.fadegpu_job_results_view.argtypes = [vp, C.POINTER(JobResults)]
     L.fadegpu_measure_alu_peak.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.fadehost_parse_clips.argtypes = [C.POINTER(C.c_uint32), i32, C.POINTER(C.c_uint32)]
     L.fadehost_parse_clips.restype = None

@@ -8,8 +8,8 @@ from dataclasses import dataclass, field
 
 import numpy as np
 
-from ._lib import (BatchView, FadeGpuError, HostRecord, Inputs, PairResult, PairsIn, Params, RegionsIn, Result,
-                   ResultsView, Stats, lib)
+from ._lib import (BatchView, FadeGpuError, HostRecord, Inputs, JobResults, PairResult, PairsIn, Params, RegionsIn,
+                   Result, ResultsView, Stats, lib)
 
 MAX_OPS = 10
 R_ALIGNED, R_ART_LEFT, R_ART_RIGHT, R_OPS_TRUNC, R_GENERIC, R_OVERSIZE, R_SCORE_ONLY = 1, 2, 4, 8, 16, 32, 64
@@ -19,6 +19,7 @@ F_TAGS_ONLY = 4
 F_NO_SHORTCUT = 8
 F_HOST_BINNING = 16
 F_SYNC_SUBMIT = 32
+JOB_SCORE_ONLY = 1
 RESULT_DTYPE = np.dtype([("score", "<i4"), ("end_query", "<i4"), ("end_ref", "<i4"), ("beg_query", "<i4"),
                          ("beg_ref", "<i4"), ("n_ops", "<i4"), ("flags", "<u4"), ("read", "<i4"),
                          ("ops", "<u4", (MAX_OPS,))])
@@ -156,6 +157,7 @@ class Context:
         self.device = device
         self.contig_names: list[str] = []
         self._batches = weakref.WeakSet()      # freed before the ctx: a batch must not outlive it
+        self._jobs = weakref.WeakSet()         # the same for jobs
 
     def _check(self, rc: int):
         if rc:
@@ -262,6 +264,25 @@ class Context:
         self._check(lib().fadegpu_score_regions(self._h, n, C.byref(rin), rec.ctypes.data, C.byref(st)))
         return ScoreResults(rec, st)
 
+    def submit_pairs(self, queries, targets, max_ops: int | None = None, *, score_only: bool = False,
+                     query_offsets=None, target_offsets=None) -> "Job":
+        """fadegpu_submit_pairs on a new job: align_pairs (score_pairs with score_only=True) that returns once the
+        inputs are copied; the kernels run while the caller goes on, and Job.wait() gives the call's results"""
+        return self._new_job(_pairs_job(queries, targets, max_ops, score_only, query_offsets, target_offsets))
+
+    def submit_regions(self, queries, tids, starts, ends, strands=None, max_ops: int | None = None, *,
+                       score_only: bool = False, query_offsets=None) -> "Job":
+        """fadegpu_submit_regions on a new job: align_regions (score_regions with score_only=True); see submit_pairs"""
+        return self._new_job(_regions_job(queries, tids, starts, ends, strands, max_ops, score_only, query_offsets))
+
+    def _new_job(self, call) -> "Job":
+        job = Job(self)
+        try:
+            return job._submit(call)
+        except BaseException:
+            job.close()
+            raise
+
     def alloc_batch(self, max_reads: int, max_seq_bytes: int) -> "Batch":
         return Batch(self, max_reads, max_seq_bytes)
 
@@ -269,7 +290,94 @@ class Context:
         if self._h:
             for b in list(self._batches):
                 b.close()
+            for j in list(self._jobs):
+                j.close()
             lib().fadegpu_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _job_max_ops(qo, max_ops, score_only: bool) -> int:
+    if score_only:
+        if max_ops:
+            raise ValueError("a score-only job has no CIGAR: max_ops must be 0 or None")
+        return 0
+    return default_max_ops(qo) if max_ops is None else max_ops
+
+
+def _pairs_job(queries, targets, max_ops, score_only, query_offsets, target_offsets):
+    """the packed and validated arguments of fadegpu_submit_pairs (and the arrays they point into)"""
+    q, qo, t, to = pack_pairs(queries, targets, query_offsets, target_offsets)
+    max_ops = _job_max_ops(qo, max_ops, score_only)
+    pin = PairsIn(q.ctypes.data, qo.ctypes.data, t.ctypes.data, to.ctypes.data)
+    return "fadegpu_submit_pairs", len(qo) - 1, pin, max_ops, score_only, (q, qo, t, to)
+
+
+def _regions_job(queries, tids, starts, ends, strands, max_ops, score_only, query_offsets):
+    q, qo, tid, start, end, strand = pack_regions(queries, tids, starts, ends, strands, query_offsets)
+    max_ops = _job_max_ops(qo, max_ops, score_only)
+    rin = RegionsIn(q.ctypes.data, qo.ctypes.data, tid.ctypes.data, start.ctypes.data, end.ctypes.data,
+                    strand.ctypes.data)
+    return "fadegpu_submit_regions", len(qo) - 1, rin, max_ops, score_only, (q, qo, tid, start, end, strand)
+
+
+class Job:
+    """One pair or region call in flight (Context.submit_pairs / submit_regions).  wait() gives what the synchronous
+    call would have returned: PairResults, or ScoreResults for a score-only job.  A job can be closed before it is
+    waited for (close waits for it); the ctx closes its jobs when it is closed."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        self._h = C.c_void_p()
+        ctx._check(lib().fadegpu_job_create(ctx._h, C.byref(self._h)))
+        ctx._jobs.add(self)
+        self.score_only = False
+
+    def submit_pairs(self, queries, targets, max_ops: int | None = None, *, score_only: bool = False,
+                     query_offsets=None, target_offsets=None) -> "Job":
+        """fadegpu_submit_pairs: inputs and max_ops as in Context.align_pairs (max_ops defaults to 3 * the longest
+        query, and must be 0 or None with score_only).  A job is reused once waited for: its buffers grow with use."""
+        return self._submit(_pairs_job(queries, targets, max_ops, score_only, query_offsets, target_offsets))
+
+    def submit_regions(self, queries, tids, starts, ends, strands=None, max_ops: int | None = None, *,
+                       score_only: bool = False, query_offsets=None) -> "Job":
+        """fadegpu_submit_regions: inputs and max_ops as in Context.align_regions; see submit_pairs"""
+        return self._submit(_regions_job(queries, tids, starts, ends, strands, max_ops, score_only, query_offsets))
+
+    def _submit(self, call) -> "Job":
+        fn, n, inp, max_ops, score_only, _arrays = call     # (the arrays are read during the call only)
+        self.ctx._check(getattr(lib(), fn)(self.ctx._h, self._h, n, C.byref(inp), max_ops,
+                                           JOB_SCORE_ONLY if score_only else 0))
+        self.score_only = score_only
+        return self
+
+    def wait(self):
+        st = Stats()
+        self.ctx._check(lib().fadegpu_job_wait(self.ctx._h, self._h, C.byref(st)))
+        v = JobResults()
+        self.ctx._check(lib().fadegpu_job_results_view(self._h, C.byref(v)))
+        n, m = int(v.n), int(v.max_ops)
+        rec = _np_view(C.cast(v.records, C.POINTER(C.c_uint8)), n * PAIR_RESULT_DTYPE.itemsize, np.uint8)
+        rec = rec.view(PAIR_RESULT_DTYPE).copy()
+        if self.score_only:
+            return ScoreResults(rec, st)
+        ops = _np_view(C.cast(v.ops, C.POINTER(C.c_uint32)), n * m, np.uint32).reshape(n, m).copy()
+        return PairResults(rec, ops, st)
+
+    def close(self):
+        if self._h:
+            lib().fadegpu_job_destroy(self._h)
             self._h = C.c_void_p()
 
     def __enter__(self):

@@ -8,6 +8,9 @@
 // view), then fills on `stream` and traceback rounds on `tstream` over alternating scratch sets (three by default),
 // result_index_kernel and the copies home on `stream3`.  FADEGPU_F_HOST_BINNING keeps the first
 // implementation, which evaluates the floor and the windows and sorts on the host.
+// A pair or region call (fadegpu_align_* / fadegpu_score_*, or a job of fadegpu_submit_pairs / _regions) is a stage
+// half on the caller's thread (staging, upload, prep and classify on stream2) and a device half (plan, scatter, kernels,
+// results on stream3), which the ctx thread runs for jobs.
 // There is no CPU fallback: every compute entry point needs a CUDA device.
 #include <cuda_runtime.h>
 #include <algorithm>
@@ -84,34 +87,73 @@ struct fadegpu_ctx {
     cudaStream_t stream3 = nullptr;      // result copies to the host, off the compute stream
     int64_t *d_clen = nullptr, *d_coff = nullptr;   // contig tables for the device-side binning
     std::string err;
-    // asynchronous submits: fadegpu_submit queues the batch, this thread waits for the binning
-    // histogram, plans and launches; the caller goes on filling / reading other batches
+    // asynchronous submits: fadegpu_submit queues the batch (fadegpu_submit_pairs / _regions the job), this thread
+    // waits for the binning histogram, plans and launches; the caller goes on filling / reading other batches or jobs
+    struct Queued { fadegpu_batch *b; int64_t n; fadegpu_job *j; };   // a batch of n reads, or a job
     std::thread worker;
     std::mutex q_mu;
     std::condition_variable q_cv, done_cv;
-    std::deque<std::pair<fadegpu_batch *, int64_t>> jobs;
+    std::deque<Queued> queue;
     bool worker_stop = false, worker_busy = false;
     std::mutex submit_mu;                 // one submit body at a time (they size shared scratch and order the streams)
     std::vector<fadegpu_batch *> batches; // the caller's batches (guarded by q_mu): fadegpu_align_pairs / _regions refuse to
                                           // run while one of them is in flight
-    // fadegpu_align_pairs / fadegpu_align_regions: an internal batch (descriptors, binning arrays, result records) that
-    // grows with use, the staging of the raw inputs, and the targets of a pair call packed as a reference of their own
-    struct PairBufs {
-        fadegpu_batch *b = nullptr;
-        char *h_stage = nullptr, *d_raw = nullptr;          // pinned staging / device copy of offsets + ASCII
-        size_t stage_bytes = 0, raw_bytes = 0;
-        uint32_t *d_two = nullptr, *d_n = nullptr, *d_x = nullptr, *d_chunk_x = nullptr;
-        size_t two_bytes = 0, n_bytes = 0, x_bytes = 0, chunk_bytes = 0;
-        int64_t *d_xpos = nullptr, *d_clen = nullptr, *d_coff = nullptr;
-        size_t xpos_bytes = 0, clen_bytes = 0, coff_bytes = 0;
-        uint8_t *d_xchr = nullptr;
-        size_t xchr_bytes = 0;
-        uint32_t *d_spill = nullptr, *d_ops = nullptr;
-        size_t spill_bytes = 0, ops_bytes = 0;
-        fadegpu_pair_result *d_res = nullptr;
-        size_t res_bytes = 0;
-        int32_t *d_bad = nullptr;
-    } pairs;
+    // fadegpu_align_* / fadegpu_score_* run on this job; fadegpu_job_create hands out the others (guarded by q_mu),
+    // freed with the ctx.  jobs_in_flight counts those submitted and not yet waited for.
+    fadegpu_job *sync_job = nullptr;
+    std::vector<fadegpu_job *> jobs;
+    int jobs_in_flight = 0;
+};
+
+// What a pair call and a region call do differently after the stage half of their shared body (stage_call), kept
+// with the job until its device half has run.  Both stage the query offsets at byte 0 of the upload; the rest of the
+// layout is the caller's.
+struct StagedCall {
+    const char *fn = nullptr, *item = nullptr;   // the call's and an item's name, for messages
+    int64_t n = 0, qbytes = 0, n_over = 0;       // items, query letters, oversize items (counted by the host validation)
+    int32_t max_ops = 0;
+    bool score_only = false;                     // fadegpu_score_*: score and end cell, no traceback (max_ops is 0)
+    size_t raw = 0;                              // bytes staged and uploaded
+    size_t o_tbeg = 0, o_tend = 0;               // byte offsets of the int64 window bounds of every item in the upload
+    // after the binning histogram is home: the reference the SW kernels read; counts its launches
+    std::function<int(fadegpu_job *j, RefDev *ref, int *launches)> reference;
+};
+
+// One pair or region call: an internal batch (descriptors, binning arrays, result records), the staging of the raw
+// inputs, the targets of a pair call packed as a reference of their own, the records and ops of the call in pinned
+// memory (fadegpu_job_results_view).  Everything grows with use.
+struct fadegpu_job {
+    fadegpu_ctx *ctx = nullptr;
+    fadegpu_batch *b = nullptr;
+    char *h_stage = nullptr, *d_raw = nullptr;          // pinned staging / device copy of offsets + ASCII
+    size_t stage_bytes = 0, raw_bytes = 0;
+    uint32_t *d_two = nullptr, *d_n = nullptr, *d_x = nullptr, *d_chunk_x = nullptr;
+    size_t two_bytes = 0, n_bytes = 0, x_bytes = 0, chunk_bytes = 0;
+    int64_t *d_xpos = nullptr, *d_clen = nullptr, *d_coff = nullptr;
+    size_t xpos_bytes = 0, clen_bytes = 0, coff_bytes = 0;
+    uint8_t *d_xchr = nullptr;
+    size_t xchr_bytes = 0;
+    uint32_t *d_spill = nullptr, *d_ops = nullptr;
+    size_t spill_bytes = 0, ops_bytes = 0;
+    fadegpu_pair_result *d_res = nullptr;
+    size_t res_bytes = 0;
+    int32_t *d_bad = nullptr;
+    fadegpu_pair_result *h_res = nullptr;               // pinned records and ops of the last submit
+    uint32_t *h_ops = nullptr;
+    size_t h_res_bytes = 0, h_ops_bytes = 0;
+    // the call between its stage half and its wait: where the records go, what the device half needs, the stats
+    StagedCall sc;
+    PairArgs pa{};
+    fadegpu_pair_result *out = nullptr;
+    uint32_t *ops_out = nullptr;
+    int n_prep = 0;
+    int64_t h2d = 0;
+    fadegpu_stats st{};
+    int64_t n_res = -1;                                 // records of the last successful wait (-1: none)
+    // guarded by ctx->q_mu
+    bool in_flight = false, queued = false;
+    int rc = 0;                                         // outcome of a device half run by the ctx thread
+    std::string err;
 };
 
 struct AlnTmp {       // a read that needs SW, captured in read order (sequential pass), before sorting
@@ -233,6 +275,18 @@ void free_reference(fadegpu_ctx *c)
     free_dev(c->d_clen); free_dev(c->d_coff);
     c->n_x = 0; c->ref_bytes = 0; c->n_contigs = 0; c->total_bases = c->padded_bases = 0;
     c->names.clear(); c->clen.clear(); c->coff.clear();
+}
+
+// the job must not be queued; fadegpu_free_batch waits for the ctx's streams before anything is freed
+void free_job(fadegpu_job *j)
+{
+    if (!j) return;
+    if (j->b) fadegpu_free_batch(j->b);
+    free_host(j->h_stage); free_host(j->h_res); free_host(j->h_ops);
+    free_dev(j->d_raw); free_dev(j->d_two); free_dev(j->d_n); free_dev(j->d_x); free_dev(j->d_chunk_x);
+    free_dev(j->d_xpos); free_dev(j->d_xchr); free_dev(j->d_clen); free_dev(j->d_coff); free_dev(j->d_spill);
+    free_dev(j->d_ops); free_dev(j->d_res); free_dev(j->d_bad);
+    delete j;
 }
 
 int upload_contig_tables(fadegpu_ctx *c)
@@ -635,14 +689,9 @@ void fadegpu_destroy(fadegpu_ctx *c)
         c->worker.join();                 // finishes the queued submits first
     }
     cudaSetDevice(c->device);
-    {
-        fadegpu_ctx::PairBufs &pb = c->pairs;
-        if (pb.b) fadegpu_free_batch(pb.b);
-        free_host(pb.h_stage);
-        free_dev(pb.d_raw); free_dev(pb.d_two); free_dev(pb.d_n); free_dev(pb.d_x); free_dev(pb.d_chunk_x);
-        free_dev(pb.d_xpos); free_dev(pb.d_xchr); free_dev(pb.d_clen); free_dev(pb.d_coff); free_dev(pb.d_spill);
-        free_dev(pb.d_ops); free_dev(pb.d_res); free_dev(pb.d_bad);
-    }
+    for (fadegpu_job *j : c->jobs) free_job(j);   // (each waits for the streams first)
+    c->jobs.clear();
+    free_job(c->sync_job);
     if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->stream2) { cudaStreamSynchronize(c->stream2); cudaStreamDestroy(c->stream2); }
     if (c->stream3) { cudaStreamSynchronize(c->stream3); cudaStreamDestroy(c->stream3); }
@@ -904,12 +953,14 @@ static int ensure_host_staging(fadegpu_ctx *c, fadegpu_batch *b)
 static int gather_reads(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, const fadegpu_inputs &in);
 static int queue_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, int mode, int64_t seq_bytes);
 static bool batch_in_flight(fadegpu_ctx *c, fadegpu_batch *b);
+static int refuse_jobs_in_flight(fadegpu_ctx *c, const char *fn);
 
 int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, const fadegpu_inputs *in)
 {
     if (!c || !b || b->ctx != c || !in) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: bad ctx/batch/inputs");
     if (!c->d_two) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: no reference loaded");
     if (batch_in_flight(c, b)) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: batch already in flight (call fadegpu_wait)");
+    { int rc = refuse_jobs_in_flight(c, "fadegpu_submit"); if (rc) return rc; }
     if (n_reads < 0 || n_reads > b->v.max_reads) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: n_reads out of range");
     if (n_reads > 0 && (!in->seq4 || !in->seq_off || !in->l_qseq || !in->tid || !in->pos || !in->aligned_len ||
                         !in->clip_left || !in->clip_right))
@@ -1387,7 +1438,22 @@ static int queue_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, int mode, i
     }
     b->queued = true; b->submit_rc = 0; b->mode = mode; b->job_seq_bytes = seq_bytes;
     b->in_flight = true;
-    c->jobs.emplace_back(b, n);
+    c->queue.push_back({ b, n, nullptr });
+    c->q_cv.notify_one();
+    return FADEGPU_OK;
+}
+
+static int launch_job(fadegpu_ctx *c, fadegpu_job *j);
+
+// queue the device half of a staged job for the ctx thread (caller holds q_mu)
+static int queue_job(fadegpu_ctx *c, fadegpu_job *j)
+{
+    if (!c->worker.joinable()) {
+        try { c->worker = std::thread(worker_main, c); }
+        catch (const std::exception &e) { return fail(c, FADEGPU_E_STATE, std::string(j->sc.fn) + ": cannot start the submit thread: " + e.what()); }
+    }
+    j->queued = true; j->rc = 0;
+    c->queue.push_back({ nullptr, 0, j });
     c->q_cv.notify_one();
     return FADEGPU_OK;
 }
@@ -1397,25 +1463,27 @@ static void worker_main(fadegpu_ctx *c)
     cudaSetDevice(c->device);
     std::unique_lock<std::mutex> lk(c->q_mu);
     for (;;) {
-        c->q_cv.wait(lk, [&] { return c->worker_stop || !c->jobs.empty(); });
-        if (c->jobs.empty()) return;
-        auto job = c->jobs.front();
-        c->jobs.pop_front();
+        c->q_cv.wait(lk, [&] { return c->worker_stop || !c->queue.empty(); });
+        if (c->queue.empty()) return;
+        const fadegpu_ctx::Queued q = c->queue.front();
+        c->queue.pop_front();
         c->worker_busy = true;
-        const int mode = job.first->mode;
-        const int64_t seq_bytes = job.first->job_seq_bytes;
+        const int mode = q.b ? q.b->mode : 0;
+        const int64_t seq_bytes = q.b ? q.b->job_seq_bytes : 0;
         lk.unlock();
         int rc;
         std::string err;
         {
             std::lock_guard<std::mutex> g(c->submit_mu);
-            rc = submit_stages(c, job.first, job.second, mode, seq_bytes);
+            rc = q.j ? launch_job(c, q.j) : submit_stages(c, q.b, q.n, mode, seq_bytes);
             if (rc) { std::lock_guard<std::mutex> ge(g_err_mu); err = c->err; }
         }
         lk.lock();
-        job.first->submit_rc = rc;
-        job.first->submit_err = err;
-        job.first->queued = false;
+        if (q.j) {
+            q.j->rc = rc; q.j->err = err; q.j->queued = false;
+        } else {
+            q.b->submit_rc = rc; q.b->submit_err = err; q.b->queued = false;
+        }
         c->worker_busy = false;
         c->done_cv.notify_all();
     }
@@ -1425,7 +1493,17 @@ static void worker_main(fadegpu_ctx *c)
 static void drain_submits(fadegpu_ctx *c)
 {
     std::unique_lock<std::mutex> lk(c->q_mu);
-    c->done_cv.wait(lk, [&] { return c->jobs.empty() && !c->worker_busy; });
+    c->done_cv.wait(lk, [&] { return c->queue.empty() && !c->worker_busy; });
+}
+
+// FADEGPU_E_STATE while a job of the ctx is submitted and not yet waited for (annotate batches and jobs are not in
+// flight together)
+static int refuse_jobs_in_flight(fadegpu_ctx *c, const char *fn)
+{
+    std::lock_guard<std::mutex> lk(c->q_mu);
+    if (c->jobs_in_flight > 0)
+        return fail(c, FADEGPU_E_STATE, std::string(fn) + ": a job of this ctx is in flight (call fadegpu_job_wait)");
+    return 0;
 }
 
 // a batch is "in flight" from its submit to its wait; the flag is shared with the ctx thread
@@ -1445,6 +1523,7 @@ int fadegpu_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads)
     if (!(c->p.flags & FADEGPU_F_HOST_BINNING)) {
         if (!c->d_two) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: no reference loaded");
         if (batch_in_flight(c, b)) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: batch already in flight (call fadegpu_wait)");
+        { int rc = refuse_jobs_in_flight(c, "fadegpu_submit"); if (rc) return rc; }
         return queue_submit(c, b, n_reads, MODE_VIEW, 0);
     }
     fadegpu_inputs in = view_inputs(v);
@@ -1460,6 +1539,7 @@ int fadegpu_submit_compact(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, in
         return fail(c, FADEGPU_E_ARG, "fadegpu_submit_compact: seq_bytes out of range");
     if (!c->d_two) return fail(c, FADEGPU_E_STATE, "fadegpu_submit_compact: no reference loaded");
     if (batch_in_flight(c, b)) return fail(c, FADEGPU_E_STATE, "fadegpu_submit_compact: batch already in flight (call fadegpu_wait)");
+    { int rc = refuse_jobs_in_flight(c, "fadegpu_submit_compact"); if (rc) return rc; }
     if (c->p.flags & FADEGPU_F_HOST_BINNING) {
         // A/B switch: expand the compact records into the view's arrays and take the host path
         fadegpu_batch_view &w = b->v;
@@ -1684,72 +1764,56 @@ static int refuse_in_flight(fadegpu_ctx *c, const char *fn)
     return 0;
 }
 
-// What a pair call and a region call do differently around their shared body (align_staged).  Both stage the query
-// offsets at byte 0 of the upload; the rest of the layout is the caller's.
-struct StagedCall {
-    const char *fn, *item;        // the call's and an item's name, for messages
-    int64_t n, qbytes, n_over;    // items, query letters, oversize items (counted by the host validation)
-    int32_t max_ops;
-    bool score_only;              // fadegpu_score_*: score and end cell, no traceback (max_ops is 0)
-    size_t raw;                   // bytes staged and uploaded
-    size_t o_tbeg, o_tend;        // byte offsets of the int64 window bounds of every item in the upload (results init)
-    std::function<void(char *h_stage)> stage;
-    // on stream2, after the upload: the binning inputs and the queries of b (failures reported to *d_bad), and ba's
-    // contig table; counts its launches
-    std::function<int(fadegpu_batch *b, const char *d_raw, BinArgs &ba, int *launches)> prep;
-    // after the binning histogram is home: the reference the SW kernels read; counts its launches
-    std::function<int(fadegpu_batch *b, RefDev *ref, int *launches)> reference;
-};
+// The caller's part of a pair or region call: copy its arrays into the job's pinned staging
+using StageFn = std::function<void(char *h_stage)>;
+// on stream2, after the upload: the binning inputs and the queries of j->b (failures reported to j->d_bad), and ba's
+// contig table; counts its launches
+using PrepFn = std::function<int(fadegpu_job *j, const char *d_raw, BinArgs &ba, int *launches)>;
 
-// The raw inputs go to the device through pinned staging on stream2, where the caller's prep kernels write the
-// per-item binning inputs and the queries; the binning, the launch plan and run_plan are those of a device-binned
-// submit, on the ctx's internal pair batch, with every alignment traced back and the full CIGARs spilled (score-only
-// calls: only the end cell is found, nothing is spilled); the records come back in item order on stream3.
-static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_result *out, uint32_t *ops_out,
-                        fadegpu_stats *stats_out, std::chrono::steady_clock::time_point t_begin)
+// Stage half of a pair or region call, on the caller's thread: the raw inputs go to the device through the job's pinned
+// staging on stream2, where the caller's prep kernels write the per-item binning inputs and the queries, and the binning
+// classify kernel histograms them; the histogram is on its way home when this returns.  The device half (launch_job)
+// does the rest.
+static int stage_call(fadegpu_ctx *c, fadegpu_job *j, const StagedCall &sc, const StageFn &stage, const PrepFn &prep)
 {
+    j->sc = sc;
+    j->st = fadegpu_stats{};
+    j->st.n_reads = sc.n;
+    j->st.n_oversize = sc.n_over;
+    if (sc.n == 0) return FADEGPU_OK;
     const int64_t n = sc.n, qbytes = sc.qbytes;
     const int32_t max_ops = sc.max_ops;
-    fadegpu_stats st{};
-    st.n_reads = n;
-    st.n_oversize = sc.n_over;
-    if (n == 0) {
-        if (stats_out) *stats_out = st;
-        return FADEGPU_OK;
-    }
-    std::lock_guard<std::mutex> submit_guard(c->submit_mu);
     CU(c, cudaSetDevice(c->device));
-    fadegpu_ctx::PairBufs &pb = c->pairs;
-    if (!pb.b || pb.b->v.max_reads < n || pb.b->v.max_seq_bytes < qbytes + 16) {
+    if (!j->b || j->b->v.max_reads < n || j->b->v.max_seq_bytes < qbytes + 16) {
         int64_t nr = n, sb = qbytes + 16;
-        if (pb.b) {
-            nr = std::max(nr, pb.b->v.max_reads); sb = std::max(sb, pb.b->v.max_seq_bytes);
-            fadegpu_free_batch(pb.b);
-            pb.b = nullptr;
+        if (j->b) {
+            nr = std::max(nr, j->b->v.max_reads); sb = std::max(sb, j->b->v.max_seq_bytes);
+            fadegpu_free_batch(j->b);
+            j->b = nullptr;
         }
-        int rc = fadegpu_alloc_batch(c, nr, sb, &pb.b);
+        int rc = fadegpu_alloc_batch(c, nr, sb, &j->b);
         if (rc) return rc;
     }
-    fadegpu_batch *b = pb.b;
+    fadegpu_batch *b = j->b;
     const size_t raw = sc.raw;
-    if (pb.stage_bytes < raw) {
-        free_host(pb.h_stage);
-        pb.stage_bytes = 0;
-        CU(c, cudaHostAlloc((void **)&pb.h_stage, raw, cudaHostAllocDefault));
-        pb.stage_bytes = raw;
+    if (j->stage_bytes < raw) {
+        free_host(j->h_stage);
+        j->stage_bytes = 0;
+        CU(c, cudaHostAlloc((void **)&j->h_stage, raw, cudaHostAllocDefault));
+        j->stage_bytes = raw;
     }
-    sc.stage(pb.h_stage);
+    stage(j->h_stage);
     {
         int rc = 0;
         auto grow = [&](auto **p, size_t *have, size_t bytes) { if (!rc) rc = ensure_dev(c, (void **)p, have, std::max<size_t>(bytes, 16)); };
-        grow(&pb.d_raw, &pb.raw_bytes, raw);
-        grow(&pb.d_res, &pb.res_bytes, (size_t)n * sizeof(fadegpu_pair_result));
+        grow(&j->d_raw, &j->raw_bytes, raw);
+        grow(&j->d_res, &j->res_bytes, (size_t)n * sizeof(fadegpu_pair_result));
         if (max_ops > 0) {
-            grow(&pb.d_spill, &pb.spill_bytes, (size_t)n * (size_t)max_ops * 4);
-            grow(&pb.d_ops, &pb.ops_bytes, (size_t)n * (size_t)max_ops * 4);
+            grow(&j->d_spill, &j->spill_bytes, (size_t)n * (size_t)max_ops * 4);
+            grow(&j->d_ops, &j->ops_bytes, (size_t)n * (size_t)max_ops * 4);
         }
         if (rc) return rc;
-        if (!pb.d_bad) CU(c, cudaMalloc((void **)&pb.d_bad, sizeof(int32_t)));
+        if (!j->d_bad) CU(c, cudaMalloc((void **)&j->d_bad, sizeof(int32_t)));
     }
     // ---- upload, packing and binning on stream2 ----
     b->n_reads = n;
@@ -1761,14 +1825,15 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
     memset(b->h_stats, 0, 128);
     cudaStream_t s2 = c->stream2;
     CU(c, cudaEventRecord(b->ev[0], s2));
-    CU(c, cudaMemcpyAsync(pb.d_raw, pb.h_stage, raw, cudaMemcpyHostToDevice, s2));
-    int64_t h2d = (int64_t)raw;
+    CU(c, cudaMemcpyAsync(j->d_raw, j->h_stage, raw, cudaMemcpyHostToDevice, s2));
+    j->h2d = (int64_t)raw;
     CU(c, cudaEventRecord(b->ev[4], s2));
     CU(c, cudaMemsetAsync(b->d_hist, 0, (size_t)BIN_KEYS * 4, s2));
     CU(c, cudaMemsetAsync(b->d_cursor, 0, (size_t)BIN_KEYS * 4, s2));
     CU(c, cudaMemsetAsync(b->d_stats, 0, 128, s2));
-    CU(c, cudaMemsetAsync(pb.d_bad, 0x7f, sizeof(int32_t), s2));   // > any item index
-    BinArgs ba{};
+    CU(c, cudaMemsetAsync(j->d_bad, 0x7f, sizeof(int32_t), s2));   // > any item index
+    BinArgs &ba = b->ba;
+    ba = BinArgs{};
     ba.seq4 = b->d_in_seq4; ba.seq_off = b->d_in_seq_off; ba.l_qseq = b->d_in_lq; ba.tid = b->d_in_tid; ba.pos = b->d_in_pos;
     ba.aligned_len = b->d_in_alen; ba.clip_left = b->d_in_cl; ba.clip_right = b->d_in_cr;
     ba.read = nullptr; ba.seq_cursor = nullptr; ba.src_off = b->d_src_off; ba.gate = nullptr; ba.host_meta = nullptr;
@@ -1777,13 +1842,29 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
     ba.n = n; ba.seq_total = qbytes; ba.window = 0; ba.min_length = 0; ba.flags = c->p.flags;
     ba.key = b->d_key; ba.tlen = b->d_tlen; ba.start = b->d_start; ba.hist = b->d_hist; ba.stats = b->d_stats;
     ba.keybase = b->d_keybase; ba.cursor = b->d_cursor; ba.aln = b->d_aln; ba.aln_start = b->d_aln_start;
-    int n_prep = 0;
-    { int rc = sc.prep(b, pb.d_raw, ba, &n_prep); if (rc) return rc; }
+    j->n_prep = 0;
+    { int rc = prep(j, j->d_raw, ba, &j->n_prep); if (rc) return rc; }
     CU(c, launch_bin_classify(ba, c->sm_count, s2));
     CU(c, cudaMemcpyAsync(b->h_hist, b->d_hist, (size_t)BIN_KEYS * 4, cudaMemcpyDeviceToHost, s2));
     CU(c, cudaMemcpyAsync(b->h_stats, b->d_stats, 128, cudaMemcpyDeviceToHost, s2));
-    CU(c, cudaMemcpyAsync(b->h_over, pb.d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaMemcpyAsync(b->h_over, j->d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s2));
     CU(c, cudaEventRecord(b->ev_prep, s2));
+    return FADEGPU_OK;
+}
+
+// Device half of a staged call, under submit_mu (it sizes the shared scratch): once the binning histogram is home, the
+// launch plan and run_plan of a device-binned submit on the job's batch, with every alignment traced back and the full
+// CIGARs spilled (score-only calls: only the end cell is found, nothing is spilled); the records come back in item
+// order to j->out / j->ops_out on stream3.  Queued jobs run it on the ctx thread while the caller stages the next.
+static int launch_job(fadegpu_ctx *c, fadegpu_job *j)
+{
+    const StagedCall &sc = j->sc;
+    if (sc.n == 0) return FADEGPU_OK;
+    const int64_t n = sc.n;
+    const int32_t max_ops = sc.max_ops;
+    fadegpu_batch *b = j->b;
+    cudaStream_t s2 = c->stream2;
+    CU(c, cudaSetDevice(c->device));
     CU(c, cudaEventSynchronize(b->ev_prep));
     const int32_t bad = b->h_over[0];
     if (bad >= 0 && bad < n)
@@ -1791,22 +1872,24 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
                                           " holds a letter outside the BAM nt16 alphabet =ACMGRSVTWYHKDBN");
     if (b->h_stats[6] & 1ull) return fail(c, FADEGPU_E_CUDA, std::string(sc.fn) + ": internal error (query offsets)");
     const int64_t n_aln = (int64_t)b->h_stats[1];
+    int n_prep = j->n_prep;
+    int64_t h2d = j->h2d;
     PlanTarget pt{};
-    { int rc = sc.reference(b, &pt.ref, &n_prep); if (rc) return rc; }
+    { int rc = sc.reference(j, &pt.ref, &n_prep); if (rc) return rc; }
     { int rc = plan_from_histogram(c, b, n_aln); if (rc) return rc; }
     if (n_aln > 0) {
         CU(c, cudaMemcpyAsync(b->d_keybase, b->h_keybase, (size_t)BIN_KEYS * 4, cudaMemcpyHostToDevice, s2));
         if (b->n_items > 0)
             CU(c, cudaMemcpyAsync(b->d_items, b->h_items, (size_t)b->n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, s2));
         h2d += (int64_t)BIN_KEYS * 4 + b->n_items * (int64_t)sizeof(WarpItem);
-        CU(c, launch_bin_scatter(ba, c->sm_count, s2));
+        CU(c, launch_bin_scatter(b->ba, c->sm_count, s2));
     }
     CU(c, cudaEventRecord(b->ev_ready, s2));
     // ---- SW kernels: the batch's plan against the caller's reference ----
     CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
     CU(c, cudaEventRecord(b->ev[1], c->stream));
     pt.tags_only = 0;   // every item is traced back (or has its end cell found), whatever the ctx's FADEGPU_F_TAGS_ONLY
-    pt.ops_spill = max_ops > 0 ? pb.d_spill : nullptr;
+    pt.ops_spill = max_ops > 0 ? j->d_spill : nullptr;
     pt.ops_cap = max_ops;
     pt.end_only = sc.score_only;
     int nl = 0;
@@ -1815,18 +1898,19 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
     cudaStream_t s3 = c->stream3;
     { int rc = join_kernels(c, b, s3); if (rc) return rc; }
     CU(c, cudaEventRecord(b->ev[2], s3));
-    CU(c, launch_pair_results(n, reinterpret_cast<const int64_t *>(pb.d_raw), reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tbeg),
-                              reinterpret_cast<const int64_t *>(pb.d_raw + sc.o_tend), b->d_aln, b->d_out, (int)n_aln,
-                              sc.score_only, pb.d_spill, max_ops, reinterpret_cast<PairResult *>(pb.d_res), pb.d_ops,
+    // the results kernel writes the ops of the aligned items only: empty and oversize items keep these zeros (rather
+    // than whatever an earlier call of this job left there)
+    if (max_ops > 0) CU(c, cudaMemsetAsync(j->d_ops, 0, (size_t)n * (size_t)max_ops * 4, s3));
+    CU(c, launch_pair_results(n, reinterpret_cast<const int64_t *>(j->d_raw), reinterpret_cast<const int64_t *>(j->d_raw + sc.o_tbeg),
+                              reinterpret_cast<const int64_t *>(j->d_raw + sc.o_tend), b->d_aln, b->d_out, (int)n_aln,
+                              sc.score_only, j->d_spill, max_ops, reinterpret_cast<PairResult *>(j->d_res), j->d_ops,
                               b->d_stats + 7, c->sm_count, s3));
-    CU(c, cudaMemcpyAsync(out, pb.d_res, (size_t)n * sizeof(fadegpu_pair_result), cudaMemcpyDeviceToHost, s3));
+    CU(c, cudaMemcpyAsync(j->out, j->d_res, (size_t)n * sizeof(fadegpu_pair_result), cudaMemcpyDeviceToHost, s3));
     if (max_ops > 0)
-        CU(c, cudaMemcpyAsync(ops_out, pb.d_ops, (size_t)n * (size_t)max_ops * 4, cudaMemcpyDeviceToHost, s3));
+        CU(c, cudaMemcpyAsync(j->ops_out, j->d_ops, (size_t)n * (size_t)max_ops * 4, cudaMemcpyDeviceToHost, s3));
     CU(c, cudaMemcpyAsync(b->h_stats + 7, b->d_stats + 7, 8, cudaMemcpyDeviceToHost, s3));
     CU(c, cudaEventRecord(b->ev[3], s3));
-    CU(c, cudaEventSynchronize(b->ev[3]));
-    if ((int64_t)b->h_stats[7] != n_aln)
-        return fail(c, FADEGPU_E_CUDA, std::string(sc.fn) + ": a kernel did not produce a result record (internal error)");
+    fadegpu_stats &st = j->st;
     st.n_aligned = n_aln;
     st.n_generic = b->st.n_generic;
     st.cells = (int64_t)b->h_stats[0];
@@ -1834,13 +1918,82 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
     st.d2h_bytes = n * (int64_t)(sizeof(fadegpu_pair_result) + 4 * (size_t)max_ops) + (int64_t)BIN_KEYS * 4 + 128 + 4 + 8;
     st.kernel_launches = nl + n_prep + 1 + (n_aln > 0 ? 2 : 1);
     st.scratch_bytes = b->st.scratch_bytes;
-    float t;
-    if (cudaEventElapsedTime(&t, b->ev[1], b->ev[2]) == cudaSuccess) st.kernel_ms = t;
-    if (cudaEventElapsedTime(&t, b->ev[0], b->ev[3]) == cudaSuccess) st.total_ms = t;
     st.host_threads = c->host_threads;
-    st.host_submit_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
-    b->st = st;
-    if (stats_out) *stats_out = st;
+    return FADEGPU_OK;
+}
+
+// The records of a launched call are home: the device's count of result records, and the device times
+static int finish_job(fadegpu_ctx *c, fadegpu_job *j)
+{
+    if (j->sc.n == 0) return FADEGPU_OK;
+    fadegpu_batch *b = j->b;
+    CU(c, cudaEventSynchronize(b->ev[3]));
+    if ((int64_t)b->h_stats[7] != j->st.n_aligned)
+        return fail(c, FADEGPU_E_CUDA, std::string(j->sc.fn) + ": a kernel did not produce a result record (internal error)");
+    float t;
+    if (cudaEventElapsedTime(&t, b->ev[1], b->ev[2]) == cudaSuccess) j->st.kernel_ms = t;
+    if (cudaEventElapsedTime(&t, b->ev[0], b->ev[3]) == cudaSuccess) j->st.total_ms = t;
+    b->st = j->st;
+    return FADEGPU_OK;
+}
+
+// A validated pair or region call.  Synchronous (job == nullptr): after the device halves of the jobs queued before it,
+// both halves on the ctx's own job, the records straight into the caller's arrays.  A job: its pinned records, the
+// stage half here and the device half queued for the ctx thread (here with FADEGPU_F_SYNC_SUBMIT).
+static int run_call(fadegpu_ctx *c, fadegpu_job *job, const StagedCall &sc, const StageFn &stage, const PrepFn &prep,
+                    fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out,
+                    std::chrono::steady_clock::time_point t_begin)
+{
+    auto ms_since_begin = [&] {
+        return std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    };
+    if (!job) {
+        drain_submits(c);
+        std::lock_guard<std::mutex> submit_guard(c->submit_mu);
+        if (!c->sync_job) {
+            c->sync_job = new (std::nothrow) fadegpu_job();
+            if (!c->sync_job) return fail(c, FADEGPU_E_OOM, std::string(sc.fn) + ": out of host memory");
+            c->sync_job->ctx = c;
+        }
+        fadegpu_job *j = c->sync_job;
+        j->out = out; j->ops_out = ops_out;
+        int rc = stage_call(c, j, sc, stage, prep);
+        if (!rc) rc = launch_job(c, j);
+        if (!rc) rc = finish_job(c, j);
+        if (rc) return rc;
+        if (sc.n > 0) j->st.host_submit_ms = ms_since_begin();
+        if (stats_out) *stats_out = j->st;
+        return FADEGPU_OK;
+    }
+    fadegpu_job *j = job;
+    j->n_res = -1;
+    const size_t res_bytes = (size_t)sc.n * sizeof(fadegpu_pair_result), ops_bytes = (size_t)sc.n * (size_t)sc.max_ops * 4;
+    CU(c, cudaSetDevice(c->device));
+    if (j->h_res_bytes < res_bytes) {
+        free_host(j->h_res);
+        j->h_res_bytes = 0;
+        CU(c, cudaHostAlloc((void **)&j->h_res, res_bytes, cudaHostAllocDefault));
+        j->h_res_bytes = res_bytes;
+    }
+    if (j->h_ops_bytes < ops_bytes) {
+        free_host(j->h_ops);
+        j->h_ops_bytes = 0;
+        CU(c, cudaHostAlloc((void **)&j->h_ops, ops_bytes, cudaHostAllocDefault));
+        j->h_ops_bytes = ops_bytes;
+    }
+    j->out = j->h_res; j->ops_out = j->h_ops;
+    { int rc = stage_call(c, j, sc, stage, prep); if (rc) return rc; }
+    const bool here = (c->p.flags & FADEGPU_F_SYNC_SUBMIT) != 0;
+    if (here) {
+        std::lock_guard<std::mutex> submit_guard(c->submit_mu);
+        int rc = launch_job(c, j);
+        if (rc) return rc;
+    }
+    if (sc.n > 0) j->st.host_submit_ms = ms_since_begin();
+    std::lock_guard<std::mutex> lk(c->q_mu);
+    if (!here) { int rc = queue_job(c, j); if (rc) return rc; }
+    j->in_flight = true;
+    ++c->jobs_in_flight;
     return FADEGPU_OK;
 }
 
@@ -1848,13 +2001,14 @@ static int align_staged(fadegpu_ctx *c, const StagedCall &sc, fadegpu_pair_resul
 // pair_pack_targets_kernel and pair_xlist_kernel pack the targets as a reference of their own, whose contigs the
 // targets are.
 static int pairs_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n_pairs, const fadegpu_pairs *in,
-                      int32_t max_ops, fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+                      int32_t max_ops, fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out,
+                      fadegpu_job *job)
 {
     const std::string at = std::string(fn) + ": ";
     if (!c) return fail(nullptr, FADEGPU_E_ARG, at + "null ctx");
     if (n_pairs < 0 || n_pairs > ((int64_t)1 << 30) || max_ops < 0)
         return fail(c, FADEGPU_E_ARG, at + "n_pairs or max_ops out of range");
-    if (n_pairs > 0 && (!in || !in->query_off || !in->target_off || !out || (max_ops > 0 && !ops_out)))
+    if (n_pairs > 0 && (!in || !in->query_off || !in->target_off || (!job && (!out || (max_ops > 0 && !ops_out)))))
         return fail(c, FADEGPU_E_ARG, at + "null argument");
     { int rc = refuse_in_flight(c, fn); if (rc) return rc; }
     const auto t_begin = std::chrono::steady_clock::now();
@@ -1878,78 +2032,82 @@ static int pairs_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n
     const size_t o_t = o_q + align16((size_t)qbytes);
     const int64_t n_words = n + (tbytes >> 5) + 2;   // target k starts at 32 * (k + toff[k] / 32)
     const int64_t n_chunks = (n_words + PAIR_CHUNK_WORDS - 1) / PAIR_CHUNK_WORDS;
-    fadegpu_ctx::PairBufs &pb = c->pairs;
-    PairArgs pa{};
     StagedCall sc;
     sc.fn = fn; sc.item = "pair";
     sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops; sc.score_only = score_only;
     sc.raw = o_t + align16((size_t)tbytes);
     sc.o_tbeg = o_toff; sc.o_tend = o_toff + 8;   // target k spans toff[k] .. toff[k + 1]
-    sc.stage = [&](char *h) {
+    auto stage = [&](char *h) {
         int64_t *hq = reinterpret_cast<int64_t *>(h), *ht = reinterpret_cast<int64_t *>(h + o_toff);
         const int64_t q0 = in->query_off[0], t0 = in->target_off[0];
         for (int64_t k = 0; k <= n; ++k) { hq[k] = in->query_off[k] - q0; ht[k] = in->target_off[k] - t0; }
         if (qbytes) parallel_copy(h + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
         if (tbytes) parallel_copy(h + o_t, in->target + t0, (size_t)tbytes, c->host_threads);
     };
-    sc.prep = [&](fadegpu_batch *b, const char *d, BinArgs &ba, int *launches) -> int {
+    auto prep = [&](fadegpu_job *j, const char *d, BinArgs &ba, int *launches) -> int {
+        fadegpu_batch *b = j->b;
         int rc = 0;
         auto grow = [&](auto **p, size_t *have, size_t bytes) { if (!rc) rc = ensure_dev(c, (void **)p, have, std::max<size_t>(bytes, 16)); };
-        grow(&pb.d_two, &pb.two_bytes, (size_t)n_words * 8); grow(&pb.d_n, &pb.n_bytes, (size_t)n_words * 4);
-        grow(&pb.d_x, &pb.x_bytes, (size_t)n_words * 4); grow(&pb.d_chunk_x, &pb.chunk_bytes, (size_t)n_chunks * 4);
-        grow(&pb.d_clen, &pb.clen_bytes, (size_t)n * 8); grow(&pb.d_coff, &pb.coff_bytes, (size_t)n * 8);
+        grow(&j->d_two, &j->two_bytes, (size_t)n_words * 8); grow(&j->d_n, &j->n_bytes, (size_t)n_words * 4);
+        grow(&j->d_x, &j->x_bytes, (size_t)n_words * 4); grow(&j->d_chunk_x, &j->chunk_bytes, (size_t)n_chunks * 4);
+        grow(&j->d_clen, &j->clen_bytes, (size_t)n * 8); grow(&j->d_coff, &j->coff_bytes, (size_t)n * 8);
         if (rc) return rc;
+        PairArgs &pa = j->pa;
+        pa = PairArgs{};
         pa.n = n;
         pa.qoff = reinterpret_cast<const int64_t *>(d); pa.toff = reinterpret_cast<const int64_t *>(d + o_toff);
         pa.query = d + o_q; pa.target = d + o_t;
         pa.seq_off = b->d_in_seq_off; pa.pos = b->d_in_pos; pa.l_qseq = b->d_in_lq; pa.tid = b->d_in_tid;
         pa.aligned_len = b->d_in_alen; pa.clip_left = b->d_in_cl; pa.clip_right = b->d_in_cr;
-        pa.clen = pb.d_clen; pa.coff = pb.d_coff; pa.seq4 = b->d_in_seq4; pa.bad = pb.d_bad;
-        pa.two = pb.d_two; pa.nmask = pb.d_n; pa.xmask = pb.d_x; pa.n_words = n_words;
-        pa.chunk_x = pb.d_chunk_x; pa.n_x = b->d_stats + 12;
+        pa.clen = j->d_clen; pa.coff = j->d_coff; pa.seq4 = b->d_in_seq4; pa.bad = j->d_bad;
+        pa.two = j->d_two; pa.nmask = j->d_n; pa.xmask = j->d_x; pa.n_words = n_words;
+        pa.chunk_x = j->d_chunk_x; pa.n_x = b->d_stats + 12;
         CU(c, launch_pair_prep(pa, c->sm_count, c->stream2));
         CU(c, launch_pair_pack_targets(pa, c->stream2));
         *launches += 2;
-        ba.clen = pb.d_clen; ba.coff = pb.d_coff; ba.n_contigs = (int32_t)n;   // contigs = targets
+        ba.clen = j->d_clen; ba.coff = j->d_coff; ba.n_contigs = (int32_t)n;   // contigs = targets
         return 0;
     };
-    sc.reference = [&](fadegpu_batch *b, RefDev *ref, int *launches) -> int {
-        const int64_t n_x = (int64_t)b->h_stats[12];
-        int rc = ensure_dev(c, (void **)&pb.d_xpos, &pb.xpos_bytes, std::max<size_t>(16, (size_t)n_x * 8));
-        if (!rc) rc = ensure_dev(c, (void **)&pb.d_xchr, &pb.xchr_bytes, std::max<size_t>(16, (size_t)n_x));
+    // (runs in the device half, possibly on the ctx thread: it captures nothing of this frame)
+    sc.reference = [c](fadegpu_job *j, RefDev *ref, int *launches) -> int {
+        PairArgs &pa = j->pa;
+        const int64_t n_x = (int64_t)j->b->h_stats[12];
+        int rc = ensure_dev(c, (void **)&j->d_xpos, &j->xpos_bytes, std::max<size_t>(16, (size_t)n_x * 8));
+        if (!rc) rc = ensure_dev(c, (void **)&j->d_xchr, &j->xchr_bytes, std::max<size_t>(16, (size_t)n_x));
         if (rc) return rc;
-        pa.xpos = pb.d_xpos; pa.xchr = pb.d_xchr;
+        pa.xpos = j->d_xpos; pa.xchr = j->d_xchr;
         if (n_x > 0) { CU(c, launch_pair_xlist(pa, c->stream2)); ++*launches; }
-        ref->planes.two = pb.d_two; ref->planes.nmask = pb.d_n; ref->planes.xmask = pb.d_x;
-        ref->xpos = pb.d_xpos; ref->xchr = pb.d_xchr; ref->n_x = n_x;
+        ref->planes.two = j->d_two; ref->planes.nmask = j->d_n; ref->planes.xmask = j->d_x;
+        ref->xpos = j->d_xpos; ref->xchr = j->d_xchr; ref->n_x = n_x;
         return 0;
     };
-    return align_staged(c, sc, out, ops_out, stats_out, t_begin);
+    return run_call(c, job, sc, stage, prep, out, ops_out, stats_out, t_begin);
 }
 
 int fadegpu_align_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
                         fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
 {
-    return pairs_call(c, "fadegpu_align_pairs", false, n_pairs, in, max_ops, out, ops_out, stats_out);
+    return pairs_call(c, "fadegpu_align_pairs", false, n_pairs, in, max_ops, out, ops_out, stats_out, nullptr);
 }
 
 int fadegpu_score_pairs(fadegpu_ctx *c, int64_t n_pairs, const fadegpu_pairs *in, fadegpu_pair_result *out,
                         fadegpu_stats *stats_out)
 {
-    return pairs_call(c, "fadegpu_score_pairs", true, n_pairs, in, 0, out, nullptr, stats_out);
+    return pairs_call(c, "fadegpu_score_pairs", true, n_pairs, in, 0, out, nullptr, stats_out, nullptr);
 }
 
 // Regions: only the queries and the intervals are staged; region_prep_kernel writes the per-region binning inputs and
 // the queries, the binning runs on the ctx's contig table and the SW kernels read the resident reference.
 static int regions_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n_regions, const fadegpu_regions *in,
-                        int32_t max_ops, fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
+                        int32_t max_ops, fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out,
+                        fadegpu_job *job)
 {
     const std::string at0 = std::string(fn) + ": ";
     if (!c) return fail(nullptr, FADEGPU_E_ARG, at0 + "null ctx");
     if (n_regions < 0 || n_regions > ((int64_t)1 << 30) || max_ops < 0)
         return fail(c, FADEGPU_E_ARG, at0 + "n_regions or max_ops out of range");
-    if (n_regions > 0 && (!in || !in->query_off || !in->tid || !in->start || !in->end || !in->strand || !out ||
-                          (max_ops > 0 && !ops_out)))
+    if (n_regions > 0 && (!in || !in->query_off || !in->tid || !in->start || !in->end || !in->strand ||
+                          (!job && (!out || (max_ops > 0 && !ops_out)))))
         return fail(c, FADEGPU_E_ARG, at0 + "null argument");
     { int rc = refuse_in_flight(c, fn); if (rc) return rc; }
     if (c->n_contigs <= 0) return fail(c, FADEGPU_E_STATE, at0 + "no reference is loaded");
@@ -1989,7 +2147,7 @@ static int regions_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t
     sc.n = n; sc.qbytes = qbytes; sc.n_over = n_over; sc.max_ops = max_ops; sc.score_only = score_only;
     sc.raw = o_q + align16((size_t)qbytes);
     sc.o_tbeg = o_start; sc.o_tend = o_end;
-    sc.stage = [&](char *h) {
+    auto stage = [&](char *h) {
         int64_t *hq = reinterpret_cast<int64_t *>(h);
         const int64_t q0 = in->query_off[0];
         for (int64_t k = 0; k <= n; ++k) hq[k] = in->query_off[k] - q0;
@@ -1999,7 +2157,8 @@ static int regions_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t
         memcpy(h + o_strand, in->strand, (size_t)n);
         if (qbytes) parallel_copy(h + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
     };
-    sc.prep = [&](fadegpu_batch *b, const char *d, BinArgs &ba, int *launches) -> int {
+    auto prep = [&](fadegpu_job *j, const char *d, BinArgs &ba, int *launches) -> int {
+        fadegpu_batch *b = j->b;
         RegionArgs ra{};
         ra.n = n;
         ra.query = d + o_q; ra.qoff = reinterpret_cast<const int64_t *>(d);
@@ -2008,27 +2167,126 @@ static int regions_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t
         ra.strand = reinterpret_cast<const uint8_t *>(d + o_strand);
         ra.seq_off = b->d_in_seq_off; ra.pos = b->d_in_pos; ra.l_qseq = b->d_in_lq; ra.tid = b->d_in_tid;
         ra.aligned_len = b->d_in_alen; ra.clip_left = b->d_in_cl; ra.clip_right = b->d_in_cr;
-        ra.seq4 = b->d_in_seq4; ra.bad = c->pairs.d_bad;
+        ra.seq4 = b->d_in_seq4; ra.bad = j->d_bad;
         CU(c, launch_region_prep(ra, c->sm_count, c->stream2));
         *launches += 1;
         // the intervals were validated above, so the window arithmetic clamps nothing: gstart = coff[tid] + start
         ba.clen = c->d_clen; ba.coff = c->d_coff; ba.n_contigs = c->n_contigs;
         return 0;
     };
-    sc.reference = [&](fadegpu_batch *, RefDev *ref, int *) -> int { *ref = ref_dev(c); return 0; };
-    return align_staged(c, sc, out, ops_out, stats_out, t_begin);
+    sc.reference = [c](fadegpu_job *, RefDev *ref, int *) -> int { *ref = ref_dev(c); return 0; };
+    return run_call(c, job, sc, stage, prep, out, ops_out, stats_out, t_begin);
 }
 
 int fadegpu_align_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regions *in, int32_t max_ops,
                           fadegpu_pair_result *out, uint32_t *ops_out, fadegpu_stats *stats_out)
 {
-    return regions_call(c, "fadegpu_align_regions", false, n_regions, in, max_ops, out, ops_out, stats_out);
+    return regions_call(c, "fadegpu_align_regions", false, n_regions, in, max_ops, out, ops_out, stats_out, nullptr);
 }
 
 int fadegpu_score_regions(fadegpu_ctx *c, int64_t n_regions, const fadegpu_regions *in, fadegpu_pair_result *out,
                           fadegpu_stats *stats_out)
 {
-    return regions_call(c, "fadegpu_score_regions", true, n_regions, in, 0, out, nullptr, stats_out);
+    return regions_call(c, "fadegpu_score_regions", true, n_regions, in, 0, out, nullptr, stats_out, nullptr);
+}
+
+// ---- jobs: queued pair and region calls ----
+
+int fadegpu_job_create(fadegpu_ctx *c, fadegpu_job **out)
+{
+    if (!c || !out) return fail(c, FADEGPU_E_ARG, "fadegpu_job_create: null argument");
+    *out = nullptr;
+    fadegpu_job *j = new (std::nothrow) fadegpu_job();
+    if (!j) return fail(c, FADEGPU_E_OOM, "fadegpu_job_create: out of host memory");
+    j->ctx = c;
+    { std::lock_guard<std::mutex> lk(c->q_mu); c->jobs.push_back(j); }
+    *out = j;
+    return FADEGPU_OK;
+}
+
+void fadegpu_job_destroy(fadegpu_job *j)
+{
+    if (!j) return;
+    fadegpu_ctx *c = j->ctx;
+    {
+        std::unique_lock<std::mutex> lk(c->q_mu);
+        c->done_cv.wait(lk, [&] { return !j->queued; });
+        if (j->in_flight) { j->in_flight = false; --c->jobs_in_flight; }
+        c->jobs.erase(std::remove(c->jobs.begin(), c->jobs.end(), j), c->jobs.end());
+    }
+    cudaSetDevice(c->device);
+    free_job(j);
+}
+
+// what every submit checks before the call's own validation: the ctx, the job's state, the job flags
+static int check_job_submit(fadegpu_ctx *c, fadegpu_job *j, const char *fn, int32_t max_ops, uint32_t job_flags)
+{
+    const std::string at = std::string(fn) + ": ";
+    if (!c || !j) return fail(c, FADEGPU_E_ARG, at + "null ctx or job");
+    if (j->ctx != c) return fail(c, FADEGPU_E_STATE, at + "the job belongs to another ctx");
+    if (job_flags & ~FADEGPU_JOB_SCORE_ONLY) return fail(c, FADEGPU_E_ARG, at + "unknown job flags");
+    if ((job_flags & FADEGPU_JOB_SCORE_ONLY) && max_ops != 0)
+        return fail(c, FADEGPU_E_ARG, at + "max_ops must be 0 with FADEGPU_JOB_SCORE_ONLY");
+    {
+        std::lock_guard<std::mutex> lk(c->q_mu);
+        if (!j->in_flight) return 0;
+    }
+    return fail(c, FADEGPU_E_STATE, at + "job already in flight (call fadegpu_job_wait)");
+}
+
+int fadegpu_submit_pairs(fadegpu_ctx *c, fadegpu_job *j, int64_t n_pairs, const fadegpu_pairs *in, int32_t max_ops,
+                         uint32_t job_flags)
+{
+    const char *fn = "fadegpu_submit_pairs";
+    { int rc = check_job_submit(c, j, fn, max_ops, job_flags); if (rc) return rc; }
+    return pairs_call(c, fn, (job_flags & FADEGPU_JOB_SCORE_ONLY) != 0, n_pairs, in, max_ops, nullptr, nullptr, nullptr, j);
+}
+
+int fadegpu_submit_regions(fadegpu_ctx *c, fadegpu_job *j, int64_t n_regions, const fadegpu_regions *in,
+                           int32_t max_ops, uint32_t job_flags)
+{
+    const char *fn = "fadegpu_submit_regions";
+    { int rc = check_job_submit(c, j, fn, max_ops, job_flags); if (rc) return rc; }
+    return regions_call(c, fn, (job_flags & FADEGPU_JOB_SCORE_ONLY) != 0, n_regions, in, max_ops, nullptr, nullptr,
+                        nullptr, j);
+}
+
+int fadegpu_job_wait(fadegpu_ctx *c, fadegpu_job *j, fadegpu_stats *stats_out)
+{
+    if (!c || !j) return fail(c, FADEGPU_E_ARG, "fadegpu_job_wait: null ctx or job");
+    if (j->ctx != c) return fail(c, FADEGPU_E_STATE, "fadegpu_job_wait: the job belongs to another ctx");
+    int rc;
+    std::string err;
+    {   // a queued device half reports its outcome here
+        std::unique_lock<std::mutex> lk(c->q_mu);
+        if (!j->in_flight) { lk.unlock(); return fail(c, FADEGPU_E_STATE, "fadegpu_job_wait: job not submitted"); }
+        c->done_cv.wait(lk, [&] { return !j->queued; });
+        j->in_flight = false;
+        --c->jobs_in_flight;
+        rc = j->rc; err = j->err;
+        j->rc = 0;
+    }
+    if (rc) return fail(c, rc, err);
+    CU(c, cudaSetDevice(c->device));
+    { int r = finish_job(c, j); if (r) return r; }
+    j->n_res = j->sc.n;
+    if (stats_out) *stats_out = j->st;
+    return FADEGPU_OK;
+}
+
+int fadegpu_job_results_view(const fadegpu_job *j, fadegpu_job_results *r)
+{
+    if (!j || !r) return fail(j ? j->ctx : nullptr, FADEGPU_E_ARG, "fadegpu_job_results_view: null argument");
+    bool in_flight;
+    { std::lock_guard<std::mutex> lk(j->ctx->q_mu); in_flight = j->in_flight; }
+    if (in_flight) return fail(j->ctx, FADEGPU_E_STATE, "fadegpu_job_results_view: job in flight (call fadegpu_job_wait)");
+    const int64_t n = std::max<int64_t>(0, j->n_res);
+    r->n = n;
+    r->records = n > 0 ? j->h_res : nullptr;
+    r->ops = n > 0 && j->sc.max_ops > 0 ? j->h_ops : nullptr;
+    r->max_ops = j->n_res >= 0 ? j->sc.max_ops : 0;
+    r->reserved = 0;
+    return FADEGPU_OK;
 }
 
 int fadegpu_measure_alu_peak(fadegpu_ctx *c, double *ops_per_sec_out, double *sm_clock_mhz_out)

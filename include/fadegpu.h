@@ -25,8 +25,9 @@
  * never throws or aborts.  There is NO CPU fallback: without a CUDA device (or with the kernels
  * failing to launch) calls fail with FADEGPU_E_CUDA / FADEGPU_E_NODEV.
  * Threading: a ctx (and its batches) is driven by one host thread at a time; distinct ctxs may be
- * driven concurrently.  A ctx owns one helper thread (started by the first fadegpu_submit) that
- * plans and launches queued batches.  All buffers handed out are owned by the library.
+ * driven concurrently.  A ctx owns one helper thread (started by the first queued submit of a batch
+ * or a job) that plans and launches queued batches and jobs.  All buffers handed out are owned by
+ * the library.
  */
 #ifndef FADEGPU_H
 #define FADEGPU_H
@@ -344,6 +345,59 @@ int fadegpu_score_pairs(fadegpu_ctx *ctx, int64_t n_pairs, const fadegpu_pairs *
                         fadegpu_pair_result *out, fadegpu_stats *stats_out);
 int fadegpu_score_regions(fadegpu_ctx *ctx, int64_t n_regions, const fadegpu_regions *in,
                           fadegpu_pair_result *out, fadegpu_stats *stats_out);
+
+/* ---- Jobs: pair and region calls submitted now and collected later, several in flight on one ctx ----
+ * A job is one fadegpu_align_* / fadegpu_score_* call split in two: fadegpu_submit_pairs / fadegpu_submit_regions stage
+ *   the inputs, upload them and start the binning, then return; the ctx's helper thread plans and launches the kernels
+ *   and queues the records home; fadegpu_job_wait blocks until they are there.  While the host stages job k+1, the GPU
+ *   runs job k: the upload and binning of k+1 and the result copies of k-1 overlap the kernels of k.  The device work
+ *   of a job is exactly the synchronous call's.
+ * Results: after fadegpu_job_wait, fadegpu_job_results_view gives the records (in PAIR / REGION ORDER) and the ops,
+ *   byte-identical to those of the synchronous call on the same input, ctx and flags: fadegpu_align_pairs /
+ *   fadegpu_align_regions, or with FADEGPU_JOB_SCORE_ONLY fadegpu_score_pairs / fadegpu_score_regions (max_ops must then
+ *   be 0).  Letters, empty and oversize items, max_ops / FADEGPU_R_OPS_TRUNC and the ctx's flags all follow that call.
+ *   The view points into pinned memory owned by the job, where the result copies land; it stays valid until the job's
+ *   next submit or its destroy.  While the job is in flight the view call fails with FADEGPU_E_STATE; before the
+ *   first successful wait it gives n = 0.
+ * Inputs: host arrays (pageable is fine), read only during the submit, which copies them into the job's pinned staging:
+ *   the caller may overwrite them as soon as it returns.
+ * Errors: the host-side checks run at submit, with the FADEGPU_E_ARG cases and messages of the synchronous call under
+ *   the submit function's name; a refused submit leaves the job idle.  Errors found on the device (a query letter
+ *   outside nt16, the internal "no result record" check) are returned by fadegpu_job_wait of that job only, with the
+ *   synchronous messages; other jobs in flight are not affected.  FADEGPU_E_STATE: a submit of a job in flight, a wait
+ *   on a job not submitted since its last wait, a region submit with no reference loaded, a job used with a ctx other
+ *   than its own, a job submit while an annotate batch of the ctx is in flight, and fadegpu_submit /
+ *   fadegpu_submit_compact / fadegpu_submit_inputs while a job of the ctx is in flight.  Batches and jobs are not in
+ *   flight together; waited batches keep their results and fadegpu_replay_* keep working.
+ * Synchronous calls made while jobs are in flight run after them, in submit order; their records do not change.
+ * FADEGPU_F_SYNC_SUBMIT: a submit plans and launches on the calling thread, and device-found errors are returned by the
+ *   submit itself (the job is then idle).
+ * Stats (fadegpu_job_wait's stats_out, may be NULL): the fields the synchronous call fills.  n_*, cells, h2d_bytes,
+ *   d2h_bytes and kernel_launches equal the synchronous call's; kernel_ms and total_ms come from the job's own events
+ *   and can include overlapped work of neighbouring jobs; host_submit_ms is the wall time of the submit call.
+ * Lifetime: fadegpu_job_destroy waits for the job first if it is in flight.  fadegpu_destroy waits for the jobs in
+ *   flight and frees every job of the ctx (their handles are then invalid).  The helper thread is the ctx's one, started
+ *   by its first queued submit of either kind and joined by fadegpu_destroy.  A ctx and its jobs are driven by one host
+ *   thread at a time. */
+typedef struct fadegpu_job fadegpu_job;             /* opaque: staging, device buffers and pinned records of one call */
+int fadegpu_job_create(fadegpu_ctx *ctx, fadegpu_job **out);
+void fadegpu_job_destroy(fadegpu_job *job);
+
+#define FADEGPU_JOB_SCORE_ONLY 1u                  /* the fadegpu_score_* semantics: score and end cell, no traceback */
+int fadegpu_submit_pairs(fadegpu_ctx *ctx, fadegpu_job *job, int64_t n_pairs, const fadegpu_pairs *in,
+                         int32_t max_ops, uint32_t job_flags);
+int fadegpu_submit_regions(fadegpu_ctx *ctx, fadegpu_job *job, int64_t n_regions, const fadegpu_regions *in,
+                           int32_t max_ops, uint32_t job_flags);
+int fadegpu_job_wait(fadegpu_ctx *ctx, fadegpu_job *job, fadegpu_stats *stats_out);
+
+typedef struct fadegpu_job_results {
+    int64_t n;                                      /* items of the last submit */
+    const fadegpu_pair_result *records;             /* [n], item order; NULL when n == 0 */
+    const uint32_t *ops;                            /* [n * max_ops], as ops_out of the synchronous call; NULL when
+                                                       max_ops == 0 or n == 0 */
+    int32_t max_ops, reserved;
+} fadegpu_job_results;                              /* 32 bytes */
+int fadegpu_job_results_view(const fadegpu_job *job, fadegpu_job_results *r);
 
 /* INT16x2 ALU roofline denominator (SURVEY 8d): measures packed VIMNMX/VIADDMNMX issue rate.
  * ops_per_sec_out = packed (2-lane) instructions * 32 threads per second over the whole GPU. */

@@ -43,6 +43,24 @@ def line(name, rnd, n, wall, st):
           f"h2d {st.h2d_bytes} B, d2h {st.d2h_bytes} B, {st.kernel_launches} launches, {st.n_generic} generic")
 
 
+def c2_alignments(ctx, rd, ref):
+    """one annotate batch of the reads rd on ctx (reference ref loaded), and every alignment it ran: (batch, read
+    indices, forward letters, reverse-complement letters, window letters, window starts, window ends)"""
+    b = ctx.alloc_batch(rd.n, int(rd.seq_off[rd.n]))
+    b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right).run()
+    al = np.nonzero(b.flags[:rd.n] & api.R_ALIGNED)[0]
+    W = ctx.params.window_size
+    fwd, rcs, ts = [], [], []
+    starts = b.win_start[al].astype(np.int64)
+    ends = np.minimum(rd.pos[al] + rd.aligned_len[al] + W, len(ref)).astype(np.int64)
+    for r, s, e in zip(al, starts, ends):
+        so, lq = int(rd.seq_off[r]), int(rd.l_qseq[r])
+        fwd.append(orc.decode_nt16(rd.seq4[so:so + (lq + 1) // 2], lq))
+        rcs.append(orc.revcomp_nt16(rd.seq4[so:so + (lq + 1) // 2], lq))
+        ts.append(ref[int(s):int(e)])
+    return b, al, fwd, rcs, ts, starts, ends
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--reads", type=int, default=1_000_000)
@@ -60,18 +78,7 @@ def main():
           f"generated in {time.time() - t0:.1f} s")
     with Context(0) as ctx:
         ctx.load_reference(["chrS"], [ref])
-        b = ctx.alloc_batch(rd.n, int(rd.seq_off[rd.n]))
-        b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right).run()
-        al = np.nonzero(b.flags[:rd.n] & api.R_ALIGNED)[0]
-        W = ctx.params.window_size
-        fwd, rcs, ts = [], [], []
-        starts = b.win_start[al].astype(np.int64)
-        ends = np.minimum(rd.pos[al] + rd.aligned_len[al] + W, len(ref)).astype(np.int64)
-        for r, s, e in zip(al, starts, ends):
-            so, lq = int(rd.seq_off[r]), int(rd.l_qseq[r])
-            fwd.append(orc.decode_nt16(rd.seq4[so:so + (lq + 1) // 2], lq))
-            rcs.append(orc.revcomp_nt16(rd.seq4[so:so + (lq + 1) // 2], lq))
-            ts.append(ref[int(s):int(e)])
+        b, al, fwd, rcs, ts, starts, ends = c2_alignments(ctx, rd, ref)
         rq, rqo, tids, starts, ends, strands = api.pack_regions(fwd, np.zeros(len(al)), starts, ends, np.ones(len(al)))
         q, qo, t, to = api.pack_pairs(rcs, ts)
         n = len(al)
