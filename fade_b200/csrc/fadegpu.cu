@@ -9,8 +9,9 @@
 // result_index_kernel and the copies home on `stream3`.  FADEGPU_F_HOST_BINNING keeps the first
 // implementation, which evaluates the floor and the windows and sorts on the host.
 // A pair or region call (fadegpu_align_* / fadegpu_score_*, or a job of fadegpu_submit_pairs / _regions) is a stage
-// half on the caller's thread (staging, upload, prep and classify on stream2) and a device half (plan, scatter, kernels,
-// results on stream3), which the ctx thread runs for jobs.
+// half on the caller's thread (stage_call: staging, upload, prep and classify on stream2) and a device half
+// (launch_job: plan, scatter, kernels, results on stream3), which the ctx thread runs for jobs.  A device-binned submit
+// and the two halves of a call run one binning sequence on their BinState.
 // There is no CPU fallback: every compute entry point needs a CUDA device.
 #include <cuda_runtime.h>
 #include <algorithm>
@@ -119,12 +120,53 @@ struct StagedCall {
     std::function<int(fadegpu_job *j, RefDev *ref, int *launches)> reference;
 };
 
-// One pair or region call: an internal batch (descriptors, binning arrays, result records), the staging of the raw
-// inputs, the targets of a pair call packed as a reference of their own, the records and ops of the call in pinned
-// memory (fadegpu_job_results_view).  Everything grows with use.
+struct Launch {
+    int R;            // 13/19/32 = packed kernels, 0 = generic list
+    int aln_first, n_aln;
+    int item_first, n_items;
+    int tw_stride;
+    int nblk_max;
+    int qmax, tmax;   // generic only
+};
+
+// The device-binning core of an annotate batch and of a pair / region job: the binning inputs on the device, the
+// histogram and the launch plan built from it, the sorted descriptors, the result records and the events that order
+// them (alloc_bin_state, free_bin_state).
+struct BinState {
+    int64_t max_items = 0, max_seq_bytes = 0, cap_items = 0;   // (cap_items: warp items)
+    // binning inputs; d_in_seq4: 16-byte slots that keep the source's alignment phase
+    uint8_t *d_in_seq4 = nullptr;
+    int64_t *d_in_seq_off = nullptr, *d_in_pos = nullptr;
+    int32_t *d_in_lq = nullptr, *d_in_tid = nullptr, *d_in_alen = nullptr, *d_in_cl = nullptr, *d_in_cr = nullptr;
+    // classify and scatter
+    int32_t *d_key = nullptr, *d_tlen = nullptr, *d_hist = nullptr, *d_keybase = nullptr, *d_cursor = nullptr;
+    int64_t *d_start = nullptr, *d_aln_start = nullptr, *d_src_off = nullptr;
+    int32_t *d_over = nullptr, *h_over = nullptr;      // items left unaligned because their window exceeds 2^31 cells
+    unsigned long long *d_stats = nullptr, *h_stats = nullptr;
+    int32_t *h_hist = nullptr, *h_keybase = nullptr;   // (h_*: pinned)
+    BinArgs ba{};                                      // the binning of the last submit (for replays); n == 0: none
+    // launch plan, descriptors in sorted order, result records
+    std::vector<Launch> plan;
+    std::vector<int32_t> sorted_tlen;
+    int64_t n_aln = 0, n_items = 0, n_generic = 0, scratch_bytes = 0;
+    AlnDesc *d_aln = nullptr;
+    WarpItem *h_items = nullptr, *d_items = nullptr;
+    AlnOut *d_out = nullptr;
+    uint32_t *d_flags = nullptr;
+    uint2 *d_fillres = nullptr;
+    // start of the uploads, first fill may start (compute stream), end of the kernels, results home,
+    // inputs ready (upload stream), end of the last fill
+    cudaEvent_t ev[6] = { nullptr, nullptr, nullptr, nullptr, nullptr, nullptr };
+    cudaEvent_t ev_prep = nullptr, ev_ready = nullptr;   // histogram home / descriptors ready (upload stream)
+    cudaEvent_t ev_kernels = nullptr;                    // end of the kernels (recorded on tstream)
+};
+
+// One pair or region call: its device-binning core, the staging of the raw inputs, the targets of a pair call packed
+// as a reference of their own, the records and ops of the call in pinned memory (fadegpu_job_results_view).
+// Everything grows with use.
 struct fadegpu_job {
     fadegpu_ctx *ctx = nullptr;
-    fadegpu_batch *b = nullptr;
+    BinState bs;
     char *h_stage = nullptr, *d_raw = nullptr;          // pinned staging / device copy of offsets + ASCII
     size_t stage_bytes = 0, raw_bytes = 0;
     uint32_t *d_two = nullptr, *d_n = nullptr, *d_x = nullptr, *d_chunk_x = nullptr;
@@ -137,7 +179,7 @@ struct fadegpu_job {
     size_t spill_bytes = 0, ops_bytes = 0;
     fadegpu_pair_result *d_res = nullptr;
     size_t res_bytes = 0;
-    int32_t *d_bad = nullptr;
+    int32_t *d_bad = nullptr, *h_bad = nullptr;         // lowest item index with a bad query letter (h_bad: pinned)
     fadegpu_pair_result *h_res = nullptr;               // pinned records and ops of the last submit
     uint32_t *h_ops = nullptr;
     size_t h_res_bytes = 0, h_ops_bytes = 0;
@@ -163,56 +205,30 @@ struct AlnTmp {       // a read that needs SW, captured in read order (sequentia
     uint32_t clip_left, clip_right;
 };
 
-struct Launch {
-    int R;            // 13/19/32 = packed kernels, 0 = generic list
-    int aln_first, n_aln;
-    int item_first, n_items;
-    int tw_stride;
-    int nblk_max;
-    int qmax, tmax;   // generic only
-};
-
 struct fadegpu_batch {
     fadegpu_ctx *ctx = nullptr;
     fadegpu_batch_view v{};
-    // staging (pinned) and device mirrors
-    AlnDesc *h_aln = nullptr, *d_aln = nullptr;
-    WarpItem *h_items = nullptr, *d_items = nullptr;
-    uint8_t *h_seq = nullptr, *d_seq = nullptr;
-    AlnOut *h_out = nullptr, *d_out = nullptr;
-    uint32_t *d_flags = nullptr;
-    uint2 *d_fillres = nullptr;
-    int64_t cap_items = 0, cap_seq = 0;
-    std::vector<Launch> plan;
-    int64_t n_reads = 0, n_aln = 0, n_items = 0, seq_bytes = 0;
-    int qmax_all = 0, tmax_all = 0;
+    BinState bs;
+    AlnOut *h_out = nullptr;                   // [max_reads] pinned result records
+    int64_t n_reads = 0;
     fadegpu_stats st{};
-    // start of the uploads, first fill may start (compute stream), end of the kernels, results home,
-    // inputs ready (upload stream), end of the last fill
-    cudaEvent_t ev[6] = { nullptr, nullptr, nullptr, nullptr, nullptr, nullptr };
     bool in_flight = false;
-    // scratch for the host binning
+    // host binning: staging (pinned descriptors and bases, allocated on first use) and scratch
+    AlnDesc *h_aln = nullptr;
+    uint8_t *h_seq = nullptr, *d_seq = nullptr;
+    int64_t cap_seq = 0;
     std::vector<std::vector<AlnTmp>> tl_aln;   // per host thread
     std::vector<uint32_t> order;               // alignment indices sorted by (class, window length desc)
     int32_t *h_ridx = nullptr;                 // [max_reads] per read: index into the results, -1 = none
     std::vector<AlnTmp> all_aln;
     std::vector<int32_t> cnt;
     std::vector<int64_t> soff, aln_start;
-    std::vector<int32_t> sorted_tlen;
     // ---- device-side binning (submits from the pinned view) ----
     bool dev_binning = false;          // the last submit used it
-    uint8_t *d_in_seq4 = nullptr;
-    int64_t *d_in_seq_off = nullptr, *d_in_pos = nullptr, *d_start = nullptr, *d_aln_start = nullptr;
-    int32_t *d_in_lq = nullptr, *d_in_tid = nullptr, *d_in_alen = nullptr, *d_in_cl = nullptr, *d_in_cr = nullptr;
-    int32_t *d_key = nullptr, *d_tlen = nullptr, *d_hist = nullptr, *d_keybase = nullptr, *d_cursor = nullptr;
     int32_t *d_ridx = nullptr;                         // per read: index into the results (built on the device, copied home)
     uint8_t *d_rflags = nullptr;
     uint8_t *d_gate = nullptr;                         // compact inputs: the one byte per read that is uploaded
     const uint4 *d_view_meta = nullptr;                // device address of the pinned view's 32-byte records
-    int32_t *d_over = nullptr, *h_over = nullptr;      // reads left unaligned because their window exceeds 2^31 cells
-    unsigned long long *d_stats = nullptr;
-    int32_t *h_hist = nullptr, *h_keybase = nullptr;   // pinned
-    unsigned long long *h_stats = nullptr;            // pinned
     int64_t *h_aln_start = nullptr;                   // pinned
     // reads that pass the length floor, gathered by the host in read order (pinned, allocated on first use)
     uint8_t *h_c_seq4 = nullptr;
@@ -221,17 +237,12 @@ struct fadegpu_batch {
     int32_t *d_in_read = nullptr;
     int64_t n_c = 0, seq_c = 0;                        // gathered reads / their sequence bytes
     bool pulled = false;
-    int64_t *d_src_off = nullptr;
     const uint8_t *d_view_seq4 = nullptr;              // device address of the pinned view's seq4
     std::vector<int32_t> idx;                          // gather scratch
-    BinArgs ba{};                                      // the binning of the last submit (for replays)
-    bool ba_valid = false;
     AlnDesc *d_aln_scratch = nullptr;                  // replays scatter into these instead of the live descriptors
     int64_t *d_i64_scratch = nullptr;
-    cudaEvent_t ev_prep = nullptr, ev_ready = nullptr;
     int mode = 0;                                      // SubmitMode of the queued / last submit
     int64_t job_seq_bytes = 0;
-    cudaEvent_t ev_kernels = nullptr;                  // end of the batch's kernels (recorded on tstream)
     // asynchronous submit (guarded by ctx->q_mu)
     bool queued = false;
     int submit_rc = 0;
@@ -277,12 +288,67 @@ void free_reference(fadegpu_ctx *c)
     c->names.clear(); c->clen.clear(); c->coff.clear();
 }
 
-// the job must not be queued; fadegpu_free_batch waits for the ctx's streams before anything is freed
+// an allocated core is freed once the ctx's streams are done with whatever they have queued
+void free_bin_state(fadegpu_ctx *c, BinState &s)
+{
+    if (s.max_items) {
+        cudaSetDevice(c->device);
+        for (cudaStream_t q : { c->stream, c->tstream, c->stream2, c->stream3 }) if (q) cudaStreamSynchronize(q);
+    }
+    free_host(s.h_items); free_dev(s.d_aln); free_dev(s.d_items); free_dev(s.d_out); free_dev(s.d_flags); free_dev(s.d_fillres);
+    free_dev(s.d_in_seq4); free_dev(s.d_in_seq_off); free_dev(s.d_in_pos); free_dev(s.d_in_lq); free_dev(s.d_in_tid);
+    free_dev(s.d_in_alen); free_dev(s.d_in_cl); free_dev(s.d_in_cr); free_dev(s.d_key); free_dev(s.d_tlen); free_dev(s.d_start);
+    free_dev(s.d_aln_start); free_dev(s.d_src_off); free_dev(s.d_hist); free_dev(s.d_keybase); free_dev(s.d_cursor);
+    free_dev(s.d_over); free_host(s.h_over); free_dev(s.d_stats);
+    free_host(s.h_hist); free_host(s.h_keybase); free_host(s.h_stats);
+    for (cudaEvent_t e : { s.ev_prep, s.ev_ready, s.ev_kernels }) if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : s.ev) if (e) cudaEventDestroy(e);
+    s = BinState{};
+}
+
+// Allocates the core and wires s.ba to its arrays (the caller sets the rest of s.ba before each classify); on failure
+// nothing stays allocated.
+int alloc_bin_state(fadegpu_ctx *c, BinState &s, int64_t max_items, int64_t max_seq_bytes)
+{
+    const size_t n = (size_t)max_items;
+    s.cap_items = (max_items + 7) / 8 + 8;
+    cudaError_t e = cudaSuccess;
+    auto H = [&](auto **p, size_t bytes) { if (e == cudaSuccess) e = cudaHostAlloc((void **)p, std::max<size_t>(bytes, 16), cudaHostAllocDefault); };
+    auto D = [&](auto **p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc((void **)p, std::max<size_t>(bytes, 16)); };
+    H(&s.h_items, (size_t)s.cap_items * sizeof(WarpItem));
+    D(&s.d_aln, n * sizeof(AlnDesc)); D(&s.d_items, (size_t)s.cap_items * sizeof(WarpItem));
+    D(&s.d_out, n * sizeof(AlnOut)); D(&s.d_flags, n * 4);
+    D(&s.d_fillres, (size_t)s.cap_items * 32 * sizeof(uint2));
+    D(&s.d_in_seq4, (size_t)max_seq_bytes + 32 * n + 16); D(&s.d_in_seq_off, (n + 1) * 8); D(&s.d_in_pos, n * 8);
+    D(&s.d_in_lq, n * 4); D(&s.d_in_tid, n * 4); D(&s.d_in_alen, n * 4); D(&s.d_in_cl, n * 4); D(&s.d_in_cr, n * 4);
+    D(&s.d_key, n * 4); D(&s.d_tlen, n * 4); D(&s.d_start, n * 8); D(&s.d_aln_start, n * 8); D(&s.d_src_off, n * 8);
+    D(&s.d_hist, (size_t)BIN_KEYS * 4); D(&s.d_keybase, (size_t)BIN_KEYS * 4); D(&s.d_cursor, (size_t)BIN_KEYS * 4);
+    D(&s.d_over, (size_t)OVER_CAP * 4); H(&s.h_over, (size_t)OVER_CAP * 4); D(&s.d_stats, 128);
+    H(&s.h_hist, (size_t)BIN_KEYS * 4); H(&s.h_keybase, (size_t)BIN_KEYS * 4); H(&s.h_stats, 128);
+    if (e == cudaSuccess) e = cudaEventCreate(&s.ev_prep);
+    if (e == cudaSuccess) e = cudaEventCreate(&s.ev_ready);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s.ev_kernels, cudaEventDisableTiming);
+    for (auto &ev : s.ev) if (e == cudaSuccess) e = cudaEventCreate(&ev);
+    if (e != cudaSuccess) {
+        free_bin_state(c, s);
+        return cuda_fail(c, e, "fadegpu_alloc_batch");   // (a job's core grows through the same allocation)
+    }
+    s.max_items = max_items; s.max_seq_bytes = max_seq_bytes;
+    BinArgs &ba = s.ba;
+    ba.seq4 = s.d_in_seq4; ba.seq_off = s.d_in_seq_off; ba.l_qseq = s.d_in_lq; ba.tid = s.d_in_tid; ba.pos = s.d_in_pos;
+    ba.aligned_len = s.d_in_alen; ba.clip_left = s.d_in_cl; ba.clip_right = s.d_in_cr;
+    ba.src_off = s.d_src_off; ba.over_list = s.d_over;
+    ba.key = s.d_key; ba.tlen = s.d_tlen; ba.start = s.d_start; ba.hist = s.d_hist; ba.stats = s.d_stats;
+    ba.keybase = s.d_keybase; ba.cursor = s.d_cursor; ba.aln = s.d_aln; ba.aln_start = s.d_aln_start;
+    return 0;
+}
+
+// the job must not be queued; the ctx's streams are synchronised before anything is freed
 void free_job(fadegpu_job *j)
 {
     if (!j) return;
-    if (j->b) fadegpu_free_batch(j->b);
-    free_host(j->h_stage); free_host(j->h_res); free_host(j->h_ops);
+    free_bin_state(j->ctx, j->bs);
+    free_host(j->h_stage); free_host(j->h_res); free_host(j->h_ops); free_host(j->h_bad);
     free_dev(j->d_raw); free_dev(j->d_two); free_dev(j->d_n); free_dev(j->d_x); free_dev(j->d_chunk_x);
     free_dev(j->d_xpos); free_dev(j->d_xchr); free_dev(j->d_clen); free_dev(j->d_coff); free_dev(j->d_spill);
     free_dev(j->d_ops); free_dev(j->d_res); free_dev(j->d_bad);
@@ -355,14 +421,14 @@ size_t gen_slot_bytes(int qmax, int tmax)
 
 // Launch plan from the sorted order: cls_first[rk] = first sorted position of row class rk (the
 // generic list is rank N_ROW_CLASSES), sorted_tlen[pos] = window length at sorted position pos.
-// Fills b->plan, b->h_items and grows the ctx scratch buffers.
-int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *cls_first, const int32_t *sorted_tlen,
+// Fills s.plan, s.h_items and grows the ctx scratch buffers.
+int build_plan(fadegpu_ctx *c, BinState &s, int64_t n_aln, const int64_t *cls_first, const int32_t *sorted_tlen,
                int qmax_all, int tmax_all, int gen_qmax, int gen_tmax)
 {
     int64_t n_items = 0;
     size_t ck_needed = 0, gen_needed = 0, trace_needed = 0;
-    b->plan.clear();
-    b->st.n_generic = 0;
+    s.plan.clear();
+    s.n_generic = 0;
     for (int rk = 0; rk <= N_ROW_CLASSES; ++rk) {
         const int R = rk < N_ROW_CLASSES ? ROW_CLASSES[rk] : 0;
         const int64_t first_aln = cls_first[rk], last_aln = cls_first[rk + 1];
@@ -370,9 +436,9 @@ int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *c
         if (R == 0) {
             Launch L{};
             L.R = 0; L.aln_first = (int)first_aln; L.n_aln = (int)(last_aln - first_aln); L.qmax = gen_qmax; L.tmax = gen_tmax;
-            b->plan.push_back(L);
+            s.plan.push_back(L);
             gen_needed = std::max(gen_needed, gen_slot_bytes(gen_qmax, gen_tmax));
-            b->st.n_generic += last_aln - first_aln;
+            s.n_generic += last_aln - first_aln;
             continue;
         }
         // warp items of 8 alignments; split into launches that fit the checkpoint scratch
@@ -388,8 +454,8 @@ int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *c
                 const int nblk = num_blocks(sorted_tlen[a1]);  // longest of the 8 (sorted descending)
                 const size_t wds = (size_t)(nblk - 1) * cw * 32;
                 if (a1 > a0 && (words + wds) * 4 > (size_t)c->p.scratch_bytes) break;
-                if (n_items >= b->cap_items) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: internal error (item capacity)");
-                WarpItem &it = b->h_items[n_items++];
+                if (n_items >= s.cap_items) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: internal error (item capacity)");
+                WarpItem &it = s.h_items[n_items++];
                 it.ck_off = (int64_t)words;
                 it.first = (int32_t)(a1 - a0);
                 it.nblk = (int16_t)nblk;
@@ -405,17 +471,15 @@ int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *c
             L.nblk_max = nblk_max;
             ck_needed = std::max(ck_needed, words * 4);
             trace_needed = std::max(trace_needed, trace_scratch_bytes(R, L.n_aln));
-            b->plan.push_back(L);
+            s.plan.push_back(L);
             a0 = a1;
         }
     }
-    b->n_aln = n_aln; b->n_items = n_items;
-    b->qmax_all = qmax_all; b->tmax_all = tmax_all;
-    b->st.n_aligned = n_aln;
-    b->st.scratch_bytes = (int64_t)ck_needed;
+    s.n_aln = n_aln; s.n_items = n_items;
+    s.scratch_bytes = (int64_t)ck_needed;
     // a slot for wildcard alignments discovered on the device, sized for the largest problem
     if (n_aln > 0) gen_needed = std::max(gen_needed, gen_slot_bytes(qmax_all, tmax_all));
-    for (int l = 0; l < (b->plan.empty() ? 0 : c->n_sets); ++l) {
+    for (int l = 0; l < (s.plan.empty() ? 0 : c->n_sets); ++l) {
         fadegpu_ctx::ScratchSet &ln = c->scratch[l];
         if (ck_needed) { int rc = ensure_dev(c, (void **)&ln.d_ck, &ln.ck_bytes, ck_needed); if (rc) return rc; }
         if (trace_needed) { int rc = ensure_dev(c, (void **)&ln.d_trace, &ln.trace_bytes, trace_needed); if (rc) return rc; }
@@ -428,28 +492,30 @@ int build_plan(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln, const int64_t *c
     return 0;
 }
 
-// Queue every kernel of the batch's plan: fills on c->stream (after `dep`: the batch's inputs, or the
-// start of a timed replay), traceback + generic on c->tstream, consecutive launches on alternating
-// scratch sets.  On return b->ev_kernels marks the end of the batch's kernels; the caller joins it.
-// With stage timers every launch is synchronised.
-// What a plan runs against: the resident reference (submits) or the packed targets of a pair call, whether alignments
-// whose score rules out both predicates skip the traceback (FADEGPU_F_TAGS_ONLY), and the optional full-CIGAR spill
-// rings (ops_cap words per alignment of the batch, in its sorted order).  end_only (score-only calls): no alignment is
-// traced back; the traceback launches only find the end cell.
+// What a plan runs against: the resident reference (submits) or the packed targets of a pair call, the query bases its
+// descriptors point into, whether alignments whose score rules out both predicates skip the traceback
+// (FADEGPU_F_TAGS_ONLY), and the optional full-CIGAR spill rings (ops_cap words per alignment, in sorted order).
+// end_only (score-only calls): no alignment is traced back; the traceback launches only find the end cell.
 struct PlanTarget {
     RefDev ref;
+    const uint8_t *seq;
     int tags_only;
     uint32_t *ops_spill;
     int ops_cap;
     bool end_only;
 };
 
-PlanTarget batch_target(const fadegpu_ctx *c)
+// an annotate batch's plan: its queries are staged by the host binning (d_seq) or in the device mirror (d_in_seq4)
+PlanTarget batch_target(const fadegpu_ctx *c, const fadegpu_batch *b)
 {
-    return PlanTarget{ ref_dev(c), (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0, nullptr, 0, false };
+    return PlanTarget{ ref_dev(c), b->dev_binning ? b->bs.d_in_seq4 : b->d_seq, (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0,
+                       nullptr, 0, false };
 }
 
-int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill_ms, float *trace_ms, float *gen_ms,
+// Queue every kernel of the plan: fills on c->stream (after `dep`: the inputs, or the start of a timed replay),
+// traceback + generic on c->tstream, consecutive launches on alternating scratch sets.  On return bs.ev_kernels marks
+// the end of the kernels; the caller joins it.  With stage timers every launch is synchronised.
+int run_plan(fadegpu_ctx *c, BinState &bs, const PlanTarget &pt, float *fill_ms, float *trace_ms, float *gen_ms,
              int *launches, cudaEvent_t dep)
 {
     const bool timed = fill_ms != nullptr;
@@ -461,24 +527,23 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill
     int nl = 0;
     cudaStream_t sf = c->stream, st = c->tstream;
     if (dep) CU(c, cudaStreamWaitEvent(sf, dep, 0));
-    for (const Launch &L : b->plan) {
+    for (const Launch &L : bs.plan) {
         fadegpu_ctx::ScratchSet &ln = c->scratch[c->next_set++ % (unsigned)c->n_sets];
         // the scratch set is free again once its previous traceback is through
         if (ln.used) CU(c, cudaStreamWaitEvent(sf, ln.ev_trace, 0));
         ln.used = true;
-        const uint8_t *seq = b->dev_binning ? b->d_in_seq4 : b->d_seq;
         if (L.R != 0) {
             KernelArgs a;
-            a.aln = b->d_aln + L.aln_first;
+            a.aln = bs.d_aln + L.aln_first;
             a.n_aln = L.n_aln;
-            a.items = b->d_items + L.item_first;
+            a.items = bs.d_items + L.item_first;
             a.n_items = L.n_items;
-            a.seq = seq;
+            a.seq = pt.seq;
             a.ref = pt.ref;
             a.ck = ln.d_ck;
-            a.fillres = b->d_fillres + (size_t)L.item_first * 32;
-            a.aln_flags = b->d_flags + L.aln_first;
-            a.out = b->d_out + L.aln_first;
+            a.fillres = bs.d_fillres + (size_t)L.item_first * 32;
+            a.aln_flags = bs.d_flags + L.aln_first;
+            a.out = bs.d_out + L.aln_first;
             a.k = c->k;
             a.min_length = c->p.min_length;
             a.tw_stride = L.tw_stride;
@@ -533,8 +598,8 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill
             CU(c, cudaEventRecord(ln.ev_trace, st));
         } else {
             GenericArgs ga;
-            ga.aln = b->d_aln + L.aln_first; ga.n_aln = L.n_aln; ga.aln_flags = nullptr; ga.seq = seq;
-            ga.ref = pt.ref; ga.out = b->d_out + L.aln_first; ga.cursor = ln.d_cursor; ga.scratch = ln.d_gen;
+            ga.aln = bs.d_aln + L.aln_first; ga.n_aln = L.n_aln; ga.aln_flags = nullptr; ga.seq = pt.seq;
+            ga.ref = pt.ref; ga.out = bs.d_out + L.aln_first; ga.cursor = ln.d_cursor; ga.scratch = ln.d_gen;
             ga.qmax = L.qmax; ga.tmax = L.tmax;
             ga.slot_bytes = (int64_t)gen_slot_bytes(L.qmax, L.tmax);
             ga.n_slots = (int)std::max<size_t>(1, std::min<size_t>(GEN_SLOTS_MAX, ln.gen_bytes / (size_t)ga.slot_bytes));
@@ -560,17 +625,87 @@ int run_plan(fadegpu_ctx *c, fadegpu_batch *b, const PlanTarget &pt, float *fill
         }
     }
     if (timed) { cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(e2); }
-    CU(c, cudaEventRecord(b->ev[5], sf));          // end of the batch's last fill (timeline diagnostics)
+    CU(c, cudaEventRecord(bs.ev[5], sf));          // end of the batch's last fill (timeline diagnostics)
     // every launch ends on tstream, in launch order: its tail is the batch's
-    CU(c, cudaEventRecord(b->ev_kernels, b->plan.empty() ? sf : st));
+    CU(c, cudaEventRecord(bs.ev_kernels, bs.plan.empty() ? sf : st));
     if (launches) *launches = nl;
     return 0;
 }
 
-// the stream `s` continues after the batch's kernels
-int join_kernels(fadegpu_ctx *c, fadegpu_batch *b, cudaStream_t s)
+// ---- The device-binning sequence of a device-binned submit and of a pair / region call, in the order the stream
+// overlap of DESIGN.md 4.4 and 4.10 depends on: bin_zero, (caller's prep) bin_classify, (host waits for ev_prep)
+// plan_from_histogram, bin_scatter, (caller records ev_ready) run_kernels. ----
+
+// on stream2, before the classify kernel and anything else that counts into the stats
+int bin_zero(fadegpu_ctx *c, BinState &s)
 {
-    CU(c, cudaStreamWaitEvent(s, b->ev_kernels, 0));
+    CU(c, cudaMemsetAsync(s.d_hist, 0, (size_t)BIN_KEYS * 4, c->stream2));
+    CU(c, cudaMemsetAsync(s.d_cursor, 0, (size_t)BIN_KEYS * 4, c->stream2));
+    CU(c, cudaMemsetAsync(s.d_stats, 0, 128, c->stream2));
+    return 0;
+}
+
+// Classify on stream2, then the histogram, the stats and `list_bytes` of the caller's list (a batch's over-list, a
+// job's bad-letter slot) go home; ev_prep marks their arrival.
+int bin_classify(fadegpu_ctx *c, BinState &s, void *h_list, const void *d_list, size_t list_bytes)
+{
+    cudaStream_t s2 = c->stream2;
+    CU(c, launch_bin_classify(s.ba, c->sm_count, s2));
+    CU(c, cudaMemcpyAsync(s.h_hist, s.d_hist, (size_t)BIN_KEYS * 4, cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaMemcpyAsync(s.h_stats, s.d_stats, 128, cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaMemcpyAsync(h_list, d_list, list_bytes, cudaMemcpyDeviceToHost, s2));
+    CU(c, cudaEventRecord(s.ev_prep, s2));
+    return 0;
+}
+
+// Launch plan from the binning histogram of the device (s.h_hist, s.h_stats) that classified n_aln alignments; also
+// fills s.h_keybase, the first sorted position of every key, for bin_scatter_kernel.
+int plan_from_histogram(fadegpu_ctx *c, BinState &s, int64_t n_aln)
+{
+    int64_t cls_first[N_ROW_CLASSES + 2];
+    std::vector<int32_t> &stl = s.sorted_tlen;
+    stl.resize((size_t)n_aln);
+    int64_t run = 0;
+    for (int rk = 0; rk <= N_ROW_CLASSES; ++rk) {
+        cls_first[rk] = run;
+        const int k0 = rk * KEYS_PER_CLASS, k1 = k0 + KEYS_PER_CLASS;
+        for (int key = k0; key < k1; ++key) {
+            const int32_t cnt = s.h_hist[key];
+            s.h_keybase[key] = (int32_t)run;
+            if (!cnt) continue;
+            const int tl = rk == N_ROW_CLASSES ? (int)s.h_stats[5] : key_tlen(key - k0);
+            std::fill(stl.begin() + run, stl.begin() + run + cnt, tl);
+            run += cnt;
+        }
+    }
+    cls_first[N_ROW_CLASSES + 1] = run;
+    if (run != n_aln) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: internal error (histogram does not add up)");
+    return build_plan(c, s, n_aln, cls_first, stl.data(), std::max(1, (int)s.h_stats[2]), std::max(1, (int)s.h_stats[3]),
+                      std::max(1, (int)s.h_stats[4]), std::max(1, (int)s.h_stats[5]));
+}
+
+// After plan_from_histogram, on stream2: the keybase and the plan's warp items go up (BIN_KEYS * 4 +
+// n_items * sizeof(WarpItem) bytes) and the scatter kernel writes the sorted descriptors
+int bin_scatter(fadegpu_ctx *c, BinState &s)
+{
+    if (s.n_aln == 0) return 0;
+    cudaStream_t s2 = c->stream2;
+    CU(c, cudaMemcpyAsync(s.d_keybase, s.h_keybase, (size_t)BIN_KEYS * 4, cudaMemcpyHostToDevice, s2));
+    if (s.n_items > 0)
+        CU(c, cudaMemcpyAsync(s.d_items, s.h_items, (size_t)s.n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, s2));
+    CU(c, launch_bin_scatter(s.ba, c->sm_count, s2));
+    return 0;
+}
+
+// Once the caller has recorded ev_ready on stream2: the compute stream waits for it and runs the plan against pt, and
+// stream3 continues after the kernels; ev[1] and ev[2] bracket them.
+int run_kernels(fadegpu_ctx *c, BinState &s, const PlanTarget &pt, int *launches)
+{
+    CU(c, cudaStreamWaitEvent(c->stream, s.ev_ready, 0));
+    CU(c, cudaEventRecord(s.ev[1], c->stream));
+    { int rc = run_plan(c, s, pt, nullptr, nullptr, nullptr, launches, s.ev_ready); if (rc) return rc; }
+    CU(c, cudaStreamWaitEvent(c->stream3, s.ev_kernels, 0));
+    CU(c, cudaEventRecord(s.ev[2], c->stream3));
     return 0;
 }
 
@@ -849,29 +984,18 @@ void fadegpu_free_batch(fadegpu_batch *b)
         c->done_cv.wait(lk, [&] { return !b->queued; });
         c->batches.erase(std::remove(c->batches.begin(), c->batches.end(), b), c->batches.end());
     }
-    if (c) { cudaSetDevice(c->device); if (c->stream) cudaStreamSynchronize(c->stream); if (c->tstream) cudaStreamSynchronize(c->tstream); if (c->stream2) cudaStreamSynchronize(c->stream2); if (c->stream3) cudaStreamSynchronize(c->stream3); }
+    free_bin_state(c, b->bs);
     fadegpu_batch_view &v = b->v;
     free_host(v.seq4); free_host(v.seq_off); free_host(v.l_qseq); free_host(v.tid); free_host(v.pos);
     free_host(v.aligned_len); free_host(v.clip_left); free_host(v.clip_right);
     free_host(v.gate); free_host(v.meta);
     free_host(v.flags); free_host(v.score); free_host(v.beg_query); free_host(v.end_query);
     free_host(v.beg_ref); free_host(v.end_ref); free_host(v.win_start); free_host(v.n_ops); free_host(v.ops);
-    free_host(b->h_aln); free_host(b->h_items); free_host(b->h_seq); free_host(b->h_out); free_host(b->h_ridx);
-    free_dev(b->d_aln); free_dev(b->d_items); free_dev(b->d_seq); free_dev(b->d_out); free_dev(b->d_flags);
-    free_dev(b->d_fillres);
-    free_dev(b->d_in_seq4); free_dev(b->d_in_seq_off); free_dev(b->d_in_pos); free_dev(b->d_in_lq); free_dev(b->d_in_tid);
-    free_dev(b->d_in_alen); free_dev(b->d_in_cl); free_dev(b->d_in_cr); free_dev(b->d_key); free_dev(b->d_tlen); free_dev(b->d_start);
-    free_dev(b->d_aln_start); free_dev(b->d_hist); free_dev(b->d_keybase); free_dev(b->d_cursor);
-    free_dev(b->d_ridx); free_dev(b->d_rflags);
-    free_dev(b->d_gate); free_dev(b->d_over); free_host(b->h_over); free_dev(b->d_stats);
-    free_host(b->h_hist); free_host(b->h_keybase); free_host(b->h_stats); free_host(b->h_aln_start);
+    free_host(b->h_aln); free_host(b->h_seq); free_host(b->h_out); free_host(b->h_ridx); free_host(b->h_aln_start);
+    free_dev(b->d_seq); free_dev(b->d_ridx); free_dev(b->d_rflags); free_dev(b->d_gate);
     free_host(b->h_c_seq4); free_host(b->h_c_seq_off); free_host(b->h_c_pos); free_host(b->h_c_lq); free_host(b->h_c_tid);
-    free_host(b->h_c_alen); free_host(b->h_c_cl); free_host(b->h_c_cr); free_host(b->h_c_read); free_dev(b->d_in_read); free_dev(b->d_src_off);
+    free_host(b->h_c_alen); free_host(b->h_c_cl); free_host(b->h_c_cr); free_host(b->h_c_read); free_dev(b->d_in_read);
     free_dev(b->d_aln_scratch); free_dev(b->d_i64_scratch);
-    if (b->ev_prep) cudaEventDestroy(b->ev_prep);
-    if (b->ev_ready) cudaEventDestroy(b->ev_ready);
-    if (b->ev_kernels) cudaEventDestroy(b->ev_kernels);
-    for (auto &e : b->ev) if (e) { cudaEventDestroy(e); e = nullptr; }
     delete b;
 }
 
@@ -888,7 +1012,6 @@ int fadegpu_alloc_batch(fadegpu_ctx *c, int64_t max_reads, int64_t max_seq_bytes
     fadegpu_batch_view &v = b->v;
     v.max_reads = max_reads; v.max_seq_bytes = max_seq_bytes;
     const size_t n = (size_t)max_reads;
-    b->cap_items = (max_reads + 7) / 8 + 8;
     b->cap_seq = max_seq_bytes + 16;
     cudaError_t e = cudaSuccess;
     auto H = [&](auto **p, size_t bytes) { if (e == cudaSuccess) e = cudaHostAlloc((void **)p, std::max<size_t>(bytes, 16), cudaHostAllocDefault); };
@@ -900,34 +1023,14 @@ int fadegpu_alloc_batch(fadegpu_ctx *c, int64_t max_reads, int64_t max_seq_bytes
         H(&v.score, n * 4); H(&v.beg_query, n * 4); H(&v.end_query, n * 4); H(&v.beg_ref, n * 4);
         H(&v.end_ref, n * 4); H(&v.win_start, n * 8); H(&v.n_ops, n * 4); H(&v.ops, n * 4 * FADEGPU_MAX_OPS);
     }
-    H(&b->h_items, (size_t)b->cap_items * sizeof(WarpItem));
-    H(&b->h_out, n * sizeof(AlnOut)); H(&b->h_ridx, n * 4);
+    H(&b->h_out, n * sizeof(AlnOut)); H(&b->h_ridx, n * 4); H(&b->h_aln_start, n * 8);
     // h_aln / h_seq / d_seq (staging of the host-binning path) are allocated on its first use
-    D(&b->d_aln, n * sizeof(AlnDesc)); D(&b->d_items, (size_t)b->cap_items * sizeof(WarpItem));
-    D(&b->d_out, n * sizeof(AlnOut)); D(&b->d_flags, n * 4);
-    D(&b->d_fillres, (size_t)b->cap_items * 32 * sizeof(uint2));
-    // device-side binning: mirrors of the inputs, keys, histogram, per-read result index
-    // d_in_seq4: 16-byte slots that keep the source's alignment phase
-    D(&b->d_in_seq4, (size_t)max_seq_bytes + 32 * n + 16); D(&b->d_in_seq_off, (n + 1) * 8); D(&b->d_in_pos, n * 8);
-    D(&b->d_in_read, n * 4);
-    D(&b->d_in_lq, n * 4); D(&b->d_in_tid, n * 4); D(&b->d_in_alen, n * 4); D(&b->d_in_cl, n * 4); D(&b->d_in_cr, n * 4);
-    D(&b->d_key, n * 4); D(&b->d_tlen, n * 4); D(&b->d_start, n * 8); D(&b->d_aln_start, n * 8);
-    D(&b->d_hist, (size_t)BIN_KEYS * 4); D(&b->d_keybase, (size_t)BIN_KEYS * 4); D(&b->d_cursor, (size_t)BIN_KEYS * 4);
-    D(&b->d_ridx, n * 4); D(&b->d_rflags, n);
-    D(&b->d_gate, n); D(&b->d_over, (size_t)OVER_CAP * 4); H(&b->h_over, (size_t)OVER_CAP * 4);
-    D(&b->d_stats, 128); D(&b->d_src_off, n * 8);
-    H(&b->h_hist, (size_t)BIN_KEYS * 4); H(&b->h_keybase, (size_t)BIN_KEYS * 4); H(&b->h_stats, 128); H(&b->h_aln_start, n * 8);
+    // device-side binning beyond the core: gathered read indices, per-read result index and flags, gate bytes
+    D(&b->d_in_read, n * 4); D(&b->d_ridx, n * 4); D(&b->d_rflags, n); D(&b->d_gate, n);
     if (e == cudaSuccess) e = cudaHostGetDevicePointer((void **)&b->d_view_seq4, v.seq4, 0);
     if (e == cudaSuccess) e = cudaHostGetDevicePointer((void **)&b->d_view_meta, v.meta, 0);
-    if (e == cudaSuccess) e = cudaEventCreate(&b->ev_prep);
-    if (e == cudaSuccess) e = cudaEventCreate(&b->ev_ready);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->ev_kernels, cudaEventDisableTiming);
-    for (auto &ev : b->ev) if (e == cudaSuccess) e = cudaEventCreate(&ev);
-    if (e != cudaSuccess) {
-        int rc = cuda_fail(c, e, "fadegpu_alloc_batch");
-        fadegpu_free_batch(b);
-        return rc;
-    }
+    const int rc = e != cudaSuccess ? cuda_fail(c, e, "fadegpu_alloc_batch") : alloc_bin_state(c, b->bs, max_reads, max_seq_bytes);
+    if (rc) { fadegpu_free_batch(b); return rc; }
     { std::lock_guard<std::mutex> lk(c->q_mu); c->batches.push_back(b); }
     *out = b;
     return FADEGPU_OK;
@@ -976,7 +1079,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     { int rc = ensure_host_staging(c, b); if (rc) return rc; }
     const int64_t n = n_reads;
     b->n_reads = n;
-    b->plan.clear();
+    b->bs.plan.clear();
     b->dev_binning = false;
     memset(&b->st, 0, sizeof(b->st));
     b->st.n_reads = n;
@@ -1022,7 +1125,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
             if (end - start > 0x7fffffff || (end - start) * (int64_t)ql > ((int64_t)1 << 31)) {
                 // (the reference would need a multi-GB trace for this ONE read) left unaligned and reported
 #pragma omp critical(fadegpu_oversize)
-                { if (n_over < OVER_CAP) b->h_over[n_over] = (int32_t)r; ++n_over; }
+                { if (n_over < OVER_CAP) b->bs.h_over[n_over] = (int32_t)r; ++n_over; }
                 continue;
             }
             const int tlen = (int)(end - start);
@@ -1146,7 +1249,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
 
     b->st.host_gather_ms = ms_since(t_gather);
     // ---- 4. launch plan ----
-    std::vector<int32_t> &stl = b->sorted_tlen;
+    std::vector<int32_t> &stl = b->bs.sorted_tlen;
     stl.resize((size_t)n_aln);
     for (int64_t kx = 0; kx < n_aln; ++kx) {   // long windows share keys: the plan uses the key's upper end for all of them
         const AlnTmp &t = all[order[(size_t)kx]];
@@ -1154,33 +1257,30 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     }
     int gq = 1, gt = 1;
     for (int64_t kx = cls_first[N_ROW_CLASSES]; kx < n_aln; ++kx) { gq = std::max(gq, b->h_aln[kx].qlen); gt = std::max(gt, b->h_aln[kx].tlen); }
-    b->seq_bytes = seq_bytes;
-    { int rc = build_plan(c, b, n_aln, cls_first, stl.data(), qmax_all, tmax_all, gq, gt); if (rc) return rc; }
-    const int64_t n_items = b->n_items;
+    BinState &bs = b->bs;
+    { int rc = build_plan(c, bs, n_aln, cls_first, stl.data(), qmax_all, tmax_all, gq, gt); if (rc) return rc; }
+    b->st.n_aligned = n_aln; b->st.n_generic = bs.n_generic; b->st.scratch_bytes = bs.scratch_bytes;
+    const int64_t n_items = bs.n_items;
 
     // ---- 5. queue copies and kernels ----
     // copies in on stream2, kernels on the compute stream, copies out on stream3: the DMA of one
     // batch overlaps the kernels of its neighbours
-    CU(c, cudaEventRecord(b->ev[0], c->stream2));
+    CU(c, cudaEventRecord(bs.ev[0], c->stream2));
     if (n_aln > 0) {
-        CU(c, cudaMemcpyAsync(b->d_aln, b->h_aln, (size_t)n_aln * sizeof(AlnDesc), cudaMemcpyHostToDevice, c->stream2));
+        CU(c, cudaMemcpyAsync(bs.d_aln, b->h_aln, (size_t)n_aln * sizeof(AlnDesc), cudaMemcpyHostToDevice, c->stream2));
         if (n_items > 0)
-            CU(c, cudaMemcpyAsync(b->d_items, b->h_items, (size_t)n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, c->stream2));
+            CU(c, cudaMemcpyAsync(bs.d_items, bs.h_items, (size_t)n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, c->stream2));
         CU(c, cudaMemcpyAsync(b->d_seq, b->h_seq, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream2));
     }
     b->st.h2d_bytes = n_aln * (int64_t)sizeof(AlnDesc) + n_items * (int64_t)sizeof(WarpItem) + seq_bytes;
-    CU(c, cudaEventRecord(b->ev_ready, c->stream2));
-    CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
-    CU(c, cudaEventRecord(b->ev[1], c->stream));
+    CU(c, cudaEventRecord(bs.ev_ready, c->stream2));
     int nl = 0;
-    { int rc = run_plan(c, b, batch_target(c), nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
+    { int rc = run_kernels(c, bs, batch_target(c, b), &nl); if (rc) return rc; }
     b->st.kernel_launches = nl;
-    { int rc = join_kernels(c, b, c->stream3); if (rc) return rc; }
-    CU(c, cudaEventRecord(b->ev[2], c->stream3));
     if (n_aln > 0)
-        CU(c, cudaMemcpyAsync(b->h_out, b->d_out, (size_t)n_aln * sizeof(AlnOut), cudaMemcpyDeviceToHost, c->stream3));
+        CU(c, cudaMemcpyAsync(b->h_out, bs.d_out, (size_t)n_aln * sizeof(AlnOut), cudaMemcpyDeviceToHost, c->stream3));
     b->st.d2h_bytes = n_aln * (int64_t)sizeof(AlnOut);
-    CU(c, cudaEventRecord(b->ev[3], c->stream3));
+    CU(c, cudaEventRecord(bs.ev[3], c->stream3));
     b->in_flight = true;
     b->st.host_submit_ms = ms_since(t_begin);
     return FADEGPU_OK;
@@ -1268,32 +1368,6 @@ enum SubmitMode : int {
     MODE_COMPACT = 2     // fadegpu_submit_compact: one gate byte per read is DMA'd, the GPU fetches the rest it needs
 };
 
-// Launch plan from the binning histogram of the device (b->h_hist, b->h_stats) that classified n_aln alignments; also
-// fills b->h_keybase, the first sorted position of every key, for bin_scatter_kernel.
-static int plan_from_histogram(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_aln)
-{
-    int64_t cls_first[N_ROW_CLASSES + 2];
-    std::vector<int32_t> &stl = b->sorted_tlen;
-    stl.resize((size_t)n_aln);
-    int64_t run = 0;
-    for (int rk = 0; rk <= N_ROW_CLASSES; ++rk) {
-        cls_first[rk] = run;
-        const int k0 = rk * KEYS_PER_CLASS, k1 = k0 + KEYS_PER_CLASS;
-        for (int key = k0; key < k1; ++key) {
-            const int32_t cnt = b->h_hist[key];
-            b->h_keybase[key] = (int32_t)run;
-            if (!cnt) continue;
-            const int tl = rk == N_ROW_CLASSES ? (int)b->h_stats[5] : key_tlen(key - k0);
-            std::fill(stl.begin() + run, stl.begin() + run + cnt, tl);
-            run += cnt;
-        }
-    }
-    cls_first[N_ROW_CLASSES + 1] = run;
-    if (run != n_aln) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: internal error (histogram does not add up)");
-    return build_plan(c, b, n_aln, cls_first, stl.data(), std::max(1, (int)b->h_stats[2]), std::max(1, (int)b->h_stats[3]),
-                      std::max(1, (int)b->h_stats[4]), std::max(1, (int)b->h_stats[5]));
-}
-
 // Stage B: the inputs go to the GPU, a classify kernel applies the length floor (analysis.d:34) and the window
 // arithmetic (analysis.d:45-59) and histograms the reads that need SW by (row class, window length), the host
 // turns the 96 KB histogram into the launch plan, a scatter kernel writes the sorted descriptors, the GPU pulls the
@@ -1306,8 +1380,9 @@ static int submit_device_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_rea
         return std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
     };
     const bool pull = mode != MODE_GATHERED;
+    BinState &bs = b->bs;
     b->n_reads = n_reads;
-    b->plan.clear();
+    bs.plan.clear();
     b->dev_binning = true;
     b->mode = mode;
     {
@@ -1316,93 +1391,75 @@ static int submit_device_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_rea
         b->st.host_gather_ms = g; b->st.host_threads = th;
     }
     b->st.n_reads = n_reads;
-    b->n_aln = 0; b->n_items = 0;
-    b->ba_valid = false;
+    bs.n_aln = 0; bs.n_items = 0; bs.ba.n = 0;
     cudaStream_t s2 = c->stream2;
-    CU(c, cudaEventRecord(b->ev[0], s2));
+    CU(c, cudaEventRecord(bs.ev[0], s2));
     b->pulled = pull;
     const fadegpu_batch_view &v = b->v;
     const int64_t n = pull ? n_reads : b->n_c;
     const int64_t seq_total = mode == MODE_COMPACT ? seq_bytes : mode == MODE_VIEW ? (n > 0 ? v.seq_off[n] : 0) : b->seq_c;
     int64_t n_aln = 0, up_bytes = 0;
-    memset(b->h_stats, 0, 128);
+    memset(bs.h_stats, 0, 128);
     if (n > 0) {
         auto up = [&](void *d, const void *h, size_t bytes) { up_bytes += (int64_t)bytes; return cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s2); };
         if (mode == MODE_COMPACT) CU(c, up(b->d_gate, v.gate, (size_t)n));
         else {
-            if (!pull) CU(c, up(b->d_in_seq4, b->h_c_seq4, (size_t)seq_total));
-            CU(c, up(b->d_in_seq_off, pull ? v.seq_off : b->h_c_seq_off, (size_t)(n + 1) * 8));
-            CU(c, up(b->d_in_lq, pull ? v.l_qseq : b->h_c_lq, (size_t)n * 4)); CU(c, up(b->d_in_tid, pull ? v.tid : b->h_c_tid, (size_t)n * 4));
-            CU(c, up(b->d_in_pos, pull ? v.pos : b->h_c_pos, (size_t)n * 8)); CU(c, up(b->d_in_alen, pull ? v.aligned_len : b->h_c_alen, (size_t)n * 4));
-            CU(c, up(b->d_in_cl, pull ? v.clip_left : b->h_c_cl, (size_t)n * 4)); CU(c, up(b->d_in_cr, pull ? v.clip_right : b->h_c_cr, (size_t)n * 4));
+            if (!pull) CU(c, up(bs.d_in_seq4, b->h_c_seq4, (size_t)seq_total));
+            CU(c, up(bs.d_in_seq_off, pull ? v.seq_off : b->h_c_seq_off, (size_t)(n + 1) * 8));
+            CU(c, up(bs.d_in_lq, pull ? v.l_qseq : b->h_c_lq, (size_t)n * 4)); CU(c, up(bs.d_in_tid, pull ? v.tid : b->h_c_tid, (size_t)n * 4));
+            CU(c, up(bs.d_in_pos, pull ? v.pos : b->h_c_pos, (size_t)n * 8)); CU(c, up(bs.d_in_alen, pull ? v.aligned_len : b->h_c_alen, (size_t)n * 4));
+            CU(c, up(bs.d_in_cl, pull ? v.clip_left : b->h_c_cl, (size_t)n * 4)); CU(c, up(bs.d_in_cr, pull ? v.clip_right : b->h_c_cr, (size_t)n * 4));
             if (!pull) CU(c, up(b->d_in_read, b->h_c_read, (size_t)n * 4));
         }
-        CU(c, cudaMemsetAsync(b->d_hist, 0, (size_t)BIN_KEYS * 4, s2));
-        CU(c, cudaMemsetAsync(b->d_cursor, 0, (size_t)BIN_KEYS * 4, s2));
-        CU(c, cudaMemsetAsync(b->d_stats, 0, 128, s2));
-        BinArgs ba{};
-        ba.seq4 = b->d_in_seq4; ba.seq_off = b->d_in_seq_off; ba.l_qseq = b->d_in_lq; ba.tid = b->d_in_tid; ba.pos = b->d_in_pos;
-        ba.aligned_len = b->d_in_alen; ba.clip_left = b->d_in_cl; ba.clip_right = b->d_in_cr;
+        { int rc = bin_zero(c, bs); if (rc) return rc; }
+        BinArgs &ba = bs.ba;
         ba.read = pull ? nullptr : b->d_in_read;
-        ba.seq_cursor = pull ? b->d_stats + 8 : nullptr; ba.src_off = b->d_src_off;
-        ba.gate = mode == MODE_COMPACT ? b->d_gate : nullptr; ba.host_meta = b->d_view_meta; ba.over_list = b->d_over;
+        ba.seq_cursor = pull ? bs.d_stats + 8 : nullptr;
+        ba.gate = mode == MODE_COMPACT ? b->d_gate : nullptr; ba.host_meta = b->d_view_meta;
         ba.n = n; ba.seq_total = seq_total; ba.clen = c->d_clen; ba.coff = c->d_coff; ba.n_contigs = c->n_contigs;
         ba.window = c->p.window_size; ba.min_length = c->p.min_length; ba.flags = c->p.flags;
-        ba.key = b->d_key; ba.tlen = b->d_tlen; ba.start = b->d_start; ba.hist = b->d_hist; ba.stats = b->d_stats;
-        ba.keybase = b->d_keybase; ba.cursor = b->d_cursor; ba.aln = b->d_aln; ba.aln_start = b->d_aln_start;
-        b->ba = ba; b->ba_valid = true;
-        CU(c, launch_bin_classify(ba, c->sm_count, s2));
-        CU(c, cudaMemcpyAsync(b->h_hist, b->d_hist, (size_t)BIN_KEYS * 4, cudaMemcpyDeviceToHost, s2));
-        CU(c, cudaMemcpyAsync(b->h_stats, b->d_stats, 128, cudaMemcpyDeviceToHost, s2));
-        CU(c, cudaMemcpyAsync(b->h_over, b->d_over, (size_t)OVER_CAP * 4, cudaMemcpyDeviceToHost, s2));
-        CU(c, cudaEventRecord(b->ev_prep, s2));
-        CU(c, cudaEventSynchronize(b->ev_prep));   // the previous batch keeps computing on c->stream meanwhile
+        { int rc = bin_classify(c, bs, bs.h_over, bs.d_over, (size_t)OVER_CAP * 4); if (rc) return rc; }
+        CU(c, cudaEventSynchronize(bs.ev_prep));   // the previous batch keeps computing on c->stream meanwhile
         b->st.host_classify_ms = ms_since(t_begin);
-        if (b->h_stats[6] & 1ull) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: seq_off / l_qseq inconsistent");
-        b->st.n_oversize = (int64_t)b->h_stats[11];
+        if (bs.h_stats[6] & 1ull) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: seq_off / l_qseq inconsistent");
+        b->st.n_oversize = (int64_t)bs.h_stats[11];
         // ---- plan from the histogram ----
         const auto t_sort = std::chrono::steady_clock::now();
-        n_aln = (int64_t)b->h_stats[1];
-        b->st.cells = (int64_t)b->h_stats[0];
-        { int rc = plan_from_histogram(c, b, n_aln); if (rc) return rc; }
+        n_aln = (int64_t)bs.h_stats[1];
+        b->st.cells = (int64_t)bs.h_stats[0];
+        { int rc = plan_from_histogram(c, bs, n_aln); if (rc) return rc; }
         b->st.host_sort_ms = ms_since(t_sort);
-        if (n_aln > 0) {
-            CU(c, up(b->d_keybase, b->h_keybase, (size_t)BIN_KEYS * 4));
-            if (b->n_items > 0) CU(c, up(b->d_items, b->h_items, (size_t)b->n_items * sizeof(WarpItem)));
-            CU(c, launch_bin_scatter(ba, c->sm_count, s2));
-            if (pull) CU(c, launch_seq_pull(b->d_view_seq4, b->d_aln, b->d_src_off, (int)n_aln, b->d_in_seq4, c->sm_count, s2));
-        }
+        b->st.n_aligned = n_aln; b->st.n_generic = bs.n_generic; b->st.scratch_bytes = bs.scratch_bytes;
+        if (n_aln > 0) up_bytes += (int64_t)BIN_KEYS * 4 + bs.n_items * (int64_t)sizeof(WarpItem);
+        { int rc = bin_scatter(c, bs); if (rc) return rc; }
+        if (pull && n_aln > 0) CU(c, launch_seq_pull(b->d_view_seq4, bs.d_aln, bs.d_src_off, (int)n_aln, bs.d_in_seq4, c->sm_count, s2));
     }
     if (n_reads > 0) {
         CU(c, cudaMemsetAsync(b->d_rflags, 0, (size_t)n_reads, s2));
         CU(c, cudaMemsetAsync(b->d_ridx, 0xff, (size_t)n_reads * 4, s2));
     }
-    CU(c, cudaEventRecord(b->ev_ready, s2));
-    CU(c, cudaEventRecord(b->ev[4], s2));
-    // ---- compute stream ----
-    CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
-    CU(c, cudaEventRecord(b->ev[1], c->stream));
+    CU(c, cudaEventRecord(bs.ev_ready, s2));
+    CU(c, cudaEventRecord(bs.ev[4], s2));
+    // ---- compute stream; results go home on stream3 while the next batch computes ----
     int nl = 0;
-    { int rc = run_plan(c, b, batch_target(c), nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
+    { int rc = run_kernels(c, bs, batch_target(c, b), &nl); if (rc) return rc; }
     b->st.kernel_launches = nl + (n > 0 ? 1 : 0) + (n_aln > 0 ? (pull ? 3 : 2) : 0);
-    cudaStream_t s3 = c->stream3;                    // results go home while the next batch computes
-    { int rc = join_kernels(c, b, s3); if (rc) return rc; }
-    CU(c, cudaEventRecord(b->ev[2], s3));
-    if (n_aln > 0) CU(c, launch_result_index(b->d_out, (int)n_aln, n_reads, b->d_rflags, b->d_ridx, b->d_stats + 7, c->sm_count, s3));
+    cudaStream_t s3 = c->stream3;
+    if (n_aln > 0) CU(c, launch_result_index(bs.d_out, (int)n_aln, n_reads, b->d_rflags, b->d_ridx, bs.d_stats + 7, c->sm_count, s3));
     if (n_reads > 0) {
         CU(c, cudaMemcpyAsync(b->v.flags, b->d_rflags, (size_t)n_reads, cudaMemcpyDeviceToHost, s3));
         CU(c, cudaMemcpyAsync(b->h_ridx, b->d_ridx, (size_t)n_reads * 4, cudaMemcpyDeviceToHost, s3));
     }
-    if (n_aln > 0) CU(c, cudaMemcpyAsync(b->h_stats + 7, b->d_stats + 7, 8, cudaMemcpyDeviceToHost, s3));
+    if (n_aln > 0) CU(c, cudaMemcpyAsync(bs.h_stats + 7, bs.d_stats + 7, 8, cudaMemcpyDeviceToHost, s3));
     if (n_aln > 0) {
-        CU(c, cudaMemcpyAsync(b->h_out, b->d_out, (size_t)n_aln * sizeof(AlnOut), cudaMemcpyDeviceToHost, s3));
-        CU(c, cudaMemcpyAsync(b->h_aln_start, b->d_aln_start, (size_t)n_aln * 8, cudaMemcpyDeviceToHost, s3));
+        CU(c, cudaMemcpyAsync(b->h_out, bs.d_out, (size_t)n_aln * sizeof(AlnOut), cudaMemcpyDeviceToHost, s3));
+        CU(c, cudaMemcpyAsync(b->h_aln_start, bs.d_aln_start, (size_t)n_aln * 8, cudaMemcpyDeviceToHost, s3));
     }
     // (the bytes the GPU fetched itself -- bases, compact records -- are added from the device's counters)
-    b->st.h2d_bytes = up_bytes + (pull ? (int64_t)b->h_stats[10] * (int64_t)sizeof(fadegpu_read_meta) : 0);
+    b->st.h2d_bytes = up_bytes + (pull ? (int64_t)bs.h_stats[10] * (int64_t)sizeof(fadegpu_read_meta) : 0);
     b->st.d2h_bytes = n_aln * (int64_t)(sizeof(AlnOut) + 8) + n_reads * 5 + (n > 0 ? (int64_t)BIN_KEYS * 4 + 128 + OVER_CAP * 4 : 0);
-    if (pull && n_aln > 0) CU(c, cudaMemcpyAsync(b->h_stats + 8, b->d_stats + 8, 8, cudaMemcpyDeviceToHost, s3));   // bases pulled
-    CU(c, cudaEventRecord(b->ev[3], s3));
+    if (pull && n_aln > 0) CU(c, cudaMemcpyAsync(bs.h_stats + 8, bs.d_stats + 8, 8, cudaMemcpyDeviceToHost, s3));   // bases pulled
+    CU(c, cudaEventRecord(bs.ev[3], s3));
     b->in_flight = true;
     b->st.host_submit_ms = ms_since(t_begin);
     return FADEGPU_OK;
@@ -1571,12 +1628,12 @@ int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
         }
     }
     CU(c, cudaSetDevice(c->device));
-    CU(c, cudaEventSynchronize(b->ev[3]));
+    CU(c, cudaEventSynchronize(b->bs.ev[3]));
     float t;
-    if (cudaEventElapsedTime(&t, b->ev[1], b->ev[2]) == cudaSuccess) b->st.kernel_ms = t;
-    if (cudaEventElapsedTime(&t, b->ev[0], b->ev[3]) == cudaSuccess) b->st.total_ms = t;
+    if (cudaEventElapsedTime(&t, b->bs.ev[1], b->bs.ev[2]) == cudaSuccess) b->st.kernel_ms = t;
+    if (cudaEventElapsedTime(&t, b->bs.ev[0], b->bs.ev[3]) == cudaSuccess) b->st.total_ms = t;
     if (b->dev_binning && b->pulled) {
-        if (b->n_aln > 0) b->st.h2d_bytes += (int64_t)b->h_stats[8];
+        if (b->bs.n_aln > 0) b->st.h2d_bytes += (int64_t)b->bs.h_stats[8];
         b->pulled = false;
     }
     // Device-binned submits: flags[] and the per-read index into the results were built on the device; only the
@@ -1588,17 +1645,17 @@ int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
     // (no parallel region unless there is real work: its threads would spin for milliseconds afterwards on the
     // cores the ctx thread needs to queue the next batch)
     const bool walk = scatter || !b->dev_binning;
-    const int nthr = walk ? (int)std::max<int64_t>(1, std::min<int64_t>(c->host_threads, b->n_aln / 8192 + 1)) : 1;
+    const int nthr = walk ? (int)std::max<int64_t>(1, std::min<int64_t>(c->host_threads, b->bs.n_aln / 8192 + 1)) : 1;
     const int64_t *wstart = b->dev_binning ? b->h_aln_start : b->aln_start.data();
     int64_t bad = 0;
     if (b->dev_binning) {
-        if (b->n_aln > 0 && (int64_t)b->h_stats[7] != b->n_aln) bad = 1;   // result records counted on the device
+        if (b->bs.n_aln > 0 && (int64_t)b->bs.h_stats[7] != b->bs.n_aln) bad = 1;   // result records counted on the device
     } else {
         memset(v.flags, 0, (size_t)n);   // the other per-read outputs are defined only where FADEGPU_R_ALIGNED is set
         memset(b->h_ridx, 0xff, (size_t)n * sizeof(int32_t));
     }
 #pragma omp parallel for schedule(static) reduction(+ : bad) num_threads(nthr) if (nthr > 1)
-    for (int64_t k = 0; k < (walk ? b->n_aln : 0); ++k) {
+    for (int64_t k = 0; k < (walk ? b->bs.n_aln : 0); ++k) {
         const AlnOut &o = b->h_out[k];
         const int64_t r = o.read;
         if (r < 0 || r >= n || (o.flags & 0x80000000u) || !(o.flags & 1u) || (!b->dev_binning && b->h_aln[k].read != (int32_t)r)) { ++bad; continue; }
@@ -1613,7 +1670,7 @@ int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
         memcpy(v.ops + (size_t)r * FADEGPU_MAX_OPS, o.ops, sizeof(o.ops));
     }
     for (int64_t k = 0; k < std::min<int64_t>(b->st.n_oversize, OVER_CAP); ++k) {
-        const int64_t r = b->h_over[k];
+        const int64_t r = b->bs.h_over[k];
         if (r >= 0 && r < n) v.flags[r] = FADEGPU_R_OVERSIZE;
     }
     b->st.host_wait_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_scatter).count();
@@ -1626,7 +1683,7 @@ int fadegpu_get_results(const fadegpu_batch *b, fadegpu_results_view *r)
     if (!b || !r) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_get_results: null argument");
     if (b->in_flight) return fail(b->ctx, FADEGPU_E_STATE, "fadegpu_get_results: batch in flight (call fadegpu_wait)");
     static_assert(sizeof(fadegpu_result) == sizeof(AlnOut), "fadegpu_result must mirror AlnOut");
-    r->n_results = b->n_aln;
+    r->n_results = b->bs.n_aln;
     r->results = reinterpret_cast<const fadegpu_result *>(b->h_out);
     r->win_start = b->dev_binning ? b->h_aln_start : b->aln_start.data();
     r->result_index = b->h_ridx;
@@ -1644,7 +1701,7 @@ int fadegpu_get_timeline(const fadegpu_batch *b, const fadegpu_batch *origin, fl
 {
     if (!b || !origin || !ms || b->ctx != origin->ctx) return fail(b ? b->ctx : nullptr, FADEGPU_E_ARG, "fadegpu_get_timeline: bad arguments");
     for (int k = 0; k < 6; ++k)
-        if (cudaEventElapsedTime(&ms[k], origin->ev[0], b->ev[k]) != cudaSuccess) { cudaGetLastError(); ms[k] = -1.f; }
+        if (cudaEventElapsedTime(&ms[k], origin->bs.ev[0], b->bs.ev[k]) != cudaSuccess) { cudaGetLastError(); ms[k] = -1.f; }
     return FADEGPU_OK;
 }
 
@@ -1655,26 +1712,25 @@ int fadegpu_get_timeline(const fadegpu_batch *b, const fadegpu_batch *origin, fl
 static int replay_binning(fadegpu_ctx *c, fadegpu_batch *b, cudaEvent_t *dep)
 {
     *dep = nullptr;
-    if (!b->dev_binning || !b->ba_valid) return 0;
+    if (!b->dev_binning || b->bs.ba.n == 0) return 0;
     const size_t n = (size_t)b->v.max_reads;
     if (!b->d_aln_scratch) {
         CU(c, cudaMalloc((void **)&b->d_aln_scratch, n * sizeof(AlnDesc)));
         CU(c, cudaMalloc((void **)&b->d_i64_scratch, 2 * n * sizeof(int64_t)));
     }
+    BinState &bs = b->bs;
     cudaStream_t s2 = c->stream2;
-    CU(c, cudaMemsetAsync(b->d_hist, 0, (size_t)BIN_KEYS * 4, s2));
-    CU(c, cudaMemsetAsync(b->d_cursor, 0, (size_t)BIN_KEYS * 4, s2));
-    CU(c, cudaMemsetAsync(b->d_stats, 0, 128, s2));
-    BinArgs ba = b->ba;
+    { int rc = bin_zero(c, bs); if (rc) return rc; }
+    BinArgs ba = bs.ba;
     ba.gate = nullptr;        // compact inputs: the records fetched by the submit are resident in the device mirrors
     CU(c, launch_bin_classify(ba, c->sm_count, s2));
-    if (b->n_aln > 0) {
+    if (bs.n_aln > 0) {
         ba.aln = b->d_aln_scratch; ba.aln_start = b->d_i64_scratch; ba.src_off = b->d_i64_scratch + n;
-        if (ba.seq_cursor) ba.seq_cursor = b->d_stats + 9;
+        if (ba.seq_cursor) ba.seq_cursor = bs.d_stats + 9;
         CU(c, launch_bin_scatter(ba, c->sm_count, s2));
     }
-    CU(c, cudaEventRecord(b->ev_ready, s2));
-    *dep = b->ev_ready;
+    CU(c, cudaEventRecord(bs.ev_ready, s2));
+    *dep = bs.ev_ready;
     return 0;
 }
 
@@ -1682,14 +1738,7 @@ static int replay_pass(fadegpu_ctx *c, fadegpu_batch *b)
 {
     cudaEvent_t dep = nullptr;
     { int rc = replay_binning(c, b, &dep); if (rc) return rc; }
-    { int rc = run_plan(c, b, batch_target(c), nullptr, nullptr, nullptr, nullptr, dep); if (rc) return rc; }
-    return 0;
-}
-
-// the ctx stream continues after everything a replay pass of b queued
-static int replay_join(fadegpu_ctx *c, fadegpu_batch *b)
-{
-    { int rc = join_kernels(c, b, c->stream); if (rc) return rc; }
+    { int rc = run_plan(c, b->bs, batch_target(c, b), nullptr, nullptr, nullptr, nullptr, dep); if (rc) return rc; }
     return 0;
 }
 
@@ -1700,7 +1749,7 @@ int fadegpu_replay_batches(fadegpu_ctx *c, fadegpu_batch *const *batches, int32_
         fadegpu_batch *b = batches[i];
         if (!b || b->ctx != c) return fail(c, FADEGPU_E_ARG, "fadegpu_replay_batches: bad batch");
         if (b->in_flight) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_batches: batch in flight");
-        if (b->plan.empty() && b->n_aln > 0) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_batches: nothing submitted");
+        if (b->bs.plan.empty() && b->bs.n_aln > 0) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_batches: nothing submitted");
     }
     drain_submits(c);
     std::lock_guard<std::mutex> submit_guard(c->submit_mu);
@@ -1712,8 +1761,9 @@ int fadegpu_replay_batches(fadegpu_ctx *c, fadegpu_batch *const *batches, int32_
     CU(c, cudaStreamWaitEvent(c->stream2, e0, 0));
     for (int32_t it = 0; it < iters; ++it)
         for (int32_t i = 0; i < n_batches; ++i) { int rc = replay_pass(c, batches[i]); if (rc) return rc; }
-    // the streams are in order, so the last pass of every batch covers the earlier ones
-    for (int32_t i = 0; i < n_batches; ++i) { int rc = replay_join(c, batches[i]); if (rc) return rc; }
+    // the ctx stream continues after the kernels of every batch; the streams are in order, so the last pass of every
+    // batch covers the earlier ones
+    for (int32_t i = 0; i < n_batches; ++i) CU(c, cudaStreamWaitEvent(c->stream, batches[i]->bs.ev_kernels, 0));
     CU(c, cudaEventRecord(e1, c->stream));
     CU(c, cudaEventSynchronize(e1));
     float ms = 0;
@@ -1727,13 +1777,13 @@ int fadegpu_replay_kernels(fadegpu_ctx *c, fadegpu_batch *b, int32_t iters, floa
 {
     if (!c || !b || b->ctx != c || iters <= 0) return fail(c, FADEGPU_E_ARG, "fadegpu_replay_kernels: bad arguments");
     if (b->in_flight) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_kernels: batch in flight");
-    if (b->plan.empty() && b->n_aln > 0) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_kernels: nothing submitted");
+    if (b->bs.plan.empty() && b->bs.n_aln > 0) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_kernels: nothing submitted");
     drain_submits(c);
     {   // one pass with per-stage events (serialising: fill / traceback / generic), then the timed passes
         std::lock_guard<std::mutex> submit_guard(c->submit_mu);
         CU(c, cudaSetDevice(c->device));
         float f = 0, t = 0, g = 0;
-        int rc = run_plan(c, b, batch_target(c), &f, &t, &g, nullptr, nullptr);
+        int rc = run_plan(c, b->bs, batch_target(c, b), &f, &t, &g, nullptr, nullptr);
         if (rc) return rc;
         b->st.fill_ms = f; b->st.trace_ms = t; b->st.generic_ms = g;
     }
@@ -1766,7 +1816,7 @@ static int refuse_in_flight(fadegpu_ctx *c, const char *fn)
 
 // The caller's part of a pair or region call: copy its arrays into the job's pinned staging
 using StageFn = std::function<void(char *h_stage)>;
-// on stream2, after the upload: the binning inputs and the queries of j->b (failures reported to j->d_bad), and ba's
+// on stream2, after the upload: the binning inputs and the queries of j->bs (failures reported to j->d_bad), and ba's
 // contig table; counts its launches
 using PrepFn = std::function<int(fadegpu_job *j, const char *d_raw, BinArgs &ba, int *launches)>;
 
@@ -1784,17 +1834,13 @@ static int stage_call(fadegpu_ctx *c, fadegpu_job *j, const StagedCall &sc, cons
     const int64_t n = sc.n, qbytes = sc.qbytes;
     const int32_t max_ops = sc.max_ops;
     CU(c, cudaSetDevice(c->device));
-    if (!j->b || j->b->v.max_reads < n || j->b->v.max_seq_bytes < qbytes + 16) {
-        int64_t nr = n, sb = qbytes + 16;
-        if (j->b) {
-            nr = std::max(nr, j->b->v.max_reads); sb = std::max(sb, j->b->v.max_seq_bytes);
-            fadegpu_free_batch(j->b);
-            j->b = nullptr;
-        }
-        int rc = fadegpu_alloc_batch(c, nr, sb, &j->b);
+    BinState &bs = j->bs;
+    if (bs.max_items < n || bs.max_seq_bytes < qbytes + 16) {
+        const int64_t nr = std::max(n, bs.max_items), sb = std::max(qbytes + 16, bs.max_seq_bytes);
+        free_bin_state(c, bs);
+        int rc = alloc_bin_state(c, bs, nr, sb);
         if (rc) return rc;
     }
-    fadegpu_batch *b = j->b;
     const size_t raw = sc.raw;
     if (j->stage_bytes < raw) {
         free_host(j->h_stage);
@@ -1814,42 +1860,25 @@ static int stage_call(fadegpu_ctx *c, fadegpu_job *j, const StagedCall &sc, cons
         }
         if (rc) return rc;
         if (!j->d_bad) CU(c, cudaMalloc((void **)&j->d_bad, sizeof(int32_t)));
+        if (!j->h_bad) CU(c, cudaHostAlloc((void **)&j->h_bad, sizeof(int32_t), cudaHostAllocDefault));
     }
     // ---- upload, packing and binning on stream2 ----
-    b->n_reads = n;
-    b->plan.clear();
-    b->dev_binning = true;
-    b->ba_valid = false;
-    b->n_aln = 0; b->n_items = 0;
-    memset(&b->st, 0, sizeof(b->st));
-    memset(b->h_stats, 0, 128);
+    bs.plan.clear();
+    bs.n_aln = 0; bs.n_items = 0;
+    memset(bs.h_stats, 0, 128);
     cudaStream_t s2 = c->stream2;
-    CU(c, cudaEventRecord(b->ev[0], s2));
+    CU(c, cudaEventRecord(bs.ev[0], s2));
     CU(c, cudaMemcpyAsync(j->d_raw, j->h_stage, raw, cudaMemcpyHostToDevice, s2));
     j->h2d = (int64_t)raw;
-    CU(c, cudaEventRecord(b->ev[4], s2));
-    CU(c, cudaMemsetAsync(b->d_hist, 0, (size_t)BIN_KEYS * 4, s2));
-    CU(c, cudaMemsetAsync(b->d_cursor, 0, (size_t)BIN_KEYS * 4, s2));
-    CU(c, cudaMemsetAsync(b->d_stats, 0, 128, s2));
+    CU(c, cudaEventRecord(bs.ev[4], s2));
+    { int rc = bin_zero(c, bs); if (rc) return rc; }
     CU(c, cudaMemsetAsync(j->d_bad, 0x7f, sizeof(int32_t), s2));   // > any item index
-    BinArgs &ba = b->ba;
-    ba = BinArgs{};
-    ba.seq4 = b->d_in_seq4; ba.seq_off = b->d_in_seq_off; ba.l_qseq = b->d_in_lq; ba.tid = b->d_in_tid; ba.pos = b->d_in_pos;
-    ba.aligned_len = b->d_in_alen; ba.clip_left = b->d_in_cl; ba.clip_right = b->d_in_cr;
-    ba.read = nullptr; ba.seq_cursor = nullptr; ba.src_off = b->d_src_off; ba.gate = nullptr; ba.host_meta = nullptr;
-    ba.over_list = b->d_over;
+    BinArgs &ba = bs.ba;
     // window 0 and floor 0: the window of item k is exactly its target / interval, every non-empty item is aligned
     ba.n = n; ba.seq_total = qbytes; ba.window = 0; ba.min_length = 0; ba.flags = c->p.flags;
-    ba.key = b->d_key; ba.tlen = b->d_tlen; ba.start = b->d_start; ba.hist = b->d_hist; ba.stats = b->d_stats;
-    ba.keybase = b->d_keybase; ba.cursor = b->d_cursor; ba.aln = b->d_aln; ba.aln_start = b->d_aln_start;
     j->n_prep = 0;
     { int rc = prep(j, j->d_raw, ba, &j->n_prep); if (rc) return rc; }
-    CU(c, launch_bin_classify(ba, c->sm_count, s2));
-    CU(c, cudaMemcpyAsync(b->h_hist, b->d_hist, (size_t)BIN_KEYS * 4, cudaMemcpyDeviceToHost, s2));
-    CU(c, cudaMemcpyAsync(b->h_stats, b->d_stats, 128, cudaMemcpyDeviceToHost, s2));
-    CU(c, cudaMemcpyAsync(b->h_over, j->d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, s2));
-    CU(c, cudaEventRecord(b->ev_prep, s2));
-    return FADEGPU_OK;
+    return bin_classify(c, bs, j->h_bad, j->d_bad, sizeof(int32_t));
 }
 
 // Device half of a staged call, under submit_mu (it sizes the shared scratch): once the binning histogram is home, the
@@ -1862,62 +1891,53 @@ static int launch_job(fadegpu_ctx *c, fadegpu_job *j)
     if (sc.n == 0) return FADEGPU_OK;
     const int64_t n = sc.n;
     const int32_t max_ops = sc.max_ops;
-    fadegpu_batch *b = j->b;
-    cudaStream_t s2 = c->stream2;
+    BinState &bs = j->bs;
     CU(c, cudaSetDevice(c->device));
-    CU(c, cudaEventSynchronize(b->ev_prep));
-    const int32_t bad = b->h_over[0];
+    CU(c, cudaEventSynchronize(bs.ev_prep));
+    const int32_t bad = *j->h_bad;
     if (bad >= 0 && bad < n)
         return fail(c, FADEGPU_E_ARG, std::string(sc.fn) + ": the query of " + sc.item + " " + std::to_string(bad) +
                                           " holds a letter outside the BAM nt16 alphabet =ACMGRSVTWYHKDBN");
-    if (b->h_stats[6] & 1ull) return fail(c, FADEGPU_E_CUDA, std::string(sc.fn) + ": internal error (query offsets)");
-    const int64_t n_aln = (int64_t)b->h_stats[1];
+    if (bs.h_stats[6] & 1ull) return fail(c, FADEGPU_E_CUDA, std::string(sc.fn) + ": internal error (query offsets)");
+    const int64_t n_aln = (int64_t)bs.h_stats[1];
     int n_prep = j->n_prep;
     int64_t h2d = j->h2d;
     PlanTarget pt{};
     { int rc = sc.reference(j, &pt.ref, &n_prep); if (rc) return rc; }
-    { int rc = plan_from_histogram(c, b, n_aln); if (rc) return rc; }
-    if (n_aln > 0) {
-        CU(c, cudaMemcpyAsync(b->d_keybase, b->h_keybase, (size_t)BIN_KEYS * 4, cudaMemcpyHostToDevice, s2));
-        if (b->n_items > 0)
-            CU(c, cudaMemcpyAsync(b->d_items, b->h_items, (size_t)b->n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, s2));
-        h2d += (int64_t)BIN_KEYS * 4 + b->n_items * (int64_t)sizeof(WarpItem);
-        CU(c, launch_bin_scatter(b->ba, c->sm_count, s2));
-    }
-    CU(c, cudaEventRecord(b->ev_ready, s2));
-    // ---- SW kernels: the batch's plan against the caller's reference ----
-    CU(c, cudaStreamWaitEvent(c->stream, b->ev_ready, 0));
-    CU(c, cudaEventRecord(b->ev[1], c->stream));
+    { int rc = plan_from_histogram(c, bs, n_aln); if (rc) return rc; }
+    if (n_aln > 0) h2d += (int64_t)BIN_KEYS * 4 + bs.n_items * (int64_t)sizeof(WarpItem);
+    { int rc = bin_scatter(c, bs); if (rc) return rc; }
+    CU(c, cudaEventRecord(bs.ev_ready, c->stream2));
+    // ---- SW kernels: the plan against the caller's reference ----
+    pt.seq = bs.d_in_seq4;
     pt.tags_only = 0;   // every item is traced back (or has its end cell found), whatever the ctx's FADEGPU_F_TAGS_ONLY
     pt.ops_spill = max_ops > 0 ? j->d_spill : nullptr;
     pt.ops_cap = max_ops;
     pt.end_only = sc.score_only;
     int nl = 0;
-    { int rc = run_plan(c, b, pt, nullptr, nullptr, nullptr, &nl, b->ev_ready); if (rc) return rc; }
+    { int rc = run_kernels(c, bs, pt, &nl); if (rc) return rc; }
     // ---- records in item order, home on stream3 ----
     cudaStream_t s3 = c->stream3;
-    { int rc = join_kernels(c, b, s3); if (rc) return rc; }
-    CU(c, cudaEventRecord(b->ev[2], s3));
     // the results kernel writes the ops of the aligned items only: empty and oversize items keep these zeros (rather
     // than whatever an earlier call of this job left there)
     if (max_ops > 0) CU(c, cudaMemsetAsync(j->d_ops, 0, (size_t)n * (size_t)max_ops * 4, s3));
     CU(c, launch_pair_results(n, reinterpret_cast<const int64_t *>(j->d_raw), reinterpret_cast<const int64_t *>(j->d_raw + sc.o_tbeg),
-                              reinterpret_cast<const int64_t *>(j->d_raw + sc.o_tend), b->d_aln, b->d_out, (int)n_aln,
+                              reinterpret_cast<const int64_t *>(j->d_raw + sc.o_tend), bs.d_aln, bs.d_out, (int)n_aln,
                               sc.score_only, j->d_spill, max_ops, reinterpret_cast<PairResult *>(j->d_res), j->d_ops,
-                              b->d_stats + 7, c->sm_count, s3));
+                              bs.d_stats + 7, c->sm_count, s3));
     CU(c, cudaMemcpyAsync(j->out, j->d_res, (size_t)n * sizeof(fadegpu_pair_result), cudaMemcpyDeviceToHost, s3));
     if (max_ops > 0)
         CU(c, cudaMemcpyAsync(j->ops_out, j->d_ops, (size_t)n * (size_t)max_ops * 4, cudaMemcpyDeviceToHost, s3));
-    CU(c, cudaMemcpyAsync(b->h_stats + 7, b->d_stats + 7, 8, cudaMemcpyDeviceToHost, s3));
-    CU(c, cudaEventRecord(b->ev[3], s3));
+    CU(c, cudaMemcpyAsync(bs.h_stats + 7, bs.d_stats + 7, 8, cudaMemcpyDeviceToHost, s3));
+    CU(c, cudaEventRecord(bs.ev[3], s3));
     fadegpu_stats &st = j->st;
     st.n_aligned = n_aln;
-    st.n_generic = b->st.n_generic;
-    st.cells = (int64_t)b->h_stats[0];
+    st.n_generic = bs.n_generic;
+    st.cells = (int64_t)bs.h_stats[0];
     st.h2d_bytes = h2d;
     st.d2h_bytes = n * (int64_t)(sizeof(fadegpu_pair_result) + 4 * (size_t)max_ops) + (int64_t)BIN_KEYS * 4 + 128 + 4 + 8;
     st.kernel_launches = nl + n_prep + 1 + (n_aln > 0 ? 2 : 1);
-    st.scratch_bytes = b->st.scratch_bytes;
+    st.scratch_bytes = bs.scratch_bytes;
     st.host_threads = c->host_threads;
     return FADEGPU_OK;
 }
@@ -1926,14 +1946,13 @@ static int launch_job(fadegpu_ctx *c, fadegpu_job *j)
 static int finish_job(fadegpu_ctx *c, fadegpu_job *j)
 {
     if (j->sc.n == 0) return FADEGPU_OK;
-    fadegpu_batch *b = j->b;
-    CU(c, cudaEventSynchronize(b->ev[3]));
-    if ((int64_t)b->h_stats[7] != j->st.n_aligned)
+    const BinState &bs = j->bs;
+    CU(c, cudaEventSynchronize(bs.ev[3]));
+    if ((int64_t)bs.h_stats[7] != j->st.n_aligned)
         return fail(c, FADEGPU_E_CUDA, std::string(j->sc.fn) + ": a kernel did not produce a result record (internal error)");
     float t;
-    if (cudaEventElapsedTime(&t, b->ev[1], b->ev[2]) == cudaSuccess) j->st.kernel_ms = t;
-    if (cudaEventElapsedTime(&t, b->ev[0], b->ev[3]) == cudaSuccess) j->st.total_ms = t;
-    b->st = j->st;
+    if (cudaEventElapsedTime(&t, bs.ev[1], bs.ev[2]) == cudaSuccess) j->st.kernel_ms = t;
+    if (cudaEventElapsedTime(&t, bs.ev[0], bs.ev[3]) == cudaSuccess) j->st.total_ms = t;
     return FADEGPU_OK;
 }
 
@@ -2045,7 +2064,7 @@ static int pairs_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n
         if (tbytes) parallel_copy(h + o_t, in->target + t0, (size_t)tbytes, c->host_threads);
     };
     auto prep = [&](fadegpu_job *j, const char *d, BinArgs &ba, int *launches) -> int {
-        fadegpu_batch *b = j->b;
+        BinState &bs = j->bs;
         int rc = 0;
         auto grow = [&](auto **p, size_t *have, size_t bytes) { if (!rc) rc = ensure_dev(c, (void **)p, have, std::max<size_t>(bytes, 16)); };
         grow(&j->d_two, &j->two_bytes, (size_t)n_words * 8); grow(&j->d_n, &j->n_bytes, (size_t)n_words * 4);
@@ -2057,11 +2076,11 @@ static int pairs_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n
         pa.n = n;
         pa.qoff = reinterpret_cast<const int64_t *>(d); pa.toff = reinterpret_cast<const int64_t *>(d + o_toff);
         pa.query = d + o_q; pa.target = d + o_t;
-        pa.seq_off = b->d_in_seq_off; pa.pos = b->d_in_pos; pa.l_qseq = b->d_in_lq; pa.tid = b->d_in_tid;
-        pa.aligned_len = b->d_in_alen; pa.clip_left = b->d_in_cl; pa.clip_right = b->d_in_cr;
-        pa.clen = j->d_clen; pa.coff = j->d_coff; pa.seq4 = b->d_in_seq4; pa.bad = j->d_bad;
+        pa.seq_off = bs.d_in_seq_off; pa.pos = bs.d_in_pos; pa.l_qseq = bs.d_in_lq; pa.tid = bs.d_in_tid;
+        pa.aligned_len = bs.d_in_alen; pa.clip_left = bs.d_in_cl; pa.clip_right = bs.d_in_cr;
+        pa.clen = j->d_clen; pa.coff = j->d_coff; pa.seq4 = bs.d_in_seq4; pa.bad = j->d_bad;
         pa.two = j->d_two; pa.nmask = j->d_n; pa.xmask = j->d_x; pa.n_words = n_words;
-        pa.chunk_x = j->d_chunk_x; pa.n_x = b->d_stats + 12;
+        pa.chunk_x = j->d_chunk_x; pa.n_x = bs.d_stats + 12;
         CU(c, launch_pair_prep(pa, c->sm_count, c->stream2));
         CU(c, launch_pair_pack_targets(pa, c->stream2));
         *launches += 2;
@@ -2071,7 +2090,7 @@ static int pairs_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t n
     // (runs in the device half, possibly on the ctx thread: it captures nothing of this frame)
     sc.reference = [c](fadegpu_job *j, RefDev *ref, int *launches) -> int {
         PairArgs &pa = j->pa;
-        const int64_t n_x = (int64_t)j->b->h_stats[12];
+        const int64_t n_x = (int64_t)j->bs.h_stats[12];
         int rc = ensure_dev(c, (void **)&j->d_xpos, &j->xpos_bytes, std::max<size_t>(16, (size_t)n_x * 8));
         if (!rc) rc = ensure_dev(c, (void **)&j->d_xchr, &j->xchr_bytes, std::max<size_t>(16, (size_t)n_x));
         if (rc) return rc;
@@ -2158,16 +2177,16 @@ static int regions_call(fadegpu_ctx *c, const char *fn, bool score_only, int64_t
         if (qbytes) parallel_copy(h + o_q, in->query + q0, (size_t)qbytes, c->host_threads);
     };
     auto prep = [&](fadegpu_job *j, const char *d, BinArgs &ba, int *launches) -> int {
-        fadegpu_batch *b = j->b;
+        BinState &bs = j->bs;
         RegionArgs ra{};
         ra.n = n;
         ra.query = d + o_q; ra.qoff = reinterpret_cast<const int64_t *>(d);
         ra.rtid = reinterpret_cast<const int32_t *>(d + o_tid);
         ra.start = reinterpret_cast<const int64_t *>(d + o_start); ra.end = reinterpret_cast<const int64_t *>(d + o_end);
         ra.strand = reinterpret_cast<const uint8_t *>(d + o_strand);
-        ra.seq_off = b->d_in_seq_off; ra.pos = b->d_in_pos; ra.l_qseq = b->d_in_lq; ra.tid = b->d_in_tid;
-        ra.aligned_len = b->d_in_alen; ra.clip_left = b->d_in_cl; ra.clip_right = b->d_in_cr;
-        ra.seq4 = b->d_in_seq4; ra.bad = j->d_bad;
+        ra.seq_off = bs.d_in_seq_off; ra.pos = bs.d_in_pos; ra.l_qseq = bs.d_in_lq; ra.tid = bs.d_in_tid;
+        ra.aligned_len = bs.d_in_alen; ra.clip_left = bs.d_in_cl; ra.clip_right = bs.d_in_cr;
+        ra.seq4 = bs.d_in_seq4; ra.bad = j->d_bad;
         CU(c, launch_region_prep(ra, c->sm_count, c->stream2));
         *launches += 1;
         // the intervals were validated above, so the window arithmetic clamps nothing: gstart = coff[tid] + start
