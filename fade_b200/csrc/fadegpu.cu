@@ -6,8 +6,8 @@
 // source/analysis.d:34, window arithmetic of source/analysis.d:45-59, histogram), launch plan from the
 // histogram, bin_scatter_kernel (sorted descriptors), seq_pull_kernel (bases fetched from the pinned
 // view), then fills on `stream` and traceback rounds on `tstream` over alternating scratch sets (three by default),
-// result_index_kernel and the copies home on `stream3`.  FADEGPU_F_HOST_BINNING keeps the first
-// implementation, which evaluates the floor and the windows and sorts on the host.
+// result_index_kernel and the copies home on `stream3`.  FADEGPU_F_HOST_BINNING evaluates the floor and
+// the windows and sorts on the host, then plans from its histogram and runs the kernels on the same BinState.
 // A pair or region call (fadegpu_align_* / fadegpu_score_*, or a job of fadegpu_submit_pairs / _regions) is a stage
 // half on the caller's thread (stage_call: staging, upload, prep and classify on stream2) and a device half
 // (launch_job: plan, scatter, kernels, results on stream3), which the ctx thread runs for jobs.  A device-binned submit
@@ -201,7 +201,7 @@ struct fadegpu_job {
 struct AlnTmp {       // a read that needs SW, captured in read order (sequential pass), before sorting
     int64_t start;    // window start inside the contig
     int64_t so;       // byte offset of its bases inside the caller's seq4
-    int32_t read, tlen, cls, qlen, tid, key;
+    int32_t read, tlen, qlen, tid, key;
     uint32_t clip_left, clip_right;
 };
 
@@ -210,26 +210,26 @@ struct fadegpu_batch {
     fadegpu_batch_view v{};
     BinState bs;
     AlnOut *h_out = nullptr;                   // [max_reads] pinned result records
+    int64_t *h_aln_start = nullptr;            // [max_reads] pinned window start of each record
     int64_t n_reads = 0;
     fadegpu_stats st{};
     bool in_flight = false;
     // host binning: staging (pinned descriptors and bases, allocated on first use) and scratch
     AlnDesc *h_aln = nullptr;
-    uint8_t *h_seq = nullptr, *d_seq = nullptr;
+    uint8_t *h_seq = nullptr;
     int64_t cap_seq = 0;
     std::vector<std::vector<AlnTmp>> tl_aln;   // per host thread
     std::vector<uint32_t> order;               // alignment indices sorted by (class, window length desc)
     int32_t *h_ridx = nullptr;                 // [max_reads] per read: index into the results, -1 = none
     std::vector<AlnTmp> all_aln;
     std::vector<int32_t> cnt;
-    std::vector<int64_t> soff, aln_start;
+    std::vector<int64_t> soff;
     // ---- device-side binning (submits from the pinned view) ----
     bool dev_binning = false;          // the last submit used it
     int32_t *d_ridx = nullptr;                         // per read: index into the results (built on the device, copied home)
     uint8_t *d_rflags = nullptr;
     uint8_t *d_gate = nullptr;                         // compact inputs: the one byte per read that is uploaded
     const uint4 *d_view_meta = nullptr;                // device address of the pinned view's 32-byte records
-    int64_t *h_aln_start = nullptr;                   // pinned
     // reads that pass the length floor, gathered by the host in read order (pinned, allocated on first use)
     uint8_t *h_c_seq4 = nullptr;
     int64_t *h_c_seq_off = nullptr, *h_c_pos = nullptr;
@@ -374,21 +374,6 @@ RefDev ref_dev(const fadegpu_ctx *c)
     return r;
 }
 
-// rank of a row class inside ROW_CLASSES; N_ROW_CLASSES = the generic list
-int cls_rank(int cls)
-{
-    for (int k = 0; k < N_ROW_CLASSES; ++k) if (ROW_CLASSES[k] == cls) return k;
-    return N_ROW_CLASSES;
-}
-
-int class_of(const fadegpu_ctx *c, int qlen, int tlen)
-{
-    if (c->p.flags & FADEGPU_F_FORCE_GENERIC) return 0;
-    if (qlen > QMAX_FAST || tlen > TMAX_PACKED) return 0;
-    for (int k = 0; k < N_ROW_CLASSES; ++k) if (qlen <= FG * ROW_CLASSES[k]) return ROW_CLASSES[k];
-    return 0;
-}
-
 size_t ck_words_of(int R) { return (size_t)(2 * R + 2); }
 
 int ensure_dev(fadegpu_ctx *c, void **p, size_t *have, size_t bytes)
@@ -420,11 +405,14 @@ size_t gen_slot_bytes(int qmax, int tmax)
 }
 
 // Launch plan from the sorted order: cls_first[rk] = first sorted position of row class rk (the
-// generic list is rank N_ROW_CLASSES), sorted_tlen[pos] = window length at sorted position pos.
-// Fills s.plan, s.h_items and grows the ctx scratch buffers.
-int build_plan(fadegpu_ctx *c, BinState &s, int64_t n_aln, const int64_t *cls_first, const int32_t *sorted_tlen,
-               int qmax_all, int tmax_all, int gen_qmax, int gen_tmax)
+// generic list is rank N_ROW_CLASSES), s.sorted_tlen[pos] = window length at sorted position pos,
+// s.h_stats[2..5] = the maxima of the binning.  Fills s.plan, s.h_items and grows the ctx scratch buffers.
+int build_plan(fadegpu_ctx *c, BinState &s, const int64_t *cls_first)
 {
+    const int64_t n_aln = cls_first[N_ROW_CLASSES + 1];
+    const int32_t *sorted_tlen = s.sorted_tlen.data();
+    const int qmax_all = std::max(1, (int)s.h_stats[2]), tmax_all = std::max(1, (int)s.h_stats[3]);
+    const int gen_qmax = std::max(1, (int)s.h_stats[4]), gen_tmax = std::max(1, (int)s.h_stats[5]);
     int64_t n_items = 0;
     size_t ck_needed = 0, gen_needed = 0, trace_needed = 0;
     s.plan.clear();
@@ -505,11 +493,10 @@ struct PlanTarget {
     bool end_only;
 };
 
-// an annotate batch's plan: its queries are staged by the host binning (d_seq) or in the device mirror (d_in_seq4)
+// an annotate batch's plan: both binnings stage its queries in the device mirror (d_in_seq4)
 PlanTarget batch_target(const fadegpu_ctx *c, const fadegpu_batch *b)
 {
-    return PlanTarget{ ref_dev(c), b->dev_binning ? b->bs.d_in_seq4 : b->d_seq, (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0,
-                       nullptr, 0, false };
+    return PlanTarget{ ref_dev(c), b->bs.d_in_seq4, (c->p.flags & FADEGPU_F_TAGS_ONLY) ? 1 : 0, nullptr, 0, false };
 }
 
 // Queue every kernel of the plan: fills on c->stream (after `dep`: the inputs, or the start of a timed replay),
@@ -658,8 +645,8 @@ int bin_classify(fadegpu_ctx *c, BinState &s, void *h_list, const void *d_list, 
     return 0;
 }
 
-// Launch plan from the binning histogram of the device (s.h_hist, s.h_stats) that classified n_aln alignments; also
-// fills s.h_keybase, the first sorted position of every key, for bin_scatter_kernel.
+// Launch plan from the binning histogram (s.h_hist, s.h_stats: from the device, or summed by the host binning) that
+// classified n_aln alignments; also fills s.h_keybase, the first sorted position of every key, for the scatter.
 int plan_from_histogram(fadegpu_ctx *c, BinState &s, int64_t n_aln)
 {
     int64_t cls_first[N_ROW_CLASSES + 2];
@@ -680,8 +667,7 @@ int plan_from_histogram(fadegpu_ctx *c, BinState &s, int64_t n_aln)
     }
     cls_first[N_ROW_CLASSES + 1] = run;
     if (run != n_aln) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: internal error (histogram does not add up)");
-    return build_plan(c, s, n_aln, cls_first, stl.data(), std::max(1, (int)s.h_stats[2]), std::max(1, (int)s.h_stats[3]),
-                      std::max(1, (int)s.h_stats[4]), std::max(1, (int)s.h_stats[5]));
+    return build_plan(c, s, cls_first);
 }
 
 // After plan_from_histogram, on stream2: the keybase and the plan's warp items go up (BIN_KEYS * 4 +
@@ -992,7 +978,7 @@ void fadegpu_free_batch(fadegpu_batch *b)
     free_host(v.flags); free_host(v.score); free_host(v.beg_query); free_host(v.end_query);
     free_host(v.beg_ref); free_host(v.end_ref); free_host(v.win_start); free_host(v.n_ops); free_host(v.ops);
     free_host(b->h_aln); free_host(b->h_seq); free_host(b->h_out); free_host(b->h_ridx); free_host(b->h_aln_start);
-    free_dev(b->d_seq); free_dev(b->d_ridx); free_dev(b->d_rflags); free_dev(b->d_gate);
+    free_dev(b->d_ridx); free_dev(b->d_rflags); free_dev(b->d_gate);
     free_host(b->h_c_seq4); free_host(b->h_c_seq_off); free_host(b->h_c_pos); free_host(b->h_c_lq); free_host(b->h_c_tid);
     free_host(b->h_c_alen); free_host(b->h_c_cl); free_host(b->h_c_cr); free_host(b->h_c_read); free_dev(b->d_in_read);
     free_dev(b->d_aln_scratch); free_dev(b->d_i64_scratch);
@@ -1024,7 +1010,7 @@ int fadegpu_alloc_batch(fadegpu_ctx *c, int64_t max_reads, int64_t max_seq_bytes
         H(&v.end_ref, n * 4); H(&v.win_start, n * 8); H(&v.n_ops, n * 4); H(&v.ops, n * 4 * FADEGPU_MAX_OPS);
     }
     H(&b->h_out, n * sizeof(AlnOut)); H(&b->h_ridx, n * 4); H(&b->h_aln_start, n * 8);
-    // h_aln / h_seq / d_seq (staging of the host-binning path) are allocated on its first use
+    // h_aln / h_seq (staging of the host-binning path) are allocated on its first use
     // device-side binning beyond the core: gathered read indices, per-read result index and flags, gate bytes
     D(&b->d_in_read, n * 4); D(&b->d_ridx, n * 4); D(&b->d_rflags, n); D(&b->d_gate, n);
     if (e == cudaSuccess) e = cudaHostGetDevicePointer((void **)&b->d_view_seq4, v.seq4, 0);
@@ -1049,7 +1035,6 @@ static int ensure_host_staging(fadegpu_ctx *c, fadegpu_batch *b)
     const size_t n = (size_t)b->v.max_reads;
     CU(c, cudaHostAlloc((void **)&b->h_aln, n * sizeof(AlnDesc), cudaHostAllocDefault));
     CU(c, cudaHostAlloc((void **)&b->h_seq, (size_t)b->cap_seq, cudaHostAllocDefault));
-    CU(c, cudaMalloc((void **)&b->d_seq, (size_t)b->cap_seq));
     return 0;
 }
 
@@ -1078,8 +1063,10 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     CU(c, cudaSetDevice(c->device));
     { int rc = ensure_host_staging(c, b); if (rc) return rc; }
     const int64_t n = n_reads;
+    BinState &bs = b->bs;
     b->n_reads = n;
-    b->bs.plan.clear();
+    bs.plan.clear();
+    bs.ba.n = 0;   // nothing binned on the device: replays run the plan only
     b->dev_binning = false;
     memset(&b->st, 0, sizeof(b->st));
     b->st.n_reads = n;
@@ -1095,9 +1082,9 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     const uint32_t floor_u = (uint32_t)c->p.min_length;  // uint <= int compare of analysis.d:34
     const int64_t W = c->p.window_size;
     const int64_t seq_total = n > 0 ? in->seq_off[n] : 0;
-    int64_t cells = 0, n_over = 0;
-    int bad = 0;
-#pragma omp parallel num_threads(nthr) reduction(+ : cells) reduction(| : bad)
+    int64_t cells = 0, n_over = 0, seq_bytes = 0;
+    int bad = 0, qmax = 0, tmax = 0, qmax_g = 0, tmax_g = 0;
+#pragma omp parallel num_threads(nthr) reduction(+ : cells, seq_bytes) reduction(| : bad) reduction(max : qmax, tmax, qmax_g, tmax_g)
     {
         int tix = 0, tn = 1;
 #ifdef _OPENMP
@@ -1125,25 +1112,28 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
             if (end - start > 0x7fffffff || (end - start) * (int64_t)ql > ((int64_t)1 << 31)) {
                 // (the reference would need a multi-GB trace for this ONE read) left unaligned and reported
 #pragma omp critical(fadegpu_oversize)
-                { if (n_over < OVER_CAP) b->bs.h_over[n_over] = (int32_t)r; ++n_over; }
+                { if (n_over < OVER_CAP) bs.h_over[n_over] = (int32_t)r; ++n_over; }
                 continue;
             }
             const int tlen = (int)(end - start);
-            const int cls = class_of(c, ql, tlen);
-            const int rk = cls_rank(cls);
+            const int rk = bin_rank(ql, tlen, c->p.flags & FADEGPU_F_FORCE_GENERIC);
             // key = class rank (row classes, then the generic list) then descending window length (generic: input order)
-            const int key = bin_key(rk, tlen);
-            loc.push_back(AlnTmp{ start, so, (int32_t)r, tlen, cls, ql, tid, key, cl, cr });
+            loc.push_back(AlnTmp{ start, so, (int32_t)r, tlen, ql, tid, bin_key(rk, tlen), cl, cr });
             cells += (int64_t)ql * tlen;
+            seq_bytes += (ql + 1) / 2;
+            qmax = std::max(qmax, ql); tmax = std::max(tmax, tlen);
+            if (rk == N_ROW_CLASSES) { qmax_g = std::max(qmax_g, ql); tmax_g = std::max(tmax_g, tlen); }
         }
     }
     if (bad & 1) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: seq_off / l_qseq inconsistent");
     b->st.cells = cells;
     b->st.n_oversize = n_over;
     b->st.host_classify_ms = ms_since(t_begin);
+    // (they go up into bs.d_in_seq4, which holds max_seq_bytes + 32 n + 16 bytes)
+    if (seq_bytes > b->cap_seq) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: read bases exceed max_seq_bytes");
     const auto t_sort = std::chrono::steady_clock::now();
 
-    // ---- 2. bin by class, counting sort by window length (longest first) ----
+    // ---- 2. bin by class, counting sort by window length (longest first), launch plan ----
     int64_t n_aln = 0;
     for (int t = 0; t < nthr; ++t) n_aln += (int64_t)b->tl_aln[(size_t)t].size();
     std::vector<AlnTmp> &all = b->all_aln;
@@ -1151,12 +1141,12 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     all.resize((size_t)n_aln);
     order.resize((size_t)n_aln);
     // parallel, stable counting sort of the INDICES: per-thread histograms over the thread's own
-    // (read-ordered) slice, one prefix pass over (key, thread), per-thread scatter
+    // (read-ordered) slice, their sum planned like a device histogram, per-thread start of every key
+    // (key, then thread), per-thread scatter
     const int KEYS = BIN_KEYS;
     std::vector<int32_t> &hist = b->cnt;
     hist.resize((size_t)nthr * (size_t)(KEYS + 1));
     std::vector<int64_t> toff((size_t)nthr + 1, 0);
-    std::vector<int> kmin((size_t)nthr, KEYS), kmax((size_t)nthr, -1);
     for (int t = 0; t < nthr; ++t) toff[(size_t)t + 1] = toff[(size_t)t] + (int64_t)b->tl_aln[(size_t)t].size();
 #pragma omp parallel num_threads(nthr)
     {
@@ -1169,29 +1159,29 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
             int32_t *h = hist.data() + (size_t)t * (size_t)(KEYS + 1);
             memset(h, 0, (size_t)(KEYS + 1) * sizeof(int32_t));
             if (!loc.empty()) memcpy(all.data() + toff[(size_t)t], loc.data(), loc.size() * sizeof(AlnTmp));
-            int lo = KEYS, hi = -1;
-            for (const AlnTmp &a : loc) { ++h[a.key]; lo = std::min(lo, a.key); hi = std::max(hi, a.key); }
-            kmin[(size_t)t] = lo; kmax[(size_t)t] = hi;
+            for (const AlnTmp &a : loc) ++h[a.key];
         }
     }
-    int64_t cls_first[N_ROW_CLASSES + 2];
-    {
-        int64_t run = 0;
-        int klo = KEYS, khi = -1;
-        for (int t = 0; t < nthr; ++t) { klo = std::min(klo, kmin[(size_t)t]); khi = std::max(khi, kmax[(size_t)t]); }
-        for (int rk = 0; rk <= N_ROW_CLASSES; ++rk) cls_first[rk] = -1;
-        for (int key = std::max(klo, 0); key <= khi; ++key) {
-            const int rk = key / KEYS_PER_CLASS;
-            if (cls_first[rk] < 0) cls_first[rk] = run;   // first key seen of this class
-            for (int t = 0; t < nthr; ++t) {
-                int32_t &hv = hist[(size_t)t * (size_t)(KEYS + 1) + (size_t)key];
-                const int32_t c0 = hv;
-                hv = (int32_t)run;
-                run += c0;
-            }
+#pragma omp parallel for schedule(static) num_threads(nthr)
+    for (int key = 0; key < KEYS; ++key) {
+        int32_t sum = 0;
+        for (int t = 0; t < nthr; ++t) sum += hist[(size_t)t * (size_t)(KEYS + 1) + (size_t)key];
+        bs.h_hist[key] = sum;
+    }
+    memset(bs.h_stats, 0, 128);   // the layout bin_classify_kernel writes
+    bs.h_stats[0] = (unsigned long long)cells; bs.h_stats[1] = (unsigned long long)n_aln;
+    bs.h_stats[2] = qmax; bs.h_stats[3] = tmax; bs.h_stats[4] = qmax_g; bs.h_stats[5] = tmax_g;
+    { int rc = plan_from_histogram(c, bs, n_aln); if (rc) return rc; }
+    b->st.n_aligned = n_aln; b->st.n_generic = bs.n_generic; b->st.scratch_bytes = bs.scratch_bytes;
+    for (int key = 0; key < KEYS; ++key) {
+        if (!bs.h_hist[key]) continue;
+        int32_t run = bs.h_keybase[key];
+        for (int t = 0; t < nthr; ++t) {
+            int32_t &hv = hist[(size_t)t * (size_t)(KEYS + 1) + (size_t)key];
+            const int32_t c0 = hv;
+            hv = run;
+            run += c0;
         }
-        cls_first[N_ROW_CLASSES + 1] = n_aln;
-        for (int rk = N_ROW_CLASSES; rk >= 0; --rk) if (cls_first[rk] < 0) cls_first[rk] = cls_first[rk + 1];   // empty classes
     }
 #pragma omp parallel num_threads(nthr)
     {
@@ -1210,22 +1200,11 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
     const auto t_gather = std::chrono::steady_clock::now();
     // ---- 3. descriptors + gathered read bases ----
     std::vector<int64_t> &soff = b->soff;
-    soff.resize((size_t)n_aln + 1);
-    int qmax_all = 1, tmax_all = 1;
-    {
-        int64_t o = 0;
-        for (int64_t kx = 0; kx < n_aln; ++kx) {
-            soff[(size_t)kx] = o;
-            const AlnTmp &a = all[order[(size_t)kx]];
-            o += (a.qlen + 1) / 2;
-            qmax_all = std::max(qmax_all, a.qlen);
-            tmax_all = std::max(tmax_all, a.tlen);
-        }
-        soff[(size_t)n_aln] = o;
+    soff.resize((size_t)n_aln);
+    for (int64_t kx = 0, o = 0; kx < n_aln; ++kx) {
+        soff[(size_t)kx] = o;
+        o += (all[order[(size_t)kx]].qlen + 1) / 2;
     }
-    const int64_t seq_bytes = soff[(size_t)n_aln];
-    if (seq_bytes > b->cap_seq) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: read bases exceed max_seq_bytes");
-    b->aln_start.resize((size_t)n_aln);
 #pragma omp parallel for schedule(static) num_threads(nthr)
     for (int64_t kx = 0; kx < n_aln; ++kx) {
         const AlnTmp &a = all[order[(size_t)kx]];
@@ -1243,26 +1222,14 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
         d.clip_right = a.clip_right;
         d.read = a.read;
         d.pad = 0;
-        b->aln_start[(size_t)kx] = a.start;
+        b->h_aln_start[kx] = a.start;
         memcpy(b->h_seq + d.seq_off, in->seq4 + a.so, (size_t)((ql + 1) / 2));
     }
 
     b->st.host_gather_ms = ms_since(t_gather);
-    // ---- 4. launch plan ----
-    std::vector<int32_t> &stl = b->bs.sorted_tlen;
-    stl.resize((size_t)n_aln);
-    for (int64_t kx = 0; kx < n_aln; ++kx) {   // long windows share keys: the plan uses the key's upper end for all of them
-        const AlnTmp &t = all[order[(size_t)kx]];
-        stl[(size_t)kx] = (t.cls != 0 && t.tlen > TMAX_FAST) ? key_tlen(t.key % KEYS_PER_CLASS) : t.tlen;
-    }
-    int gq = 1, gt = 1;
-    for (int64_t kx = cls_first[N_ROW_CLASSES]; kx < n_aln; ++kx) { gq = std::max(gq, b->h_aln[kx].qlen); gt = std::max(gt, b->h_aln[kx].tlen); }
-    BinState &bs = b->bs;
-    { int rc = build_plan(c, bs, n_aln, cls_first, stl.data(), qmax_all, tmax_all, gq, gt); if (rc) return rc; }
-    b->st.n_aligned = n_aln; b->st.n_generic = bs.n_generic; b->st.scratch_bytes = bs.scratch_bytes;
     const int64_t n_items = bs.n_items;
 
-    // ---- 5. queue copies and kernels ----
+    // ---- 4. queue copies and kernels ----
     // copies in on stream2, kernels on the compute stream, copies out on stream3: the DMA of one
     // batch overlaps the kernels of its neighbours
     CU(c, cudaEventRecord(bs.ev[0], c->stream2));
@@ -1270,7 +1237,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
         CU(c, cudaMemcpyAsync(bs.d_aln, b->h_aln, (size_t)n_aln * sizeof(AlnDesc), cudaMemcpyHostToDevice, c->stream2));
         if (n_items > 0)
             CU(c, cudaMemcpyAsync(bs.d_items, bs.h_items, (size_t)n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, c->stream2));
-        CU(c, cudaMemcpyAsync(b->d_seq, b->h_seq, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream2));
+        CU(c, cudaMemcpyAsync(bs.d_in_seq4, b->h_seq, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream2));
     }
     b->st.h2d_bytes = n_aln * (int64_t)sizeof(AlnDesc) + n_items * (int64_t)sizeof(WarpItem) + seq_bytes;
     CU(c, cudaEventRecord(bs.ev_ready, c->stream2));
@@ -1646,7 +1613,6 @@ int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
     // cores the ctx thread needs to queue the next batch)
     const bool walk = scatter || !b->dev_binning;
     const int nthr = walk ? (int)std::max<int64_t>(1, std::min<int64_t>(c->host_threads, b->bs.n_aln / 8192 + 1)) : 1;
-    const int64_t *wstart = b->dev_binning ? b->h_aln_start : b->aln_start.data();
     int64_t bad = 0;
     if (b->dev_binning) {
         if (b->bs.n_aln > 0 && (int64_t)b->bs.h_stats[7] != b->bs.n_aln) bad = 1;   // result records counted on the device
@@ -1666,7 +1632,7 @@ int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
         if (!scatter) continue;
         v.score[r] = o.score; v.beg_query[r] = o.beg_query; v.end_query[r] = o.end_query;
         v.beg_ref[r] = o.beg_ref; v.end_ref[r] = o.end_ref; v.n_ops[r] = o.n_ops;
-        v.win_start[r] = wstart[k];
+        v.win_start[r] = b->h_aln_start[k];
         memcpy(v.ops + (size_t)r * FADEGPU_MAX_OPS, o.ops, sizeof(o.ops));
     }
     for (int64_t k = 0; k < std::min<int64_t>(b->st.n_oversize, OVER_CAP); ++k) {
@@ -1685,7 +1651,7 @@ int fadegpu_get_results(const fadegpu_batch *b, fadegpu_results_view *r)
     static_assert(sizeof(fadegpu_result) == sizeof(AlnOut), "fadegpu_result must mirror AlnOut");
     r->n_results = b->bs.n_aln;
     r->results = reinterpret_cast<const fadegpu_result *>(b->h_out);
-    r->win_start = b->dev_binning ? b->h_aln_start : b->aln_start.data();
+    r->win_start = b->h_aln_start;
     r->result_index = b->h_ridx;
     return FADEGPU_OK;
 }
@@ -1712,7 +1678,7 @@ int fadegpu_get_timeline(const fadegpu_batch *b, const fadegpu_batch *origin, fl
 static int replay_binning(fadegpu_ctx *c, fadegpu_batch *b, cudaEvent_t *dep)
 {
     *dep = nullptr;
-    if (!b->dev_binning || b->bs.ba.n == 0) return 0;
+    if (b->bs.ba.n == 0) return 0;
     const size_t n = (size_t)b->v.max_reads;
     if (!b->d_aln_scratch) {
         CU(c, cudaMalloc((void **)&b->d_aln_scratch, n * sizeof(AlnDesc)));

@@ -451,20 +451,32 @@ def test_compact_inputs_equal_view_inputs_and_oracle():
 def test_device_and_host_binning_agree(flags):
     """By default the host only gathers the reads past the length floor and the device bins them, queued
     on the ctx thread; FADEGPU_F_SYNC_SUBMIT does that on the calling thread, FADEGPU_F_HOST_BINNING bins
-    on the host.  Same records every way (ragged lengths, several contigs), from the view and from arrays."""
+    on the host.  Same records every way (ragged lengths, several contigs), from the view and from arrays, and
+    the same plan as the default flags (every binning feeds one planner)."""
     rng = random.Random(41)
     contigs = [readsets.random_ref(rng, n) for n in (9000, 2500, 600)]
     rd = readsets.build(readsets.ragged_reads(rng, contigs, 4000, max_len=320))
+
+    def plan_of(st):
+        return st.n_aligned, st.n_generic, st.cells, st.scratch_bytes
+
+    with _ctx() as ctx:
+        ctx.load_reference(["a", "b", "c"], contigs)
+        b = run_gpu(ctx, rd)
+        want = plan_of(b.stats())
+        b.close()
     with _ctx(flags=flags) as ctx:
         ctx.load_reference(["a", "b", "c"], contigs)
         b = run_gpu(ctx, rd)                       # fadegpu_submit (pinned view)
         compare(b, rd, contigs, oracle_params(ctx.params))
         st = b.stats()
         assert st.n_aligned > 800 and st.n_generic > 0
+        assert plan_of(st) == want
         rec1 = b.results()[0]
         rec1 = rec1[np.argsort(rec1["read"])].copy()
         b.submit_arrays(rd.n, rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
         b.wait()                                   # fadegpu_submit_inputs (caller-owned arrays)
+        assert plan_of(b.stats()) == want
         rec2 = b.results()[0]
         assert np.array_equal(rec1, rec2[np.argsort(rec2["read"])])
         b.run(0)                                   # empty batch through the device path
