@@ -1,13 +1,16 @@
 // fadegpu.cu -- C ABI (include/fadegpu.h) and host runtime of libfadegpu: contexts, packed
 // reference upload, pinned batch buffers, queued submits, launch planning, streams, results.
 //
-// A submit is: (fadegpu_submit_inputs only: gather of the reads past the length floor, on the
-// caller's thread) -> on the ctx thread: upload, bin_classify_kernel (length floor of
-// source/analysis.d:34, window arithmetic of source/analysis.d:45-59, histogram), launch plan from the
-// histogram, bin_scatter_kernel (sorted descriptors), seq_pull_kernel (bases fetched from the pinned
-// view), then fills on `stream` and traceback rounds on `tstream` over alternating scratch sets (three by default),
-// result_index_kernel and the copies home on `stream3`.  FADEGPU_F_HOST_BINNING evaluates the floor and
-// the windows and sorts on the host, then plans from its histogram and runs the kernels on the same BinState.
+// fadegpu_submit (the pinned view), fadegpu_submit_compact (gate bytes + compact records) and fadegpu_submit_inputs (the
+// caller's arrays) check their arguments and the ctx's state (refuse_submit) and run one sequence (submit_batch).
+// A device-binned submit is: (caller's arrays only: gather of the reads past the length floor, on the
+// caller's thread) -> submit_device_binning on the ctx thread (the caller's with FADEGPU_F_SYNC_SUBMIT): upload,
+// bin_classify_kernel (length floor of source/analysis.d:34, window arithmetic of source/analysis.d:45-59, histogram),
+// launch plan from the histogram, bin_scatter_kernel (sorted descriptors), seq_pull_kernel (bases fetched from the
+// pinned view), then fills on `stream` and traceback rounds on `tstream` over alternating scratch sets (three by
+// default), result_index_kernel and the copies home on `stream3`.  FADEGPU_F_HOST_BINNING (submit_host_binning, on the
+// caller's thread) evaluates the floor and the windows and sorts on the host, then plans from its histogram and runs
+// the kernels on the same BinState.  A batch and a job are in flight (InFlight) from their submit to their wait.
 // A pair or region call (fadegpu_align_* / fadegpu_score_*, or a job of fadegpu_submit_pairs / _regions) is a stage
 // half on the caller's thread (stage_call: staging, upload, prep and classify on stream2) and a device half
 // (launch_job: plan, scatter, kernels, results on stream3), which the ctx thread runs for jobs.  A device-binned submit
@@ -90,7 +93,8 @@ struct fadegpu_ctx {
     std::string err;
     // asynchronous submits: fadegpu_submit queues the batch (fadegpu_submit_pairs / _regions the job), this thread
     // waits for the binning histogram, plans and launches; the caller goes on filling / reading other batches or jobs
-    struct Queued { fadegpu_batch *b; int64_t n; fadegpu_job *j; };   // a batch of n reads, or a job
+    // a batch of n reads in input layout `mode` (SubmitMode; seq_bytes of compact inputs), or a job
+    struct Queued { fadegpu_batch *b; int64_t n; int mode; int64_t seq_bytes; fadegpu_job *j; };
     std::thread worker;
     std::mutex q_mu;
     std::condition_variable q_cv, done_cv;
@@ -161,6 +165,14 @@ struct BinState {
     cudaEvent_t ev_kernels = nullptr;                    // end of the kernels (recorded on tstream)
 };
 
+// A batch's or a job's submit from the submit call to its wait (guarded by ctx->q_mu): `queued` while its device half
+// waits for or runs on the ctx thread, which leaves that half's outcome here
+struct InFlight {
+    bool in_flight = false, queued = false;
+    int rc = 0;
+    std::string err;
+};
+
 // One pair or region call: its device-binning core, the staging of the raw inputs, the targets of a pair call packed
 // as a reference of their own, the records and ops of the call in pinned memory (fadegpu_job_results_view).
 // Everything grows with use.
@@ -192,10 +204,7 @@ struct fadegpu_job {
     int64_t h2d = 0;
     fadegpu_stats st{};
     int64_t n_res = -1;                                 // records of the last successful wait (-1: none)
-    // guarded by ctx->q_mu
-    bool in_flight = false, queued = false;
-    int rc = 0;                                         // outcome of a device half run by the ctx thread
-    std::string err;
+    InFlight fl;
 };
 
 struct AlnTmp {       // a read that needs SW, captured in read order (sequential pass), before sorting
@@ -213,10 +222,9 @@ struct fadegpu_batch {
     int64_t *h_aln_start = nullptr;            // [max_reads] pinned window start of each record
     int64_t n_reads = 0;
     fadegpu_stats st{};
-    bool in_flight = false;
-    // host binning: staging (pinned descriptors and bases, allocated on first use) and scratch
+    InFlight fl;
+    // host binning: staging (pinned descriptors, allocated on first use; the bases go through h_c_seq4) and scratch
     AlnDesc *h_aln = nullptr;
-    uint8_t *h_seq = nullptr;
     int64_t cap_seq = 0;
     std::vector<std::vector<AlnTmp>> tl_aln;   // per host thread
     std::vector<uint32_t> order;               // alignment indices sorted by (class, window length desc)
@@ -230,7 +238,8 @@ struct fadegpu_batch {
     uint8_t *d_rflags = nullptr;
     uint8_t *d_gate = nullptr;                         // compact inputs: the one byte per read that is uploaded
     const uint4 *d_view_meta = nullptr;                // device address of the pinned view's 32-byte records
-    // reads that pass the length floor, gathered by the host in read order (pinned, allocated on first use)
+    // reads that pass the length floor, gathered by the host in read order (pinned, allocated on first use); h_c_seq4
+    // also stages the bases of a host-binned submit
     uint8_t *h_c_seq4 = nullptr;
     int64_t *h_c_seq_off = nullptr, *h_c_pos = nullptr;
     int32_t *h_c_lq = nullptr, *h_c_tid = nullptr, *h_c_alen = nullptr, *h_c_cl = nullptr, *h_c_cr = nullptr, *h_c_read = nullptr;
@@ -241,12 +250,6 @@ struct fadegpu_batch {
     std::vector<int32_t> idx;                          // gather scratch
     AlnDesc *d_aln_scratch = nullptr;                  // replays scatter into these instead of the live descriptors
     int64_t *d_i64_scratch = nullptr;
-    int mode = 0;                                      // SubmitMode of the queued / last submit
-    int64_t job_seq_bytes = 0;
-    // asynchronous submit (guarded by ctx->q_mu)
-    bool queued = false;
-    int submit_rc = 0;
-    std::string submit_err;
 };
 
 extern "C" { static void drain_submits(fadegpu_ctx *c); }
@@ -967,7 +970,7 @@ void fadegpu_free_batch(fadegpu_batch *b)
     fadegpu_ctx *c = b->ctx;
     if (c) {
         std::unique_lock<std::mutex> lk(c->q_mu);
-        c->done_cv.wait(lk, [&] { return !b->queued; });
+        c->done_cv.wait(lk, [&] { return !b->fl.queued; });
         c->batches.erase(std::remove(c->batches.begin(), c->batches.end(), b), c->batches.end());
     }
     free_bin_state(c, b->bs);
@@ -977,7 +980,7 @@ void fadegpu_free_batch(fadegpu_batch *b)
     free_host(v.gate); free_host(v.meta);
     free_host(v.flags); free_host(v.score); free_host(v.beg_query); free_host(v.end_query);
     free_host(v.beg_ref); free_host(v.end_ref); free_host(v.win_start); free_host(v.n_ops); free_host(v.ops);
-    free_host(b->h_aln); free_host(b->h_seq); free_host(b->h_out); free_host(b->h_ridx); free_host(b->h_aln_start);
+    free_host(b->h_aln); free_host(b->h_out); free_host(b->h_ridx); free_host(b->h_aln_start);
     free_dev(b->d_ridx); free_dev(b->d_rflags); free_dev(b->d_gate);
     free_host(b->h_c_seq4); free_host(b->h_c_seq_off); free_host(b->h_c_pos); free_host(b->h_c_lq); free_host(b->h_c_tid);
     free_host(b->h_c_alen); free_host(b->h_c_cl); free_host(b->h_c_cr); free_host(b->h_c_read); free_dev(b->d_in_read);
@@ -1010,7 +1013,7 @@ int fadegpu_alloc_batch(fadegpu_ctx *c, int64_t max_reads, int64_t max_seq_bytes
         H(&v.end_ref, n * 4); H(&v.win_start, n * 8); H(&v.n_ops, n * 4); H(&v.ops, n * 4 * FADEGPU_MAX_OPS);
     }
     H(&b->h_out, n * sizeof(AlnOut)); H(&b->h_ridx, n * 4); H(&b->h_aln_start, n * 8);
-    // h_aln / h_seq (staging of the host-binning path) are allocated on its first use
+    // the host staging (h_aln, h_c_*) is allocated on first use
     // device-side binning beyond the core: gathered read indices, per-read result index and flags, gate bytes
     D(&b->d_in_read, n * 4); D(&b->d_ridx, n * 4); D(&b->d_rflags, n); D(&b->d_gate, n);
     if (e == cudaSuccess) e = cudaHostGetDevicePointer((void **)&b->d_view_seq4, v.seq4, 0);
@@ -1029,40 +1032,14 @@ int fadegpu_get_batch_view(fadegpu_batch *b, fadegpu_batch_view *view)
     return FADEGPU_OK;
 }
 
-static int ensure_host_staging(fadegpu_ctx *c, fadegpu_batch *b)
+// FADEGPU_F_HOST_BINNING, on the calling thread under submit_mu: the host evaluates the length floor and the windows
+// (analysis.d:34,45-59), sorts by (row class, window length) and gathers descriptors and bases, fills the batch's
+// histogram and stats as the classify kernel would and plans from them; uploads and kernels follow on the batch's
+// BinState as for a device-binned submit.  The independent reference for the classify kernel's arithmetic.
+static int submit_host_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, const fadegpu_inputs *in)
 {
-    if (b->h_aln) return 0;
-    const size_t n = (size_t)b->v.max_reads;
-    CU(c, cudaHostAlloc((void **)&b->h_aln, n * sizeof(AlnDesc), cudaHostAllocDefault));
-    CU(c, cudaHostAlloc((void **)&b->h_seq, (size_t)b->cap_seq, cudaHostAllocDefault));
-    return 0;
-}
-
-static int gather_reads(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, const fadegpu_inputs &in);
-static int queue_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, int mode, int64_t seq_bytes);
-static bool batch_in_flight(fadegpu_ctx *c, fadegpu_batch *b);
-static int refuse_jobs_in_flight(fadegpu_ctx *c, const char *fn);
-
-int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, const fadegpu_inputs *in)
-{
-    if (!c || !b || b->ctx != c || !in) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: bad ctx/batch/inputs");
-    if (!c->d_two) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: no reference loaded");
-    if (batch_in_flight(c, b)) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: batch already in flight (call fadegpu_wait)");
-    { int rc = refuse_jobs_in_flight(c, "fadegpu_submit"); if (rc) return rc; }
-    if (n_reads < 0 || n_reads > b->v.max_reads) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: n_reads out of range");
-    if (n_reads > 0 && (!in->seq4 || !in->seq_off || !in->l_qseq || !in->tid || !in->pos || !in->aligned_len ||
-                        !in->clip_left || !in->clip_right))
-        return fail(c, FADEGPU_E_ARG, "fadegpu_submit: null input array");
-    if (!(c->p.flags & FADEGPU_F_HOST_BINNING)) {
-        // the caller's arrays are only read here; uploads, binning and launches follow on the ctx thread
-        CU(c, cudaSetDevice(c->device));
-        { int rc = gather_reads(c, b, n_reads, *in); if (rc) return rc; }
-        return queue_submit(c, b, n_reads, 0 /* MODE_GATHERED */, 0);
-    }
-    std::lock_guard<std::mutex> submit_guard(c->submit_mu);
-    CU(c, cudaSetDevice(c->device));
-    { int rc = ensure_host_staging(c, b); if (rc) return rc; }
-    const int64_t n = n_reads;
+    if (!b->h_aln) CU(c, cudaHostAlloc((void **)&b->h_aln, (size_t)b->v.max_reads * sizeof(AlnDesc), cudaHostAllocDefault));
+    if (!b->h_c_seq4) CU(c, cudaHostAlloc((void **)&b->h_c_seq4, (size_t)b->cap_seq + 16, cudaHostAllocDefault));
     BinState &bs = b->bs;
     b->n_reads = n;
     bs.plan.clear();
@@ -1223,7 +1200,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
         d.read = a.read;
         d.pad = 0;
         b->h_aln_start[kx] = a.start;
-        memcpy(b->h_seq + d.seq_off, in->seq4 + a.so, (size_t)((ql + 1) / 2));
+        memcpy(b->h_c_seq4 + d.seq_off, in->seq4 + a.so, (size_t)((ql + 1) / 2));
     }
 
     b->st.host_gather_ms = ms_since(t_gather);
@@ -1237,7 +1214,7 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
         CU(c, cudaMemcpyAsync(bs.d_aln, b->h_aln, (size_t)n_aln * sizeof(AlnDesc), cudaMemcpyHostToDevice, c->stream2));
         if (n_items > 0)
             CU(c, cudaMemcpyAsync(bs.d_items, bs.h_items, (size_t)n_items * sizeof(WarpItem), cudaMemcpyHostToDevice, c->stream2));
-        CU(c, cudaMemcpyAsync(bs.d_in_seq4, b->h_seq, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream2));
+        CU(c, cudaMemcpyAsync(bs.d_in_seq4, b->h_c_seq4, (size_t)seq_bytes, cudaMemcpyHostToDevice, c->stream2));
     }
     b->st.h2d_bytes = n_aln * (int64_t)sizeof(AlnDesc) + n_items * (int64_t)sizeof(WarpItem) + seq_bytes;
     CU(c, cudaEventRecord(bs.ev_ready, c->stream2));
@@ -1248,7 +1225,6 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
         CU(c, cudaMemcpyAsync(b->h_out, bs.d_out, (size_t)n_aln * sizeof(AlnOut), cudaMemcpyDeviceToHost, c->stream3));
     b->st.d2h_bytes = n_aln * (int64_t)sizeof(AlnOut);
     CU(c, cudaEventRecord(bs.ev[3], c->stream3));
-    b->in_flight = true;
     b->st.host_submit_ms = ms_since(t_begin);
     return FADEGPU_OK;
 }
@@ -1260,9 +1236,9 @@ int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, con
 static int gather_reads(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, const fadegpu_inputs &in)
 {
     const auto t0 = std::chrono::steady_clock::now();
-    if (!b->h_c_seq4) {
+    if (!b->h_c_read) {   // (a host-binned submit may have allocated h_c_seq4 already)
         const size_t m = (size_t)b->v.max_reads;
-        auto H = [&](auto **p, size_t bytes) { return cudaHostAlloc((void **)p, std::max<size_t>(bytes, 16), cudaHostAllocDefault); };
+        auto H = [&](auto **p, size_t bytes) { return *p ? cudaSuccess : cudaHostAlloc((void **)p, std::max<size_t>(bytes, 16), cudaHostAllocDefault); };
         CU(c, H(&b->h_c_seq4, (size_t)b->cap_seq + 16)); CU(c, H(&b->h_c_seq_off, (m + 1) * 8)); CU(c, H(&b->h_c_pos, m * 8));
         CU(c, H(&b->h_c_lq, m * 4)); CU(c, H(&b->h_c_tid, m * 4)); CU(c, H(&b->h_c_alen, m * 4));
         CU(c, H(&b->h_c_cl, m * 4)); CU(c, H(&b->h_c_cr, m * 4)); CU(c, H(&b->h_c_read, m * 4));
@@ -1351,7 +1327,6 @@ static int submit_device_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_rea
     b->n_reads = n_reads;
     bs.plan.clear();
     b->dev_binning = true;
-    b->mode = mode;
     {
         const float g = pull ? 0.f : b->st.host_gather_ms; const int32_t th = pull ? 1 : b->st.host_threads;
         memset(&b->st, 0, sizeof(b->st));
@@ -1427,12 +1402,9 @@ static int submit_device_binning(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_rea
     b->st.d2h_bytes = n_aln * (int64_t)(sizeof(AlnOut) + 8) + n_reads * 5 + (n > 0 ? (int64_t)BIN_KEYS * 4 + 128 + OVER_CAP * 4 : 0);
     if (pull && n_aln > 0) CU(c, cudaMemcpyAsync(bs.h_stats + 8, bs.d_stats + 8, 8, cudaMemcpyDeviceToHost, s3));   // bases pulled
     CU(c, cudaEventRecord(bs.ev[3], s3));
-    b->in_flight = true;
     b->st.host_submit_ms = ms_since(t_begin);
     return FADEGPU_OK;
 }
-
-static void worker_main(fadegpu_ctx *c);
 
 static fadegpu_inputs view_inputs(const fadegpu_batch_view &v)
 {
@@ -1442,42 +1414,20 @@ static fadegpu_inputs view_inputs(const fadegpu_batch_view &v)
     return in;
 }
 
-static int submit_stages(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, int mode, int64_t seq_bytes)
-{
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: cudaSetDevice failed");
-    return submit_device_binning(c, b, n, mode, seq_bytes);
-}
-
-// queue stage B for the ctx thread
-static int queue_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, int mode, int64_t seq_bytes)
-{
-    if (c->p.flags & FADEGPU_F_SYNC_SUBMIT) {
-        std::lock_guard<std::mutex> g(c->submit_mu);
-        return submit_stages(c, b, n, mode, seq_bytes);
-    }
-    std::lock_guard<std::mutex> lk(c->q_mu);
-    if (!c->worker.joinable()) {
-        try { c->worker = std::thread(worker_main, c); }
-        catch (const std::exception &e) { return fail(c, FADEGPU_E_STATE, std::string("fadegpu_submit: cannot start the submit thread: ") + e.what()); }
-    }
-    b->queued = true; b->submit_rc = 0; b->mode = mode; b->job_seq_bytes = seq_bytes;
-    b->in_flight = true;
-    c->queue.push_back({ b, n, nullptr });
-    c->q_cv.notify_one();
-    return FADEGPU_OK;
-}
-
+static void worker_main(fadegpu_ctx *c);
 static int launch_job(fadegpu_ctx *c, fadegpu_job *j);
 
-// queue the device half of a staged job for the ctx thread (caller holds q_mu)
-static int queue_job(fadegpu_ctx *c, fadegpu_job *j)
+// queue the device half of a batch (stage B) or of a staged job for the ctx thread, started on first use (caller holds
+// q_mu)
+static int queue_half(fadegpu_ctx *c, const fadegpu_ctx::Queued &q, const char *fn)
 {
     if (!c->worker.joinable()) {
         try { c->worker = std::thread(worker_main, c); }
-        catch (const std::exception &e) { return fail(c, FADEGPU_E_STATE, std::string(j->sc.fn) + ": cannot start the submit thread: " + e.what()); }
+        catch (const std::exception &e) { return fail(c, FADEGPU_E_STATE, std::string(fn) + ": cannot start the submit thread: " + e.what()); }
     }
-    j->queued = true; j->rc = 0;
-    c->queue.push_back({ nullptr, 0, j });
+    InFlight &f = q.j ? q.j->fl : q.b->fl;
+    f.queued = true; f.rc = 0;
+    c->queue.push_back(q);
     c->q_cv.notify_one();
     return FADEGPU_OK;
 }
@@ -1492,22 +1442,17 @@ static void worker_main(fadegpu_ctx *c)
         const fadegpu_ctx::Queued q = c->queue.front();
         c->queue.pop_front();
         c->worker_busy = true;
-        const int mode = q.b ? q.b->mode : 0;
-        const int64_t seq_bytes = q.b ? q.b->job_seq_bytes : 0;
         lk.unlock();
         int rc;
         std::string err;
         {
             std::lock_guard<std::mutex> g(c->submit_mu);
-            rc = q.j ? launch_job(c, q.j) : submit_stages(c, q.b, q.n, mode, seq_bytes);
+            rc = q.j ? launch_job(c, q.j) : submit_device_binning(c, q.b, q.n, q.mode, q.seq_bytes);
             if (rc) { std::lock_guard<std::mutex> ge(g_err_mu); err = c->err; }
         }
         lk.lock();
-        if (q.j) {
-            q.j->rc = rc; q.j->err = err; q.j->queued = false;
-        } else {
-            q.b->submit_rc = rc; q.b->submit_err = err; q.b->queued = false;
-        }
+        InFlight &f = q.j ? q.j->fl : q.b->fl;
+        f.rc = rc; f.err = err; f.queued = false;
         c->worker_busy = false;
         c->done_cv.notify_all();
     }
@@ -1520,21 +1465,64 @@ static void drain_submits(fadegpu_ctx *c)
     c->done_cv.wait(lk, [&] { return c->queue.empty() && !c->worker_busy; });
 }
 
-// FADEGPU_E_STATE while a job of the ctx is submitted and not yet waited for (annotate batches and jobs are not in
-// flight together)
-static int refuse_jobs_in_flight(fadegpu_ctx *c, const char *fn)
+// The state every submit entry point checks, in this order: a reference is loaded, the batch is not in flight, and no
+// job of the ctx is (annotate batches and jobs are not in flight together).  Messages under the entry point's name.
+static int refuse_submit(fadegpu_ctx *c, const fadegpu_batch *b, bool compact)
 {
+    if (!c->d_two)
+        return compact ? fail(c, FADEGPU_E_STATE, "fadegpu_submit_compact: no reference loaded")
+                       : fail(c, FADEGPU_E_STATE, "fadegpu_submit: no reference loaded");
     std::lock_guard<std::mutex> lk(c->q_mu);
+    if (b->fl.in_flight)
+        return compact ? fail(c, FADEGPU_E_STATE, "fadegpu_submit_compact: batch already in flight (call fadegpu_wait)")
+                       : fail(c, FADEGPU_E_STATE, "fadegpu_submit: batch already in flight (call fadegpu_wait)");
+    const char *fn = compact ? "fadegpu_submit_compact" : "fadegpu_submit";
     if (c->jobs_in_flight > 0)
         return fail(c, FADEGPU_E_STATE, std::string(fn) + ": a job of this ctx is in flight (call fadegpu_job_wait)");
     return 0;
 }
 
-// a batch is "in flight" from its submit to its wait; the flag is shared with the ctx thread
-static bool batch_in_flight(fadegpu_ctx *c, fadegpu_batch *b)
+// The submit sequence of every input layout (`in`: the caller's arrays of MODE_GATHERED), after the entry point's
+// checks.  Host-binned: the inputs binned on this thread, from the view's arrays (compact records expanded into them
+// first) or the caller's.  Device-binned: the caller's arrays gathered on this thread, then stage B queued for the ctx
+// thread, or run on this one with FADEGPU_F_SYNC_SUBMIT.
+static int submit_batch(fadegpu_ctx *c, fadegpu_batch *b, int64_t n, int mode, int64_t seq_bytes, const fadegpu_inputs *in)
 {
+    if (c->p.flags & FADEGPU_F_HOST_BINNING) {
+        fadegpu_batch_view &v = b->v;
+        const fadegpu_inputs view = view_inputs(v);
+        if (mode == MODE_COMPACT) {
+            for (int64_t k = 0; k < n; ++k) {
+                const fadegpu_read_meta &m = v.meta[k];
+                v.seq_off[k] = m.seq_off; v.l_qseq[k] = m.l_qseq; v.tid[k] = m.tid; v.pos[k] = m.pos;
+                v.aligned_len[k] = m.aligned_len; v.clip_left[k] = (int32_t)m.clip_left; v.clip_right[k] = (int32_t)m.clip_right;
+            }
+            v.seq_off[n] = seq_bytes;
+        }
+        std::lock_guard<std::mutex> g(c->submit_mu);
+        CU(c, cudaSetDevice(c->device));
+        int rc = submit_host_binning(c, b, n, mode == MODE_GATHERED ? in : &view);
+        if (rc) return rc;
+    } else {
+        if (mode == MODE_GATHERED) {   // the caller's arrays are only read here
+            CU(c, cudaSetDevice(c->device));
+            int rc = gather_reads(c, b, n, *in);
+            if (rc) return rc;
+        }
+        if (!(c->p.flags & FADEGPU_F_SYNC_SUBMIT)) {
+            std::lock_guard<std::mutex> lk(c->q_mu);
+            int rc = queue_half(c, { b, n, mode, seq_bytes, nullptr }, "fadegpu_submit");
+            if (!rc) b->fl.in_flight = true;
+            return rc;
+        }
+        std::lock_guard<std::mutex> g(c->submit_mu);
+        if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, FADEGPU_E_CUDA, "fadegpu_submit: cudaSetDevice failed");
+        int rc = submit_device_binning(c, b, n, mode, seq_bytes);
+        if (rc) return rc;
+    }
     std::lock_guard<std::mutex> lk(c->q_mu);
-    return b->in_flight;
+    b->fl.in_flight = true;
+    return FADEGPU_OK;
 }
 
 int fadegpu_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads)
@@ -1544,14 +1532,8 @@ int fadegpu_submit(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads)
     if (n_reads < 0 || n_reads > v.max_reads) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: n_reads out of range");
     if (n_reads > 0 && (v.seq_off[n_reads] < 0 || v.seq_off[n_reads] > v.max_seq_bytes))
         return fail(c, FADEGPU_E_ARG, "fadegpu_submit: seq_off[n] exceeds max_seq_bytes");
-    if (!(c->p.flags & FADEGPU_F_HOST_BINNING)) {
-        if (!c->d_two) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: no reference loaded");
-        if (batch_in_flight(c, b)) return fail(c, FADEGPU_E_STATE, "fadegpu_submit: batch already in flight (call fadegpu_wait)");
-        { int rc = refuse_jobs_in_flight(c, "fadegpu_submit"); if (rc) return rc; }
-        return queue_submit(c, b, n_reads, MODE_VIEW, 0);
-    }
-    fadegpu_inputs in = view_inputs(v);
-    return fadegpu_submit_inputs(c, b, n_reads, &in);
+    { int rc = refuse_submit(c, b, false); if (rc) return rc; }
+    return submit_batch(c, b, n_reads, MODE_VIEW, 0, nullptr);
 }
 
 int fadegpu_submit_compact(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, int64_t seq_bytes)
@@ -1561,39 +1543,43 @@ int fadegpu_submit_compact(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, in
     if (n_reads < 0 || n_reads > v.max_reads) return fail(c, FADEGPU_E_ARG, "fadegpu_submit_compact: n_reads out of range");
     if (seq_bytes < 0 || seq_bytes > v.max_seq_bytes || seq_bytes > (int64_t)0xffffffffll)
         return fail(c, FADEGPU_E_ARG, "fadegpu_submit_compact: seq_bytes out of range");
-    if (!c->d_two) return fail(c, FADEGPU_E_STATE, "fadegpu_submit_compact: no reference loaded");
-    if (batch_in_flight(c, b)) return fail(c, FADEGPU_E_STATE, "fadegpu_submit_compact: batch already in flight (call fadegpu_wait)");
-    { int rc = refuse_jobs_in_flight(c, "fadegpu_submit_compact"); if (rc) return rc; }
-    if (c->p.flags & FADEGPU_F_HOST_BINNING) {
-        // A/B switch: expand the compact records into the view's arrays and take the host path
-        fadegpu_batch_view &w = b->v;
-        for (int64_t k = 0; k < n_reads; ++k) {
-            const fadegpu_read_meta &m = w.meta[k];
-            w.seq_off[k] = m.seq_off; w.l_qseq[k] = m.l_qseq; w.tid[k] = m.tid; w.pos[k] = m.pos;
-            w.aligned_len[k] = m.aligned_len; w.clip_left[k] = (int32_t)m.clip_left; w.clip_right[k] = (int32_t)m.clip_right;
-        }
-        w.seq_off[n_reads] = seq_bytes;
-        fadegpu_inputs in = view_inputs(w);
-        return fadegpu_submit_inputs(c, b, n_reads, &in);
-    }
-    return queue_submit(c, b, n_reads, MODE_COMPACT, seq_bytes);
+    { int rc = refuse_submit(c, b, true); if (rc) return rc; }
+    return submit_batch(c, b, n_reads, MODE_COMPACT, seq_bytes, nullptr);
+}
+
+// (the state is checked before n_reads and the arrays: a call that fails both reports the state)
+int fadegpu_submit_inputs(fadegpu_ctx *c, fadegpu_batch *b, int64_t n_reads, const fadegpu_inputs *in)
+{
+    if (!c || !b || b->ctx != c || !in) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: bad ctx/batch/inputs");
+    { int rc = refuse_submit(c, b, false); if (rc) return rc; }
+    if (n_reads < 0 || n_reads > b->v.max_reads) return fail(c, FADEGPU_E_ARG, "fadegpu_submit: n_reads out of range");
+    if (n_reads > 0 && (!in->seq4 || !in->seq_off || !in->l_qseq || !in->tid || !in->pos || !in->aligned_len ||
+                        !in->clip_left || !in->clip_right))
+        return fail(c, FADEGPU_E_ARG, "fadegpu_submit: null input array");
+    return submit_batch(c, b, n_reads, MODE_GATHERED, 0, in);
+}
+
+// At a wait: false if the submit is not in flight.  Otherwise, once the ctx thread is through with its queued half, the
+// submit leaves flight (and the count *n_in_flight, if given), and *rc / *err receive that half's outcome.
+static bool end_flight(fadegpu_ctx *c, InFlight &f, int *n_in_flight, int *rc, std::string *err)
+{
+    std::unique_lock<std::mutex> lk(c->q_mu);
+    if (!f.in_flight) return false;
+    c->done_cv.wait(lk, [&] { return !f.queued; });
+    f.in_flight = false;
+    if (n_in_flight) --*n_in_flight;
+    *rc = f.rc; *err = f.err;
+    f.rc = 0;
+    return true;
 }
 
 int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
 {
     if (!c || !b || b->ctx != c) return fail(c, FADEGPU_E_ARG, "fadegpu_wait: bad ctx/batch");
-    {   // a queued submit reports its outcome here
-        std::unique_lock<std::mutex> lk(c->q_mu);
-        if (!b->in_flight) { lk.unlock(); return fail(c, FADEGPU_E_STATE, "fadegpu_wait: batch not submitted"); }
-        c->done_cv.wait(lk, [&] { return !b->queued; });
-        b->in_flight = false;
-        if (b->submit_rc) {
-            const int rc = b->submit_rc;
-            b->submit_rc = 0;
-            lk.unlock();
-            return fail(c, rc, b->submit_err);
-        }
-    }
+    int rc;
+    std::string err;
+    if (!end_flight(c, b->fl, nullptr, &rc, &err)) return fail(c, FADEGPU_E_STATE, "fadegpu_wait: batch not submitted");
+    if (rc) return fail(c, rc, err);   // (a queued submit reports its outcome here)
     CU(c, cudaSetDevice(c->device));
     CU(c, cudaEventSynchronize(b->bs.ev[3]));
     float t;
@@ -1647,7 +1633,7 @@ int fadegpu_wait(fadegpu_ctx *c, fadegpu_batch *b)
 int fadegpu_get_results(const fadegpu_batch *b, fadegpu_results_view *r)
 {
     if (!b || !r) return fail(nullptr, FADEGPU_E_ARG, "fadegpu_get_results: null argument");
-    if (b->in_flight) return fail(b->ctx, FADEGPU_E_STATE, "fadegpu_get_results: batch in flight (call fadegpu_wait)");
+    if (b->fl.in_flight) return fail(b->ctx, FADEGPU_E_STATE, "fadegpu_get_results: batch in flight (call fadegpu_wait)");
     static_assert(sizeof(fadegpu_result) == sizeof(AlnOut), "fadegpu_result must mirror AlnOut");
     r->n_results = b->bs.n_aln;
     r->results = reinterpret_cast<const fadegpu_result *>(b->h_out);
@@ -1714,7 +1700,7 @@ int fadegpu_replay_batches(fadegpu_ctx *c, fadegpu_batch *const *batches, int32_
     for (int32_t i = 0; i < n_batches; ++i) {
         fadegpu_batch *b = batches[i];
         if (!b || b->ctx != c) return fail(c, FADEGPU_E_ARG, "fadegpu_replay_batches: bad batch");
-        if (b->in_flight) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_batches: batch in flight");
+        if (b->fl.in_flight) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_batches: batch in flight");
         if (b->bs.plan.empty() && b->bs.n_aln > 0) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_batches: nothing submitted");
     }
     drain_submits(c);
@@ -1742,7 +1728,7 @@ int fadegpu_replay_batches(fadegpu_ctx *c, fadegpu_batch *const *batches, int32_
 int fadegpu_replay_kernels(fadegpu_ctx *c, fadegpu_batch *b, int32_t iters, float *ms_out)
 {
     if (!c || !b || b->ctx != c || iters <= 0) return fail(c, FADEGPU_E_ARG, "fadegpu_replay_kernels: bad arguments");
-    if (b->in_flight) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_kernels: batch in flight");
+    if (b->fl.in_flight) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_kernels: batch in flight");
     if (b->bs.plan.empty() && b->bs.n_aln > 0) return fail(c, FADEGPU_E_STATE, "fadegpu_replay_kernels: nothing submitted");
     drain_submits(c);
     {   // one pass with per-stage events (serialising: fill / traceback / generic), then the timed passes
@@ -1775,7 +1761,7 @@ static int refuse_in_flight(fadegpu_ctx *c, const char *fn)
 {
     std::lock_guard<std::mutex> lk(c->q_mu);
     for (const fadegpu_batch *b : c->batches)
-        if (b->in_flight)
+        if (b->fl.in_flight)
             return fail(c, FADEGPU_E_STATE, std::string(fn) + ": a batch of this ctx is in flight (call fadegpu_wait)");
     return 0;
 }
@@ -1976,8 +1962,8 @@ static int run_call(fadegpu_ctx *c, fadegpu_job *job, const StagedCall &sc, cons
     }
     if (sc.n > 0) j->st.host_submit_ms = ms_since_begin();
     std::lock_guard<std::mutex> lk(c->q_mu);
-    if (!here) { int rc = queue_job(c, j); if (rc) return rc; }
-    j->in_flight = true;
+    if (!here) { int rc = queue_half(c, { nullptr, 0, 0, 0, j }, sc.fn); if (rc) return rc; }
+    j->fl.in_flight = true;
     ++c->jobs_in_flight;
     return FADEGPU_OK;
 }
@@ -2195,8 +2181,8 @@ void fadegpu_job_destroy(fadegpu_job *j)
     fadegpu_ctx *c = j->ctx;
     {
         std::unique_lock<std::mutex> lk(c->q_mu);
-        c->done_cv.wait(lk, [&] { return !j->queued; });
-        if (j->in_flight) { j->in_flight = false; --c->jobs_in_flight; }
+        c->done_cv.wait(lk, [&] { return !j->fl.queued; });
+        if (j->fl.in_flight) { j->fl.in_flight = false; --c->jobs_in_flight; }
         c->jobs.erase(std::remove(c->jobs.begin(), c->jobs.end(), j), c->jobs.end());
     }
     cudaSetDevice(c->device);
@@ -2214,7 +2200,7 @@ static int check_job_submit(fadegpu_ctx *c, fadegpu_job *j, const char *fn, int3
         return fail(c, FADEGPU_E_ARG, at + "max_ops must be 0 with FADEGPU_JOB_SCORE_ONLY");
     {
         std::lock_guard<std::mutex> lk(c->q_mu);
-        if (!j->in_flight) return 0;
+        if (!j->fl.in_flight) return 0;
     }
     return fail(c, FADEGPU_E_STATE, at + "job already in flight (call fadegpu_job_wait)");
 }
@@ -2242,16 +2228,8 @@ int fadegpu_job_wait(fadegpu_ctx *c, fadegpu_job *j, fadegpu_stats *stats_out)
     if (j->ctx != c) return fail(c, FADEGPU_E_STATE, "fadegpu_job_wait: the job belongs to another ctx");
     int rc;
     std::string err;
-    {   // a queued device half reports its outcome here
-        std::unique_lock<std::mutex> lk(c->q_mu);
-        if (!j->in_flight) { lk.unlock(); return fail(c, FADEGPU_E_STATE, "fadegpu_job_wait: job not submitted"); }
-        c->done_cv.wait(lk, [&] { return !j->queued; });
-        j->in_flight = false;
-        --c->jobs_in_flight;
-        rc = j->rc; err = j->err;
-        j->rc = 0;
-    }
-    if (rc) return fail(c, rc, err);
+    if (!end_flight(c, j->fl, &c->jobs_in_flight, &rc, &err)) return fail(c, FADEGPU_E_STATE, "fadegpu_job_wait: job not submitted");
+    if (rc) return fail(c, rc, err);   // (a queued device half reports its outcome here)
     CU(c, cudaSetDevice(c->device));
     { int r = finish_job(c, j); if (r) return r; }
     j->n_res = j->sc.n;
@@ -2263,7 +2241,7 @@ int fadegpu_job_results_view(const fadegpu_job *j, fadegpu_job_results *r)
 {
     if (!j || !r) return fail(j ? j->ctx : nullptr, FADEGPU_E_ARG, "fadegpu_job_results_view: null argument");
     bool in_flight;
-    { std::lock_guard<std::mutex> lk(j->ctx->q_mu); in_flight = j->in_flight; }
+    { std::lock_guard<std::mutex> lk(j->ctx->q_mu); in_flight = j->fl.in_flight; }
     if (in_flight) return fail(j->ctx, FADEGPU_E_STATE, "fadegpu_job_results_view: job in flight (call fadegpu_job_wait)");
     const int64_t n = std::max<int64_t>(0, j->n_res);
     r->n = n;

@@ -287,25 +287,32 @@ def test_state_and_argument_errors(c1, wild):
     assert b"another ctx" in L.fadegpu_last_error(other._h)
     names, c1c, cfg, n = sim.config_c1()
     rd = sim.make_reads(cfg, 0, 2000, c1c)
-    b = ctx.alloc_batch(rd.n, int(rd.seq_off[rd.n]))
-    b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
-    assert "a job of this ctx is in flight" in _raises(E_STATE, b.submit)
-    _raises(E_STATE, b.submit_arrays, rd.n, rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len,
-            rd.clip_left, rd.clip_right)
-    b.fill_compact(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
-    _raises(E_STATE, b.submit_compact)
-    want = _sync(ctx, "pairs", False, x)                            # a synchronous call runs after the job
-    _equal(res.wait(), want)
-    _raises(E_STATE, job.wait)                                      # waited already
-    b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
-    b.submit()
-    assert "a batch of this ctx is in flight" in _raises(E_STATE, _submit, job, "pairs", False, x)
-    _raises(E_STATE, job.submit_regions, ["ACGT"], [0], [0], [4])
-    b.wait()
-    rec0 = b.results()[0].copy()
-    _equal(_submit(job, "pairs", False, x).wait(), want)
-    assert np.array_equal(b.results()[0], rec0) and b.replay_kernels(1) > 0
-    b.close()
+    # the same exclusions on a host-binned ctx, whose batch submits run on the calling thread
+    with Context(0, default_params(flags=api.F_HOST_BINNING)) as hctx:
+        hctx.share_reference_from(ctx)
+        hjob = Job(hctx)
+        hres = _submit(hjob, "pairs", False, x)
+        for cx, jb, res in ((ctx, job, res), (hctx, hjob, hres)):
+            b = cx.alloc_batch(rd.n, int(rd.seq_off[rd.n]))
+            b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
+            assert "a job of this ctx is in flight" in _raises(E_STATE, b.submit)
+            _raises(E_STATE, b.submit_arrays, rd.n, rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len,
+                    rd.clip_left, rd.clip_right)
+            b.fill_compact(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
+            _raises(E_STATE, b.submit_compact)
+            want = _sync(cx, "pairs", False, x)                     # a synchronous call runs after the job
+            _equal(res.wait(), want)
+            _raises(E_STATE, jb.wait)                               # waited already
+            b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
+            b.submit()
+            assert "a batch of this ctx is in flight" in _raises(E_STATE, _submit, jb, "pairs", False, x)
+            _raises(E_STATE, jb.submit_regions, ["ACGT"], [0], [0], [4])
+            b.wait()
+            rec0 = b.results()[0].copy()
+            _equal(_submit(jb, "pairs", False, x).wait(), want)
+            assert np.array_equal(b.results()[0], rec0) and b.replay_kernels(1) > 0
+            b.close()
+        hjob.close()
     # max_ops with FADEGPU_JOB_SCORE_ONLY, unknown flags, no reference for regions
     assert L.fadegpu_submit_pairs(ctx._h, job._h, 0, C.byref(pin), 3, api.JOB_SCORE_ONLY) == E_ARG
     assert L.fadegpu_submit_pairs(ctx._h, job._h, 0, C.byref(pin), 0, 2) == E_ARG

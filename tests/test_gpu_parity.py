@@ -518,26 +518,44 @@ def test_many_batches_in_flight_and_replay_batches():
 
 
 def test_errors_of_a_queued_submit_surface_at_wait():
-    """inconsistent seq_off: FADEGPU_E_ARG from fadegpu_wait (queued submit) or from fadegpu_submit itself
-    (FADEGPU_F_SYNC_SUBMIT); the batch and the ctx stay usable afterwards."""
+    """inconsistent seq_off, through fadegpu_submit (view), fadegpu_submit_compact and fadegpu_submit_inputs
+    (arrays): FADEGPU_E_ARG from fadegpu_wait when the check runs in a queued submit, from the submit call itself
+    with FADEGPU_F_SYNC_SUBMIT or FADEGPU_F_HOST_BINNING and for arrays (checked while they are gathered, on the
+    calling thread); the batch and the ctx stay usable afterwards."""
     rng = random.Random(5)
     contigs = [readsets.random_ref(rng, 4000)]
     rd = readsets.build(readsets.ragged_reads(rng, contigs, 200, max_len=150))
-    for flags in (0, api.F_SYNC_SUBMIT):
+    k = int(np.flatnonzero(rd.clip_left > 10)[0])
+    bad_off = rd.seq_off.copy()
+    bad_off[k] = int(rd.seq_off[rd.n]) + 5                   # points past the end of seq4
+    fields = (rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
+
+    def submit(b, entry, seq_off):
+        if entry == "view":
+            b.fill(*fields)
+            b.seq_off[:rd.n + 1] = seq_off
+            b.submit()
+        elif entry == "compact":
+            b.fill_compact(*fields)
+            b.meta["seq_off"][:rd.n] = seq_off[:rd.n]
+            b.submit_compact()
+        else:
+            b.submit_arrays(rd.n, rd.seq4, seq_off, *fields[2:])
+
+    for flags in (0, api.F_SYNC_SUBMIT, api.F_HOST_BINNING):
         with _ctx(flags=flags) as ctx:
             ctx.load_reference(["a"], contigs)
             b = ctx.alloc_batch(rd.n, int(rd.seq_off[rd.n]))
-            b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right)
-            k = int(np.flatnonzero(rd.clip_left > 10)[0])
-            b.seq_off[k] = int(rd.seq_off[rd.n]) + 5        # points past the end of seq4
-            if flags:
-                with pytest.raises(api.FadeGpuError) as e:
-                    b.submit()
-            else:
-                b.submit()
-                with pytest.raises(api.FadeGpuError) as e:
-                    b.wait()
-            assert "seq_off" in str(e.value)
-            b.fill(rd.seq4, rd.seq_off, rd.l_qseq, rd.tid, rd.pos, rd.aligned_len, rd.clip_left, rd.clip_right).run()
-            compare(b, rd, contigs, oracle_params(ctx.params))
+            for entry in ("view", "compact", "arrays"):
+                if flags == 0 and entry != "arrays":
+                    submit(b, entry, bad_off)
+                    with pytest.raises(api.FadeGpuError) as e:
+                        b.wait()
+                else:
+                    with pytest.raises(api.FadeGpuError) as e:
+                        submit(b, entry, bad_off)
+                assert e.value.code == -1 and "seq_off" in str(e.value), (flags, entry)   # FADEGPU_E_ARG
+                submit(b, entry, rd.seq_off)
+                b.wait()
+                compare(b, rd, contigs, oracle_params(ctx.params))
             b.close()
